@@ -7,7 +7,8 @@
 A "step" is one pass of the hot path over one batch of 4,096 synthetic ciphertext pairs per GPU
 (BASELINE.json configs[2]).  `value` = whole-job ops/s with inputs resident in HBM; `e2e` = the same metric
 through the C-ABI host-buffer entry point (fhe_b200_mul_relin_host: pinned host limb arrays in, H2D + kernels
-+ D2H inside the timed region).  One JSON line on stdout from rank 0.
++ D2H inside the timed region).  One JSON line on stdout from rank 0.  `--dump-outputs DIR` also writes a fixed sample of
+the last timed step's results as .npy files, to compare two builds output for output.
 """
 from __future__ import annotations
 
@@ -102,6 +103,20 @@ SM_COUNT = 148
 WIDE_PER_CLK_PER_SM = 32  # IMAD.WIDE results per clock per SM (scripts/pipe_probe.cu: 0.25 warp-instructions / clk / SMSP)
 METRIC = "ct_ct_fhe_multiply_relin_ops_per_sec"
 WORKLOAD = "batch of 4096 ct*ct fhe_multiply+relinearize per GPU, testnet BFV params (N=4096, q=72b, t=4096)"
+DUMP_ROWS = 256  # ciphertexts kept by --dump-outputs: 256 x 128 KiB of float64 = 32 MiB
+
+
+def dump_outputs(path: str, n: int, take) -> None:
+    """--dump-outputs: a fixed sample of the results of the last timed step, so that two builds can be compared output for
+    output.  ct_out.npy: float64 [rows, 2, 2, 4096], the result ciphertexts (residues < 2^37, exact in float64);
+    ct_out_rows.npy: the batch index of each row (DUMP_ROWS indices drawn with seed 0, ascending; the whole batch if smaller).
+    `take(rows)` returns those rows of the result as uint64."""
+    import numpy as np
+
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "ct_out.npy"), take(rows).astype(np.float64))
+    np.save(os.path.join(path, "ct_out_rows.npy"), rows.astype(np.float64))
 
 
 def measured_peaks():
@@ -623,8 +638,10 @@ def run_reference(args) -> None:
         bfv.batch_mul_relin(a, b, rk, cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        bfv.batch_mul_relin(a, b, rk, cores)
+        out, _ = bfv.batch_mul_relin(a, b, rk, cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sample, lambda rows: out[rows])
     value = sample * args.steps / dt
     # the same op through the reference's BYTE surface on the CPU (packed bytes in, packed bytes out), bounded sample
     bs = None
@@ -678,7 +695,11 @@ def main() -> None:
     ap.add_argument("--no-configs", action="store_true", help="skip the quick runs of BASELINE configs 2, 4 and 5")
     ap.add_argument("--sustain-seconds", type=float, default=0.0, help="extra device-resident run of at least this long with the clock sampler (recorded under `sustained`)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="ops in the CPU-baseline sample (0 = ~20 s of CPU work)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of the last step's results "
+                    "to DIR/*.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -745,6 +766,8 @@ def main() -> None:
     fdev.set_kernel_timing(False)
     clocks = sampler.stop()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, lambda rows: out[torch.from_numpy(rows).to(dev)].cpu().numpy().view(np.uint64))
     from fhe_precompiles_b200.sharding import max_over_ranks, whole_job_rate
 
     ms_max = max_over_ranks(ms, dist)

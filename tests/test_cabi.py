@@ -66,22 +66,35 @@ def test_public_key_bytes_needs_no_gpu(lib):
     assert FHE.public_key_bytes() == open(os.path.join(ROOT, "fhe_precompiles_b200/data/network.pub"), "rb").read()
 
 
+NO_DEVICE = r"""
+import sys
+sys.path.insert(0, sys.argv[1])
+import pytest
+import torch
+assert not torch.cuda.is_available()
+from fhe_precompiles_b200 import FHE, FheError, _lib
+
+with pytest.raises(FheError) as e:
+    FHE.add_cipheri64_cipheri64(b"\x00" * 16)
+assert e.value.code == 7 and "no CPU fallback" in str(e.value)
+assert _lib.lib().fhe_b200_init(0) == -1
+from fhe_precompiles_b200 import device
+
+with pytest.raises(RuntimeError):
+    device.add(torch.zeros((1, 2, 2, 4096), dtype=torch.int64), torch.zeros((1, 2, 2, 4096), dtype=torch.int64))
+print("ok")
+"""
+
+
 def test_no_cpu_fallback():
-    """On a box without a CUDA device the product path must fail loudly, never compute on the CPU."""
-    import torch
+    """On a box without a CUDA device the product path must fail loudly, never compute on the CPU.  The check runs in a child
+    process that sees no device (CUDA_VISIBLE_DEVICES empty), so it runs on GPU machines too."""
+    import subprocess
+    import sys
 
-    if torch.cuda.is_available():
-        pytest.skip("CUDA device present")
-    from fhe_precompiles_b200 import FHE, FheError, _lib
-
-    with pytest.raises(FheError) as e:
-        FHE.add_cipheri64_cipheri64(b"\x00" * 16)
-    assert e.value.code == 7 and "no CPU fallback" in str(e.value)
-    assert _lib.lib().fhe_b200_init(0) == -1
-    from fhe_precompiles_b200 import device
-
-    with pytest.raises(RuntimeError):
-        device.add(torch.zeros((1, 2, 2, 4096), dtype=torch.int64), torch.zeros((1, 2, 2, 4096), dtype=torch.int64))
+    r = subprocess.run([sys.executable, "-c", NO_DEVICE, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                       text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stdout + r.stderr
 
 
 def test_product_does_not_import_the_oracle():
