@@ -89,6 +89,10 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_decrypt.restype = i32
     L.fhe_b200_decrypt_checked.argtypes = [i32, vp, vp, vp, vp, sz, vp]
     L.fhe_b200_decrypt_checked.restype = i32
+    L.fhe_b200_encode_values.argtypes = [i32, i32, vp, vp, vp, sz, vp]
+    L.fhe_b200_encode_values.restype = i32
+    L.fhe_b200_decode_values.argtypes = [i32, i32, vp, vp, sz, vp]
+    L.fhe_b200_decode_values.restype = i32
     L.fhe_b200_data_type_kind.argtypes = [ctypes.c_char_p]
     L.fhe_b200_data_type_kind.restype = i32
     L.fhe_b200_set_chunk_ops.argtypes = [i64]

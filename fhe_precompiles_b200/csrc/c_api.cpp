@@ -14,6 +14,7 @@
 #include <functional>
 #include <memory>
 #include <mutex>
+#include <stdexcept>
 #include <string>
 #include <thread>
 #include <vector>
@@ -22,6 +23,7 @@
 #include "engine.h"
 #include "host_pool.h"
 #include "kernels.h"
+#include "value_kernels.h"
 
 using namespace fheb;
 
@@ -371,6 +373,20 @@ int32_t fhe_b200_decrypt(int32_t device, const uint64_t *ct, const uint64_t *sk,
 int32_t fhe_b200_decrypt_checked(int32_t device, const uint64_t *ct, const uint64_t *sk, uint16_t *plain, int32_t *exhausted, size_t n,
                                  void *stream) {
     DEV_GUARD(Engine::get().decrypt_device(device, ct, sk, plain, n, (cudaStream_t)stream, exhausted));
+}
+static void check_value_args(const char *fn, int32_t kind, const uint16_t *plain) {
+    if (!value_kind_valid(kind))
+        throw std::runtime_error(std::string(fn) + ": unknown kind " + std::to_string(kind) + " (0 u256, 1 u64, 2 i64, 3 frac64)");
+    if ((uintptr_t)plain % 16) throw std::runtime_error(std::string(fn) + ": plain must be 16-byte aligned");
+}
+int32_t fhe_b200_encode_values(int32_t device, int32_t kind, const void *values, uint16_t *plain, int32_t *status, size_t n,
+                               void *stream) {
+    DEV_GUARD(check_value_args("fhe_b200_encode_values", kind, plain); device_context(device);
+              cuda_throw(launch_encode_values(kind, values, plain, status, n, (cudaStream_t)stream), "encode_values"));
+}
+int32_t fhe_b200_decode_values(int32_t device, int32_t kind, const uint16_t *plain, void *values, size_t n, void *stream) {
+    DEV_GUARD(check_value_args("fhe_b200_decode_values", kind, plain); device_context(device);
+              cuda_throw(launch_decode_values(kind, plain, values, n, (cudaStream_t)stream), "decode_values"));
 }
 int32_t fhe_b200_bfly_peak(int32_t device, int32_t mod, double *giga_bfly_per_s) {
     DEV_GUARD(device_context(device); cuda_throw(measure_bfly_peak(mod, giga_bfly_per_s), "bfly_peak"));

@@ -4,6 +4,8 @@ torch is plumbing only: it owns device memory and streams; every op is a call in
 Tensors are int64 views of uint64 words (torch has no general uint64 ops), C-contiguous:
   ciphertext [n, 2, 2, 4096], size-3 ciphertext [n, 3, 2, 4096], relin key [2, 2, 3, 4096],
   plaintext [n, 4096] int16 (coefficients < 4096).
+Typed values (encode / decode, encrypt_values / decrypt_values): u64 and i64 int64 [n] (u64 as its two's-complement view),
+u256 int64 [n, 4] (words least significant first), frac64 float64 [n].
 """
 from __future__ import annotations
 
@@ -270,6 +272,64 @@ def decrypt_checked(ct: torch.Tensor, sk: torch.Tensor):
     flags = torch.empty((ct.shape[0],), dtype=torch.int32, device=ct.device)
     _check(_lib.lib().fhe_b200_decrypt_checked(dev, ct.data_ptr(), sk.data_ptr(), plain.data_ptr(), flags.data_ptr(), ct.shape[0], _stream(dev)))
     return plain, flags
+
+
+# value kinds, numbered as fhe_b200_data_type_kind numbers them
+VALUE_KINDS = ("u256", "u64", "i64", "frac64")
+
+
+def _value_kind(kind: str) -> int:
+    if kind not in VALUE_KINDS:
+        raise ValueError(f"unknown value kind {kind!r}: expected one of {', '.join(VALUE_KINDS)}")
+    return VALUE_KINDS.index(kind)
+
+
+def _value_shape(kind: str, n: int):
+    return (n, 4) if kind == "u256" else (n,)
+
+
+def _value_dtype(kind: str):
+    return torch.float64 if kind == "frac64" else torch.int64
+
+
+def encode(kind: str, values: torch.Tensor):
+    """values ([n] int64 for u64 / i64, [n, 4] int64 for u256, [n] float64 for frac64) -> (plain [n, 4096] int16, status [n]
+    int32): sunscreen's plaintext of each value, bit-identical to the byte surface's encoder.  status[i] = 7 (and a zero row)
+    where a frac64 value is NaN, +-inf or |v| >= 2^64, 0 otherwise."""
+    k = _value_kind(kind)
+    dev = _dev(values)
+    n = values.shape[0]
+    if values.dtype != _value_dtype(kind) or tuple(values.shape) != _value_shape(kind, n):
+        raise ValueError(f"encode({kind!r}): values must be {_value_dtype(kind)} {_value_shape(kind, 'n')}")
+    plain = torch.empty((n, N), dtype=torch.int16, device=values.device)
+    status = torch.empty((n,), dtype=torch.int32, device=values.device)
+    _check(_lib.lib().fhe_b200_encode_values(dev, k, values.data_ptr(), plain.data_ptr(), status.data_ptr(), n, _stream(dev)))
+    return plain, status
+
+
+def decode(kind: str, plain: torch.Tensor) -> torch.Tensor:
+    """plain [n, 4096] int16 -> values in encode()'s layout: the byte surface's decoder applied to every row, whatever its
+    coefficients (>= 4096 wrap as the reference's do)."""
+    k = _value_kind(kind)
+    dev = _dev(plain)
+    if plain.dtype != torch.int16 or plain.dim() != 2 or plain.shape[1] != N:
+        raise ValueError("decode: plain must be int16 [n, 4096]")
+    n = plain.shape[0]
+    values = torch.empty(_value_shape(kind, n), dtype=_value_dtype(kind), device=plain.device)
+    _check(_lib.lib().fhe_b200_decode_values(dev, k, plain.data_ptr(), values.data_ptr(), n, _stream(dev)))
+    return values
+
+
+def encrypt_values(pk: torch.Tensor, kind: str, values: torch.Tensor, seeds: torch.Tensor):
+    """encode() + encrypt(): (ct [n,2,2,4096], status [n] int32 as encode() returns it)."""
+    plain, status = encode(kind, values)
+    return encrypt(pk, plain, seeds), status
+
+
+def decrypt_values(ct: torch.Tensor, sk: torch.Tensor, kind: str):
+    """decrypt_checked() + decode(): (values, exhausted [n] int32); values[i] is meaningless where exhausted[i] = 1."""
+    plain, exhausted = decrypt_checked(ct, sk)
+    return decode(kind, plain), exhausted
 
 
 def set_chunk_ops(ops: int) -> int:

@@ -159,6 +159,20 @@ size_t fhe_b200_seal_op_words(void);
  * return 5 (FailedDecryption, fhe.rs:640-643, 692-696); plain[i] is then meaningless. */
 int32_t fhe_b200_decrypt_checked(int32_t device, const uint64_t *ct, const uint64_t *sk, uint16_t *plain, int32_t *exhausted, size_t n,
                                  void *stream);
+/* Typed values <-> plaintexts on the device: sunscreen's encoders of the four operand kinds, so that a device-resident chain
+ * can start and end in values (fhe_b200_encode_values -> fhe_b200_encrypt / plain_addsub / multiply_plain ... ->
+ * fhe_b200_decrypt_checked -> fhe_b200_decode_values).  `kind` is numbered as in fhe_b200_data_type_kind: 0 u256, 1 u64, 2 i64,
+ * 3 frac64.  `values` holds one value per op, batch outermost: u64 uint64; i64 int64; u256 four uint64 words, least
+ * significant first; frac64 an IEEE double.  `plain` is [n][4096] uint16, 16-byte aligned (any cudaMalloc pointer).
+ * BIT-EXACT with the byte surface: row i of encode equals the plaintext c_fhe_*_<kind> builds from the value's big-endian
+ * serialization (Unsigned64 / Unsigned256 / Signed / Fractional<64> encoders, every one of the 4096 coefficients), and decode
+ * is the same function of EVERY uint16 plaintext as c_fhe_decrypt_<kind>'s decoder, coefficients >= 4096 included (they wrap
+ * as in the reference's release arithmetic); for frac64 that is the double the host's in-order sum gives, bit for bit.
+ * status (device, [n], may be NULL): 0, or 7 (the byte surface's code) where a frac64 value is NaN, +-inf or |v| >= 2^64;
+ * that row is all zero.  The integer kinds never fail.  Device pointers, enqueued on `stream`; n == 0 launches nothing.
+ * 0 / -1 (unknown kind, misaligned plain, no device, launch failure: see fhe_b200_last_error). */
+int32_t fhe_b200_encode_values(int32_t device, int32_t kind, const void *values, uint16_t *plain, int32_t *status, size_t n, void *stream);
+int32_t fhe_b200_decode_values(int32_t device, int32_t kind, const uint16_t *plain, void *values, size_t n, void *stream);
 /* Same op on HOST buffers (pin them for full PCIe rate): copies in, computes and copies out chunk by chunk with
  * the three phases of consecutive chunks overlapped; returns when `out` is complete. rk: host words. */
 int32_t fhe_b200_mul_relin_host(int32_t device, const uint64_t *a, const uint64_t *b, const uint64_t *rk, uint64_t *out,
