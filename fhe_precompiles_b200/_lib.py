@@ -73,7 +73,7 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_batch.argtypes = [ctypes.POINTER(BatchCall), sz, i32]
     L.fhe_b200_batch.restype = i64
     dev3 = [i32, vp, vp, vp, sz, vp]
-    for name in ("add", "sub", "multiply", "relinearize", "behz_tensor"):
+    for name in ("add", "sub", "multiply", "relinearize"):
         getattr(L, "fhe_b200_" + name).argtypes = dev3
     L.fhe_b200_negate.argtypes = [i32, vp, vp, sz, vp]
     L.fhe_b200_plain_addsub.argtypes = [i32, vp, vp, vp, sz, i32, vp]
@@ -113,8 +113,6 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_int_peak.restype = i32
     L.fhe_b200_bfly_peak.argtypes = [i32, i32, ctypes.POINTER(ctypes.c_double)]
     L.fhe_b200_bfly_peak.restype = i32
-    L.fhe_b200_set_fused.argtypes = [i32]
-    L.fhe_b200_set_fused.restype = None
     L.fhe_b200_set_call_timing.argtypes = [i32]
     L.fhe_b200_set_call_timing.restype = None
     L.fhe_b200_last_call_breakdown.argtypes = [ctypes.POINTER(ctypes.c_double)]
@@ -124,12 +122,7 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_kernel_timing_report.argtypes = [i32, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_uint64)]
     L.fhe_b200_kernel_timing_report.restype = i32
     L.fhe_b200_ntt.argtypes = [i32, vp, sz, ctypes.POINTER(i32), i32, i32, vp]
-    L.fhe_b200_behz_extend.argtypes = [i32, vp, vp, vp, sz, vp]
-    L.fhe_b200_behz_floor_sk.argtypes = [i32, vp, vp, sz, vp]
-    for name in (
-        "add", "sub", "negate", "plain_addsub", "multiply_plain", "multiply", "relinearize", "mul_relin", "ntt",
-        "behz_extend", "behz_tensor", "behz_floor_sk",
-    ):
+    for name in ("add", "sub", "negate", "plain_addsub", "multiply_plain", "multiply", "relinearize", "mul_relin", "ntt"):
         getattr(L, "fhe_b200_" + name).restype = i32
     L.fhe_b200_parse_public_key.argtypes = [vp, sz, vp, vp]
     L.fhe_b200_parse_public_key.restype = i32

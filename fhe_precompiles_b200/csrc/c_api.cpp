@@ -406,13 +406,6 @@ int64_t fhe_b200_set_chunk_ops(int64_t ops) {
         return -1;
     }
 }
-void fhe_b200_set_fused(int32_t on) {
-    try {
-        Engine::get().set_fused(on != 0);
-    } catch (const std::exception &e) {
-        set_error(e.what());
-    }
-}
 void fhe_b200_set_call_timing(int32_t on) {
     try {
         Engine::get().set_call_timing(on != 0);
@@ -467,15 +460,6 @@ int32_t fhe_b200_ntt(int32_t device, uint64_t *data, size_t n_limbs, const int32
         lm.mod[i] = mods[i];
     }
     DEV_GUARD(device_context(device); cuda_throw(launch_ntt(data, n_limbs, lm, inverse != 0, (cudaStream_t)stream), "ntt"));
-}
-int32_t fhe_b200_behz_extend(int32_t device, const uint64_t *a, const uint64_t *b, uint64_t *ext, size_t n, void *stream) {
-    DEV_GUARD(device_context(device); cuda_throw(launch_behz_extend_tap(a, b, ext, n, (cudaStream_t)stream), "behz_extend"));
-}
-int32_t fhe_b200_behz_tensor(int32_t device, const uint64_t *a, const uint64_t *b, uint64_t *tens, size_t n, void *stream) {
-    DEV_GUARD(device_context(device); cuda_throw(launch_behz_tensor(a, b, tens, n, (cudaStream_t)stream), "behz_tensor"));
-}
-int32_t fhe_b200_behz_floor_sk(int32_t device, const uint64_t *tens, uint64_t *out3, size_t n, void *stream) {
-    DEV_GUARD(device_context(device); cuda_throw(launch_floor_sk(tens, out3, n, (cudaStream_t)stream), "floor_sk"));
 }
 
 int32_t fhe_b200_parse_public_key(const uint8_t *bytes, size_t len, uint64_t *pk_words, uint64_t *rk_words) {

@@ -147,11 +147,6 @@ Engine::Engine() {
     tile_ops_ = env_size("FHE_B200_TILE_OPS", 16);
     if (tile_ops_ < 1) tile_ops_ = 1;
     chunk_ops_ = env_size("FHE_B200_CHUNK_OPS", 4096);
-    fused_ = env_size("FHE_B200_FUSED", 0) != 0;
-    {
-        const char *v = getenv("FHE_B200_SUBCHUNK_OPS");
-        subchunk_ops_ = (v && *v) ? (size_t)atoll(v) : 0;  // opt-in L2-resident fork/join pipeline (e.g. 96); 0 = off
-    }
     // byte-surface devices: FHE_B200_DEVICES="0,3" restricts single calls and batches to those GPUs (default: all).
     // Under a one-process-per-GPU launcher each rank sets it to its own device.
     if (const char *v = getenv("FHE_B200_DEVICES")) {
@@ -475,16 +470,6 @@ void Engine::release_scratch(StreamState *st) {
 void Engine::free_stream_state(StreamState &v) {
     if (v.p) cudaFree(v.p);
     v.p = nullptr;
-    ForkSet &F = v.forks;
-    if (F.ready) {
-        for (int i = 0; i < kForkStreams; i++) {
-            if (F.scratch[i]) cudaFree(F.scratch[i]);
-            cudaStreamDestroy(F.stream[i]);
-            cudaEventDestroy(F.join[i]);
-        }
-        cudaEventDestroy(F.fork);
-        F.ready = false;
-    }
 }
 size_t Engine::set_chunk_ops(long long ops) {
     std::lock_guard<std::mutex> lk(arena_mu_);
@@ -530,9 +515,9 @@ void Engine::kernel_timing_report(int device, double ms[kNumTimedKernels], uint6
     timed_.clear();
 }
 
-// kernel ids: 0 k_behz_tensor, 1 k_floor_sk, 2 k_relin_ks, 3 k_relin_finish, 4 k_ext_ntt, 5 k_tensor_intt,
-//             6 k_digit_ntt, 7 k_ks_intt, 8 k_ext_conv, 9 k_ks_finish, 10 k_rk_*_ksd (key preparation), 11 k_digit_ntt_ksd,
-//             12 k_ks_intt_ksd, 13 k_ks_finish_ksd, 14 k_tensor_floor_d, 15 k_ks_tail_ksd
+// kernel ids (device.py KERNEL_NAMES): 1 k_floor_sk_d, 3 k_relin_finish, 4 k_ext_ntt_d, 5 k_tensor_intt_d, 6 k_digit_ntt,
+//             7 k_ks_intt, 8 k_ext_conv_d, 10 k_rk_*_ksd (key preparation), 11 k_digit_ntt_ksd, 14 k_tensor_floor_d,
+//             15 k_ks_tail_ksd; 0, 2, 9, 12 and 13 are reserved and never filled
 #define TIMED(id, call, what)                                        \
     do {                                                             \
         if (timed) {                                                 \
@@ -547,87 +532,35 @@ void Engine::kernel_timing_report(int device, double ms[kNumTimedKernels], uint6
         }                                                            \
     } while (0)
 
+// Chunks of at least this many ops run the fused tails (k_tensor_floor_d, k_ks_tail_ksd), smaller ones the split tails and the
+// key switch on SEAL's key primes.  A fused tail runs three dual words one after the other in one CTA per (output polynomial,
+// op): right once its 2 or 3 CTAs per op come close to the 296 resident at a time (2 per SM), three times the critical path
+// for a single call or a small tile.
+constexpr size_t kFusedTailMinOps = 96;
+
 // BEHZ multiply of c ops: a, b -> m.c3 (size-3 ciphertexts)
 void Engine::enqueue_mul(const uint64_t *a, const uint64_t *b, const ScratchMap &m, size_t c, cudaStream_t s, bool timed) {
-    const bool dual = !fused_ && behz_mode() == 0;  // tensor product on the dual base (default) or on SEAL's 61-bit Bsk limbs
-    if (fused_) {
-        TIMED(0, launch_behz_tensor(a, b, m.tens, c, s), "behz_tensor");
+    TIMED(8, launch_ext_conv(a, b, m.nttbuf, c, s), "ext_conv");
+    TIMED(4, launch_ext_ntt(m.nttbuf, c, s), "ext_ntt");
+    if (c >= kFusedTailMinOps) {
+        TIMED(14, launch_tensor_floor(m.nttbuf, m.c3, c, s), "tensor_floor");
     } else {
-        if (ext_split() || dual) TIMED(8, launch_ext_conv(a, b, m.nttbuf, c, s), "ext_conv");
-        TIMED(4, launch_ext_ntt(a, b, m.nttbuf, c, s), "ext_ntt");
-        // three dual words one after the other in one CTA: right for chunks that fill the GPU, three times the critical path for
-        // a single call or a small tile (as for the key-switch tail below)
-        if (dual && (fuse_tail() & 1) && c >= 96) {
-            TIMED(14, launch_tensor_floor(m.nttbuf, m.c3, c, s), "tensor_floor");
-            return;
-        }
         TIMED(5, launch_tensor_intt(m.nttbuf, m.tens, c, s), "tensor_intt");
+        TIMED(1, launch_floor_sk(m.tens, m.c3, c, s), "floor_sk");
     }
-    TIMED(1, launch_floor_sk(m.tens, m.c3, c, s, dual), "floor_sk");
 }
 // relinearise c size-3 ciphertexts c3 -> out
 void Engine::enqueue_relin(const uint64_t *c3, const uint64_t *rk, uint64_t *out, const ScratchMap &m, size_t c, cudaStream_t s,
                            bool timed) {
-    if (fused_) {
-        TIMED(2, launch_relin_ks(c3, rk, m.ks, c, s), "relin_ks");
+    if (c >= kFusedTailMinOps) {
+        // the whole key switch on the dual base; m.tens (15 limbs per op, dead once c3 exists) holds the lifted key
+        TIMED(10, launch_rk_prepare_ksd(rk, m.tens, s), "rk_prepare_ksd");
+        TIMED(11, launch_digit_ntt_ksd(c3, m.dig, c, s), "digit_ntt_ksd");
+        TIMED(15, launch_ks_tail_ksd(m.dig, m.tens + 24 * kN, c3, out, c, s), "ks_tail_ksd");
     } else {
-        if (ks_dual() && c >= 96) {
-            // the whole key switch on the dual base; m.tens (15 limbs per op, dead once c3 exists) holds the lifted key
-            TIMED(10, launch_rk_prepare_ksd(rk, m.tens, s), "rk_prepare_ksd");
-            TIMED(11, launch_digit_ntt_ksd(c3, m.dig, c, s), "digit_ntt_ksd");
-            if (fuse_tail() & 2) {
-                TIMED(15, launch_ks_tail_ksd(m.dig, m.tens + 24 * kN, c3, out, c, s), "ks_tail_ksd");
-                return;
-            }
-            TIMED(12, launch_ks_intt_ksd(m.dig, m.tens + 24 * kN, m.ks, c, s), "ks_intt_ksd");
-            TIMED(13, launch_ks_finish_ksd(m.ks, c3, out, c, s), "ks_finish_ksd");
-            return;
-        }
         TIMED(6, launch_digit_ntt(c3, m.dig, c, s), "digit_ntt");
-        // the fused tail runs the three moduli one after the other in two CTAs per op: right once 2c CTAs come close to the
-        // 296 resident ones (the 128-op chunks of the host-buffer pipelines included), three times the critical path for a
-        // single call or a small tile
-        if (ks_finish_fused() && c >= 96) {
-            // m.ks (6 limbs per op) is free on this path: it holds the lane-major copy of the key
-            TIMED(9, launch_ks_finish(m.dig, rk, c3, out, c, s, m.ks), "ks_finish");
-            return;
-        }
         TIMED(7, launch_ks_intt(m.dig, rk, m.ks, c, s), "ks_intt");
-    }
-    TIMED(3, launch_relin_finish(c3, m.ks, out, c, s), "relin_finish");
-}
-
-void Engine::mul_relin_forked(StreamState *st, const uint64_t *a, const uint64_t *b, const uint64_t *rk, uint64_t *out, size_t n,
-                              cudaStream_t s) {
-    ForkSet &F = st->forks;  // owned by this (device, stream); the lease keeps it alive while we enqueue
-    const size_t sub = subchunk_ops_;
-    if (!F.ready || F.ops < sub) {
-        cuda_throw(cudaStreamSynchronize(s), "sync before fork-set rebuild");
-        for (int i = 0; i < kForkStreams; i++) {
-            if (!F.ready) {
-                cuda_throw(cudaStreamCreateWithFlags(&F.stream[i], cudaStreamNonBlocking), "cudaStreamCreate");
-                cuda_throw(cudaEventCreateWithFlags(&F.join[i], cudaEventDisableTiming), "cudaEventCreate");
-            }
-            if (F.scratch[i]) cudaFree(F.scratch[i]);
-            cuda_throw(cudaMalloc((void **)&F.scratch[i], sub * kScratchLimbsPerOp * kN * 8), "cudaMalloc(sub scratch)");
-        }
-        if (!F.ready) cuda_throw(cudaEventCreateWithFlags(&F.fork, cudaEventDisableTiming), "cudaEventCreate");
-        F.ready = true;
-        F.ops = sub;
-    }
-    cuda_throw(cudaEventRecord(F.fork, s), "fork record");
-    for (int i = 0; i < kForkStreams; i++) cuda_throw(cudaStreamWaitEvent(F.stream[i], F.fork, 0), "fork wait");
-    size_t k = 0;
-    for (size_t off = 0; off < n; off += sub, k++) {
-        const size_t c = n - off < sub ? n - off : sub;
-        const int i = (int)(k % kForkStreams);
-        ScratchMap m(F.scratch[i], sub);
-        enqueue_mul(a + off * kCtWords, b + off * kCtWords, m, c, F.stream[i], timing_);
-        enqueue_relin(m.c3, rk, out + off * kCtWords, m, c, F.stream[i], timing_);
-    }
-    for (int i = 0; i < kForkStreams; i++) {
-        cuda_throw(cudaEventRecord(F.join[i], F.stream[i]), "join record");
-        cuda_throw(cudaStreamWaitEvent(s, F.join[i], 0), "join wait");
+        TIMED(3, launch_relin_finish(c3, m.ks, out, c, s), "relin_finish");
     }
 }
 
@@ -635,13 +568,8 @@ void Engine::mul_relin(int device, const uint64_t *a, const uint64_t *b, const u
                        cudaStream_t s) {
     if (n == 0) return;
     device_context(device);
-    const bool forked = subchunk_ops_ && n > subchunk_ops_;
-    const size_t chunk = forked ? 0 : (chunk_ops_ < n ? chunk_ops_ : n);
+    const size_t chunk = chunk_ops_ < n ? chunk_ops_ : n;
     ScratchLease lease{this, lease_scratch(device, s, chunk), &Engine::release_scratch};
-    if (forked) {
-        mul_relin_forked(lease.st, a, b, rk, out, n, s);
-        return;
-    }
     ScratchMap m(lease.st->p, chunk);
     for (size_t off = 0; off < n; off += chunk) {
         const size_t c = n - off < chunk ? n - off : chunk;
@@ -676,10 +604,10 @@ void Engine::relinearize(int device, const uint64_t *c3, const uint64_t *rk, uin
 
 // ---------------------------------------------------------------- host-buffer batch (H2D | kernels | D2H overlapped)
 // Chunk schedule of the host pipelines: full chunks in the middle, a short first one (the kernels start after 0.5 ms of copies
-// instead of 1.3) and a short last one (less to drain) - both still >= 96 ops, the size from which the fused kernel set runs.
+// instead of 1.3) and a short last one (less to drain) - both still >= kFusedTailMinOps ops, so that they run the fused tails.
 // A function of (off, n, chunk) only: every loop over the same batch sees the same chunks.
 static size_t pipe_chunk(size_t off, size_t n, size_t chunk) {
-    const size_t rem = n - off, edge = 96;
+    const size_t rem = n - off, edge = kFusedTailMinOps;
     if (chunk <= edge || rem <= edge) return rem < chunk ? rem : chunk;
     if (off == 0) return edge;
     if (rem <= chunk) return rem > 2 * edge ? rem - edge : rem;

@@ -170,7 +170,6 @@ class Engine {
     // kernel ids: see kKernelNames.  report() synchronises the device.
     static constexpr int kNumTimedKernels = 16;
     void set_kernel_timing(bool on);
-    void set_fused(bool on) { fused_ = on; }  // choose k_behz_tensor/k_relin_ks (true) or the split kernels (false)
     void kernel_timing_report(int device, double ms[kNumTimedKernels], uint64_t launches[kNumTimedKernels]);
 
     // threshold-network simulation API (fhe.rs:594-779) against the embedded network keys
@@ -178,15 +177,6 @@ class Engine {
     int32_t reencrypt(Kind kind, Span in, Span net_pub, Span net_pri, std::vector<uint8_t> *out);
     int32_t decrypt(Kind kind, Span in, Span net_pub, Span net_pri, std::vector<uint8_t> *out);
 
-    // L2-resident fork/join pipeline state of one (device, stream), see subchunk_ops_
-    static constexpr int kForkStreams = 2;
-    struct ForkSet {
-        bool ready = false;
-        cudaStream_t stream[kForkStreams];
-        cudaEvent_t fork, join[kForkStreams];
-        uint64_t *scratch[kForkStreams] = {nullptr, nullptr};
-        size_t ops = 0;
-    };
     // scratch arena for `ops` concurrent multiply+relin ops, one per (device, caller stream): grown on demand, leased while
     // a caller enqueues, evicted (after synchronising its stream) when more than FHE_B200_SCRATCH_ARENAS are idle on a device
     struct StreamState {
@@ -196,7 +186,6 @@ class Engine {
         size_t ops = 0;
         int users = 0;
         uint64_t last_use = 0;
-        ForkSet forks;
     };
     StreamState *lease_scratch(int device, cudaStream_t s, size_t ops);
     void release_scratch(StreamState *st);
@@ -299,7 +288,6 @@ class Engine {
         int kernel;
         cudaEvent_t e0, e1;
     };
-    bool fused_ = false;  // FHE_B200_FUSED=1: multi-polynomial-per-CTA kernels (k_behz_tensor, k_relin_ks)
     bool timing_ = false;
     void enqueue_mul(const uint64_t *a, const uint64_t *b, const ScratchMap &m, size_t c, cudaStream_t s, bool timed);
     void enqueue_relin(const uint64_t *c3, const uint64_t *rk, uint64_t *out, const ScratchMap &m, size_t c, cudaStream_t s,
@@ -310,12 +298,6 @@ class Engine {
     std::vector<cudaEvent_t> event_pool_;
     cudaEvent_t take_event();
 
-    // L2-resident pipelining of multiply+relinearise: the batch is cut into sub-chunks whose scratch (1.7 MB per op)
-    // fits the 126 MB L2 and the sub-chunks alternate over kForkStreams internal streams, so that one sub-chunk's
-    // kernel tails overlap the other's heads while producer->consumer scratch stays on chip. 0 = off.
-    size_t subchunk_ops_ = 0;
-    void mul_relin_forked(StreamState *st, const uint64_t *a, const uint64_t *b, const uint64_t *rk, uint64_t *out, size_t n,
-                          cudaStream_t s);
     void free_stream_state(StreamState &v);
     std::vector<std::unique_ptr<StreamState>> stream_states_;
     uint64_t arena_clock_ = 0;

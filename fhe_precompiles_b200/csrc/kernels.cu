@@ -6,7 +6,7 @@
 // Device data layouts (u64 everywhere, limb-major):
 //   data-level ciphertext   [poly 0..1][limb q0,q1][4096]                 128 KiB
 //   size-3 ciphertext       [poly 0..2][limb q0,q1][4096]
-//   BEHZ tensor scratch     [poly 0..2][limb q0,q1,b0,b1,msk][4096]       (already x t)
+//   BEHZ tensor scratch     [poly 0..2][slot 0..4][4096]                  (already x t; dual words in slots 2..4)
 //   key-switch scratch      [poly 0..1][limb q0,q1,P][4096]
 //   relin key               [digit 0..1][poly 0..1][limb q0,q1,P][4096]   NTT form, as in the key file
 //   plaintext               [4096] u16 coefficients < t, zero padded
@@ -14,10 +14,6 @@
 #include <cstdio>
 
 #include "kernels.h"
-
-#ifndef FHE_B200_WIDESUM
-#define FHE_B200_WIDESUM 1  // CRT recoveries on exact two-accumulator sums (modarith.cuh WideSum); 0 = the ShoupSum form
-#endif
 
 namespace fheb {
 __constant__ DevTwLow ktl;  // defined before ntt.cuh, which reads it
@@ -40,35 +36,34 @@ cudaError_t upload_constants(const DevConsts &c, const DevTables &t, const DevTw
 // =====================================================================================
 // K1/K2: batched limb NTT (config 2 microbenchmark; also used by the parity tests)
 // =====================================================================================
-template <int MI, bool INV, bool SHFL>
+template <int MI, bool INV>
 __device__ __forceinline__ void ntt_limb_body(u64 *limb, u64 *smem, int t) {
     using M = Mod<MI>;
     u64 v[1][8];
     if (!INV) {
         load_natural(limb, v[0], t);
-        ntt_forward<M, 1, true, false, SHFL>(v, smem, kt.twf[MI], t);
+        ntt_forward<M, 1, true, false>(v, smem, kt.twf[MI], t);
         store_chunk8(limb, v[0], t);
     } else {
         load_chunk8(limb, v[0], t);
-        ntt_inverse<M, 1, true, false, SHFL>(v, smem, kt.twi[MI], t, kc.ninv[MI], kc.ninv_w[MI]);
+        ntt_inverse<M, 1, true, false>(v, smem, kt.twi[MI], t, kc.ninv[MI], kc.ninv_w[MI]);
         store_natural(limb, v[0], t);
     }
 }
 
-// SHFL: the last (intra-warp) exchange through warp shuffles instead of shared memory (A/B variant, see ntt.cuh)
-template <bool INV, bool SHFL>
+template <bool INV>
 // the forward transform fits 40 registers (3 CTAs per SM, +9 % on the 36-bit primes); the inverse does not gain from it
 __global__ void __launch_bounds__(kThreads, INV ? 2 : 3) k_ntt(u64 *data, LimbMods mods) {
     extern __shared__ __align__(16) u64 smem[];
     const int t = threadIdx.x;
     u64 *limb = data + (size_t)blockIdx.x * kN;
     switch (mods.mod[blockIdx.x % mods.n]) {
-        case MQ0: ntt_limb_body<MQ0, INV, SHFL>(limb, smem, t); break;
-        case MQ1: ntt_limb_body<MQ1, INV, SHFL>(limb, smem, t); break;
-        case MP: ntt_limb_body<MP, INV, SHFL>(limb, smem, t); break;
-        case MB0: ntt_limb_body<MB0, INV, SHFL>(limb, smem, t); break;
-        case MB1: ntt_limb_body<MB1, INV, SHFL>(limb, smem, t); break;
-        default: ntt_limb_body<MSK, INV, SHFL>(limb, smem, t); break;
+        case MQ0: ntt_limb_body<MQ0, INV>(limb, smem, t); break;
+        case MQ1: ntt_limb_body<MQ1, INV>(limb, smem, t); break;
+        case MP: ntt_limb_body<MP, INV>(limb, smem, t); break;
+        case MB0: ntt_limb_body<MB0, INV>(limb, smem, t); break;
+        case MB1: ntt_limb_body<MB1, INV>(limb, smem, t); break;
+        default: ntt_limb_body<MSK, INV>(limb, smem, t); break;
     }
 }
 
@@ -180,12 +175,20 @@ __global__ void __launch_bounds__(kThreads, 1) k_mul_plain(const u64 *__restrict
 }
 
 // =====================================================================================
-// K6+K1+K7+K2: BEHZ base extension -> forward NTT -> tensor -> inverse NTT (x t)
-//   SEAL Evaluator::bfv_multiply steps (1)-(6); RNSTool::fastbconv_m_tilde, RNSTool::sm_mrq
-// one CTA per (extended limb e = q0,q1,b0,b1,msk ; op)
+// K6-K8: BEHZ multiply   (SEAL Evaluator::bfv_multiply steps (1)-(6); RNSTool::fastbconv_m_tilde, sm_mrq, fast_floor,
+// fastbconv_sk) on the DUAL base (params.h kDualPrime, devconsts.h d_*).  bfv_multiply's result is a function of integer
+// polynomials -- the extended operands a' = (y0 + r q) / m~, their product D, f = (t D - y0') / q -- and does not depend on the
+// auxiliary primes that carry them, so they are carried by six primes below 2^30, two per 64-bit word, where a butterfly costs
+// one IMAD.HI + two IMAD per lane (8 multiplier cycles per 30 bits) instead of 6 IMAD.WIDE + 4 IMAD (32 cycles per 61 bits
+// on SEAL's Bsk primes).  The dual words live in slots e = 2..4 of the 5-limb scratch arrays (engine.h ScratchMap).
+//   k_ext_conv_d     : a' mod s_i for the 4 input polynomials                         eltwise
+//   k_ext_ntt_d      : 12 forward dual transforms, in place                           grid (12, ops)
+//   k_tensor_intt_d  : dyadic tensor + 9 inverse dual transforms (x N^-1 t)           grid (9, ops)
+//   k_floor_sk_d     : exact CRT of t D -> t_l -> y0 -> f on (s_0..s_3) -> f mod q_l   eltwise
+//   k_tensor_floor_d : k_tensor_intt_d + k_floor_sk_d in one kernel (chunks >= 96 ops) grid (3, ops)
 // =====================================================================================
 // y0 = t0 q1 + t1 q0 as a 128-bit integer (t_l canonical residues mod q_l): q_l = 2^36 - c_l, so
-// y0 = ((t0 + t1) << 36) - (t0 c1 + t1 c0), one multiply chain and a shift.  Shared by k_ext_conv and k_floor_sk.
+// y0 = ((t0 + t1) << 36) - (t0 c1 + t1 c0), one multiply chain and a shift.  Shared by k_ext_conv_d and k_floor_sk_d.
 __device__ __forceinline__ void punctured_sum(u64 t0, u64 t1, u64 &ylo, u64 &yhi) {
     constexpr u32 c0 = (u32)Mod<MQ0>::kC, c1 = (u32)Mod<MQ1>::kC;
     u32 t0l, t0h, t1l, t1h, pl, ph;
@@ -199,7 +202,10 @@ __device__ __forceinline__ void punctured_sum(u64 t0, u64 t1, u64 &ylo, u64 &yhi
     ylo = sh - pv;
     yhi = (ts >> 28) - (sh < pv ? 1 : 0);
 }
-// Shared part of the integer-domain base extension (see k_ext_conv): Z = base + m 2^61 (- q if neg)
+// Base extension in the integer domain.  SEAL's fastbconv_m_tilde + sm_mrq compute, per auxiliary prime p, (y0 + r q) m~^-1
+// mod p with r = -y0 q^-1 mod m~ centred: y0 + r q is an exact multiple of m~ = 2^32, so the value is the INTEGER
+// Z = (y0 + r q) / 2^32 (|Z| < 2^72) reduced mod p.  ext_shared forms Z once per coefficient, as base + m 2^61 (- q if neg);
+// ext_dual reduces it mod each dual prime.
 __device__ __forceinline__ void ext_shared(u64 x0, u64 x1, u64 &base, u32 &m, bool &neg) {
     const u64 t0 = shoup<Mod<MQ0>>(x0, kc.ext_in[0].w, kc.ext_in[0].ws);
     const u64 t1 = shoup<Mod<MQ1>>(x1, kc.ext_in[1].w, kc.ext_in[1].ws);
@@ -215,411 +221,7 @@ __device__ __forceinline__ void ext_shared(u64 x0, u64 x1, u64 &base, u32 &m, bo
     m = (u32)(sAB >> 61) + (sAB < A ? 8u : 0u) + (u32)(Cv >> 29);             // < 2^12
     base = (sAB & ((1ull << 61) - 1)) + ((Cv & ((1ull << 29) - 1)) << 32);  // < 2^62
 }
-template <int K>
-__device__ __forceinline__ u64 ext_limb(u64 base, u32 m, bool neg) {
-    using M = Mod<kExtLimb[2 + K]>;
-    return canon_k32<M>(base + (u64)(m * (u32)M::kC) + (neg ? kc.extNeg[K] : 0));
-}
-// Loads polynomial `poly` of a data-level ciphertext into pass-0 register layout in limb EI of the
-// extended base.  EI < 2: plain copy of the q-limb.  EI >= 2: fast base conversion through m_tilde with
-// the Montgomery correction, all per coefficient:
-//   tmp_l = x_l * (m~ * (q/q_l)^-1) mod q_l                     (canonical)
-//   r     = -(tmp_0*(q/q_0) + tmp_1*(q/q_1)) * q^-1 mod 2^32, centred
-//   x'_k  = (tmp_0*(q/q_0) + tmp_1*(q/q_1) + r*q) / 2^32  mod p_k     (integer domain: ext_shared / ext_limb)
-template <int EI>
-__device__ __forceinline__ void load_extended(const u64 *__restrict__ ct, int poly, u64 (&v)[8], int t) {
-    constexpr int MI = kExtLimb[EI];
-    using M = Mod<MI>;
-    if (EI < 2) {
-        load_natural(ct + (size_t)(poly * 2 + EI) * kN, v, t);
-    } else {
-        constexpr int K = EI - 2;
-        const u64 *x0 = ct + (size_t)(poly * 2 + 0) * kN;
-        const u64 *x1 = ct + (size_t)(poly * 2 + 1) * kN;
-#pragma unroll
-        for (int r = 0; r < 8; r++) {
-            int i = r * kThreads + t;
-            u64 base;
-            u32 m;
-            bool neg;
-            ext_shared(x0[i], x1[i], base, m, neg);
-            v[r] = ext_limb<K>(base, m, neg);
-        }
-    }
-}
 
-template <int EI>
-__device__ __forceinline__ void behz_tensor_body(const u64 *__restrict__ a, const u64 *__restrict__ b, u64 *__restrict__ tens,
-                                                 u64 *smem, int t) {
-    constexpr int MI = kExtLimb[EI];
-    using M = Mod<MI>;
-    const ulonglong2 *twf = kt.twf[MI];
-    // a0, a1: transform in buffers 0-1, then park the results in buffers 2-3 at this thread's own
-    // pass-9 slots (same slots the inverse transform later overwrites, so no cross-thread hazard)
-    {
-        u64 A[2][8];
-        load_extended<EI>(a, 0, A[0], t);
-        load_extended<EI>(a, 1, A[1], t);
-        ntt_forward<M, 2, true>(A, smem, twf, t);
-        smem_store<2, 9>(smem + 2 * kN, A, t);
-    }
-    u64 B[2][8];
-    load_extended<EI>(b, 0, B[0], t);
-    load_extended<EI>(b, 1, B[1], t);
-    ntt_forward<M, 2, true>(B, smem, twf, t);
-    u64 D[3][8];
-#pragma unroll
-    for (int r = 0; r < 8; r++) {
-        const int slot = swz(elem_index<9>(t, r));
-        const u64 a0 = smem[2 * kN + slot], a1 = smem[3 * kN + slot];
-        D[0][r] = mulmod<M>(a0, B[0][r]);
-        u64 lo = 0, hi = 0;
-        mac128(lo, hi, a0, B[1][r]);
-        mac128(lo, hi, a1, B[0][r]);
-        D[1][r] = reduce128<M>(hi, lo);
-        D[2][r] = mulmod<M>(a1, B[1][r]);
-    }
-    ntt_inverse<M, 3>(D, smem, kt.twi[MI], t, kc.ninv_t[MI], kc.ninv_t_w[MI]);
-#pragma unroll
-    for (int p = 0; p < 3; p++) store_natural(tens + (size_t)(p * 5 + EI) * kN, D[p], t);
-}
-
-__global__ void __launch_bounds__(kThreads, 1) k_behz_tensor(const u64 *__restrict__ a, const u64 *__restrict__ b,
-                                                              u64 *__restrict__ tens) {
-    extern __shared__ __align__(16) u64 smem[];
-    const size_t op = blockIdx.y;
-    const u64 *pa = a + op * 4 * kN;
-    const u64 *pb = b + op * 4 * kN;
-    u64 *pt = tens + op * 15 * kN;
-    const int t = threadIdx.x;
-    switch (blockIdx.x) {
-        case 0: behz_tensor_body<0>(pa, pb, pt, smem, t); break;
-        case 1: behz_tensor_body<1>(pa, pb, pt, smem, t); break;
-        case 2: behz_tensor_body<2>(pa, pb, pt, smem, t); break;
-        case 3: behz_tensor_body<3>(pa, pb, pt, smem, t); break;
-        default: behz_tensor_body<4>(pa, pb, pt, smem, t); break;
-    }
-}
-
-// debug / parity tap: base extension only, ext layout [4 polys a0,a1,b0,b1][5 limbs][N]
-template <int EI>
-__device__ __forceinline__ void extend_only_body(const u64 *a, const u64 *b, u64 *ext, int t) {
-    u64 v[8];
-    for (int p = 0; p < 4; p++) {
-        load_extended<EI>(p < 2 ? a : b, p & 1, v, t);
-        store_natural(ext + (size_t)(p * 5 + EI) * kN, v, t);
-    }
-}
-__global__ void __launch_bounds__(kThreads) k_behz_extend_tap(const u64 *a, const u64 *b, u64 *ext) {
-    const size_t op = blockIdx.y;
-    const u64 *pa = a + op * 4 * kN;
-    const u64 *pb = b + op * 4 * kN;
-    u64 *pe = ext + op * 20 * kN;
-    const int t = threadIdx.x;
-    switch (blockIdx.x) {
-        case 0: extend_only_body<0>(pa, pb, pe, t); break;
-        case 1: extend_only_body<1>(pa, pb, pe, t); break;
-        case 2: extend_only_body<2>(pa, pb, pe, t); break;
-        case 3: extend_only_body<3>(pa, pb, pe, t); break;
-        default: extend_only_body<4>(pa, pb, pe, t); break;
-    }
-}
-
-// =====================================================================================
-// Split variant of the BEHZ front end (default): one polynomial per CTA, 58-64 registers, 32 KiB smem,
-// two CTAs per SM.  Same arithmetic as k_behz_tensor; the NTT-domain limbs go through an L2-resident
-// scratch [op][4 polys a0,a1,b0,b1][5 limbs][N] instead of shared memory.
-//   k_ext_ntt     : base extension (limb >= 2) + forward NTT            grid (20 = poly*5+limb, ops)
-//   k_tensor_intt : dyadic tensor term + inverse NTT (x N^-1 t)          grid (15 = d*5+limb, ops)
-// =====================================================================================
-template <int EI>
-__device__ __forceinline__ void ext_ntt_body(const u64 *__restrict__ ct, int poly, u64 *__restrict__ dst, u64 *smem, int t) {
-    constexpr int MI = kExtLimb[EI];
-    using M = Mod<MI>;
-    u64 v[1][8];
-    load_extended<EI>(ct, poly, v[0], t);
-    // 36-bit limbs stay lazy (< 2^43): the tensor's 128-bit accumulate absorbs it; 61-bit limbs must be canonical
-    ntt_forward<M, 1, !M::kSmall, false>(v, smem, kt.twf[MI], t);
-    store_chunk8_lm(dst, v[0], t);
-}
-__global__ void __launch_bounds__(kThreads, 2) k_ext_ntt(const u64 *__restrict__ a, const u64 *__restrict__ b,
-                                                          u64 *__restrict__ nttbuf) {
-    extern __shared__ __align__(16) u64 smem[];
-    const size_t op = blockIdx.y;
-    const int p = blockIdx.x / 5, e = blockIdx.x % 5;
-    const u64 *ct = (p < 2 ? a : b) + op * 4 * kN;
-    u64 *dst = nttbuf + (op * 20 + blockIdx.x) * kN;
-    const int t = threadIdx.x;
-    switch (e) {
-        case 0: ext_ntt_body<0>(ct, p & 1, dst, smem, t); break;
-        case 1: ext_ntt_body<1>(ct, p & 1, dst, smem, t); break;
-        case 2: ext_ntt_body<2>(ct, p & 1, dst, smem, t); break;
-        case 3: ext_ntt_body<3>(ct, p & 1, dst, smem, t); break;
-        default: ext_ntt_body<4>(ct, p & 1, dst, smem, t); break;
-    }
-}
-
-// ---- default front end: base extension as its own elementwise kernel (FHE_B200_EXT_SPLIT=0 selects k_ext_ntt above)
-// k_ext_conv computes the three auxiliary-limb residues of every coefficient ONCE (the per-limb CTAs of k_ext_ntt each redo
-// the two q-limb products and the m~ correction) in a full-occupancy elementwise kernel and leaves them, coefficient domain,
-// in the scratch slots the transforms then work on in place.  The transform-only kernel needs 40 registers: 3 CTAs per SM
-// instead of 2.  431.9 k -> 444.7 k ops/s; the same split of the tensor product (elementwise + in-place inverse transforms)
-// was slower (the elementwise pass moves 1.1 MB per op through DRAM) and is not kept.
-// Base extension in the integer domain.  SEAL's fastbconv_m_tilde + sm_mrq compute, per Bsk prime p_k,
-// (y0 + r q) m~^-1 mod p_k with r = -y0 q^-1 mod m~ centred: y0 + r q is an exact multiple of m~ = 2^32, so the value is the
-// INTEGER Z = (y0 + r q) / 2^32 (|Z| < 2^72) reduced mod p_k.  Z is formed once, as base + m 2^61 (- q if r < 0), and every
-// p_k = 2^61 - c_k needs only base + m c_k: two low multiplies per auxiliary limb instead of three Shoup products.
-__global__ void __launch_bounds__(256) k_ext_conv(const u64 *__restrict__ a, const u64 *__restrict__ b, u64 *__restrict__ nttbuf,
-                                                  size_t n_ops) {
-    const size_t total = n_ops * 4 * (kN / 2);  // (op, poly a0 a1 b0 b1, coefficient pair): 16-byte loads and stores
-    for (size_t g = (size_t)blockIdx.x * 256 + threadIdx.x; g < total; g += (size_t)gridDim.x * 256) {
-        const size_t op = g / (4 * (kN / 2));
-        const int p = (int)((g / (kN / 2)) & 3), i = 2 * (int)(g & (kN / 2 - 1));
-        const u64 *ct = (p < 2 ? a : b) + op * 4 * kN + (size_t)(p & 1) * 2 * kN;
-        const ulonglong2 x0 = *reinterpret_cast<const ulonglong2 *>(ct + i), x1 = *reinterpret_cast<const ulonglong2 *>(ct + kN + i);
-        u64 base0, base1;
-        u32 m0, m1;
-        bool neg0, neg1;
-        ext_shared(x0.x, x1.x, base0, m0, neg0);
-        ext_shared(x0.y, x1.y, base1, m1, neg1);
-        u64 *dst = nttbuf + (op * 20 + (size_t)p * 5 + 2) * kN + i;
-        *reinterpret_cast<ulonglong2 *>(dst) = make_ulonglong2(ext_limb<0>(base0, m0, neg0), ext_limb<0>(base1, m1, neg1));
-        *reinterpret_cast<ulonglong2 *>(dst + kN) = make_ulonglong2(ext_limb<1>(base0, m0, neg0), ext_limb<1>(base1, m1, neg1));
-        *reinterpret_cast<ulonglong2 *>(dst + 2 * kN) = make_ulonglong2(ext_limb<2>(base0, m0, neg0), ext_limb<2>(base1, m1, neg1));
-    }
-}
-template <int EI>
-__device__ __forceinline__ void ntt_only_body(const u64 *__restrict__ src, u64 *__restrict__ dst, u64 *smem, int t) {
-    constexpr int MI = kExtLimb[EI];
-    using M = Mod<MI>;
-    u64 v[1][8];
-    load_natural(src, v[0], t);
-    ntt_forward<M, 1, !M::kSmall, false>(v, smem, kt.twf[MI], t);
-    store_chunk8_lm(dst, v[0], t);
-}
-// aux_only (default): grid (12, ops), the Bsk limbs only -- the q-limbs of the tensor product are recovered from its Bsk
-// limbs in k_floor_sk (exactly), so the q-limbs of the operands are never transformed.  Otherwise grid (20, ops).
-__global__ void __launch_bounds__(kThreads, 3) k_ext_ntt2(const u64 *__restrict__ a, const u64 *__restrict__ b,
-                                                           u64 *__restrict__ nttbuf, int aux_only) {
-    extern __shared__ __align__(16) u64 smem[];
-    const size_t op = blockIdx.y;
-    const int p = aux_only ? blockIdx.x / 3 : blockIdx.x / 5, e = aux_only ? 2 + blockIdx.x % 3 : blockIdx.x % 5;
-    u64 *dst = nttbuf + (op * 20 + (size_t)(p * 5 + e)) * kN;
-    // q limbs come from the operand, auxiliary limbs are transformed in place (every load precedes the first CTA barrier)
-    const u64 *src = e < 2 ? (p < 2 ? a : b) + op * 4 * kN + (size_t)((p & 1) * 2 + e) * kN : dst;
-    const int t = threadIdx.x;
-    switch (e) {
-        case 0: ntt_only_body<0>(src, dst, smem, t); break;
-        case 1: ntt_only_body<1>(src, dst, smem, t); break;
-        case 2: ntt_only_body<2>(src, dst, smem, t); break;
-        case 3: ntt_only_body<3>(src, dst, smem, t); break;
-        default: ntt_only_body<4>(src, dst, smem, t); break;
-    }
-}
-
-template <int EI>
-__device__ __forceinline__ void tensor_intt_body(const u64 *__restrict__ nb, int d, u64 *__restrict__ dst, u64 *smem, int t) {
-    constexpr int MI = kExtLimb[EI];
-    using M = Mod<MI>;
-    // nb: [4 polys][5 limbs][N] of this op; polys a0,a1,b0,b1
-    const u64 *a0 = nb + (size_t)(0 * 5 + EI) * kN, *a1 = nb + (size_t)(1 * 5 + EI) * kN;
-    const u64 *b0 = nb + (size_t)(2 * 5 + EI) * kN, *b1 = nb + (size_t)(3 * 5 + EI) * kN;
-    u64 v[1][8];
-    // two coefficients at a time, so that the products do not keep 32 operands live
-    const ulonglong2 *pa0 = lm_ptr(a0, t), *pa1 = lm_ptr(a1, t), *pb0 = lm_ptr(b0, t), *pb1 = lm_ptr(b1, t);  // pair r at [r * kLm]
-    if (d == 1) {
-#pragma unroll
-        for (int r = 0; r < 4; r++) {
-            const ulonglong2 x0 = pa0[r * kLm], y1 = pb1[r * kLm], x1 = pa1[r * kLm], y0 = pb0[r * kLm];
-            {
-                const u64 xs[2] = {x0.x, x1.x}, ys[2] = {y1.x, y0.x};
-                v[0][2 * r] = mulsum<M, 2>(xs, ys);
-            }
-            {
-                const u64 xs[2] = {x0.y, x1.y}, ys[2] = {y1.y, y0.y};
-                v[0][2 * r + 1] = mulsum<M, 2>(xs, ys);
-            }
-        }
-    } else {
-        const ulonglong2 *px = d == 0 ? pa0 : pa1, *py = d == 0 ? pb0 : pb1;
-#pragma unroll
-        for (int r = 0; r < 4; r++) {
-            const ulonglong2 x = px[r * kLm], y = py[r * kLm];
-            {
-                const u64 xs[1] = {x.x}, ys[1] = {y.x};
-                v[0][2 * r] = mulsum<M, 1>(xs, ys);
-            }
-            {
-                const u64 xs[1] = {x.y}, ys[1] = {y.y};
-                v[0][2 * r + 1] = mulsum<M, 1>(xs, ys);
-            }
-        }
-    }
-    // outputs stay in [0, 2q): k_floor_sk's Shoup / 128-bit reductions take any such value
-    ntt_inverse<M, 1, false, false>(v, smem, kt.twi[MI], t, kc.ninv_t[MI], kc.ninv_t_w[MI]);
-    store_natural(dst, v[0], t);
-}
-__global__ void __launch_bounds__(kThreads, 2) k_tensor_intt(const u64 *__restrict__ nttbuf, u64 *__restrict__ tens, int aux_only) {
-    extern __shared__ __align__(16) u64 smem[];
-    const size_t op = blockIdx.y;
-    const int d = aux_only ? blockIdx.x / 3 : blockIdx.x / 5, e = aux_only ? 2 + blockIdx.x % 3 : blockIdx.x % 5;
-    const u64 *nb = nttbuf + op * 20 * kN;
-    u64 *dst = tens + (op * 15 + (size_t)(d * 5 + e)) * kN;
-    const int t = threadIdx.x;
-    switch (e) {
-        case 0: tensor_intt_body<0>(nb, d, dst, smem, t); break;
-        case 1: tensor_intt_body<1>(nb, d, dst, smem, t); break;
-        case 2: tensor_intt_body<2>(nb, d, dst, smem, t); break;
-        case 3: tensor_intt_body<3>(nb, d, dst, smem, t); break;
-        default: tensor_intt_body<4>(nb, d, dst, smem, t); break;
-    }
-}
-
-// =====================================================================================
-// K8: fast_floor + fastbconv_sk   (SEAL RNSTool::fast_floor, RNSTool::fastbconv_sk), per coefficient
-//   tens [op][3][5][N] (x t, any representative in [0, 2q))  ->  c3 [op][3][2][N]
-// =====================================================================================
-// t_l = [t D (q/q_l)^-1]_{q_l} from the three Bsk residues of t D alone (devconsts.h: crt3, crtK, crtNB): the q-limbs of the
-// tensor product are never computed.  t D is an integer with |t D| < 2^166 and Bsk ~ 2^183, so sum y_i / p_i lies within
-// 2^-17 of the integer v and 16 bits per term are plenty; any representative of y_i works (v moves with it).
-__device__ __forceinline__ void floor_front_crt(u64 vb0, u64 vb1, u64 vsk, u64 &t0, u64 &t1) {
-    const u64 y0 = shoup_acc<Mod<MB0>, 1>(0, vb0, kc.crt3[0].w, kc.crt3[0].ws);  // [0, 4 p): < 2^63
-    const u64 y1 = shoup_acc<Mod<MB1>, 1>(0, vb1, kc.crt3[1].w, kc.crt3[1].ws);
-    const u64 y2 = shoup_acc<Mod<MSK>, 1>(0, vsk, kc.crt3[2].w, kc.crt3[2].ws);
-    const u32 v = (u32)(((y0 >> 45) + (y1 >> 45) + (y2 >> 45) + (1u << 15)) >> 16);  // <= 12
-    {
-        ShoupSum<Mod<MQ0>> s;  // three terms < 3.5 q each + v K' < 12 q
-        s.add_a1(y0, kc.crtK[0][0].w, kc.crtK[0][0].ws);
-        s.add_a1(y1, kc.crtK[1][0].w, kc.crtK[1][0].ws);
-        s.add_a1(y2, kc.crtK[2][0].w, kc.crtK[2][0].ws);
-        s.add_small(v, kc.crtNB[0].w);
-        t0 = canon_k32<Mod<MQ0>>(s.value());
-    }
-    {
-        ShoupSum<Mod<MQ1>> s;
-        s.add_a1(y0, kc.crtK[0][1].w, kc.crtK[0][1].ws);
-        s.add_a1(y1, kc.crtK[1][1].w, kc.crtK[1][1].ws);
-        s.add_a1(y2, kc.crtK[2][1].w, kc.crtK[2][1].ws);
-        s.add_small(v, kc.crtNB[1].w);
-        t1 = canon_k32<Mod<MQ1>>(s.value());
-    }
-}
-template <bool CRT>
-__device__ __forceinline__ void floor_sk_coeff(u64 v0, u64 v1, u64 vb0, u64 vb1, u64 vsk, u64 &o0, u64 &o1) {
-    using Q0 = Mod<MQ0>;
-    using Q1 = Mod<MQ1>;
-    using B0 = Mod<MB0>;
-    using B1 = Mod<MB1>;
-    using SK = Mod<MSK>;
-    {
-        // fast_floor: q-part -> Bsk, f_k = (v_k - conv_k) * q^-1 mod p_k  (constants merged)
-        u64 t0, t1;
-        if (CRT) {
-            floor_front_crt(vb0, vb1, vsk, t0, t1);
-        } else {
-            t0 = shoup<Q0>(v0, kc.inv_punct_q[0].w, kc.inv_punct_q[0].ws);
-            t1 = shoup<Q1>(v1, kc.inv_punct_q[1].w, kc.inv_punct_q[1].ws);
-        }
-        // The q-part of the value is the integer y0 = t0 q1 + t1 q0 (< 2^73); its residue mod a Bsk prime 2^61 - c is a fold.
-        u64 ylo, yhi;
-        punctured_sum(t0, t1, ylo, yhi);
-        const u64 y61 = ylo & ((1ull << 61) - 1);
-        const u32 yk = (u32)((ylo >> 61) | (yhi << 3));  // < 2^12
-        // tb_j = [(v_bj - y0) q^-1 (B/b_j)^-1]_{b_j}: one exact Shoup product (skV); canonical, it is carried into other moduli
-        const u64 xb0 = vb0 + B0::two_q - (y61 + (u64)(yk * (u32)B0::kC));
-        const u64 xb1 = vb1 + B1::two_q - (y61 + (u64)(yk * (u32)B1::kC));
-        if (CRT) {
-            // f = (t D - y0) / q is an integer below 2^96 and B = b0 b1 ~ 2^122, so its lift from (b0, b1) needs no m_sk:
-            // f = tb0 b1 + tb1 b0 - v' B with v' = round(tb0 / b0 + tb1 / b1), exactly what fastbconv_sk's Shenoy-Kumaresan
-            // correction produces (both are the exact f mod q_l); any representative of tb_j works (v' moves with it)
-            const u64 tb0 = shoup_acc<B0, 1>(0, xb0, kc.skV[0], kc.skVs[0]);  // [0, 4 p)
-            const u64 tb1 = shoup_acc<B1, 1>(0, xb1, kc.skV[1], kc.skVs[1]);
-            const u32 vp = (u32)(((tb0 >> 45) + (tb1 >> 45) + (1u << 15)) >> 16);  // <= 8
-            {
-                ShoupSum<Q0> s;  // two terms < 3.5 q each + v' (q - B mod q) < 8 q
-                s.add_a1(tb0, kc.pBq[0][0].w, kc.pBq[0][0].ws);
-                s.add_a1(tb1, kc.pBq[1][0].w, kc.pBq[1][0].ws);
-                s.add_small(vp, kc.nBq[0].w);
-                o0 = canon_k32<Q0>(s.value());
-            }
-            {
-                ShoupSum<Q1> s;
-                s.add_a1(tb0, kc.pBq[0][1].w, kc.pBq[0][1].ws);
-                s.add_a1(tb1, kc.pBq[1][1].w, kc.pBq[1][1].ws);
-                s.add_small(vp, kc.nBq[1].w);
-                o1 = canon_k32<Q1>(s.value());
-            }
-            return;
-        }
-        const u64 tb0 = canon_k32<B0>(shoup_lazy<B0>(xb0, kc.skV[0], kc.skVs[0]));
-        const u64 tb1 = canon_k32<B1>(shoup_lazy<B1>(xb1, kc.skV[1], kc.skVs[1]));
-        // alpha = [(tb0 b1 + tb1 b0  -  (v_msk - y0) q^-1) B^-1]_{m_sk}, and b_j == -(m_sk - b_j) (mod m_sk) is 19 bits:
-        // w = tb0 skD[1] + tb1 skD[0] (82 bits, two multiply chains), folded below 2^63
-        u64 alpha;
-        {
-            u32 al, ah, bl, bh;
-            unpack64(tb0, al, ah);
-            unpack64(tb1, bl, bh);
-            const u64 wlo = mad_wide(al, kc.skD[1], mul_wide(bl, kc.skD[0]));
-            const u64 whi = mad_wide(ah, kc.skD[1], mul_wide(bh, kc.skD[0]));  // weight 2^32, < 2^49
-            const u64 wr = wlo + ((whi & ((1ull << 29) - 1)) << 32) + mul_wide((u32)(whi >> 29), (u32)SK::kC);
-            const u64 xs = vsk + SK::two_q - (y61 + (u64)(yk * (u32)SK::kC));
-            ShoupSum<SK> s;  // two terms < 1.5 q each
-            s.add(wr, kc.nib.w, kc.nib.ws);
-            s.add(xs, kc.alK2, kc.alK2s);
-            alpha = canon_k32<SK>(s.value());
-        }
-        bool neg = alpha > (SK::q >> 1);
-        u64 am = neg ? SK::q - alpha : alpha;
-        {  // 36-bit targets: approximate quotients, three terms < 3.2 q each (< 2^40)
-            const Shoup kb = neg ? kc.Bq[0] : kc.nBq[0];
-            ShoupSum<Q0> s;
-            s.add_a1(tb0, kc.pBq[0][0].w, kc.pBq[0][0].ws);
-            s.add_a1(tb1, kc.pBq[1][0].w, kc.pBq[1][0].ws);
-            s.add_a1(am, kb.w, kb.ws);
-            o0 = canon_k32<Q0>(s.value());
-        }
-        {
-            const Shoup kb = neg ? kc.Bq[1] : kc.nBq[1];
-            ShoupSum<Q1> s;
-            s.add_a1(tb0, kc.pBq[0][1].w, kc.pBq[0][1].ws);
-            s.add_a1(tb1, kc.pBq[1][1].w, kc.pBq[1][1].ws);
-            s.add_a1(am, kb.w, kb.ws);
-            o1 = canon_k32<Q1>(s.value());
-        }
-    }
-}
-template <bool CRT>
-__global__ void __launch_bounds__(256) k_floor_sk(const u64 *__restrict__ tens, u64 *__restrict__ c3, size_t n_ops) {
-    const size_t total = n_ops * 3 * (kN / 2);  // (op, poly, coefficient pair): 16-byte loads and stores
-    const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x; g < total; g += stride) {
-        const size_t opp = g / (kN / 2);  // op*3 + poly
-        const int i = 2 * (int)(g % (kN / 2));
-        const ulonglong2 *in = reinterpret_cast<const ulonglong2 *>(tens + opp * 5 * kN + i);
-        ulonglong2 v0 = make_ulonglong2(0, 0), v1 = v0;
-        if (!CRT) v0 = in[0], v1 = in[kN / 2];  // CRT: the q-limb slots of `tens` are never written
-        const ulonglong2 vb0 = in[2 * (kN / 2)], vb1 = in[3 * (kN / 2)], vsk = in[4 * (kN / 2)];
-        u64 ax, ay, bx, by;  // limb q0 / q1 of the two coefficients
-        floor_sk_coeff<CRT>(v0.x, v1.x, vb0.x, vb1.x, vsk.x, ax, bx);
-        floor_sk_coeff<CRT>(v0.y, v1.y, vb0.y, vb1.y, vsk.y, ay, by);
-        ulonglong2 *out = reinterpret_cast<ulonglong2 *>(c3 + opp * 2 * kN + i);
-        out[0] = make_ulonglong2(ax, ay);
-        out[kN / 2] = make_ulonglong2(bx, by);
-    }
-}
-
-// =====================================================================================
-// K6d-K8d: the BEHZ multiply on the DUAL base (default; params.h kDualPrime, devconsts.h d_*).  bfv_multiply's result is
-// a function of integer polynomials -- the extended operands a' = (y0 + r q) / m~, their product D, f = (t D - y0') / q --
-// and does not depend on the auxiliary primes that carry them, so they are carried by six primes below 2^30, two per
-// 64-bit word, where a butterfly costs one IMAD.HI + two IMAD per lane (8 multiplier cycles per 30 bits) instead of
-// 6 IMAD.WIDE + 4 IMAD (32 cycles per 61 bits).  Same scratch slots as the 61-bit limbs (e = 2..4 of the 5-limb arrays).
-//   k_ext_conv_d    : a' mod s_i for the 4 input polynomials                         eltwise
-//   k_ext_ntt_d     : 12 forward dual transforms, in place                           grid (12, ops)
-//   k_tensor_intt_d : dyadic tensor + 9 inverse dual transforms (x N^-1 t)           grid (9, ops)
-//   k_floor_sk_d    : exact CRT of t D -> t_l -> y0 -> f on (s_0..s_3) -> f mod q_l   eltwise
-// =====================================================================================
 template <int D>
 __device__ __forceinline__ u64 ext_dual(u64 base, u32 m, bool neg) {
     u32 bl, bh, r[2];
@@ -635,6 +237,9 @@ __device__ __forceinline__ u64 ext_dual(u64 base, u32 m, bool neg) {
     }
     return pack64(r[0], r[1]);
 }
+// The extension is its own full-occupancy elementwise kernel: the shared part is computed once per coefficient (a CTA per dual
+// word would redo it three times) and the residues are left, coefficient domain, in the scratch slots that k_ext_ntt_d then
+// transforms in place with 40 registers, 3 CTAs per SM.
 __global__ void __launch_bounds__(256) k_ext_conv_d(const u64 *__restrict__ a, const u64 *__restrict__ b, u64 *__restrict__ nttbuf,
                                                     size_t n_ops) {
     const size_t total = n_ops * 4 * (kN / 2);
@@ -654,15 +259,14 @@ __global__ void __launch_bounds__(256) k_ext_conv_d(const u64 *__restrict__ a, c
         *reinterpret_cast<ulonglong2 *>(dst + 2 * kN) = make_ulonglong2(ext_dual<2>(base0, m0, neg0), ext_dual<2>(base1, m1, neg1));
     }
 }
-template <int D, bool SHFL>
+template <int D>
 __device__ __forceinline__ void ntt_dual_body(u64 *__restrict__ limb, u64 *smem, int t) {
     using M = ModDual<D>;
     u64 v[1][8];
     load_natural(limb, v[0], t);
-    ntt_forward<M, 1, false, false, SHFL>(v, smem, kt.twf[M::kIndex], t);  // values stay in [0, 4s)
+    ntt_forward<M, 1, false, false>(v, smem, kt.twf[M::kIndex], t);  // values stay in [0, 4s)
     store_chunk8_lm(limb, v[0], t);
 }
-template <bool SHFL>
 __global__ void __launch_bounds__(kThreads, 3) k_ext_ntt_d(u64 *__restrict__ nttbuf) {
     extern __shared__ __align__(16) u64 smem[];
     const size_t op = blockIdx.y;
@@ -670,49 +274,10 @@ __global__ void __launch_bounds__(kThreads, 3) k_ext_ntt_d(u64 *__restrict__ ntt
     u64 *limb = nttbuf + (op * 20 + (size_t)(p * 5 + 2 + d)) * kN;
     const int t = threadIdx.x;
     switch (d) {
-        case 0: ntt_dual_body<0, SHFL>(limb, smem, t); break;
-        case 1: ntt_dual_body<1, SHFL>(limb, smem, t); break;
-        default: ntt_dual_body<2, SHFL>(limb, smem, t); break;
+        case 0: ntt_dual_body<0>(limb, smem, t); break;
+        case 1: ntt_dual_body<1>(limb, smem, t); break;
+        default: ntt_dual_body<2>(limb, smem, t); break;
     }
-}
-// FHE_B200_EXT_FUSED=1: base extension and the three dual transforms of one input polynomial in one CTA -- the shared part
-// of the extension is computed once per coefficient and parked in shared memory at the thread's own eight slots (62-bit base as a
-// word, m and the sign as 16 bits), so the extended operands never make the round trip through HBM that k_ext_conv_d +
-// k_ext_ntt_d give them (0.7 MB per op) and the transforms keep their 40 registers: 72 KiB per CTA, 3 CTAs per SM.
-// grid (4 polys, ops).
-template <int D>
-__device__ __forceinline__ void ext_ntt_fused_limb(const u64 *park, const unsigned short *park_m, u64 *__restrict__ dst, u64 *smem, int t) {
-    using M = ModDual<D>;
-    u64 v[1][8];
-#pragma unroll
-    for (int r = 0; r < 8; r++) {
-        const u32 mm = park_m[r * kThreads + t];
-        v[0][r] = ext_dual<D>(park[r * kThreads + t], mm & 0x7fffu, (mm >> 15) != 0);
-    }
-    ntt_forward<M, 1, false, true>(v, smem, kt.twf[M::kIndex], t);
-    store_chunk8_lm(dst, v[0], t);
-}
-__global__ void __launch_bounds__(kThreads, 3) k_ext_ntt_f_d(const u64 *__restrict__ a, const u64 *__restrict__ b, u64 *__restrict__ nttbuf) {
-    extern __shared__ __align__(16) u64 smem[];  // [kN] exchange buffer | [kN] base | [kN] u16 m + sign
-    const size_t op = blockIdx.y;
-    const int p = blockIdx.x, t = threadIdx.x;
-    const u64 *ct = (p < 2 ? a : b) + op * 4 * kN + (size_t)(p & 1) * 2 * kN;
-    u64 *park = smem + kN;
-    unsigned short *park_m = reinterpret_cast<unsigned short *>(smem + 2 * kN);
-#pragma unroll 1
-    for (int r = 0; r < 8; r++) {
-        const int i = r * kThreads + t;
-        u64 base;
-        u32 m;
-        bool neg;
-        ext_shared(ct[i], ct[kN + i], base, m, neg);
-        park[i] = base;
-        park_m[i] = (unsigned short)(m | (neg ? 0x8000u : 0u));
-    }
-    u64 *dst = nttbuf + (op * 20 + (size_t)p * 5 + 2) * kN;
-    ext_ntt_fused_limb<0>(park, park_m, dst, smem, t);
-    ext_ntt_fused_limb<1>(park, park_m, dst + kN, smem, t);
-    ext_ntt_fused_limb<2>(park, park_m, dst + 2 * kN, smem, t);
 }
 // one lane of the dyadic tensor: operands in [0, 4s) -> product(s) mod s in [0, 2s)
 template <int NP>
@@ -726,7 +291,7 @@ __device__ __forceinline__ u32 dual_mulsum(const u32 (&x)[NP], const u32 (&y)[NP
     return csub32(barrett61(P, mu61, s), 2 * s);
 }
 // the dyadic tensor of dual word D for output polynomial d + its inverse transform, left in registers (lanes in [0, 2s))
-template <int D, bool SHFL, bool kTrailSync>
+template <int D, bool kTrailSync>
 __device__ __forceinline__ void tensor_intt_dual_regs(const u64 *__restrict__ nb, int d, u64 (&v)[1][8], u64 *smem, int t) {
     using M = ModDual<D>;
     constexpr int E = 2 + D;
@@ -766,15 +331,14 @@ __device__ __forceinline__ void tensor_intt_dual_regs(const u64 *__restrict__ nb
             v[0][2 * r + 1] = one(x.y, y.y);
         }
     }
-    ntt_inverse<M, 1, false, kTrailSync, SHFL>(v, smem, kt.twi[M::kIndex], t, kc.d_ninv_t[D], kc.d_ninv_t_w[D]);  // [0, 2s)
+    ntt_inverse<M, 1, false, kTrailSync>(v, smem, kt.twi[M::kIndex], t, kc.d_ninv_t[D], kc.d_ninv_t_w[D]);  // [0, 2s)
 }
-template <int D, bool SHFL>
+template <int D>
 __device__ __forceinline__ void tensor_intt_dual_body(const u64 *__restrict__ nb, int d, u64 *__restrict__ dst, u64 *smem, int t) {
     u64 v[1][8];
-    tensor_intt_dual_regs<D, SHFL, false>(nb, d, v, smem, t);
+    tensor_intt_dual_regs<D, false>(nb, d, v, smem, t);
     store_natural(dst, v[0], t);
 }
-template <bool SHFL>
 __global__ void __launch_bounds__(kThreads, 3) k_tensor_intt_d(const u64 *__restrict__ nttbuf, u64 *__restrict__ tens) {
     extern __shared__ __align__(16) u64 smem[];
     const size_t op = blockIdx.y;
@@ -783,9 +347,9 @@ __global__ void __launch_bounds__(kThreads, 3) k_tensor_intt_d(const u64 *__rest
     u64 *dst = tens + (op * 15 + (size_t)(d * 5 + 2 + e)) * kN;
     const int t = threadIdx.x;
     switch (e) {
-        case 0: tensor_intt_dual_body<0, SHFL>(nb, d, dst, smem, t); break;
-        case 1: tensor_intt_dual_body<1, SHFL>(nb, d, dst, smem, t); break;
-        default: tensor_intt_dual_body<2, SHFL>(nb, d, dst, smem, t); break;
+        case 0: tensor_intt_dual_body<0>(nb, d, dst, smem, t); break;
+        case 1: tensor_intt_dual_body<1>(nb, d, dst, smem, t); break;
+        default: tensor_intt_dual_body<2>(nb, d, dst, smem, t); break;
     }
 }
 __device__ __forceinline__ u32 dual_prime(int i) {
@@ -810,7 +374,6 @@ __device__ __forceinline__ void floor_sk_coeff_d(u64 w0, u64 w1, u64 w2, u64 &o0
     }
     const u32 v = est >> 16;  // t D = sum y_i (S/s_i) - v S exactly
     u64 t0, t1;
-#if FHE_B200_WIDESUM
     {
         WideSum<Q0> s;  // exact sum of the six products + v KN, one reduction (modarith.cuh)
 #pragma unroll
@@ -825,22 +388,6 @@ __device__ __forceinline__ void floor_sk_coeff_d(u64 w0, u64 w1, u64 w2, u64 &o0
         s.add_small(v, kc.d_KN[1]);
         t1 = s.value();
     }
-#else
-    {
-        ShoupSum<Q0> s;  // six terms < q + 1 each + v KN < 13 q
-#pragma unroll
-        for (int i = 0; i < 6; i++) s.add32(y[i], kc.d_K[i][0].w, kc.d_K[i][0].ws);
-        s.add_small(v, kc.d_KN[0]);
-        t0 = canon_k32<Q0>(s.value());
-    }
-    {
-        ShoupSum<Q1> s;
-#pragma unroll
-        for (int i = 0; i < 6; i++) s.add32(y[i], kc.d_K[i][1].w, kc.d_K[i][1].ws);
-        s.add_small(v, kc.d_KN[1]);
-        t1 = canon_k32<Q1>(s.value());
-    }
-#endif
     // fast_floor: y0 = t0 q1 + t1 q0 (the q-part of t D with its fast-base-conversion overflow), f = (t D - y0) / q on s_0..s_3
     u64 ylo, yhi;
     punctured_sum(t0, t1, ylo, yhi);
@@ -855,7 +402,6 @@ __device__ __forceinline__ void floor_sk_coeff_d(u64 w0, u64 w1, u64 w2, u64 &o0
         est2 += tb[i] >> 14;
     }
     const u32 vp = est2 >> 16;  // f = sum tb_i (S4/s_i) - v' S4 exactly (|f| / S4 < 2^-24)
-#if FHE_B200_WIDESUM
     {
         WideSum<Q0> s;
 #pragma unroll
@@ -870,22 +416,6 @@ __device__ __forceinline__ void floor_sk_coeff_d(u64 w0, u64 w1, u64 w2, u64 &o0
         s.add_small(vp, kc.d_NS4[1]);
         o1 = s.value();
     }
-#else
-    {
-        ShoupSum<Q0> s;
-#pragma unroll
-        for (int i = 0; i < 4; i++) s.add32(tb[i], kc.d_P[i][0].w, kc.d_P[i][0].ws);
-        s.add_small(vp, kc.d_NS4[0]);
-        o0 = canon_k32<Q0>(s.value());
-    }
-    {
-        ShoupSum<Q1> s;
-#pragma unroll
-        for (int i = 0; i < 4; i++) s.add32(tb[i], kc.d_P[i][1].w, kc.d_P[i][1].ws);
-        s.add_small(vp, kc.d_NS4[1]);
-        o1 = canon_k32<Q1>(s.value());
-    }
-#endif
 }
 __global__ void __launch_bounds__(256, 3) k_floor_sk_d(const u64 *__restrict__ tens, u64 *__restrict__ c3, size_t n_ops) {
     const size_t total = n_ops * 3 * (kN / 2);
@@ -904,11 +434,11 @@ __global__ void __launch_bounds__(256, 3) k_floor_sk_d(const u64 *__restrict__ t
     }
 }
 
-// ---- K7d + K8d in one kernel (default for chunks >= 96 ops; FHE_B200_FUSE_TAIL=0 keeps the two kernels): one CTA per (output polynomial d, op) runs the three
+// ---- K7d + K8d in one kernel (chunks >= 96 ops; smaller ones run the two kernels above): one CTA per (output polynomial d, op) runs the three
 // dual words one after the other -- dyadic tensor, inverse transform -- parks the first two results at each thread's own eight
 // slots in shared memory (r * 512 + t: the coefficients it owns after every inverse transform) and finishes with
 // floor_sk_coeff_d on its eight coefficients, so the tensor product never goes through HBM (0.59 MB per op less DRAM traffic:
-// the batch runs into the board's power limit, where bytes not moved are clock).  Same structure as k_ks_finish: 2 CTAs per SM.
+// the batch runs into the board's power limit, where bytes not moved are clock).  Same structure as k_ks_tail_ksd: 2 CTAs per SM.
 __global__ void __launch_bounds__(kThreads, 2) k_tensor_floor_d(const u64 *__restrict__ nttbuf, u64 *__restrict__ c3) {
     extern __shared__ __align__(16) u64 smem[];  // [3][kN]: exchange buffer, word 0, word 1
     const size_t op = blockIdx.y;
@@ -917,18 +447,18 @@ __global__ void __launch_bounds__(kThreads, 2) k_tensor_floor_d(const u64 *__res
     u64 *park0 = smem + kN, *park1 = smem + 2 * kN;
     {
         u64 v[1][8];
-        tensor_intt_dual_regs<0, false, true>(nb, d, v, smem, t);
+        tensor_intt_dual_regs<0, true>(nb, d, v, smem, t);
 #pragma unroll
         for (int r = 0; r < 8; r++) park0[r * kThreads + t] = v[0][r];
     }
     {
         u64 v[1][8];
-        tensor_intt_dual_regs<1, false, true>(nb, d, v, smem, t);
+        tensor_intt_dual_regs<1, true>(nb, d, v, smem, t);
 #pragma unroll
         for (int r = 0; r < 8; r++) park1[r * kThreads + t] = v[0][r];
     }
     u64 v[1][8];
-    tensor_intt_dual_regs<2, false, false>(nb, d, v, smem, t);
+    tensor_intt_dual_regs<2, false>(nb, d, v, smem, t);
     u64 *out = c3 + (op * 3 + d) * 2 * kN;
 #pragma unroll
     for (int r = 0; r < 8; r++) {
@@ -940,55 +470,10 @@ __global__ void __launch_bounds__(kThreads, 2) k_tensor_floor_d(const u64 *__res
 }
 
 // =====================================================================================
-// K9a: key switching core  (SEAL Evaluator::switch_key_inplace, BFV branch, up to the inverse NTTs)
-// one CTA per (key modulus J = q0,q1,P ; op): 2 digit NTTs, MAC with the relin key, 2 INTTs
-//   c3 [op][3][2][N]  ->  ks [op][2][3][N]   (coefficient form, canonical)
-// =====================================================================================
-template <int MI>
-__device__ __forceinline__ void relin_ks_body(const u64 *__restrict__ c2, const u64 *__restrict__ rk, u64 *__restrict__ ks,
-                                              u64 *smem, int t) {
-    using M = Mod<MI>;
-    u64 D[2][8];
-    load_natural(c2, D[0], t);       // digit 0: residues mod q0 as integers
-    load_natural(c2 + kN, D[1], t);  // digit 1: residues mod q1 as integers
-    // lazy forward transform absorbs the "mod p_J" of the digit (inputs < 2^36 < 4 p_J)
-    ntt_forward<M, 2, true>(D, smem, kt.twf[MI], t);
-    u64 E[2][8];
-#pragma unroll
-    for (int k = 0; k < 2; k++) {
-        u64 k0[8], k1[8];
-        load_chunk8_ldg(rk + (size_t)((0 * 2 + k) * 3 + MI) * kN, k0, t);
-        load_chunk8_ldg(rk + (size_t)((1 * 2 + k) * 3 + MI) * kN, k1, t);
-#pragma unroll
-        for (int r = 0; r < 8; r++) {
-            u64 lo = 0, hi = 0;
-            mac128(lo, hi, D[0][r], k0[r]);
-            mac128(lo, hi, D[1][r], k1[r]);
-            E[k][r] = reduce128<M>(hi, lo);
-        }
-    }
-    ntt_inverse<M, 2>(E, smem, kt.twi[MI], t, kc.ninv[MI], kc.ninv_w[MI]);
-    store_natural(ks + (size_t)(0 * 3 + MI) * kN, E[0], t);
-    store_natural(ks + (size_t)(1 * 3 + MI) * kN, E[1], t);
-}
-__global__ void __launch_bounds__(kThreads, 1) k_relin_ks(const u64 *__restrict__ c3, const u64 *__restrict__ rk,
-                                                           u64 *__restrict__ ks) {
-    extern __shared__ __align__(16) u64 smem[];
-    const size_t op = blockIdx.y;
-    const u64 *c2 = c3 + op * 6 * kN + 4 * kN;
-    u64 *pk = ks + op * 6 * kN;
-    const int t = threadIdx.x;
-    switch (blockIdx.x) {
-        case 0: relin_ks_body<MQ0>(c2, rk, pk, smem, t); break;
-        case 1: relin_ks_body<MQ1>(c2, rk, pk, smem, t); break;
-        default: relin_ks_body<MP>(c2, rk, pk, smem, t); break;
-    }
-}
-
-// =====================================================================================
-// Split variant of the key-switch core (default), same arithmetic as k_relin_ks:
-//   k_digit_ntt : NTT_J([c2]_I)                       grid (6 = I*3+J, ops)   -> dig [op][2][3][N]
-//   k_ks_intt   : INTT_J(sum_I dig[I][J] * rk[I][k][J]) grid (6 = k*3+J, ops) -> ks  [op][2][3][N]
+// K9: key switching  (SEAL Evaluator::switch_key_inplace, BFV branch) on SEAL's key primes q0, q1, P, for chunks < 96 ops
+//   k_digit_ntt    : NTT_J([c2]_I)                       grid (6 = I*3+J, ops)   -> dig [op][2][3][N]
+//   k_ks_intt      : INTT_J(sum_I dig[I][J] * rk[I][k][J]) grid (6 = k*3+J, ops) -> ks  [op][2][3][N]
+//   k_relin_finish : rounded division by P, added to (c0, c1)   (K9b below)
 // =====================================================================================
 template <int MI>
 __device__ __forceinline__ void digit_ntt_body(const u64 *__restrict__ src, u64 *__restrict__ dst, u64 *smem, int t) {
@@ -1009,76 +494,6 @@ __global__ void __launch_bounds__(kThreads, 3) k_digit_ntt(const u64 *__restrict
         case 0: digit_ntt_body<MQ0>(src, dst, smem, t); break;
         case 1: digit_ntt_body<MQ1>(src, dst, smem, t); break;
         default: digit_ntt_body<MP>(src, dst, smem, t); break;
-    }
-}
-// ---- persistent variant of k_digit_ntt with TMA staging (FHE_B200_TMA=1; A/B, profiles/r2_tma_ab.md): one CTA per resident slot
-// walks the (digit, modulus, op) work items; while it transforms item i the TMA engine (cp.async.bulk, one elected thread, no
-// registers in the other threads) brings the 32 KiB of item i + gridDim.x into the other half of a 64 KiB shared buffer, so the
-// head of every transform reads shared memory instead of waiting ~1 us for HBM.  Buffer `cur` is first the landing zone of the
-// bulk copy, then -- once every thread has taken its eight coefficients -- the exchange buffer of the transform.
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long *bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void tma_load_32k(void *dst_smem, const void *src_gmem, unsigned long long *bar) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(32768u) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(32768u), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long *bar, unsigned parity) {
-    unsigned done = 0;
-    for (int spin = 0; !done; spin++) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-        if (spin > (1 << 22)) __trap();  // a lost bulk copy must fail the launch, never hang the GPU
-    }
-}
-template <int kCtasPerSm>
-__global__ void __launch_bounds__(kThreads, kCtasPerSm) k_digit_ntt_tma(const u64 *__restrict__ c3, u64 *__restrict__ dig, unsigned total) {
-    extern __shared__ __align__(128) u64 smem[];  // [2][kN]
-    __shared__ __align__(8) unsigned long long bar[2];
-    const int t = threadIdx.x;
-    if (t == 0) {
-        mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    // the only loop-carried value is `it`: everything else is rebuilt from special registers and kernel parameters each time, so
-    // that the transform keeps its 40 registers (3 CTAs per SM)
-    const auto src_of = [&](unsigned w) { return c3 + (size_t)(w / 6) * 6 * kN + 4 * kN + (size_t)((w % 6) / 3) * kN; };
-    if (t == 0 && blockIdx.x < total) tma_load_32k(smem, src_of(blockIdx.x), &bar[0]);
-#pragma unroll 1
-    for (unsigned it = 0; blockIdx.x + it * gridDim.x < total; it++) {
-        {
-            u64 v[1][8];
-            {
-                const u64 *buf = smem + (it & 1) * kN;
-                mbar_wait(&bar[it & 1], (it >> 1) & 1);
-#pragma unroll
-                for (int r = 0; r < 8; r++) v[0][r] = buf[r * kThreads + t];
-            }
-            __syncthreads();  // every thread holds its coefficients and has left the previous item's exchange buffer
-            if (t == 0) {
-                const unsigned wn = blockIdx.x + (it + 1) * gridDim.x;
-                if (wn < total) {
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes of the last exchange first
-                    tma_load_32k(smem + ((it + 1) & 1) * kN, src_of(wn), &bar[(it + 1) & 1]);
-                }
-            }
-            switch ((blockIdx.x + it * gridDim.x) % 3) {
-                case 0: ntt_forward<Mod<MQ0>, 1, false, false>(v, smem + (it & 1) * kN, kt.twf[MQ0], t); break;
-                case 1: ntt_forward<Mod<MQ1>, 1, false, false>(v, smem + (it & 1) * kN, kt.twf[MQ1], t); break;
-                default: ntt_forward<Mod<MP>, 1, false, false>(v, smem + (it & 1) * kN, kt.twf[MP], t); break;
-            }
-            store_chunk8_lm(dig + (size_t)(blockIdx.x + it * gridDim.x) * kN, v[0], t);
-        }
     }
 }
 
@@ -1115,89 +530,16 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks_intt(const u64 *__restrict__
     }
 }
 
-// ---- default key-switch tail: k_ks_intt and k_relin_finish in one kernel, grid (2 = output polynomial k, ops).
-// The CTA runs the three moduli in the order P, q0, q1: a thread owns the same eight coefficients (r*512 + t) after every
-// inverse transform, so the P-limb values needed by the rounded division stay in its registers and the key-switch result
-// never goes through the [op][2][3][N] scratch (FHE_B200_KS_FINISH=0 selects the two separate kernels).
-template <int MI, bool KLM>
-__device__ __forceinline__ void ks_mac_intt(const u64 *__restrict__ dg, const u64 *__restrict__ rk, int k, u64 (&v)[1][8], u64 *smem,
-                                            int t) {
-    using M = Mod<MI>;
-    constexpr int ks = KLM ? kLm : 1;  // KLM: the key is a lane-major copy (k_rk_lm), else the key file's order
-    const ulonglong2 *pd0 = lm_ptr(dg + (size_t)(0 * 3 + MI) * kN, t), *pd1 = lm_ptr(dg + (size_t)(1 * 3 + MI) * kN, t);  // pair r at [r * kLm]
-    const u64 *k0 = rk + (size_t)((0 * 2 + k) * 3 + MI) * kN, *k1 = rk + (size_t)((1 * 2 + k) * 3 + MI) * kN;
-    const ulonglong2 *pk0 = KLM ? lm_ptr(k0, t) : reinterpret_cast<const ulonglong2 *>(k0 + 8 * t);
-    const ulonglong2 *pk1 = KLM ? lm_ptr(k1, t) : reinterpret_cast<const ulonglong2 *>(k1 + 8 * t);
-#pragma unroll
-    for (int r = 0; r < 4; r++) {  // two coefficients at a time: 16 operand registers live instead of 64
-        const ulonglong2 x0 = pd0[r * kLm], x1 = pd1[r * kLm], y0 = __ldg(pk0 + r * ks), y1 = __ldg(pk1 + r * ks);
-        {
-            const u64 xs[2] = {x0.x, x1.x}, ys[2] = {y0.x, y1.x};
-            v[0][2 * r] = mulsum<M, 2>(xs, ys);
-        }
-        {
-            const u64 xs[2] = {x0.y, x1.y}, ys[2] = {y0.y, y1.y};
-            v[0][2 * r + 1] = mulsum<M, 2>(xs, ys);
-        }
-    }
-    ntt_inverse<M, 1, true, true>(v, smem, kt.twi[MI], t, kc.ninv[MI], kc.ninv_w[MI]);
-}
-template <int L>
-__device__ __forceinline__ void ks_finish_limb(const u64 (&v)[8], const u64 *last, const u64 *__restrict__ pc, u64 *__restrict__ po,
-                                               int t) {
-    using Q = Mod<L>;
-#pragma unroll
-    for (int r = 0; r < 8; r++) {
-        // last < P < 4 q_l: one fold; d canonical, so the 16-bit quotient estimate applies: c3 + d P^-1 < 6 q_l, one more fold
-        const u64 tl = submod<Q>(canon_k32<Q>(last[r * kThreads + t]), kc.half_P_mod_q[L]);
-        const u64 d = submod<Q>(v[r], tl);
-        po[r * kThreads + t] = canon_k32<Q>(shoup_acc<Q, 2>(pc[r * kThreads + t], d, kc.inv_P_mod_q[L].w, kc.inv_P_mod_q[L].ws));
-    }
-}
-// the relinearisation key regrouped into the lane-major chunk layout (12 limbs, once per chunk of ops)
-__global__ void __launch_bounds__(kThreads) k_rk_lm(const u64 *__restrict__ rk, u64 *__restrict__ out) {
-    u64 v[8];
-    load_chunk8_ldg(rk + (size_t)blockIdx.x * kN, v, threadIdx.x);
-    store_chunk8_lm(out + (size_t)blockIdx.x * kN, v, threadIdx.x);
-}
-template <bool KLM>
-__global__ void __launch_bounds__(kThreads, 2) k_ks_finish(const u64 *__restrict__ dig, const u64 *__restrict__ rk,
-                                                            const u64 *__restrict__ c3, u64 *__restrict__ out) {
-    extern __shared__ __align__(16) u64 smem[];
-    u64 *last = smem + kN;  // second 32 KiB: the P-limb values, each thread's own eight slots
-    const size_t op = blockIdx.y;
-    const int k = blockIdx.x, t = threadIdx.x;
-    const u64 *dg = dig + op * 6 * kN;
-    const u64 *pc = c3 + (op * 3 + k) * 2 * kN;
-    u64 *po = out + (op * 2 + k) * 2 * kN;
-    {
-        u64 v[1][8];
-        ks_mac_intt<MP, KLM>(dg, rk, k, v, smem, t);
-#pragma unroll
-        for (int r = 0; r < 8; r++) last[r * kThreads + t] = csub<Mod<MP>>(v[0][r] + kc.half_P, Mod<MP>::q);
-    }
-    {
-        u64 v[1][8];
-        ks_mac_intt<MQ0, KLM>(dg, rk, k, v, smem, t);
-        ks_finish_limb<MQ0>(v[0], last, pc, po, t);
-    }
-    {
-        u64 v[1][8];
-        ks_mac_intt<MQ1, KLM>(dg, rk, k, v, smem, t);
-        ks_finish_limb<MQ1>(v[0], last, pc + kN, po + kN, t);
-    }
-}
-
 // =====================================================================================
-// K9d: the key switch on the dual base (default for chunks >= 96 ops; FHE_B200_KS=seal keeps SEAL's three key primes; +3 %, DESIGN.md section 8).  switch_key_inplace's sums S_km = sum_j d_j * rk_jkm mod m are the
+// K9d: the key switch on the dual base, for chunks >= 96 ops (+3 % over SEAL's three key primes, DESIGN.md section 8).  switch_key_inplace's sums S_km = sum_j d_j * rk_jkm mod m are the
 // residues of ONE integer polynomial per output k: U_k = sum_j d_j * RK_jk with the key lifted to integers RK == rk (mod q0, q1,
 // P), 0 <= RK < 3 Q.  |U_k| < 2 N 2^36 2^111 = 2^160 << S / 2, so U_k is carried exactly by the six dual primes: 6 forward + 6
 // inverse DUAL transforms instead of 6 + 6 on 36/37-bit primes, and U_k mod (q0, q1, P) follows by the same CRT-with-rounding
 // as in k_floor_sk_d.  Same bits as SEAL (the oracle follows SEAL; prototyped in Python first).
 //   k_rk_intt_ksd / k_rk_lift_ksd / k_rk_ntt_ksd : the key -> coefficient form -> integer lift mod s_i -> dual NTT (per call)
 //   k_digit_ntt_ksd : dual NTT of the two digits ([c2]_{q_j} as integers)          grid (6 = j*3+w, ops) -> dig [op][2][3][N]
-//   k_ks_intt_ksd   : MAC with the lifted key + inverse dual NTT                   grid (6 = k*3+w, ops) -> ks  [op][2][3][N]
-//   k_ks_finish_ksd : U mod (P, q0, q1), rounded division by P, add to (c0, c1)    eltwise
+//   k_ks_tail_ksd   : MAC with the lifted key + inverse dual NTTs, U mod (P, q0, q1), rounded division by P, add to (c0, c1)
+//                     grid (2 = k, ops) -> out [op][2][2][N]
 // =====================================================================================
 template <int MI>
 __device__ __forceinline__ void rk_intt_body(const u64 *__restrict__ src, u64 *__restrict__ dst, u64 *smem, int t) {
@@ -1301,26 +643,6 @@ __device__ __forceinline__ void ks_intt_ksd_regs(const u64 *__restrict__ dg, con
     }
     ntt_inverse<M, 1, false, kTrailSync>(v, smem, kt.twi[M::kIndex], t, kc.d_ninv[D], kc.d_ninv_w[D]);  // [0, 2s)
 }
-template <int D>
-__device__ __forceinline__ void ks_intt_ksd_body(const u64 *__restrict__ dg, const u64 *__restrict__ rkd, int k, u64 *__restrict__ dst,
-                                                 u64 *smem, int t) {
-    u64 v[1][8];
-    ks_intt_ksd_regs<D, false>(dg, rkd, k, v, smem, t);
-    store_natural(dst, v[0], t);
-}
-__global__ void __launch_bounds__(kThreads, 3) k_ks_intt_ksd(const u64 *__restrict__ dig, const u64 *__restrict__ rkd, u64 *__restrict__ ks) {
-    extern __shared__ __align__(16) u64 smem[];
-    const size_t op = blockIdx.y;
-    const int k = blockIdx.x / 3, w = blockIdx.x % 3;
-    const u64 *dg = dig + op * 6 * kN;
-    u64 *dst = ks + (op * 6 + blockIdx.x) * kN;
-    const int t = threadIdx.x;
-    switch (w) {
-        case 0: ks_intt_ksd_body<0>(dg, rkd, k, dst, smem, t); break;
-        case 1: ks_intt_ksd_body<1>(dg, rkd, k, dst, smem, t); break;
-        default: ks_intt_ksd_body<2>(dg, rkd, k, dst, smem, t); break;
-    }
-}
 // one coefficient: the three dual words of U_k (lanes in [0, 2s)), c3's limbs -> the two output limbs
 __device__ __forceinline__ void ks_finish_coeff_ksd(u64 w0, u64 w1, u64 w2, u64 c0, u64 c1, u64 &o0, u64 &o1) {
     using Q0 = Mod<MQ0>;
@@ -1337,7 +659,6 @@ __device__ __forceinline__ void ks_finish_coeff_ksd(u64 w0, u64 w1, u64 w2, u64 
         est += y[i] >> 14;
     }
     const u32 v = est >> 16;  // U = sum y_i (S/s_i) - v S exactly (|U| / S < 2^-19)
-#if FHE_B200_WIDESUM
     u64 sp;
     {
         WideSum<PP> s;
@@ -1370,62 +691,9 @@ __device__ __forceinline__ void ks_finish_coeff_ksd(u64 w0, u64 w1, u64 w2, u64 
         s.lo += c1 + kc.ksHd[1];
         o1 = s.value();
     }
-#else
-    u64 sp, s0, s1;
-    {
-        ShoupSum<PP> s;
-#pragma unroll
-        for (int i = 0; i < 6; i++) s.add32(y[i], kc.ksK[i][2].w, kc.ksK[i][2].ws);
-        s.add_small(v, kc.ksKN[2]);
-        sp = canon_k32<PP>(s.value());
-    }
-    {
-        ShoupSum<Q0> s;
-#pragma unroll
-        for (int i = 0; i < 6; i++) s.add32(y[i], kc.ksK[i][0].w, kc.ksK[i][0].ws);
-        s.add_small(v, kc.ksKN[0]);
-        s0 = canon_k32<Q0>(s.value());
-    }
-    {
-        ShoupSum<Q1> s;
-#pragma unroll
-        for (int i = 0; i < 6; i++) s.add32(y[i], kc.ksK[i][1].w, kc.ksK[i][1].ws);
-        s.add_small(v, kc.ksKN[1]);
-        s1 = canon_k32<Q1>(s.value());
-    }
-    // RNSTool::divide_and_round_q_last: (S_l - ((S_P + P/2 mod P) mod q_l - (P/2 mod q_l))) P^-1, added to c3
-    const u64 last = csub<PP>(sp + kc.half_P, PP::q);
-    {
-        const u64 tl = submod<Q0>(canon_k32<Q0>(last), kc.half_P_mod_q[0]);
-        o0 = canon_k32<Q0>(shoup_acc<Q0, 2>(c0, submod<Q0>(s0, tl), kc.inv_P_mod_q[0].w, kc.inv_P_mod_q[0].ws));
-    }
-    {
-        const u64 tl = submod<Q1>(canon_k32<Q1>(last), kc.half_P_mod_q[1]);
-        o1 = canon_k32<Q1>(shoup_acc<Q1, 2>(c1, submod<Q1>(s1, tl), kc.inv_P_mod_q[1].w, kc.inv_P_mod_q[1].ws));
-    }
-#endif
-}
-__global__ void __launch_bounds__(256, 3) k_ks_finish_ksd(const u64 *__restrict__ ks, const u64 *__restrict__ c3, u64 *__restrict__ out,
-                                                           size_t n_ops) {
-    const size_t total = n_ops * 2 * (kN / 2);  // (op, k, coefficient pair)
-    const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x; g < total; g += stride) {
-        const size_t op = g / kN;
-        const int k = (int)((g / (kN / 2)) & 1), i = 2 * (int)(g % (kN / 2));
-        const ulonglong2 *in = reinterpret_cast<const ulonglong2 *>(ks + (op * 6 + (size_t)k * 3) * kN + i);
-        const ulonglong2 w0 = in[0], w1 = in[kN / 2], w2 = in[2 * (kN / 2)];
-        const ulonglong2 *pc = reinterpret_cast<const ulonglong2 *>(c3 + (op * 3 + k) * 2 * kN + i);
-        const ulonglong2 c0 = pc[0], c1 = pc[kN / 2];
-        u64 ax, ay, bx, by;
-        ks_finish_coeff_ksd(w0.x, w1.x, w2.x, c0.x, c1.x, ax, bx);
-        ks_finish_coeff_ksd(w0.y, w1.y, w2.y, c0.y, c1.y, ay, by);
-        ulonglong2 *po = reinterpret_cast<ulonglong2 *>(out + (op * 2 + k) * 2 * kN + i);
-        po[0] = make_ulonglong2(ax, ay);
-        po[kN / 2] = make_ulonglong2(bx, by);
-    }
 }
 
-// ---- k_ks_intt_ksd + k_ks_finish_ksd in one kernel (default for chunks >= 96 ops; FHE_B200_FUSE_TAIL=0 keeps the two kernels): one CTA per (output polynomial k, op), the three dual
+// ---- the tail of the key switch in one kernel: one CTA per (output polynomial k, op), the three dual
 // words of U_k one after the other with the first two parked in shared memory (as k_tensor_floor_d): U_k never goes through HBM
 __global__ void __launch_bounds__(kThreads, 2) k_ks_tail_ksd(const u64 *__restrict__ dig, const u64 *__restrict__ rkd,
                                                               const u64 *__restrict__ c3, u64 *__restrict__ out) {
@@ -2029,28 +1297,13 @@ cudaError_t measure_int_peak(int mode, double *tera_ops_per_s) {
 // =====================================================================================
 // launchers
 // =====================================================================================
-static const int kSmem1 = 1 * kN * 8, kSmem2 = 2 * kN * 8, kSmem3 = 3 * kN * 8, kSmem4 = 4 * kN * 8;
-static const int kSmemExtF = 2 * kN * 8 + kN * 2;  // k_ext_ntt_f_d: exchange buffer + parked base + parked (m, sign)
+static const int kSmem1 = 1 * kN * 8, kSmem2 = 2 * kN * 8, kSmem3 = 3 * kN * 8;
 
 cudaError_t kernels_configure() {
     cudaError_t e;
     e = cudaFuncSetAttribute(k_mul_plain, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem3);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_behz_tensor, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem4);
-    if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_encrypt_seal, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_relin_ks, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_digit_ntt_tma<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_digit_ntt_tma<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_ks_finish<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_ks_finish<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_ext_ntt_f_d, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemExtF);
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_tensor_floor_d, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem3);
     if (e != cudaSuccess) return e;
@@ -2071,14 +1324,8 @@ static int eltwise_grid(size_t n, int block) {
 
 cudaError_t launch_ntt(u64 *data, size_t n_limbs, const LimbMods &mods, bool inverse, cudaStream_t s) {
     if (n_limbs == 0) return cudaSuccess;
-    static const bool shfl = [] {
-        const char *v = getenv("FHE_B200_NTT_SHFL");
-        return v && *v == '1';
-    }();
-    if (inverse && shfl) k_ntt<true, true><<<(unsigned)n_limbs, kThreads, kSmem1, s>>>(data, mods);
-    else if (inverse) k_ntt<true, false><<<(unsigned)n_limbs, kThreads, kSmem1, s>>>(data, mods);
-    else if (shfl) k_ntt<false, true><<<(unsigned)n_limbs, kThreads, kSmem1, s>>>(data, mods);
-    else k_ntt<false, false><<<(unsigned)n_limbs, kThreads, kSmem1, s>>>(data, mods);
+    if (inverse) k_ntt<true><<<(unsigned)n_limbs, kThreads, kSmem1, s>>>(data, mods);
+    else k_ntt<false><<<(unsigned)n_limbs, kThreads, kSmem1, s>>>(data, mods);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
@@ -2110,95 +1357,29 @@ cudaError_t launch_mul_plain(const u64 *ct, const unsigned short *plain, u64 *ou
     return cudaGetLastError();
 }
 
-cudaError_t launch_behz_extend_tap(const u64 *a, const u64 *b, u64 *ext, size_t n_ops, cudaStream_t s) {
-    if (n_ops == 0) return cudaSuccess;
-    k_behz_extend_tap<<<dim3(5, (unsigned)n_ops), kThreads, 0, s>>>(a, b, ext);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-cudaError_t launch_behz_tensor(const u64 *a, const u64 *b, u64 *tens, size_t n_ops, cudaStream_t s) {
-    if (n_ops == 0) return cudaSuccess;
-    k_behz_tensor<<<dim3(5, (unsigned)n_ops), kThreads, kSmem4, s>>>(a, b, tens);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-static int ext_split_mode() {
-    static const int mode = [] {
-        const char *v = getenv("FHE_B200_EXT_SPLIT");
-        return (v && *v == '0') ? 0 : 1;
-    }();
-    return mode;
-}
-bool ext_split() { return ext_split_mode() != 0; }
-// How bfv_multiply's tensor product is carried (same bits in every mode):
-//   0 "dual" (default): six primes below 2^30, two per word (k_*_d above): 21 dual transforms
-//   1 "bsk"           : SEAL's three 61-bit Bsk primes, q-limbs recovered from them in k_floor_sk: 21 transforms on 61-bit primes
-//   2 "seal"          : SEAL's form, q-limbs transformed too: 35 transforms (FHE_B200_BEHZ=seal or FHE_B200_QLIMB_NTT=1)
-static int behz_mode_() {
-    static const int mode = [] {
-        const char *q = getenv("FHE_B200_QLIMB_NTT");
-        if (q && *q == '1') return 2;
-        const char *v = getenv("FHE_B200_BEHZ");
-        if (v && !strcmp(v, "seal")) return 2;
-        if (v && !strcmp(v, "bsk")) return 1;
-        return 0;
-    }();
-    return mode;
-}
-int behz_mode() { return behz_mode_(); }
-static bool dual_shfl() {  // the last exchange of the dual transforms through warp shuffles instead of shared memory (A/B)
-    static const bool on = [] {
-        const char *v = getenv("FHE_B200_DUAL_SHFL");
-        return v && *v == '1';
-    }();
-    return on;
-}
-static bool ext_fused_d() {
-    static const bool on = [] {
-        const char *v = getenv("FHE_B200_EXT_FUSED");
-        return v && *v == '1';
-    }();
-    return on;
-}
-static int qlimb_ntt_mode() { return behz_mode_() == 2; }
-bool qlimb_ntt() { return qlimb_ntt_mode() != 0; }
 cudaError_t launch_ext_conv(const u64 *a, const u64 *b, u64 *nttbuf, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
-    if (behz_mode_() == 0 && ext_fused_d()) return cudaSuccess;  // the fused kernel of launch_ext_ntt does the extension
-    if (behz_mode_() == 0) k_ext_conv_d<<<eltwise_grid(n_ops * 4 * (kN / 2), 256), 256, 0, s>>>(a, b, nttbuf, n_ops);
-    else k_ext_conv<<<eltwise_grid(n_ops * 4 * (kN / 2), 256), 256, 0, s>>>(a, b, nttbuf, n_ops);
+    k_ext_conv_d<<<eltwise_grid(n_ops * 4 * (kN / 2), 256), 256, 0, s>>>(a, b, nttbuf, n_ops);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
-// with ext_split(): the transforms only (launch_ext_conv must have filled the auxiliary limbs); otherwise extension + transforms
-cudaError_t launch_ext_ntt(const u64 *a, const u64 *b, u64 *nttbuf, size_t n_ops, cudaStream_t s) {
+cudaError_t launch_ext_ntt(u64 *nttbuf, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
-    if (behz_mode_() == 0 && ext_fused_d()) k_ext_ntt_f_d<<<dim3(4, (unsigned)n_ops), kThreads, kSmemExtF, s>>>(a, b, nttbuf);
-    else if (behz_mode_() == 0 && dual_shfl()) k_ext_ntt_d<true><<<dim3(12, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf);
-    else if (behz_mode_() == 0) k_ext_ntt_d<false><<<dim3(12, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf);
-    else if (ext_split_mode() && !qlimb_ntt_mode()) k_ext_ntt2<<<dim3(12, (unsigned)n_ops), kThreads, kSmem1, s>>>(a, b, nttbuf, 1);
-    else if (ext_split_mode()) k_ext_ntt2<<<dim3(20, (unsigned)n_ops), kThreads, kSmem1, s>>>(a, b, nttbuf, 0);
-    else k_ext_ntt<<<dim3(20, (unsigned)n_ops), kThreads, kSmem1, s>>>(a, b, nttbuf);
+    k_ext_ntt_d<<<dim3(12, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
 cudaError_t launch_tensor_intt(const u64 *nttbuf, u64 *tens, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
-    if (behz_mode_() == 0 && dual_shfl()) k_tensor_intt_d<true><<<dim3(9, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf, tens);
-    else if (behz_mode_() == 0) k_tensor_intt_d<false><<<dim3(9, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf, tens);
-    else if (qlimb_ntt_mode()) k_tensor_intt<<<dim3(15, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf, tens, 0);
-    else k_tensor_intt<<<dim3(9, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf, tens, 1);
+    k_tensor_intt_d<<<dim3(9, (unsigned)n_ops), kThreads, kSmem1, s>>>(nttbuf, tens);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
-// FHE_B200_FUSE_TAIL: bit 0 = tensor product + floor in one kernel (k_tensor_floor_d), bit 1 = key-switch MAC / inverse transforms +
-// division by P in one kernel (k_ks_tail_ksd).  Both trade a launch's occupancy (2 CTAs per SM) for 0.6 / 0.4 MB per op of HBM traffic.
-int fuse_tail() {
-    static const int mode = [] {
-        const char *v = getenv("FHE_B200_FUSE_TAIL");
-        return v ? atoi(v) : 3;  // default: both (964 k against 940 k ops/s in a short run, 958 k against 895 k sustained under the power cap)
-    }();
-    return mode;
+cudaError_t launch_floor_sk(const u64 *tens, u64 *c3, size_t n_ops, cudaStream_t s) {
+    if (n_ops == 0) return cudaSuccess;
+    k_floor_sk_d<<<eltwise_grid(n_ops * 3 * (kN / 2), 256), 256, 0, s>>>(tens, c3, n_ops);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError();
 }
 cudaError_t launch_tensor_floor(const u64 *nttbuf, u64 *c3, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
@@ -2212,21 +1393,8 @@ cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u6
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
-static int tma_mode() {  // 0 off (default), 1: 3 CTAs per SM (40 registers, spills), 2: 2 CTAs per SM (64 registers)
-    static const int mode = [] {
-        const char *v = getenv("FHE_B200_TMA");
-        return v ? atoi(v) : 0;
-    }();
-    return mode;
-}
 cudaError_t launch_digit_ntt(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
-    if (tma_mode() && n_ops >= 148) {
-        if (tma_mode() == 2) k_digit_ntt_tma<2><<<148 * 2, kThreads, kSmem2, s>>>(c3, dig, (unsigned)(6 * n_ops));
-        else k_digit_ntt_tma<3><<<148 * 3, kThreads, kSmem2, s>>>(c3, dig, (unsigned)(6 * n_ops));
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        return cudaGetLastError();
-    }
     k_digit_ntt<<<dim3(6, (unsigned)n_ops), kThreads, kSmem1, s>>>(c3, dig);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
@@ -2235,26 +1403,6 @@ cudaError_t launch_ks_intt(const u64 *dig, const u64 *rk, u64 *ks, size_t n_ops,
     if (n_ops == 0) return cudaSuccess;
     k_ks_intt<<<dim3(6, (unsigned)n_ops), kThreads, kSmem1, s>>>(dig, rk, ks);
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-static int ks_finish_mode() {
-    static const int mode = [] {
-        const char *v = getenv("FHE_B200_KS_FINISH");
-        return (v && *v == '0') ? 0 : 1;
-    }();
-    return mode;
-}
-bool ks_finish_fused() { return ks_finish_mode() != 0; }
-cudaError_t launch_ks_finish(const u64 *dig, const u64 *rk, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s, u64 *rk_lm) {
-    if (n_ops == 0) return cudaSuccess;
-    if (rk_lm) {  // room for a lane-major copy of the key (12 limbs): coalesced key reads in the MAC
-        k_rk_lm<<<12, kThreads, 0, s>>>(rk, rk_lm);
-        k_ks_finish<true><<<dim3(2, (unsigned)n_ops), kThreads, kSmem2, s>>>(dig, rk_lm, c3, out);
-        g_launches.fetch_add(2, std::memory_order_relaxed);
-    } else {
-        k_ks_finish<false><<<dim3(2, (unsigned)n_ops), kThreads, kSmem2, s>>>(dig, rk, c3, out);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-    }
     return cudaGetLastError();
 }
 cudaError_t launch_decrypt(const u64 *ct, const u64 *sk, u64 *xbuf, unsigned short *plain, size_t n_ops, cudaStream_t s,
@@ -2288,29 +1436,8 @@ cudaError_t launch_seal_sample(u64 *streams, signed char *samples, int *failed, 
     (void)samples;  // the samples are written behind each op's stream words (see kernels.h)
     return cudaGetLastError();
 }
-cudaError_t launch_floor_sk(const u64 *tens, u64 *c3, size_t n_ops, cudaStream_t s, bool dual) {
-    if (n_ops == 0) return cudaSuccess;
-    if (dual) k_floor_sk_d<<<eltwise_grid(n_ops * 3 * (kN / 2), 256), 256, 0, s>>>(tens, c3, n_ops);
-    else if (qlimb_ntt_mode()) k_floor_sk<false><<<eltwise_grid(n_ops * 3 * (kN / 2), 256), 256, 0, s>>>(tens, c3, n_ops);
-    else k_floor_sk<true><<<eltwise_grid(n_ops * 3 * (kN / 2), 256), 256, 0, s>>>(tens, c3, n_ops);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-cudaError_t launch_relin_ks(const u64 *c3, const u64 *rk, u64 *ks, size_t n_ops, cudaStream_t s) {
-    if (n_ops == 0) return cudaSuccess;
-    k_relin_ks<<<dim3(3, (unsigned)n_ops), kThreads, kSmem2, s>>>(c3, rk, ks);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-bool ks_dual() {
-    static const bool on = [] {
-        const char *v = getenv("FHE_B200_KS");
-        return !(v && !strcmp(v, "seal"));  // default since the CRT recoveries run on WideSum: +3 % over SEAL's three key primes
-    }();
-    return on;
-}
-// the key switch on the dual base in four steps; tmp = 36 limbs of scratch (coefficient-form key, lifted key, dual-NTT key at
-// tmp + 24 limbs)
+// the key of the key switch on the dual base, once per chunk; tmp = 36 limbs of scratch (coefficient-form key, lifted key,
+// dual-NTT key at tmp + 24 limbs)
 cudaError_t launch_rk_prepare_ksd(const u64 *rk, u64 *tmp, cudaStream_t s) {
     u64 *coef = tmp, *lifted = tmp + 12 * kN, *rkd = tmp + 24 * kN;
     k_rk_intt_ksd<<<12, kThreads, kSmem1, s>>>(rk, coef);
@@ -2322,18 +1449,6 @@ cudaError_t launch_rk_prepare_ksd(const u64 *rk, u64 *tmp, cudaStream_t s) {
 cudaError_t launch_digit_ntt_ksd(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
     k_digit_ntt_ksd<<<dim3(6, (unsigned)n_ops), kThreads, kSmem1, s>>>(c3, dig);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-cudaError_t launch_ks_intt_ksd(const u64 *dig, const u64 *rkd, u64 *ks, size_t n_ops, cudaStream_t s) {
-    if (n_ops == 0) return cudaSuccess;
-    k_ks_intt_ksd<<<dim3(6, (unsigned)n_ops), kThreads, kSmem1, s>>>(dig, rkd, ks);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return cudaGetLastError();
-}
-cudaError_t launch_ks_finish_ksd(const u64 *ks, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s) {
-    if (n_ops == 0) return cudaSuccess;
-    k_ks_finish_ksd<<<eltwise_grid(n_ops * 2 * (kN / 2), 256), 256, 0, s>>>(ks, c3, out, n_ops);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }

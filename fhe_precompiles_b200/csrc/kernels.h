@@ -21,20 +21,17 @@ cudaError_t launch_eltwise(const u64 *a, const u64 *b, u64 *out, size_t n_ops, i
 // mode bit0: subtract, bit1: negate result
 cudaError_t launch_plain_addsub(const u64 *ct, const unsigned short *plain, u64 *out, size_t n_ops, int mode, cudaStream_t s);
 cudaError_t launch_mul_plain(const u64 *ct, const unsigned short *plain, u64 *out, size_t n_ops, cudaStream_t s);
-cudaError_t launch_behz_extend_tap(const u64 *a, const u64 *b, u64 *ext, size_t n_ops, cudaStream_t s);
-cudaError_t launch_behz_tensor(const u64 *a, const u64 *b, u64 *tens, size_t n_ops, cudaStream_t s);
-// split (one polynomial per CTA) variants; scratch: nttbuf [n][4][5][N], dig [n][2][3][N]
-bool ext_split();  // default: the base extension is its own elementwise kernel (FHE_B200_EXT_SPLIT=0: inside the transform kernel)
+// BEHZ multiply on the dual base; scratch: nttbuf [n][4][5][N], tens [n][3][5][N]
 cudaError_t launch_ext_conv(const u64 *a, const u64 *b, u64 *nttbuf, size_t n_ops, cudaStream_t s);
-cudaError_t launch_ext_ntt(const u64 *a, const u64 *b, u64 *nttbuf, size_t n_ops, cudaStream_t s);
+cudaError_t launch_ext_ntt(u64 *nttbuf, size_t n_ops, cudaStream_t s);  // in place, after launch_ext_conv
+// then either launch_tensor_intt + launch_floor_sk, or both in one kernel (launch_tensor_floor) -> c3 [n][3][2][N]
 cudaError_t launch_tensor_intt(const u64 *nttbuf, u64 *tens, size_t n_ops, cudaStream_t s);
-// fused tails of the dual pipeline (FHE_B200_FUSE_TAIL bit 0 / bit 1): tensor product + floor -> c3; key-switch MAC, inverse
-// transforms and division by P -> out
-int fuse_tail();
+cudaError_t launch_floor_sk(const u64 *tens, u64 *c3, size_t n_ops, cudaStream_t s);
 cudaError_t launch_tensor_floor(const u64 *nttbuf, u64 *c3, size_t n_ops, cudaStream_t s);
-cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s);
+// key switch on SEAL's key primes: launch_digit_ntt -> launch_ks_intt -> launch_relin_finish; dig, ks [n][2][3][N]
 cudaError_t launch_digit_ntt(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s);
 cudaError_t launch_ks_intt(const u64 *dig, const u64 *rk, u64 *ks, size_t n_ops, cudaStream_t s);
+cudaError_t launch_relin_finish(const u64 *c3, const u64 *ks, u64 *out, size_t n_ops, cudaStream_t s);
 // decrypt n size-2 ciphertexts with sk [>=2 limbs][N] (NTT form): xbuf scratch [n][2][N], plain out [n][N] u16
 // exhausted (optional, [n_ops] ints on the device): set to 1 where the invariant noise budget is 0
 cudaError_t launch_decrypt(const u64 *ct, const u64 *sk, u64 *xbuf, unsigned short *plain, size_t n_ops, cudaStream_t s,
@@ -49,22 +46,11 @@ cudaError_t launch_encrypt(const u64 *pk, const unsigned short *plain, const u64
 // int8 sample polynomials, which the kernel writes there.  failed[i] = 1 if the draws ran out.
 constexpr size_t kSealOpWords = 28 * 512 + 3 * 4096 / 8;
 cudaError_t launch_seal_sample(u64 *streams, signed char *samples, int *failed, size_t n_ops, cudaStream_t s);
-// dual: `tens` holds the tensor product on the dual base (launch_ext_conv / ext_ntt / tensor_intt in behz_mode() 0); otherwise on
-// SEAL's 61-bit Bsk limbs (the fused kernel, the stage taps, behz_mode() 1 and 2)
-cudaError_t launch_floor_sk(const u64 *tens, u64 *c3, size_t n_ops, cudaStream_t s, bool dual = false);
-cudaError_t launch_relin_ks(const u64 *c3, const u64 *rk, u64 *ks, size_t n_ops, cudaStream_t s);
-int behz_mode();        // 0 dual base (default), 1 SEAL's Bsk primes + q-limb recovery, 2 SEAL's form (FHE_B200_BEHZ=dual|bsk|seal)
-bool qlimb_ntt();       // FHE_B200_QLIMB_NTT=1: transform the q-limbs of the tensor product as SEAL does instead of recovering them from the Bsk limbs
-bool ks_finish_fused();  // default: key-switch MAC + inverse transforms + rounded division by P in one kernel (FHE_B200_KS_FINISH=0: two)
-// rk_lm: optional scratch of 12 limbs for a lane-major copy of the key (made on the stream before the kernel)
-cudaError_t launch_ks_finish(const u64 *dig, const u64 *rk, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s, u64 *rk_lm = nullptr);
-bool ks_dual();  // FHE_B200_KS=dual: the key switch on the dual base too (opt-in A/B; default: on SEAL's 36/37-bit primes; same bits)
+// key switch on the dual base: launch_rk_prepare_ksd (per chunk) -> launch_digit_ntt_ksd -> launch_ks_tail_ksd
 // tmp36: 36 limbs of scratch; the dual-NTT key ends up at tmp36 + 24 limbs
 cudaError_t launch_rk_prepare_ksd(const u64 *rk, u64 *tmp36, cudaStream_t s);
 cudaError_t launch_digit_ntt_ksd(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s);
-cudaError_t launch_ks_intt_ksd(const u64 *dig, const u64 *rkd, u64 *ks, size_t n_ops, cudaStream_t s);
-cudaError_t launch_ks_finish_ksd(const u64 *ks, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s);
-cudaError_t launch_relin_finish(const u64 *c3, const u64 *ks, u64 *out, size_t n_ops, cudaStream_t s);
+cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s);
 
 uint64_t launch_count();
 void count_launches(uint64_t n);  // kernels replayed through a CUDA graph (the launchers only count at capture time)

@@ -198,80 +198,11 @@ __device__ __forceinline__ void dual_inv_bfly_last(u64 &X, u64 &Y, u64 sc, u64 s
     Y = pack64(d_0, d_1);
 }
 
-// sum_k x_k * w_k mod q for precomputed Shoup pairs (w_k, ws_k): the products' low 64 bits and the quotient estimates
-// H_k are accumulated separately and -(sum H_k) * q is applied once, so a term costs its partial products only and the
-// whole sum one reduction.  Everything is mod 2^64 (wrap-around in either accumulator is harmless) and the result is
-// exact as long as the true value sum_k (x_k w_k - H_k q) stays below 2^64:
-//   add      exact quotient, any 64-bit x : term in [0, q + x q / 2^64)                 FMA pipe 5 wide + 2 low
-//   add_a1   drops the x_lo*ws_lo partial product (H low by <= 2): adds another 2q       4 wide + 2 low
-// value(): one wide + one low multiply.  (The compiler's 128-bit mad/madc + fold sequence for the same sum issued twice
-// the multiplier cycles: duplicated partial products for the carries and multiplications by a zero high word.)
-template <class M>
-struct ShoupSum {
-    u64 lo = 0, hs = 0;
-    __device__ __forceinline__ void low_product(u32 xl, u32 xh, u64 w) {
-        u32 wl, wh, al, ah;
-        unpack64(w, wl, wh);
-        unpack64(mad_wide(xl, wl, lo), al, ah);
-        ah = mad_lo(xl, wh, ah);
-        ah = mad_lo(xh, wl, ah);
-        lo = pack64(al, ah);
-    }
-    __device__ __forceinline__ void add(u64 x, u64 w, u64 ws) {
-        u32 xl, xh, sl, sh, tl, th, ul, uh, vl, vh;
-        unpack64(x, xl, xh);
-        unpack64(ws, sl, sh);
-        unpack64(mul_wide(xl, sl), tl, th);
-        unpack64(mul_wide(xh, sl), ul, uh);
-        unpack64(mul_wide(xl, sh), vl, vh);
-        const u64 mc = (u64)ul + (u64)vl + (u64)th;  // middle column: one three-input add, two carries (see shoup_acc)
-        hs = mad_wide(xh, sh, hs) + (u64)uh + (u64)vh + (mc >> 32);
-        low_product(xl, xh, w);
-    }
-    __device__ __forceinline__ void add_a1(u64 x, u64 w, u64 ws) {
-        u32 xl, xh, sl, sh, ul, uh, vl, vh;
-        unpack64(x, xl, xh);
-        unpack64(ws, sl, sh);
-        unpack64(mul_wide(xh, sl), ul, uh);
-        unpack64(mul_wide(xl, sh), vl, vh);
-        hs = mad_wide(xh, sh, hs) + (u64)uh + (u64)vh;
-        low_product(xl, xh, w);
-    }
-    // 32-bit x: exact quotient from two partial products, term in [0, 2q)                               3 wide + 1 low
-    __device__ __forceinline__ void add32(u32 x, u64 w, u64 ws) {
-        u32 sl, sh, wl, wh, al, ah;
-        unpack64(ws, sl, sh);
-        unpack64(w, wl, wh);
-        hs += mad_wide(x, sh, mul_wide(x, sl) >> 32) >> 32;  // floor(x ws / 2^64), exact
-        unpack64(mad_wide(x, wl, lo), al, ah);
-        ah = mad_lo(x, wh, ah);
-        lo = pack64(al, ah);
-    }
-    // x * w for a small x (the product itself stays far below 2^64: no quotient term)                  1 wide + 1 low
-    __device__ __forceinline__ void add_small(u32 x, u64 w) {
-        u32 wl, wh, al, ah;
-        unpack64(w, wl, wh);
-        unpack64(mad_wide(x, wl, lo), al, ah);
-        ah = mad_lo(x, wh, ah);
-        lo = pack64(al, ah);
-    }
-    // sum - (sum H) q  =  sum + (sum H) c - ((sum H) << B)   (mod 2^64)
-    __device__ __forceinline__ u64 value() const {
-        constexpr u32 c = (u32)M::kC;
-        u32 hl, hh, al, ah;
-        unpack64(hs, hl, hh);
-        unpack64(mad_wide(hl, c, lo), al, ah);
-        ah = mad_lo(hh, c, ah);
-        ah -= hl << (M::kBits - 32);
-        return pack64(al, ah);
-    }
-};
-
 // Exact sum of up to seven products x_k * w_k with x_k < 2^31 (a dual-lane residue in [0, 2s)) and constants w_k < q < 2^37,
 // reduced ONCE: the low 30 bits of every w_k feed `lo` (each product < 2^61), the remaining <= 7 bits feed `hi` (each < 2^38),
 // and value() folds lo + hi 2^30 with q = 2^B - c.  A term costs two wide multiplies (8 multiplier-pipe cycles) against three
-// wide + one low (14) for a ShoupSum term, whose per-term quotient estimate buys nothing when the factors are this short; the
-// result is the canonical residue, so callers that canonicalised a ShoupSum value get the same bits.
+// wide + one low (14) for a term with its own Shoup quotient estimate, which buys nothing when the factors are this short; the
+// result is the canonical residue.
 template <class M>
 struct WideSum {
     static constexpr int kHiBits = M::kBits - 30;  // 6 or 7
@@ -327,8 +258,8 @@ __device__ __forceinline__ u64 canon(u64 x) {
 }
 
 // sum of NP (1 or 2) products x_i * y_i of two VARIABLES (no precomputed quotient), on explicit 32-bit partial products.
-// The compiler's lowering of mad.lo.cc.u64 / madc.hi.u64 + reduce128 recomputes partial products for the carries and
-// multiplies by zero high words; these issue 6-9 wide multiplies per call instead of 10-16.
+// The compiler's lowering of a 128-bit mad.lo.cc.u64 / madc.hi.u64 accumulate and its reduction recomputes partial products
+// for the carries and multiplies by zero high words; these issue 6-9 wide multiplies per call instead of 10-16.
 //
 // 61-bit primes, operands < 2^61, result in [0, 2q).  V = p00 + mid 2^32 + p11 2^64 (mid, p11 accumulate over the
 // products in mad.wide chains, no carries).  Quotient Q = qe + floor(qe c / 2^61) with qe ~ floor(V / 2^61) from the
@@ -415,35 +346,6 @@ __device__ __forceinline__ u64 reduce64(u64 x) {
     if (!M::kSmall) return canon<M>(x);  // fold(x) <= 2^61 - 1 + 7c < 2q
     u64 r = x - mulhi64(x, M::r1) * M::q;
     return csub<M>(r, M::q);
-}
-
-// (hi:lo) mod q, canonical -- the job of SEAL barrett_reduce_128, done with the primes' 2^b - c shape
-// instead of a Barrett quotient (about half the instructions; profiles/r1b -> r1c).
-//   61-bit primes: any (hi:lo) < 2^125.   2^64 = 8 * 2^61 == 8c, so z == lo + hi*8c; fold the 83-bit product once
-//                  more, absorb the (rare) 64-bit wrap, finish with the 61-bit fold.
-//   36/37-bit primes: (hi:lo) < 2^99.     z = d0 + d1*2^b with d1 < 2^63; d1 is folded twice to < 2^b + 2^28 so that
-//                  d0 + d1'*c < 2^56 fits a word; two more folds leave < 2q.
-template <class M>
-__device__ __forceinline__ u64 reduce128(u64 hi, u64 lo) {
-    if (!M::kSmall) {
-        constexpr u64 e = 8 * M::kC;  // 2^64 mod q  (< 2^22)
-        const u64 p_lo = hi * e;
-        const u64 p_hi = __umul64hi(hi, e);
-        const u64 s = lo + p_lo;
-        const u64 t = p_hi + (s < lo);
-        u64 r = s + t * e;
-        if (r < s) r += e;  // wrapped past 2^64 == e
-        return canon<M>(r);
-    } else {
-        constexpr int b = M::kBits;
-        const u64 d0 = lo & M::kMask;
-        u64 d1 = (lo >> b) | (hi << (64 - b));
-        d1 = fold<M>(d1);  // < 2^b + 2^(63-b) c  < 2^46
-        d1 = fold<M>(d1);  // < 2^b + 2^10 c
-        u64 x = d0 + d1 * M::kC;  // < 2^56
-        x = fold<M>(x);           // < 2^b + 2^20 c < 2^39
-        return canon<M>(x);       // fold -> < 2^b + 8c < 2q, then one conditional subtraction
-    }
 }
 
 // canonical a*b mod q; operands below 2^44 (36/37-bit primes) or 2^61 (61-bit primes)

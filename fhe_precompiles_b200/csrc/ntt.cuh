@@ -207,35 +207,12 @@ __device__ __forceinline__ void smem_load(const u64 *smem, u64 (&v)[NP][8], int 
         for (int r = 0; r < 8; r++) v[p][r] = smem[p * kN + (base ^ PassSlot<S0>::x(r)) + PassSlot<S0>::a(r)];
 }
 
-// A/B variant of the LAST exchange (between the passes with first stage 6 and 9): it is an 8 x 8 transpose inside groups of 8
-// consecutive lanes -- register r of lane l becomes register l of lane r -- so it can be done with warp shuffles instead of
-// shared memory: three butterfly steps (lane xor 1, 2, 4), four 64-bit exchanges each = 24 SHFL.32 + ~96 selects per thread
-// against 8 STS.64 + 8 LDS.64.  Measured slower (profiles/r2_shuffle_ab.md: the selects land on the ALU pipe, which the
-// butterflies already load to ~55 %), so shared memory stays the default; FHE_B200_NTT_SHFL=1 selects this path in k_ntt.
-template <int NP>
-__device__ __forceinline__ void shfl_transpose8(u64 (&v)[NP][8], int t) {
-#pragma unroll
-    for (int p = 0; p < NP; p++)
-#pragma unroll
-        for (int s = 1; s < 8; s <<= 1) {
-            const bool up = (t & s) != 0;
-#pragma unroll
-            for (int i = 0; i < 8; i++)
-                if (!(i & s)) {
-                    const u64 send = up ? v[p][i] : v[p][i | s];
-                    const u64 recv = __shfl_xor_sync(0xffffffffu, send, s);
-                    if (up) v[p][i] = recv;
-                    else v[p][i | s] = recv;
-                }
-        }
-}
-
 // ---------------------------------------------------------------- whole transforms on registers
 // Forward NTT of NP polynomials.
 //  in : v holds coefficients elem_index<0>(t, r) = r*512 + t   (natural order; small primes < 2^42, large < 2q)
 //  out: v holds NTT values at positions elem_index<9>(t, r) = 8*t + r, reduced to [0, q) if kCanon
 //       (else small primes < in + 48q, large primes < 8q).  Large-prime inputs must be < 2q.
-template <class M, int NP, bool kCanon, bool kTrailSync = true, bool kShflLast = false>
+template <class M, int NP, bool kCanon, bool kTrailSync = true>
 __device__ __forceinline__ void ntt_forward(u64 (&v)[NP][8], u64 *smem, const ulonglong2 *__restrict__ tw, int t) {
     fwd_pass<M, NP, 0>(v, tw, pass_upper<0>(t));
     smem_store<NP, 0>(smem, v, t);
@@ -246,13 +223,9 @@ __device__ __forceinline__ void ntt_forward(u64 (&v)[NP][8], u64 *smem, const ul
     sync_group64(t);
     smem_load<NP, 6>(smem, v, t);
     fwd_pass<M, NP, 6>(v, tw, pass_upper<6>(t));
-    if (kShflLast) {
-        shfl_transpose8<NP>(v, t);
-    } else {
-        smem_store<NP, 6>(smem, v, t);
-        __syncwarp();
-        smem_load<NP, 9>(smem, v, t);
-    }
+    smem_store<NP, 6>(smem, v, t);
+    __syncwarp();
+    smem_load<NP, 9>(smem, v, t);
     fwd_pass<M, NP, 9>(v, tw, pass_upper<9>(t));
     if constexpr (kCanon && !M::kDual) {
 #pragma unroll
@@ -267,17 +240,13 @@ __device__ __forceinline__ void ntt_forward(u64 (&v)[NP][8], u64 *smem, const ul
 //  in : v holds NTT values at positions 8*t + r, each < 2q (small primes: < 4q)
 //  out: v holds coefficients r*512 + t, multiplied by the scalar sc (scw = sc * last-stage twiddle), in [0, q)
 //       ([0, 2q) if !kCanon)
-template <class M, int NP, bool kCanon = true, bool kTrailSync = true, bool kShflLast = false>
+template <class M, int NP, bool kCanon = true, bool kTrailSync = true>
 __device__ __forceinline__ void ntt_inverse(u64 (&v)[NP][8], u64 *smem, const ulonglong2 *__restrict__ tw, int t, const Shoup &sc,
                                             const Shoup &scw) {
     inv_pass<M, NP, 9, 0>(v, tw, pass_upper<9>(t));
-    if (kShflLast) {
-        shfl_transpose8<NP>(v, t);
-    } else {
-        smem_store<NP, 9>(smem, v, t);
-        __syncwarp();
-        smem_load<NP, 6>(smem, v, t);
-    }
+    smem_store<NP, 9>(smem, v, t);
+    __syncwarp();
+    smem_load<NP, 6>(smem, v, t);
     inv_pass<M, NP, 6, 3>(v, tw, pass_upper<6>(t));
     smem_store<NP, 6>(smem, v, t);
     sync_group64(t);

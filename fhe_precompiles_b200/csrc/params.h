@@ -42,9 +42,6 @@ constexpr int kTwPass9 = 7 * 512;
 constexpr int kTwEntries = kN + kTwPass9;
 constexpr int kNumTab = kNumMod + kNumDual;  // twiddle tables: the six 64-bit-lane moduli, then the three dual limbs
 
-// limb order of the extended BEHZ base q U Bsk used in all 5-limb device buffers
-constexpr int kExtLimb[5] = {MQ0, MQ1, MB0, MB1, MSK};
-
 // floor(2^128 / q) as (hi, lo), q < 2^63 and not a power of two
 struct U128c {
     u64 hi, lo;

@@ -112,21 +112,6 @@ def ntt_(data: torch.Tensor, mods: Sequence[int], inverse: bool = False) -> torc
     return data
 
 
-def behz_extend(a, b):
-    return _binary(_lib.lib().fhe_b200_behz_extend, a, b, (a.shape[0], 4, 5, N))
-
-
-def behz_tensor(a, b):
-    return _binary(_lib.lib().fhe_b200_behz_tensor, a, b, (a.shape[0], 3, 5, N))
-
-
-def behz_floor_sk(tens):
-    dev = _dev(tens)
-    out = torch.empty((tens.shape[0], 3, 2, N), dtype=torch.int64, device=tens.device)
-    _check(_lib.lib().fhe_b200_behz_floor_sk(dev, tens.data_ptr(), out.data_ptr(), tens.shape[0], _stream(dev)))
-    return out
-
-
 def mul_relin_host(a: torch.Tensor, b: torch.Tensor, rk: torch.Tensor, out: torch.Tensor, device: int = 0) -> torch.Tensor:
     """a, b, out: HOST tensors [n,2,2,4096] int64 (pinned for full PCIe rate); rk: host [2,2,3,4096]."""
     for t in (a, b, rk, out):
@@ -219,11 +204,6 @@ def bfly_peak(device: int = 0, mod: int = 0) -> float:
     v = ctypes.c_double()
     _check(_lib.lib().fhe_b200_bfly_peak(device, mod, ctypes.byref(v)))
     return float(v.value)
-
-
-def set_fused(on: bool) -> None:
-    """Select the multi-polynomial-per-CTA kernels (True) or the one-polynomial-per-CTA kernels (False, default)."""
-    _lib.lib().fhe_b200_set_fused(int(on))
 
 
 def encrypt(pk: torch.Tensor, plain: torch.Tensor, seeds: torch.Tensor) -> torch.Tensor:

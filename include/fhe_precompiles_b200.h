@@ -212,12 +212,10 @@ int32_t fhe_b200_data_type_kind(const char *data_type);
 /* Ops per chunk of the device-resident entry points (default 4,096, FHE_B200_CHUNK_OPS): a batch larger than this runs chunk
  * after chunk through one scratch arena.  ops <= 0 only queries.  Returns the previous value (-1 without a device). */
 int64_t fhe_b200_set_chunk_ops(int64_t ops);
-/* Kernel variant of multiply / relinearise: 0 (default) one polynomial per CTA (k_ext_ntt, k_tensor_intt,
- * k_digit_ntt, k_ks_intt); 1 multi-polynomial CTAs (k_behz_tensor, k_relin_ks). Same results. */
-void fhe_b200_set_fused(int32_t on);
 /* Per-kernel timing of fhe_b200_mul_relin (CUDA events around each launch, on the caller's stream).
- * ms / launches are indexed 0 k_behz_tensor, 1 k_floor_sk, 2 k_relin_ks, 3 k_relin_finish, 4 k_ext_ntt,
- * 5 k_tensor_intt, 6 k_digit_ntt, 7 k_ks_intt; the report synchronises the device and resets the accumulators. */
+ * ms / launches are indexed 1 k_floor_sk_d, 3 k_relin_finish, 4 k_ext_ntt_d, 5 k_tensor_intt_d, 6 k_digit_ntt, 7 k_ks_intt,
+ * 8 k_ext_conv_d, 10 k_rk_*_ksd (key preparation), 11 k_digit_ntt_ksd, 14 k_tensor_floor_d, 15 k_ks_tail_ksd; slots 0, 2, 9,
+ * 12 and 13 are reserved and stay zero.  The report synchronises the device and resets the accumulators. */
 /* Phase timing of the byte surface (SURVEY 8d: parse+inflate / H2D / kernels / D2H / deflate).  When on, every binary
  * precompile call records, for the calling thread: us[0] framing + key lookup, us[1] operand decode (bincode + zstd inflate
  * + range checks), us[2] H2D, us[3] kernels, us[4] D2H (CUDA events on the lane's stream), us[5] result encode, us[6] total. */
@@ -229,11 +227,6 @@ int32_t fhe_b200_kernel_timing_report(int32_t device, double ms[16], uint64_t la
  * (0 q0, 1 q1, 2 P, 3 b0, 4 b1, 5 m_sk). inverse != 0: bit-reversed -> natural, scaled by N^-1. */
 int32_t fhe_b200_ntt(int32_t device, uint64_t *data, size_t n_limbs, const int32_t *mods, int32_t n_mods, int32_t inverse,
                      void *stream);
-/* Stage taps used by the parity tests: BEHZ base extension [n][4][5][4096], tensor [n][3][5][4096] (x t),
- * floor + Shenoy-Kumaresan [n][3][2][4096]. */
-int32_t fhe_b200_behz_extend(int32_t device, const uint64_t *a, const uint64_t *b, uint64_t *ext, size_t n, void *stream);
-int32_t fhe_b200_behz_tensor(int32_t device, const uint64_t *a, const uint64_t *b, uint64_t *tens, size_t n, void *stream);
-int32_t fhe_b200_behz_floor_sk(int32_t device, const uint64_t *tens, uint64_t *out3, size_t n, void *stream);
 
 /* Host-side format helpers (no GPU needed): parse a sunscreen PublicKey and write its relinearisation key
  * (2*2*3*4096 words) and/or public key (2*3*4096 words); either pointer may be NULL. lib.rs error code. */

@@ -5,7 +5,7 @@ before any kernel was written -- pure CPU:
     on six NTT primes below 2^30 (product 2^180), recovering t_l = t D (q/q_l)^-1 mod q_l by CRT with rounding, forming
     y0 = t_0 q_1 + t_1 q_0 and lifting f = (t D - y0) / q from four of the primes by rounding gives SEAL's size-3 result bit
     for bit;
-  * key switch (default; FHE_B200_KS=seal opts out): U_k = sum_j d_j * RK_jk over Z with the key lifted to integers, |U_k| < 2^161,
+  * key switch (what the library runs for chunks of 96 ops and more): U_k = sum_j d_j * RK_jk over Z with the key lifted to integers, |U_k| < 2^161,
     carried on the same six primes; U_k mod (q0, q1, P) by the same CRT gives SEAL's relinearised ciphertext bit for bit.
 
 usage: python scripts/check_dual_base.py [pairs]      (tests/test_integer_domain.py runs one pair)"""

@@ -37,21 +37,14 @@ def main():
     b = torch.from_numpy(np.tile(base[::-1], (reps, 1, 1, 1))[:n].view(np.int64).copy()).cuda()
     rk = torch.from_numpy(keys.rk.view(np.int64)).cuda()
     out = torch.empty_like(a)
-    for fused in (True, False):
-        device.set_fused(fused)
-        ms = timeit(lambda: device.mul_relin(a, b, rk, out=out))
-        print(f"mul_relin n={n} fused={fused}: {ms:.3f} ms  -> {n / ms * 1e3:.0f} ops/s")
-        device.set_kernel_timing(True)
-        device.mul_relin(a, b, rk, out=out)
-        rep = device.kernel_timing_report(0)
-        device.set_kernel_timing(False)
-        print("   ", {k: round(v[0] / n * 1e3, 3) for k, v in rep.items()}, "us/op")
-    ms = timeit(lambda: device.behz_tensor(a, b))
-    print(f"  behz_tensor: {ms:.3f} ms ({ms / n * 1e3:.2f} us/op)")
-    tens = device.behz_tensor(a, b)
-    ms = timeit(lambda: device.behz_floor_sk(tens))
-    print(f"  floor_sk:    {ms:.3f} ms ({ms / n * 1e3:.2f} us/op)")
-    c3 = device.behz_floor_sk(tens)
+    ms = timeit(lambda: device.mul_relin(a, b, rk, out=out))
+    print(f"mul_relin n={n}: {ms:.3f} ms  -> {n / ms * 1e3:.0f} ops/s")
+    device.set_kernel_timing(True)
+    device.mul_relin(a, b, rk, out=out)
+    rep = device.kernel_timing_report(0)
+    device.set_kernel_timing(False)
+    print("   ", {k: round(v[0] / n * 1e3, 3) for k, v in rep.items()}, "us/op")
+    c3 = device.multiply(a, b)
     ms = timeit(lambda: device.relinearize(c3, rk))
     print(f"  relinearize: {ms:.3f} ms ({ms / n * 1e3:.2f} us/op)")
     ms = timeit(lambda: device.add(a, b))

@@ -12,12 +12,9 @@ rng = np.random.default_rng(0)
 a, b = t(random_ct(rng, 3)), t(random_ct(rng, 3))
 rk, pk, sk = t(keys.net_rk), t(keys.net_pk), t(keys.net_sk)
 pl = torch.randint(0, 4096, (3, N), dtype=torch.int16, device="cuda")
-for fused in (False, True):
-    d.set_fused(fused)
-    out = d.mul_relin(a, b, rk)
+out = d.mul_relin(a, b, rk)
 d.add(a, b); d.sub(a, b); d.negate(a); d.plain_addsub(a, pl, 3); d.multiply_plain(a, pl)
 x = t(rng.integers(0, MODULI[3], size=(6, N), dtype=np.uint64)); d.ntt_(x, [3]); d.ntt_(x, [3], inverse=True)
 ct = d.encrypt(pk, pl, torch.arange(3, dtype=torch.int64, device="cuda")); d.decrypt(ct, sk)
-d.behz_extend(a, b)
 torch.cuda.synchronize()
 print("sanitize case done", int(out[0,0,0,0]))

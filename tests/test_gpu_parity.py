@@ -123,19 +123,12 @@ def test_plain_ops(dev):
     assert np.array_equal(got, want)
 
 
-def test_behz_stages(dev):
+def test_multiply_against_oracle_behz_stages(dev):
+    """multiply on edge inputs against the oracle's BEHZ stages: fastbconv_m_tilde + sm_mrq, NTT + tensor + INTT * t,
+    fast_floor + fastbconv_sk"""
     a, b = edge_ct(3, 5), edge_ct(3, 6)[::-1].copy()
-    da, db = to_dev(a), to_dev(b)
-    ext = to_np(dev.behz_extend(da, db))
-    want_ext = np.stack([bfv.behz_extend(x, y) for x, y in zip(a, b)])
-    assert np.array_equal(ext, want_ext), "fastbconv_m_tilde + sm_mrq"
-    tens = to_np(dev.behz_tensor(da, db))
-    want_tens = np.stack([bfv.behz_tensor(e) for e in want_ext])
-    assert np.array_equal(tens, want_tens), "NTT + tensor + INTT * t"
-    c3 = to_np(dev.behz_floor_sk(to_dev(want_tens)))
-    want_c3 = np.stack([bfv.behz_floor_sk(t) for t in want_tens])
-    assert np.array_equal(c3, want_c3), "fast_floor + fastbconv_sk"
-    assert np.array_equal(to_np(dev.multiply(da, db)), want_c3), "bfv_multiply"
+    want_c3 = np.stack([bfv.behz_floor_sk(bfv.behz_tensor(bfv.behz_extend(x, y))) for x, y in zip(a, b)])
+    assert np.array_equal(to_np(dev.multiply(to_dev(a), to_dev(b))), want_c3), "bfv_multiply"
 
 
 def test_relinearize_and_mul_relin(dev, keys):
@@ -145,19 +138,6 @@ def test_relinearize_and_mul_relin(dev, keys):
     want = np.stack([bfv.relinearize(c, keys.rk) for c in c3])
     assert np.array_equal(to_np(dev.relinearize(to_dev(c3), drk)), want), "switch_key_inplace"
     assert np.array_equal(to_np(dev.mul_relin(da, db, drk)), want), "multiply + relinearize"
-
-
-def test_fused_kernel_variant(dev, keys):
-    """the multi-polynomial-per-CTA kernels (k_behz_tensor, k_relin_ks) give the same bits as the default split ones"""
-    a, b = edge_ct(3, 18), edge_ct(3, 19)[::-1].copy()
-    da, db, drk = to_dev(a), to_dev(b), to_dev(keys.rk)
-    want = np.stack([bfv.mul_relin(x, y, keys.rk) for x, y in zip(a, b)])
-    try:
-        dev.set_fused(True)
-        assert np.array_equal(to_np(dev.mul_relin(da, db, drk)), want)
-    finally:
-        dev.set_fused(False)
-    assert np.array_equal(to_np(dev.mul_relin(da, db, drk)), want)
 
 
 def test_mul_relin_real_encryptions_chunked(dev, keys):
@@ -995,51 +975,30 @@ def test_device_sampler_exact_paths_on_crafted_draws(dev):
 
 
 def test_qlimb_recovery_equals_seals_form(dev, keys):
-    """The multiply is computed five ways -- default (tensor product AND key switch on the GPU's dual base, fused tails), the
-    same with split tails (FHE_B200_FUSE_TAIL=0), SEAL's form
-    (FHE_B200_QLIMB_NTT=1: 47 transforms), SEAL's 61-bit primes with the q-limbs recovered (FHE_B200_BEHZ=bsk), and the default
-    with the key switch on SEAL's three key primes (FHE_B200_KS=seal) -- same bits on random and on extreme residues, equal to
-    the oracle (which follows SEAL).  The key-switch paths only differ for batches >= 96 ops, hence the 128-op batch."""
+    """Both forms of multiply + relinearise -- chunks >= 96 ops (fused tails, key switch on the dual base) and smaller chunks
+    (split tails, key switch on SEAL's key primes) -- through mul_relin and through multiply followed by relinearize: same
+    bits on random and on extreme residues, equal to the oracle (which follows SEAL)."""
     import hashlib
-    import subprocess
-    import sys
 
-    code = r"""
-import hashlib, sys
-import numpy as np, torch
-sys.path.insert(0, %r); sys.path.insert(0, %r)
-from helpers import KeySet, random_ct, MODULI, N
-from fhe_precompiles_b200 import device
-device.init(0)
-keys = KeySet.load()
-rng = np.random.default_rng(606)
-a, b = random_ct(rng, 128), random_ct(rng, 128)
-for l in range(2):
-    a[20, :, l, :] = MODULI[l] - 1; b[20, :, l, :] = MODULI[l] - 1      # every coefficient q-1: the largest |t D|
-    a[21, :, l, :] = MODULI[l] // 2; b[21, :, l, :] = MODULI[l] // 2 + 1
-a[22] = 0; b[23] = 0
-t = lambda x: torch.from_numpy(np.ascontiguousarray(x).view(np.int64)).cuda()
-out = device.mul_relin(t(a), t(b), t(keys.rk)).cpu().numpy()
-print("SHA", hashlib.sha256(out.tobytes()).hexdigest())
-""" % (ROOT, os.path.join(ROOT, "tests"))
-    shas = {}
-    # "0": the default (tensor product and key switch on the dual base); "1": SEAL's form (47 transforms) with SEAL's key switch;
-    # "bsk": SEAL's 61-bit primes with the q-limbs recovered (33 transforms); "kss": the default with SEAL's key switch
-    # "split": the default arithmetic with the tensor product and U_k going through HBM between two kernels each
-    for mode, env in (("0", {}), ("1", {"FHE_B200_QLIMB_NTT": "1", "FHE_B200_KS": "seal"}), ("bsk", {"FHE_B200_BEHZ": "bsk"}),
-                      ("kss", {"FHE_B200_KS": "seal"}), ("split", {"FHE_B200_FUSE_TAIL": "0"})):
-        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600, env=dict(os.environ, **env))
-        assert r.returncode == 0, r.stdout + r.stderr
-        shas[mode] = [ln for ln in r.stdout.splitlines() if ln.startswith("SHA")][0]
-    assert shas["0"] == shas["1"] == shas["bsk"] == shas["kss"] == shas["split"]
     rng = np.random.default_rng(606)
     a, b = random_ct(rng, 128), random_ct(rng, 128)
     for l in range(2):
-        a[20, :, l, :] = MODULI[l] - 1; b[20, :, l, :] = MODULI[l] - 1
+        a[20, :, l, :] = MODULI[l] - 1; b[20, :, l, :] = MODULI[l] - 1      # every coefficient q-1: the largest |t D|
         a[21, :, l, :] = MODULI[l] // 2; b[21, :, l, :] = MODULI[l] // 2 + 1
     a[22] = 0; b[23] = 0
     want = np.stack([bfv.mul_relin(a[i], b[i], keys.rk) for i in range(128)])
-    assert shas["0"] == "SHA " + hashlib.sha256(want.view(np.int64).tobytes()).hexdigest()
+    sha = lambda x: hashlib.sha256(np.ascontiguousarray(x).tobytes()).hexdigest()
+    da, db, drk = to_dev(a), to_dev(b), to_dev(keys.rk)
+    shas = {}
+    prev = dev.set_chunk_ops(0)
+    try:
+        for chunk in (4096, 64):  # the default: one chunk of 128 ops; then two chunks of 64
+            dev.set_chunk_ops(chunk)
+            shas[chunk, "mul_relin"] = sha(to_np(dev.mul_relin(da, db, drk)))
+            shas[chunk, "multiply + relinearize"] = sha(to_np(dev.relinearize(dev.multiply(da, db), drk)))
+    finally:
+        dev.set_chunk_ops(prev)
+    assert shas == {k: sha(want) for k in shas}
 
 
 def test_exhausted_noise_budget_is_failed_decryption(dev, keys):
