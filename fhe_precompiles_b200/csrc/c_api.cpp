@@ -514,10 +514,6 @@ int32_t fhe_b200_zstd_inflate(int32_t device, const uint8_t *const *frames, cons
                               int32_t *status, float *elapsed_ms) {
     try {
         device_context(device);
-        {
-            const char *v = getenv("FHE_B200_ZSTD_TWO_PHASE");  // 0 one warp per frame, 1 two-phase, 2 batch-oriented, 3 (default) zstd_plan3.cuh
-            codec_set_two_phase(v && *v ? atoi(v) : 3);
-        }
         std::vector<CodecJob> jobs(n);
         std::vector<uint8_t> staged(n * kFrameSlotBytes, 0);
         for (size_t i = 0; i < n; i++) {

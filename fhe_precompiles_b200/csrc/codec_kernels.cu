@@ -1,6 +1,9 @@
 // Device side of the byte surface (SURVEY 8f-3): the zstd frames of the ciphertext operands are inflated on the GPU and the
 // result is written as a structured zstd frame on the GPU, so the host moves compressed bytes only.
-//   k_zstd_inflate : one frame per warp (zstd_dec.h; lane 0 decodes, the frame's bitstreams are sequential by construction)
+//   k_zd2_parse    : headers and FSE / Huffman tables, thread per frame (zstd_plan2.h)
+//   k_zd3_huf      : Huffman literal streams, thread per stream (zstd_plan2.h)
+//   k_zd3_seq      : FSE sequence chains, four frames per warp, tables in shared memory (zstd_plan2.h, zstd_plan3.cuh)
+//   k_zd3_exec     : sequence execution, CTA per frame (zstd_plan3.cuh, zstd_exec3.h)
 //   k_ct_unpack    : 131,169-byte SEAL payload -> [2][2][N] words; checks the 97-byte prefix against the only value a valid
 //                    data-level ciphertext can have and every residue against its modulus
 //   k_unpack40     : the same for frames in this library's own structured layout (5-byte literals), fully parallel
@@ -10,8 +13,6 @@
 
 #include "codec_kernels.h"
 #include "params.h"
-#include "zstd_dec.h"
-#include "zstd_plan2.h"
 #include "zstd_plan3.cuh"
 
 namespace fheb {
@@ -20,141 +21,51 @@ extern std::atomic<unsigned long long> g_codec_launches;
 std::atomic<unsigned long long> g_codec_launches{0};
 
 namespace {
-constexpr int kInflateWarps = 4;  // decoders per block
 constexpr u64 kQ0 = kModulus[0], kQ1 = kModulus[1];
 
-constexpr size_t kInflateSmemPerWarp = zd::kSeqTableEntries * sizeof(zd::SeqEntry) + zd::kRingBytes;
-constexpr size_t kInflateSmem = kInflateWarps * kInflateSmemPerWarp;
-
-__global__ void __launch_bounds__(kInflateWarps * 32) k_zstd_inflate(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs,
-                                                                      int32_t *status, uint8_t *work, size_t work_stride, int n) {
-    extern __shared__ __align__(16) uint8_t smem[];
-    const int warp = threadIdx.x >> 5;
-    const int j = blockIdx.x * kInflateWarps + warp;
-    if (j >= n) return;
-    const CodecJob job = jobs[j];
-    if (job.kind != kJobZstd) return;
-    uint8_t *mine = smem + (size_t)warp * kInflateSmemPerWarp;
-    zd::Work *w = (zd::Work *)(work + (size_t)j * work_stride);  // first member of the job's scratch
-    if ((threadIdx.x & 31) == 0) zd::work_bind(w, (zd::SeqEntry *)mine);
-    __syncwarp();
-    size_t dlen = 0;
-    const int rc = zd::decode_frame(frames + job.src_off, job.src_len, payloads + (size_t)j * kPayloadStride, kCtPayloadBytes, &dlen, w,
-                                    mine + zd::kSeqTableEntries * sizeof(zd::SeqEntry));
-    if ((threadIdx.x & 31) == 0) status[j] = (rc == zd::kZdOk && dlen == kCtPayloadBytes) ? kJobOk : kJobFallback;
-}
-
-// ---- two-phase inflate: thread-per-frame planning, warp-per-frame execution (zstd_dec.h, "two-phase decoding")
-constexpr int kPlanLanes = 8;  // frames per warp in phase 1: few enough that a small batch still spreads over many SMs
-struct JobScratch {            // per job, in the `work` buffer
-    zd::Work work;
-    zd::FramePlan plan;
-    uint64_t seqs[zd::kPlanMaxSeqs];
-    uint8_t lits[kCtPayloadBytes + 16];
-};
-
-// (every decoder indexes the `work` buffer with the common per-job stride, codec_work_bytes())
-__global__ void __launch_bounds__(128) k_zstd_plan(const uint8_t *frames, const CodecJob *jobs, uint8_t *work, size_t work_stride, int n) {
-    const int lane = threadIdx.x & 31;
-    const int j = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * kPlanLanes + lane;
-    if (lane >= kPlanLanes || j >= n) return;
-    const CodecJob job = jobs[j];
-    JobScratch *sc = (JobScratch *)(work + (size_t)j * work_stride);
-    sc->plan.status = zd::kZdFallback;
-    if (job.kind != kJobZstd) return;
-    zd::work_bind(&sc->work, nullptr);
-    zd::plan_frame(frames + job.src_off, job.src_len, kCtPayloadBytes, &sc->work, &sc->plan, sc->seqs, sc->lits);
-}
-
-__global__ void __launch_bounds__(kInflateWarps * 32) k_zstd_execute(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs,
-                                                                      int32_t *status, const uint8_t *work, size_t work_stride, int n) {
-    __shared__ __align__(16) uint8_t rings[kInflateWarps][zd::kRingBytes];
-    const int warp = threadIdx.x >> 5;
-    const int j = blockIdx.x * kInflateWarps + warp;
-    if (j >= n) return;
-    const CodecJob job = jobs[j];
-    if (job.kind != kJobZstd) return;
-    const JobScratch *sc = (const JobScratch *)(work + (size_t)j * work_stride);
-    size_t dlen = 0;
-    const int rc = zd::execute_plan(frames + job.src_off, &sc->plan, sc->seqs, sc->lits, payloads + (size_t)j * kPayloadStride, &dlen,
-                                    rings[warp]);
-    if ((threadIdx.x & 31) == 0) status[j] = (rc == zd::kZdOk && dlen == kCtPayloadBytes) ? kJobOk : kJobFallback;
-}
-
-// ---- batch-oriented inflate (zstd_plan2.h, the default): parse (thread per frame) -> decode (a block of five warps per 32
-// frames: warps 0..3 walk Huffman stream 0..3 of their lane's frame, warp 4 its sequence streams -- the five dependent chains of
-// a frame run concurrently and a warp never diverges between the two loop bodies) -> execute (warp per frame, byte copies)
-struct JobScratch2 {
+struct JobScratch {  // one workspace slot per job, shared by the four inflate kernels
     zd::Plan2 plan;
     zd::Work work;  // table-construction scratch of the parse step
     zd::Tables2 tabs;
     uint64_t seqs[zd::kP2MaxSeqs];
     uint8_t lits[(kCtPayloadBytes + 16 + 7) & ~(size_t)7];
 };
-union JobScratchAny {  // one workspace slot per job, whichever decoder runs
-    JobScratch a;
-    JobScratch2 b;
-};
 
-__global__ void __launch_bounds__(32) k_zd2_parse(const uint8_t *frames, const CodecJob *jobs, JobScratchAny *scratch, int n) {
+__global__ void __launch_bounds__(32) k_zd2_parse(const uint8_t *frames, const CodecJob *jobs, JobScratch *scratch, int n) {
     const int j = blockIdx.x * 32 + threadIdx.x;
     if (j >= n) return;
     const CodecJob job = jobs[j];
-    JobScratch2 *sc = &scratch[j].b;
+    JobScratch *sc = &scratch[j];
     sc->plan.status = zd::kZdFallback;
     if (job.kind != kJobZstd) return;
     zd::work_bind(&sc->work, nullptr);
     zd::plan2_parse(frames + job.src_off, job.src_len, kCtPayloadBytes, &sc->work, &sc->plan, &sc->tabs);
 }
-__global__ void __launch_bounds__(160) k_zd2_decode(const uint8_t *frames, const CodecJob *jobs, JobScratchAny *scratch, int n) {
+__global__ void __launch_bounds__(128) k_zd3_huf(const uint8_t *frames, const CodecJob *jobs, JobScratch *scratch, int n) {
     const int j = blockIdx.x * 32 + (threadIdx.x & 31), role = threadIdx.x >> 5;
     if (j >= n) return;
     const CodecJob job = jobs[j];
     if (job.kind != kJobZstd) return;
-    JobScratch2 *sc = &scratch[j].b;
-    const uint8_t *f = frames + job.src_off;
-    if (role < 4) sc->plan.huf_bad[role] = zd::plan2_huf(f, &sc->plan, &sc->tabs, sc->lits, role) ? 0 : 1;
-    else sc->plan.seq_bad = zd::plan2_seq(f, &sc->plan, &sc->tabs, sc->seqs) ? 0 : 1;
-}
-__global__ void __launch_bounds__(32) k_zd2_exec(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs, int32_t *status,
-                                                 const JobScratchAny *scratch, int n) {
-    const int j = blockIdx.x * 32 + threadIdx.x;
-    if (j >= n) return;
-    const CodecJob job = jobs[j];
-    if (job.kind != kJobZstd) return;
-    const JobScratch2 *sc = &scratch[j].b;
-    size_t dlen = 0;
-    const int rc = zd::plan2_exec(frames + job.src_off, &sc->plan, sc->seqs, sc->lits, payloads + (size_t)j * kPayloadStride, &dlen);
-    status[j] = (rc == zd::kZdOk && dlen == kCtPayloadBytes) ? kJobOk : kJobFallback;
-}
-
-// ---- fourth generation (zstd_plan3.cuh, the default): parse as above -> Huffman streams (thread per stream; ciphertext frames
-// have raw literals and skip it) and sequence chains (warp per frame, tables in shared memory) -> execution (CTA per frame)
-__global__ void __launch_bounds__(128) k_zd3_huf(const uint8_t *frames, const CodecJob *jobs, JobScratchAny *scratch, int n) {
-    const int j = blockIdx.x * 32 + (threadIdx.x & 31), role = threadIdx.x >> 5;
-    if (j >= n) return;
-    const CodecJob job = jobs[j];
-    if (job.kind != kJobZstd) return;
-    JobScratch2 *sc = &scratch[j].b;
+    JobScratch *sc = &scratch[j];
     sc->plan.huf_bad[role] = zd::plan2_huf(frames + job.src_off, &sc->plan, &sc->tabs, sc->lits, role) ? 0 : 1;
 }
-__global__ void __launch_bounds__(32) k_zd3_seq(const uint8_t *frames, const CodecJob *jobs, JobScratchAny *scratch, int n) {
+__global__ void __launch_bounds__(32) k_zd3_seq(const uint8_t *frames, const CodecJob *jobs, JobScratch *scratch, int n) {
     extern __shared__ __align__(16) uint8_t smem3[];
     const int j = blockIdx.x * zd3::kSeqFrames + (threadIdx.x >> 3);
     const bool in_range = j < n;
     const CodecJob job = in_range ? jobs[j] : CodecJob{0, 0, kJobNone, 0, 0};
-    JobScratch2 *sc = &scratch[in_range ? j : 0].b;
+    JobScratch *sc = &scratch[in_range ? j : 0];
     const bool have = in_range && job.kind == kJobZstd && sc->plan.status == zd::kZdOk;
     const bool ok = zd3::seq_frames(frames + job.src_off, &sc->plan, &sc->tabs, sc->seqs, have, (uint32_t *)smem3);
     if (have && (threadIdx.x & 7) == 0) sc->plan.seq_bad = ok ? 0 : 1;
 }
 __global__ void __launch_bounds__(zd3::kExecThreads, 1) k_zd3_exec(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs,
-                                                                     int32_t *status, JobScratchAny *scratch, int n) {
+                                                                     int32_t *status, JobScratch *scratch, int n) {
     extern __shared__ __align__(16) uint8_t smem3[];
     for (int j = blockIdx.x; j < n; j += gridDim.x) {
         const CodecJob job = jobs[j];
         if (job.kind != kJobZstd) continue;
-        JobScratch2 *sc = &scratch[j].b;
+        JobScratch *sc = &scratch[j];
         const zd::Plan2 *plan = &sc->plan;
         int rc = zd::kZdFallback;
         if (plan->status == zd::kZdOk && !plan->seq_bad && !plan->huf_bad[0] && !plan->huf_bad[1] && !plan->huf_bad[2] && !plan->huf_bad[3] &&
@@ -299,12 +210,7 @@ __global__ void __launch_bounds__(256) k_ct_pack40(const u64 *words, uint8_t *fr
 }
 }  // namespace
 
-size_t codec_work_bytes() { return sizeof(JobScratchAny); }
-
-// 0 one warp per frame, 1 two-phase (thread-per-frame plan + warp-per-frame execute), 2 batch-oriented (zstd_plan2.h),
-// 3 (default) warp-per-frame sequence chains on shared-memory tables + CTA-per-frame parallel execution (zstd_plan3.cuh)
-static std::atomic<int> g_inflate_mode{3};
-void codec_set_two_phase(int mode) { g_inflate_mode.store(mode < 0 || mode > 3 ? 3 : mode); }
+size_t codec_work_bytes() { return sizeof(JobScratch); }
 
 cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs, int32_t *status, void *work,
                                  const uint8_t *prefix, u64 *dst_a, u64 *dst_b, int n_jobs, bool any_zstd, bool any_packed,
@@ -317,8 +223,7 @@ cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const
     } else {
         any_zstd = false;  // (decoded by the kCodecDecode call)
     }
-    const int mode = g_inflate_mode.load();
-    if (any_zstd && mode == 3) {
+    if (any_zstd) {
         static std::atomic<int> configured{0};  // (per process; the attributes are per function and device-independent in effect)
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
@@ -328,30 +233,12 @@ cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const
             if (e != cudaSuccess) return e;
             configured.fetch_or(1 << dev);
         }
-        k_zd2_parse<<<(n_jobs + 31) / 32, 32, 0, s>>>(frames, jobs, (JobScratchAny *)work, n_jobs);
-        k_zd3_huf<<<(n_jobs + 31) / 32, 128, 0, s>>>(frames, jobs, (JobScratchAny *)work, n_jobs);
-        k_zd3_seq<<<(n_jobs + zd3::kSeqFrames - 1) / zd3::kSeqFrames, 32, zd3::kSeqSmem, s>>>(frames, jobs, (JobScratchAny *)work, n_jobs);
+        k_zd2_parse<<<(n_jobs + 31) / 32, 32, 0, s>>>(frames, jobs, (JobScratch *)work, n_jobs);
+        k_zd3_huf<<<(n_jobs + 31) / 32, 128, 0, s>>>(frames, jobs, (JobScratch *)work, n_jobs);
+        k_zd3_seq<<<(n_jobs + zd3::kSeqFrames - 1) / zd3::kSeqFrames, 32, zd3::kSeqSmem, s>>>(frames, jobs, (JobScratch *)work, n_jobs);
         k_zd3_exec<<<n_jobs < 2 * sms ? n_jobs : 2 * sms, zd3::kExecThreads, zd3::kExecSmem, s>>>(frames, payloads, jobs, status,
-                                                                                                    (JobScratchAny *)work, n_jobs);
+                                                                                                    (JobScratch *)work, n_jobs);
         g_codec_launches.fetch_add(4, std::memory_order_relaxed);
-    } else if (any_zstd && mode == 2) {
-        k_zd2_parse<<<(n_jobs + 31) / 32, 32, 0, s>>>(frames, jobs, (JobScratchAny *)work, n_jobs);
-        k_zd2_decode<<<(n_jobs + 31) / 32, 160, 0, s>>>(frames, jobs, (JobScratchAny *)work, n_jobs);
-        k_zd2_exec<<<(n_jobs + 31) / 32, 32, 0, s>>>(frames, payloads, jobs, status, (const JobScratchAny *)work, n_jobs);
-        g_codec_launches.fetch_add(3, std::memory_order_relaxed);
-    } else if (any_zstd && mode == 1) {
-        const int warps_per_block = 4, frames_per_block = warps_per_block * kPlanLanes;
-        k_zstd_plan<<<(n_jobs + frames_per_block - 1) / frames_per_block, warps_per_block * 32, 0, s>>>(frames, jobs, (uint8_t *)work,
-                                                                                                        codec_work_bytes(), n_jobs);
-        k_zstd_execute<<<(n_jobs + kInflateWarps - 1) / kInflateWarps, kInflateWarps * 32, 0, s>>>(frames, payloads, jobs, status,
-                                                                                                   (const uint8_t *)work, codec_work_bytes(), n_jobs);
-        g_codec_launches.fetch_add(2, std::memory_order_relaxed);
-    } else if (any_zstd) {
-        cudaError_t e = cudaFuncSetAttribute(k_zstd_inflate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem);
-        if (e != cudaSuccess) return e;
-        k_zstd_inflate<<<(n_jobs + kInflateWarps - 1) / kInflateWarps, kInflateWarps * 32, kInflateSmem, s>>>(
-            frames, payloads, jobs, status, (uint8_t *)work, codec_work_bytes(), n_jobs);
-        g_codec_launches.fetch_add(1, std::memory_order_relaxed);
     }
     if (phase == kCodecDecode) return cudaGetLastError();
     if ((had_zstd || any_payload) && dst_a) {  // (the standalone inflate entry point stops at the payloads)

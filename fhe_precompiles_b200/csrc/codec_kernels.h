@@ -39,9 +39,5 @@ cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const
 cudaError_t launch_codec_pack(const uint64_t *words, uint8_t *frames, int32_t *constant_flag, const uint8_t *prefix, int n,
                               cudaStream_t s);
 uint64_t codec_launch_count();
-// device zstd inflate: 0 = one warp per frame throughout, 1 = two-phase (thread-per-frame planning + warp-per-frame copies),
-// 2 (default) = batch-oriented (zstd_plan2.h: parse, then the four Huffman streams and the sequence stream of every frame as
-// five concurrent threads, then warp-per-frame copies)
-void codec_set_two_phase(int mode);
 
 }  // namespace fheb

@@ -215,7 +215,7 @@ class Engine {
     bool device_codec_ = true;  // FHE_B200_DEVICE_CODEC=0: tiles decode and encode everything on the host
     bool call_graphs_ = true;   // FHE_B200_CALL_GRAPHS=0: the single-call fast path launches its kernels one by one
     void drop_graphs(Lane *lane);
-    // libzstd-written operand frames inflated on the GPU (zstd_plan2.h): 0 (default) never, 1 always, 2 when a tile brings at
+    // libzstd-written operand frames inflated on the GPU (codec_kernels.cu): 0 never, 1 always, 2 (default) when a tile brings at
     // least device_zstd_min_frames_ of them; host_inflate_pct_ % of those frames are inflated by the host cores meanwhile
     int device_zstd_ = 2;
     size_t device_zstd_min_frames_ = 128, host_inflate_pct_ = 0;

@@ -1,17 +1,18 @@
-// Strict single-frame zstd (RFC 8878) decoder written for the GPU: one sequential decoder per frame, aligned 64-bit loads
-// only, all tables in a caller-provided workspace.  SURVEY 8f-3: the byte surface is bound by the host's libzstd inflate of
-// the two ciphertext operands of every call; with this the compressed frames go over PCIe as they are and are inflated on
-// the device, thousands at a time.
+// Shared parsing layer of the device zstd (RFC 8878) decoder: bit readers, FSE and Huffman table construction, and the
+// literal-length / match-length codes.  zstd_plan2.h (parse, Huffman streams, sequences) and zstd_plan3.cuh / zstd_exec3.h
+// (execution) build the decoder on it.  SURVEY 8f-3: the byte surface is bound by the host's libzstd inflate of the two
+// ciphertext operands of every call; with this the compressed frames go over PCIe as they are and are inflated on the device,
+// thousands at a time.  Aligned word loads only, all tables in a caller-provided workspace.
 //
-// Contract: anything this decoder does not reproduce EXACTLY as libzstd would -- dictionaries, checksums, several frames,
+// Contract: anything the decoder does not reproduce EXACTLY as libzstd would -- dictionaries, checksums, several frames,
 // unknown content size, offsets beyond the window, an over- or under-consumed bitstream, any malformed field -- is reported
 // as kZdFallback and the caller hands that operand to libzstd on the host, whose verdict (payload or error code) is the
 // one returned.  kZdOk therefore always means "byte-identical to libzstd's output".
 //
-// The same source compiles for the host (tests/test_zstd_dec.py drives it through a test hook against libzstd on
-// fixtures, random data at many levels and corrupted frames) and for the device (k_zstd_inflate in kernels.cu).
+// The same source compiles for the host (tests/test_zstd_dec.py drives it through tests/zd_host.cpp against libzstd on
+// fixtures, random data at many levels and corrupted frames) and for the device (codec_kernels.cu).
 // Buffers: `src` must be readable from kPad bytes before to kPad bytes after the frame (the bit readers use aligned
-// 64-bit loads); the padding's content is irrelevant.
+// word loads); the padding's content is irrelevant.
 #pragma once
 #include <cstddef>
 #include <cstdint>
@@ -22,25 +23,9 @@
 #else
 #define ZD_HD inline
 #define ZD_FN inline
-struct uint4 {  // host build: only named in the device-only flush path
-    unsigned x, y, z, w;
+struct uint2 {  // host build: a sequence-table cell as the device loads it (zstd_plan2.h pack_cell)
+    unsigned x, y;
 };
-#endif
-
-// Warp-cooperative execution on the device: all 32 lanes of a warp run the decoder in lockstep on the same frame.  Everything
-// that only READS (headers, bit streams, table lookups) is executed redundantly by every lane (same addresses: broadcast
-// loads); table construction and Huffman decoding are done by lane 0; the byte copies of literals and matches -- the
-// expensive part, a chain of dependent memory round trips when one thread does it -- are split across the lanes.
-#if defined(__CUDA_ARCH__)
-#define ZD_LANE ((int)(threadIdx.x & 31))
-#define ZD_NLANES 32
-#define ZD_SYNC() __syncwarp()
-#define ZD_BCAST(v) __shfl_sync(0xffffffffu, (v), 0)
-#else
-#define ZD_LANE 0
-#define ZD_NLANES 1
-#define ZD_SYNC() ((void)0)
-#define ZD_BCAST(v) (v)
 #endif
 
 namespace fheb {
@@ -65,11 +50,10 @@ struct SeqEntry {  // sequence-table cell with the symbol already translated (li
     uint32_t base_value;  // literal length / match length base, or 1 << offset code
 };
 
-constexpr uint32_t kRingBytes = 4096;  // recent output kept in shared memory on the device (power of two)
 constexpr size_t kSeqTableEntries = 512 + 256 + 512;
 
 struct Work {
-    SeqEntry *ll, *of, *ml;  // the three sequence tables: shared memory on the device, `store` on the host
+    SeqEntry *ll, *of, *ml;  // where seq_table builds the three sequence tables: `store`, or a block's slot (zstd_plan2.h)
     SeqEntry store[kSeqTableEntries];
     FseEntry tmp[512];  // table under construction
     uint16_t huf[1 << kHufLogMax];  // sym | nb << 8
@@ -379,604 +363,8 @@ ZD_FN size_t huf_read_tree(const uint8_t *src, size_t len, Work *w) {
     return used;
 }
 
-// one Huffman stream src[0..len) -> exactly `count` symbols at out; false unless the stream is consumed exactly
-ZD_FN bool huf_stream(const uint8_t *src, size_t len, uint8_t *out, size_t count, const Work *w) {
-    BackBits b;
-    if (!b.init(src, len)) return false;
-    const int log = w->huf_log;
-    const uint32_t mask = (1u << log) - 1;
-    uint32_t state = back_read(b, log);
-    for (size_t i = 0; i < count; i++) {
-        const uint16_t e = w->huf[state];
-        out[i] = (uint8_t)e;
-        const int nb = e >> 8;
-        state = ((state << nb) | back_read(b, nb)) & mask;
-    }
-    return b.pos == -(int64_t)log;
-}
-
-// ---------------------------------------------------------------- blocks
-struct Frame {
-    uint8_t *dst;
-    size_t cap, pos;      // output
-    size_t window;        // Window_Size
-    uint32_t rep[3];
-    // Device only.  `ring` (shared memory) always mirrors the last kRingBytes of output and is where short-range matches
-    // are resolved; output bytes reach global memory in bulk flushes, so the per-sequence warp barriers order shared memory
-    // only.  Invariant: bytes below `flushed` are in global memory, pos - flushed < kFlushChunk at every sequence boundary.
-    uint8_t *ring;
-    size_t flushed;
-};
-constexpr size_t kFlushChunk = 2048;
-constexpr uint32_t kFastBytes = 1024;  // longest literals + match written through the ring alone
-
-// ring -> global for [f->flushed, upto): 16-byte stores where the alignment allows (ring index and global offset agree mod 16)
-ZD_HD void out_flush(Frame *f, size_t upto) {
-    const size_t lo = f->flushed;
-    if (upto > lo) {
-        const size_t a = (lo + 15) & ~(size_t)15, b = upto & ~(size_t)15;
-        if (a < b) {
-            for (size_t x = lo + (size_t)ZD_LANE; x < a; x += ZD_NLANES) f->dst[x] = f->ring[x & (kRingBytes - 1)];
-            for (size_t x = a + 16 * (size_t)ZD_LANE; x < b; x += 16 * ZD_NLANES)
-                *(uint4 *)(f->dst + x) = *(const uint4 *)(f->ring + (x & (kRingBytes - 1)));
-            for (size_t x = b + (size_t)ZD_LANE; x < upto; x += ZD_NLANES) f->dst[x] = f->ring[x & (kRingBytes - 1)];
-        } else {
-            for (size_t x = lo + (size_t)ZD_LANE; x < upto; x += ZD_NLANES) f->dst[x] = f->ring[x & (kRingBytes - 1)];
-        }
-    }
-    ZD_SYNC();
-    f->flushed = upto;
-}
-// a run of `n` bytes at f->pos that does not go through the fast path: value `v` (rle >= 0) or bytes src[0..n)
-ZD_HD void out_run(Frame *f, const uint8_t *src, int rle, size_t n) {
-    if (f->ring) out_flush(f, f->pos);
-    for (size_t k = (size_t)ZD_LANE; k < n; k += ZD_NLANES) {
-        const uint8_t v = rle >= 0 ? (uint8_t)rle : src[k];
-        f->dst[f->pos + k] = v;
-        if (f->ring && n - k <= kRingBytes) f->ring[(f->pos + k) & (kRingBytes - 1)] = v;
-    }
-    ZD_SYNC();
-    f->pos += n;
-    f->flushed = f->pos;
-}
-
-// One sequence: `ll` literals from lit[*lpos..] (or the RLE byte), then `ml` bytes from `offset` back.  The lanes split the bytes.
-ZD_HD bool exec_sequence(Frame *f, const uint8_t *lit, int lit_rle, size_t regen, size_t block_start, size_t block_max, uint32_t ll,
-                         uint32_t ml, uint32_t offset, size_t *lpos_io, size_t *opos_io) {
-    const int lane = ZD_LANE;
-    uint8_t *out = f->dst;
-    uint8_t *ring = f->ring;
-    size_t lpos = *lpos_io, opos = *opos_io;
-    // execute: the lanes split the bytes
-    if (ll > regen - lpos) return false;
-    if ((size_t)ll + ml > f->cap - opos || opos + ll + ml - block_start > block_max) return false;
-    if (offset > opos + ll || offset > f->window) return false;
-    if (ring && ll + ml <= kFastBytes) {
-        // fast path: the sequence is written through the ring only, in one step.  Byte t < ll is a literal; byte ll + k of the
-        // match is byte (k mod offset) of the source period, which is one of this sequence's own literals, a byte the ring
-        // still holds after this sequence's writes, or -- further back -- a byte already flushed to global memory
-        // (pos - flushed < kFlushChunk at every sequence boundary, so everything older than the ring is in `out`).
-        // Slots written never alias slots read: both lie within one ring length.
-        const size_t from = opos + ll - offset, end = opos + ll + ml;
-        for (uint32_t t = (uint32_t)lane; t < ll + ml; t += ZD_NLANES) {
-            uint8_t v;
-            if (t < ll) {
-                v = lit_rle >= 0 ? (uint8_t)lit_rle : lit[lpos + t];
-            } else {
-                const uint32_t k = t - ll;
-                const size_t sidx = from + (offset >= ml ? k : k % offset);
-                if (sidx >= opos) v = lit_rle >= 0 ? (uint8_t)lit_rle : lit[lpos + (sidx - opos)];
-                else if (sidx + kRingBytes >= end) v = ring[sidx & (kRingBytes - 1)];
-                else v = out[sidx];
-            }
-            ring[(opos + t) & (kRingBytes - 1)] = v;
-        }
-        lpos += ll;
-        opos = end;
-        ZD_SYNC();
-        f->pos = opos;
-        if (opos - f->flushed >= kFlushChunk) out_flush(f, f->flushed + ((opos - f->flushed) & ~(kFlushChunk - 1)));
-    } else {
-        // general path (also the host's): everything below pos is in `out`
-        f->pos = opos;
-        out_run(f, lit_rle >= 0 ? nullptr : lit + lpos, lit_rle, ll);
-        lpos += ll;
-        opos += ll;
-        const size_t from = opos - offset;
-        for (uint32_t k = (uint32_t)lane; k < ml; k += ZD_NLANES) {
-            const uint8_t v = out[from + (offset >= ml ? k : k % offset)];
-            out[opos + k] = v;
-            if (ring && ml - k <= kRingBytes) ring[(opos + k) & (kRingBytes - 1)] = v;
-        }
-        ZD_SYNC();
-        opos += ml;
-        f->pos = opos;
-        f->flushed = opos;
-    }
-
-    *lpos_io = lpos;
-    *opos_io = opos;
-    return true;
-}
-
-ZD_FN int compressed_block(const uint8_t *src, size_t len, Frame *f, Work *w, size_t block_max) {
-    if (len < 2) return kZdFallback;
-    // ---- literals section
-    const uint8_t b0 = byte_at(src, 0);
-    const int ltype = b0 & 3, sf = (b0 >> 2) & 3;
-    size_t hdr, regen, comp = 0;
-    int streams = 1;
-    if (ltype < 2) {
-        if (sf == 0 || sf == 2) {
-            hdr = 1;
-            regen = b0 >> 3;
-        } else if (sf == 1) {
-            hdr = 2;
-            regen = (size_t)(le_at(src, 0, 2) >> 4);
-        } else {
-            hdr = 3;
-            regen = (size_t)(le_at(src, 0, 3) >> 4);
-        }
-        if (hdr > len) return kZdFallback;
-        comp = ltype == 0 ? regen : 1;
-    } else {
-        if (sf <= 1) {
-            hdr = 3;
-            const uint32_t v = (uint32_t)le_at(src, 0, 3);
-            regen = (v >> 4) & 0x3FF;
-            comp = v >> 14;
-            streams = sf == 0 ? 1 : 4;
-        } else if (sf == 2) {
-            hdr = 4;
-            const uint32_t v = (uint32_t)le_at(src, 0, 4);
-            regen = (v >> 4) & 0x3FFF;
-            comp = v >> 18;
-            streams = 4;
-        } else {
-            hdr = 5;
-            const uint64_t v = le_at(src, 0, 5);
-            regen = (size_t)((v >> 4) & 0x3FFFF);
-            comp = (size_t)(v >> 22);
-            streams = 4;
-        }
-        if (hdr > len) return kZdFallback;
-    }
-    if (regen > block_max || hdr + comp > len) return kZdFallback;
-    const uint8_t *lit = nullptr;  // literal source: raw bytes inside src, or w->lit
-    int lit_rle = -1;
-    const uint8_t *lsrc = src + hdr;
-    if (ltype == 0) {
-        lit = lsrc;
-    } else if (ltype == 1) {
-        lit_rle = byte_at(lsrc, 0);
-    } else {
-        int ok = 1;
-        if (ZD_LANE == 0) {  // Huffman: table and streams by lane 0
-            size_t used = 0;
-            if (ltype == 2) {
-                used = huf_read_tree(lsrc, comp, w);
-                ok = used != 0;
-            } else {
-                ok = w->have_huf;
-            }
-            const uint8_t *hs = lsrc + used;
-            const size_t hlen = comp - used;
-            if (ok && streams == 1) {
-                ok = huf_stream(hs, hlen, w->lit, regen, w);
-            } else if (ok) {
-                ok = !(hlen < 6 + 4 || regen < 6);  // libzstd: >= 10 bytes and >= 6 literals for four streams
-                const size_t s1 = ok ? (size_t)le_at(hs, 0, 2) : 0, s2 = ok ? (size_t)le_at(hs, 2, 2) : 0, s3 = ok ? (size_t)le_at(hs, 4, 2) : 0;
-                const size_t seg = (regen + 3) / 4;
-                ok = ok && 6 + s1 + s2 + s3 < hlen && 3 * seg <= regen;
-                if (ok) {
-                    const size_t s4 = hlen - 6 - s1 - s2 - s3;
-                    const uint8_t *p = hs + 6;
-                    ok = huf_stream(p, s1, w->lit, seg, w) && huf_stream(p + s1, s2, w->lit + seg, seg, w) &&
-                         huf_stream(p + s1 + s2, s3, w->lit + 2 * seg, seg, w) &&
-                         huf_stream(p + s1 + s2 + s3, s4, w->lit + 3 * seg, regen - 3 * seg, w);
-                }
-            }
-        }
-        ZD_SYNC();
-        ok = ZD_BCAST(ok);
-        if (!ok) return kZdFallback;
-        lit = w->lit;
-    }
-
-    // ---- sequences section
-    const uint8_t *ss = src + hdr + comp;
-    size_t sl = len - hdr - comp;
-    if (sl < 1) return kZdFallback;
-    size_t nseq = byte_at(ss, 0), sh = 1;
-    if (nseq >= 128) {
-        if (nseq == 255) {
-            if (sl < 3) return kZdFallback;
-            nseq = (size_t)le_at(ss, 1, 2) + 0x7F00;
-            sh = 3;
-        } else {
-            if (sl < 2) return kZdFallback;
-            nseq = ((nseq - 128) << 8) + byte_at(ss, 1);
-            sh = 2;
-        }
-    }
-    const int lane = ZD_LANE;
-    size_t lpos = 0;
-    size_t opos = f->pos;
-    const size_t block_start = opos;
-    if (nseq == 0) {
-        if (sl != 1) return kZdFallback;
-    } else {
-        if (sl < sh + 1) return kZdFallback;
-        const uint8_t modes = byte_at(ss, sh);
-        if (modes & 3) return kZdFallback;
-        int tables_end = -1;  // offset of the bitstream, or -1
-        if (lane == 0) {      // table construction by lane 0
-            size_t p = sh + 1;
-            int used = seq_table(modes >> 6, ss + p, sl - p, 0, w);
-            if (used >= 0) {
-                p += (size_t)used;
-                used = seq_table((modes >> 4) & 3, ss + p, sl - p, 1, w);
-            }
-            if (used >= 0) {
-                p += (size_t)used;
-                used = seq_table((modes >> 2) & 3, ss + p, sl - p, 2, w);
-            }
-            if (used >= 0 && p + (size_t)used < sl) tables_end = (int)(p + (size_t)used);
-        }
-        ZD_SYNC();
-        tables_end = ZD_BCAST(tables_end);
-        if (tables_end < 0) return kZdFallback;
-        const size_t p = (size_t)tables_end;
-        BackBits b;
-        if (!b.init(ss + p, sl - p)) return kZdFallback;
-        const SeqEntry *tll = w->ll, *tof = w->of, *tml = w->ml;
-        uint32_t st_ll = back_read(b, w->ll_log), st_of = back_read(b, w->of_log), st_ml = back_read(b, w->ml_log);
-        if (b.pos < 0) return kZdFallback;
-        uint32_t r0 = f->rep[0], r1 = f->rep[1], r2 = f->rep[2];
-        uint8_t *out = f->dst;
-        uint8_t *ring = f->ring;
-        for (size_t i = 0; i < nseq; i++) {
-            const SeqEntry el = tll[st_ll], eo = tof[st_of], em = tml[st_ml];
-            const uint32_t ofv = eo.base_value + back_read(b, eo.add_bits);
-            const uint32_t ml = em.base_value + back_read(b, em.add_bits);
-            const uint32_t ll = el.base_value + back_read(b, el.add_bits);
-            uint32_t offset;
-            if (ofv > 3) {
-                offset = ofv - 3;
-                r2 = r1, r1 = r0, r0 = offset;
-            } else {
-                const uint32_t idx = ofv - 1 + (ll == 0 ? 1 : 0);
-                if (idx == 0) {
-                    offset = r0;
-                } else {
-                    if (idx == 3 && r0 == 1) return kZdFallback;  // offset 0: libzstd patches it up; let it decide
-                    offset = idx == 1 ? r1 : idx == 2 ? r2 : r0 - 1;
-                    if (idx != 1) r2 = r1;
-                    r1 = r0, r0 = offset;
-                }
-            }
-            if (i + 1 < nseq) {
-                st_ll = el.next_base + back_read(b, el.nb);
-                st_ml = em.next_base + back_read(b, em.nb);
-                st_of = eo.next_base + back_read(b, eo.nb);
-            }
-            if (b.pos < 0) return kZdFallback;
-            if (!exec_sequence(f, lit, lit_rle, regen, block_start, block_max, ll, ml, offset, &lpos, &opos)) return kZdFallback;
-        }
-        if (b.pos != 0) return kZdFallback;  // libzstd insists on an exactly consumed stream in recent versions only
-        f->rep[0] = r0, f->rep[1] = r1, f->rep[2] = r2;
-    }
-    // trailing literals
-    const size_t rest = regen - lpos;
-    if (rest > f->cap - opos || opos + rest - block_start > block_max) return kZdFallback;
-    f->pos = opos;
-    out_run(f, lit_rle >= 0 ? nullptr : lit + lpos, lit_rle, rest);
-    return kZdOk;
-}
-
-// One frame src[0..slen) -> dst[0..*dlen).  `cap` bounds the output; the frame must declare its content size.
-ZD_FN int decode_frame(const uint8_t *src, size_t slen, uint8_t *dst, size_t cap, size_t *dlen, Work *w, uint8_t *ring = nullptr) {
-    if (slen < 6 || le_at(src, 0, 4) != 0xFD2FB528ull) return kZdFallback;
-    const uint8_t fhd = byte_at(src, 4);
-    const int fcs_flag = fhd >> 6, single = (fhd >> 5) & 1;
-    if (fhd & 0x1F) return kZdFallback;  // unused / reserved bit, checksum, dictionary: libzstd's business
-    size_t pos = 5;
-    size_t window = 0;
-    if (!single) {
-        if (pos >= slen) return kZdFallback;
-        const uint8_t wd = byte_at(src, pos++);
-        const int wlog = 10 + (wd >> 3);
-        if (wlog > 31) return kZdFallback;
-        window = ((size_t)1 << wlog) + (((size_t)1 << wlog) >> 3) * (wd & 7);
-    }
-    const int fcs_bytes = fcs_flag == 0 ? (single ? 1 : 0) : fcs_flag == 1 ? 2 : fcs_flag == 2 ? 4 : 8;
-    if (fcs_bytes == 0 || pos + (size_t)fcs_bytes > slen) return kZdFallback;  // unknown content size
-    uint64_t fcs = le_at(src, pos, fcs_bytes);
-    if (fcs_bytes == 2) fcs += 256;
-    pos += (size_t)fcs_bytes;
-    if (fcs > cap) return kZdFallback;
-    if (single) window = (size_t)fcs;
-    const size_t block_max = window < kBlockMax ? window : kBlockMax;
-    Frame f{dst, (size_t)fcs, 0, window, {1, 4, 8}, ring, 0};
-    if (ZD_LANE == 0) w->have_ll = w->have_of = w->have_ml = w->have_huf = 0;
-    ZD_SYNC();
-    for (;;) {
-        if (pos + 3 > slen) return kZdFallback;
-        const uint32_t bh = (uint32_t)le_at(src, pos, 3);
-        pos += 3;
-        const int last = bh & 1, type = (bh >> 1) & 3;
-        const size_t bsize = bh >> 3;
-        if (type == 3) return kZdFallback;
-        if (type == 0) {
-            if (bsize > block_max || pos + bsize > slen || bsize > f.cap - f.pos) return kZdFallback;
-            out_run(&f, src + pos, -1, bsize);
-            pos += bsize;
-        } else if (type == 1) {
-            if (bsize > block_max || pos + 1 > slen || bsize > f.cap - f.pos) return kZdFallback;
-            const uint8_t v = byte_at(src, pos);
-            out_run(&f, nullptr, v, bsize);
-            pos += 1;
-        } else {
-            if (bsize > block_max || bsize < 2 || pos + bsize > slen) return kZdFallback;
-            if (compressed_block(src + pos, bsize, &f, w, block_max) != kZdOk) return kZdFallback;
-            pos += bsize;
-        }
-        if (last) break;
-    }
-    if (pos != slen || f.pos != (size_t)fcs) return kZdFallback;
-    *dlen = f.pos;
-    return kZdOk;
-}
-
-// ---------------------------------------------------------------- two-phase decoding (device: many frames in flight)
-// A frame's bitstreams are sequential, so one frame cannot use more than one thread for them -- but 32 frames can share a
-// warp.  Phase 1 (plan_frame, ONE THREAD per frame) walks the frame, decodes Huffman literals and turns every sequence
-// into a packed (literal length, match length, resolved offset) record; phase 2 (execute_plan, one warp per frame) only
-// copies bytes.  Same contract as decode_frame: kZdOk means byte-identical to libzstd, everything else goes back to the host.
-constexpr uint32_t kPlanMaxBlocks = 8;
-constexpr uint32_t kPlanMaxSeqs = 40960;
-
-struct BlockPlan {
-    uint32_t type;        // 0 raw, 1 RLE, 2 compressed
-    uint32_t src_off;     // raw: first byte; RLE: the byte; compressed: raw literals (when lit_in_src)
-    uint32_t size;        // raw / RLE: decompressed size
-    uint32_t lit_off;     // literals in the plan's literal buffer (Huffman) -- or in src (raw literals)
-    uint32_t lit_in_src;
-    int32_t lit_rle;      // >= 0: RLE literals
-    uint32_t regen, nseq, seq_off;
-};
-struct FramePlan {
-    int32_t status;
-    uint32_t nblocks, content, window;
-    BlockPlan blocks[kPlanMaxBlocks];
-};
+// a sequence record: literal length (18 bits) | match length (18) | resolved offset (28)
 ZD_HD uint64_t seq_pack(uint32_t ll, uint32_t ml, uint32_t offset) { return (uint64_t)ll | (uint64_t)ml << 18 | (uint64_t)offset << 36; }
-
-// phase 1.  `lits` holds the Huffman-decoded literals of all blocks (capacity `cap` + 8), `seqs` kPlanMaxSeqs records.
-ZD_FN int plan_frame(const uint8_t *src, size_t slen, size_t cap, Work *w, FramePlan *plan, uint64_t *seqs, uint8_t *lits) {
-    plan->status = kZdFallback;
-    if (slen < 6 || le_at(src, 0, 4) != 0xFD2FB528ull) return kZdFallback;
-    const uint8_t fhd = byte_at(src, 4);
-    const int fcs_flag = fhd >> 6, single = (fhd >> 5) & 1;
-    if (fhd & 0x1F) return kZdFallback;
-    size_t pos = 5, window = 0;
-    if (!single) {
-        if (pos >= slen) return kZdFallback;
-        const uint8_t wd = byte_at(src, pos++);
-        const int wlog = 10 + (wd >> 3);
-        if (wlog > 27) return kZdFallback;
-        window = ((size_t)1 << wlog) + (((size_t)1 << wlog) >> 3) * (wd & 7);
-    }
-    const int fcs_bytes = fcs_flag == 0 ? (single ? 1 : 0) : fcs_flag == 1 ? 2 : fcs_flag == 2 ? 4 : 8;
-    if (fcs_bytes == 0 || pos + (size_t)fcs_bytes > slen) return kZdFallback;
-    uint64_t fcs = le_at(src, pos, fcs_bytes);
-    if (fcs_bytes == 2) fcs += 256;
-    pos += (size_t)fcs_bytes;
-    if (fcs > cap || fcs >= (1u << 27)) return kZdFallback;
-    if (single) window = (size_t)fcs;
-    const size_t block_max = window < kBlockMax ? window : kBlockMax;
-    plan->content = (uint32_t)fcs;
-    plan->window = (uint32_t)(window < (1u << 27) ? window : (1u << 27));
-    w->have_ll = w->have_of = w->have_ml = w->have_huf = 0;
-    uint32_t nblocks = 0, nseq_total = 0, lit_total = 0;
-    uint32_t r0 = 1, r1 = 4, r2 = 8;
-    for (;;) {
-        if (pos + 3 > slen || nblocks >= kPlanMaxBlocks) return kZdFallback;
-        const uint32_t bh = (uint32_t)le_at(src, pos, 3);
-        pos += 3;
-        const int last = bh & 1, type = (bh >> 1) & 3;
-        const size_t bsize = bh >> 3;
-        BlockPlan &bp = plan->blocks[nblocks++];
-        bp.type = (uint32_t)type;
-        if (type == 3 || bsize > block_max) return kZdFallback;
-        if (type == 0) {
-            if (pos + bsize > slen) return kZdFallback;
-            bp.src_off = (uint32_t)pos;
-            bp.size = (uint32_t)bsize;
-            pos += bsize;
-        } else if (type == 1) {
-            if (pos + 1 > slen) return kZdFallback;
-            bp.src_off = (uint32_t)pos;
-            bp.size = (uint32_t)bsize;
-            pos += 1;
-        } else {
-            if (bsize < 2 || pos + bsize > slen) return kZdFallback;
-            const uint8_t *b = src + pos;
-            const size_t len = bsize;
-            // literals section (same grammar as compressed_block)
-            const uint8_t b0 = byte_at(b, 0);
-            const int ltype = b0 & 3, sf = (b0 >> 2) & 3;
-            size_t hdr, regen, comp = 0;
-            int streams = 1;
-            if (ltype < 2) {
-                hdr = (sf == 0 || sf == 2) ? 1 : sf == 1 ? 2 : 3;
-                if (hdr > len) return kZdFallback;
-                regen = hdr == 1 ? (size_t)(b0 >> 3) : (size_t)(le_at(b, 0, (int)hdr) >> 4);
-                comp = ltype == 0 ? regen : 1;
-            } else {
-                hdr = sf <= 1 ? 3 : sf == 2 ? 4 : 5;
-                if (hdr > len) return kZdFallback;
-                const uint64_t v = le_at(b, 0, (int)hdr);
-                const int bits = sf <= 1 ? 10 : sf == 2 ? 14 : 18;
-                regen = (size_t)((v >> 4) & ((1u << bits) - 1));
-                comp = (size_t)(v >> (4 + bits));
-                streams = sf == 0 ? 1 : 4;
-            }
-            if (regen > block_max || hdr + comp > len) return kZdFallback;
-            bp.regen = (uint32_t)regen;
-            bp.lit_rle = -1;
-            bp.lit_in_src = 0;
-            const uint8_t *lsrc = b + hdr;
-            if (ltype == 0) {
-                bp.lit_in_src = 1;
-                bp.lit_off = (uint32_t)(pos + hdr);
-            } else if (ltype == 1) {
-                bp.lit_rle = byte_at(lsrc, 0);
-                bp.lit_off = 0;
-            } else {
-                if ((size_t)lit_total + regen > cap) return kZdFallback;
-                uint8_t *out = lits + lit_total;
-                size_t used = 0;
-                if (ltype == 2) {
-                    used = huf_read_tree(lsrc, comp, w);
-                    if (used == 0) return kZdFallback;
-                } else if (!w->have_huf) {
-                    return kZdFallback;
-                }
-                const uint8_t *hs = lsrc + used;
-                const size_t hlen = comp - used;
-                if (streams == 1) {
-                    if (!huf_stream(hs, hlen, out, regen, w)) return kZdFallback;
-                } else {
-                    if (hlen < 6 + 4 || regen < 6) return kZdFallback;
-                    const size_t s1 = (size_t)le_at(hs, 0, 2), s2 = (size_t)le_at(hs, 2, 2), s3 = (size_t)le_at(hs, 4, 2);
-                    const size_t seg = (regen + 3) / 4;
-                    if (6 + s1 + s2 + s3 >= hlen || 3 * seg > regen) return kZdFallback;
-                    const size_t s4 = hlen - 6 - s1 - s2 - s3;
-                    const uint8_t *q = hs + 6;
-                    if (!huf_stream(q, s1, out, seg, w) || !huf_stream(q + s1, s2, out + seg, seg, w) ||
-                        !huf_stream(q + s1 + s2, s3, out + 2 * seg, seg, w) ||
-                        !huf_stream(q + s1 + s2 + s3, s4, out + 3 * seg, regen - 3 * seg, w))
-                        return kZdFallback;
-                }
-                bp.lit_off = lit_total;
-                lit_total += (uint32_t)regen;
-            }
-            // sequences section
-            const uint8_t *ss = b + hdr + comp;
-            const size_t sl = len - hdr - comp;
-            if (sl < 1) return kZdFallback;
-            size_t nseq = byte_at(ss, 0), sh = 1;
-            if (nseq >= 128) {
-                if (nseq == 255) {
-                    if (sl < 3) return kZdFallback;
-                    nseq = (size_t)le_at(ss, 1, 2) + 0x7F00;
-                    sh = 3;
-                } else {
-                    if (sl < 2) return kZdFallback;
-                    nseq = ((nseq - 128) << 8) + byte_at(ss, 1);
-                    sh = 2;
-                }
-            }
-            bp.nseq = (uint32_t)nseq;
-            bp.seq_off = nseq_total;
-            if (nseq == 0) {
-                if (sl != 1) return kZdFallback;
-            } else {
-                if (nseq_total + nseq > kPlanMaxSeqs || sl < sh + 1) return kZdFallback;
-                const uint8_t modes = byte_at(ss, sh);
-                if (modes & 3) return kZdFallback;
-                size_t p = sh + 1;
-                int used = seq_table(modes >> 6, ss + p, sl - p, 0, w);
-                if (used < 0) return kZdFallback;
-                p += (size_t)used;
-                if ((used = seq_table((modes >> 4) & 3, ss + p, sl - p, 1, w)) < 0) return kZdFallback;
-                p += (size_t)used;
-                if ((used = seq_table((modes >> 2) & 3, ss + p, sl - p, 2, w)) < 0) return kZdFallback;
-                p += (size_t)used;
-                if (p >= sl) return kZdFallback;
-                BackBits bb;
-                if (!bb.init(ss + p, sl - p)) return kZdFallback;
-                const SeqEntry *tll = w->ll, *tof = w->of, *tml = w->ml;
-                uint32_t st_ll = back_read(bb, w->ll_log), st_of = back_read(bb, w->of_log), st_ml = back_read(bb, w->ml_log);
-                if (bb.pos < 0) return kZdFallback;
-                uint64_t *so = seqs + nseq_total;
-                size_t lsum = 0;
-                for (size_t i = 0; i < nseq; i++) {
-                    const SeqEntry el = tll[st_ll], eo = tof[st_of], em = tml[st_ml];
-                    const uint32_t ofv = eo.base_value + back_read(bb, eo.add_bits);
-                    const uint32_t ml = em.base_value + back_read(bb, em.add_bits);
-                    const uint32_t ll = el.base_value + back_read(bb, el.add_bits);
-                    uint32_t offset;
-                    if (ofv > 3) {
-                        offset = ofv - 3;
-                        r2 = r1, r1 = r0, r0 = offset;
-                    } else {
-                        const uint32_t idx = ofv - 1 + (ll == 0 ? 1 : 0);
-                        if (idx == 0) {
-                            offset = r0;
-                        } else {
-                            if (idx == 3 && r0 == 1) return kZdFallback;
-                            offset = idx == 1 ? r1 : idx == 2 ? r2 : r0 - 1;
-                            if (idx != 1) r2 = r1;
-                            r1 = r0, r0 = offset;
-                        }
-                    }
-                    if (i + 1 < nseq) {
-                        st_ll = el.next_base + back_read(bb, el.nb);
-                        st_ml = em.next_base + back_read(bb, em.nb);
-                        st_of = eo.next_base + back_read(bb, eo.nb);
-                    }
-                    lsum += ll;
-                    if (bb.pos < 0 || lsum > regen || offset >= (1u << 27)) return kZdFallback;
-                    so[i] = seq_pack(ll, ml, offset);
-                }
-                if (bb.pos != 0) return kZdFallback;
-                nseq_total += (uint32_t)nseq;
-            }
-            pos += bsize;
-        }
-        if (last) break;
-    }
-    if (pos != slen) return kZdFallback;
-    plan->nblocks = nblocks;
-    plan->status = kZdOk;
-    return kZdOk;
-}
-
-// phase 2 (warp-cooperative on the device, scalar on the host)
-ZD_FN int execute_plan(const uint8_t *src, const FramePlan *plan, const uint64_t *seqs, const uint8_t *lits, uint8_t *dst, size_t *dlen,
-                       uint8_t *ring = nullptr) {
-    if (plan->status != kZdOk) return kZdFallback;
-    const size_t window = plan->window;
-    const size_t block_max = window < kBlockMax ? window : kBlockMax;
-    Frame f{dst, (size_t)plan->content, 0, window, {1, 4, 8}, ring, 0};
-    for (uint32_t bi = 0; bi < plan->nblocks; bi++) {
-        const BlockPlan bp = plan->blocks[bi];
-        if (bp.type != 2) {
-            if (bp.size > f.cap - f.pos) return kZdFallback;
-            out_run(&f, bp.type == 0 ? src + bp.src_off : nullptr, bp.type == 0 ? -1 : (int)byte_at(src, bp.src_off), bp.size);
-            continue;
-        }
-        const uint8_t *lit = bp.lit_in_src ? src + bp.lit_off : lits + bp.lit_off;
-        size_t lpos = 0, opos = f.pos;
-        const size_t block_start = opos;
-        const uint64_t *so = seqs + bp.seq_off;
-        for (uint32_t i = 0; i < bp.nseq; i++) {
-            const uint64_t e = so[i];
-            if (!exec_sequence(&f, lit, bp.lit_rle, bp.regen, block_start, block_max, (uint32_t)(e & 0x3FFFF), (uint32_t)((e >> 18) & 0x3FFFF),
-                               (uint32_t)(e >> 36), &lpos, &opos))
-                return kZdFallback;
-        }
-        const size_t rest = bp.regen - lpos;
-        if (rest > f.cap - opos || opos + rest - block_start > block_max) return kZdFallback;
-        f.pos = opos;
-        out_run(&f, bp.lit_rle >= 0 ? nullptr : lit + lpos, bp.lit_rle, rest);
-    }
-    if (f.pos != (size_t)plan->content) return kZdFallback;
-    *dlen = f.pos;
-    return kZdOk;
-}
 
 }  // namespace zd
 }  // namespace fheb

@@ -1,19 +1,20 @@
-// Batch-oriented zstd inflate (RFC 8878), third generation of the device decoder (see zstd_dec.h for the contract: kZdOk
-// means byte-identical to libzstd, anything else is handed back to the host).
+// Device zstd inflate (RFC 8878) up to the execution of the sequences (see zstd_dec.h for the contract: kZdOk means
+// byte-identical to libzstd, anything else is handed back to the host).
 //
 // A frame's bitstreams are chains of dependent steps -- one GPU thread walks them at ~10x a host core's cost per step -- so
 // throughput comes from (a) thousands of frames in flight and (b) splitting a frame into its INDEPENDENT chains and keeping
 // each chain's inner loop to a few dozen instructions:
 //   parse   one thread per frame   frame / block / section headers, Huffman and FSE table construction (per block, in global
-//                                  scratch), descriptors of every bitstream                                (plan2_parse)
-//   huf     one thread per (frame, Huffman stream): the four literal streams of a block decode concurrently  (plan2_huf)
-//   seq     one thread per frame   FSE sequence streams -> (literal length, match length, resolved offset)   (plan2_seq)
-//   exec    one thread per frame   sequence execution on registers: 64-bit appends, aligned word stores        (plan2_exec)
-// huf and seq are independent of each other and run on two streams.  The bit readers use one aligned 32-bit load per 32 bits
-// consumed and keep the unread bits left-aligned in a 64-bit register; tables are read through the read-only path.
+//                                  scratch), descriptors of every bitstream                      (plan2_parse; k_zd2_parse)
+//   huf     one thread per (frame, Huffman stream): the four literal streams of a block decode concurrently
+//                                                                                                 (plan2_huf; k_zd3_huf)
+//   seq     one lane per frame     FSE sequence chain -> (literal length, match length, resolved offset) records, with the
+//                                  block's tables staged in shared memory                          (seq_block; k_zd3_seq)
+// zstd_plan3.cuh executes the records (k_zd3_exec).  The bit readers use one aligned 32-bit load per 32 bits consumed and keep
+// the unread bits left-aligned in a 64-bit register; the Huffman tables are read through the read-only path.
 //
-// The same source compiles for the host (tests/zd_host.cpp: zd_decode_v2, compared with libzstd on fixtures, many levels and
-// mutated frames) and for the device (codec_kernels.cu).
+// The same source compiles for the host (tests/zd_host.cpp, compared with libzstd on fixtures, many levels and mutated frames)
+// and for the device (codec_kernels.cu).
 #pragma once
 #include "zstd_dec.h"
 
@@ -118,7 +119,7 @@ struct Back32 {
 };
 
 // ---------------------------------------------------------------- parse
-// Everything plan_frame (zstd_dec.h) checks, minus the two hot loops.  `w` is table-construction scratch.
+// Every header and table of the frame, checked; the bitstreams are only located.  `w` is table-construction scratch.
 ZD_FN int plan2_parse(const uint8_t *src, size_t slen, size_t cap, Work *w, Plan2 *plan, Tables2 *tabs) {
     plan->status = kZdFallback;
     plan->seq_bad = 0;
@@ -247,7 +248,7 @@ ZD_FN int plan2_parse(const uint8_t *src, size_t slen, size_t cap, Work *w, Plan
                 }
                 lit_total += (uint32_t)regen;
             }
-            // ---- sequences section: count, table descriptions (built here), then the bitstream (decoded by plan2_seq)
+            // ---- sequences section: count, table descriptions (built here), then the bitstream (decoded by seq_block)
             const uint8_t *ss = b + hdr + comp;
             const size_t sl = len - hdr - comp;
             if (sl < 1) return kZdFallback;
@@ -345,188 +346,171 @@ ZD_FN bool plan2_huf(const uint8_t *src, const Plan2 *plan, const Tables2 *tabs,
 }
 
 // ---------------------------------------------------------------- sequences
-struct Cell2 {
-    uint32_t x, y;  // x = next_base | nb << 16 | add_bits << 24, y = base_value: the bytes of a SeqEntry
-};
+// The FSE sequence chain of a block, as k_zd3_seq runs it (zstd_plan3.cuh seq_frames stages the tables and calls seq_block).
+constexpr int kTabCells = 512 + 256 + 512;  // LL (log <= 9), OF (<= 8), ML (<= 9)
+constexpr int kLutCells = 36 + 53;          // base values of the literal-length and match-length codes (one copy per CTA)
+
+// A table cell in shared memory: next state base (10 bits) | state bits << 10 (4) | value bits << 14 (5) | code << 19 (6).  The
+// value's BASE is a function of the code alone (RFC 8878 3.1.1.3.2.1.1) and is not on the chain that links one sequence to the
+// next - only the bit counts are - so it comes from a small per-CTA table after the fact and a cell is 4 bytes instead of 8.
 static_assert(sizeof(SeqEntry) == 8, "SeqEntry is read as one 8-byte cell");
-ZD_HD Cell2 ld_cell(const SeqEntry *e) {
-#if defined(__CUDA_ARCH__)
-    const uint2 v = __ldg((const uint2 *)e);
-    return Cell2{v.x, v.y};
-#else
-    Cell2 c;
-    c.x = (uint32_t)e->next_base | (uint32_t)e->nb << 16 | (uint32_t)e->add_bits << 24;
-    c.y = e->base_value;
-    return c;
-#endif
-}
-ZD_FN bool plan2_seq(const uint8_t *src, const Plan2 *plan, const Tables2 *tabs, uint64_t *seqs) {
-    if (plan->status != kZdOk) return true;
-    uint32_t r0 = 1, r1 = 4, r2 = 8;
-    for (uint32_t bi = 0; bi < plan->nblocks; bi++) {
-        const Block2 &bp = plan->blocks[bi];
-        if (bp.type != 2 || bp.nseq == 0) continue;
-        Back32 b;
-        if (!b.init(src + bp.bs_off, bp.bs_len)) return false;
-        const SeqEntry *tll = tabs->ll[bp.ll_tab], *tof = tabs->of[bp.of_tab], *tml = tabs->ml[bp.ml_tab];
-        b.refill();
-        uint32_t st_ll = b.read((int)bp.ll_log), st_of = b.read((int)bp.of_log), st_ml = b.read((int)bp.ml_log);
-        if (b.left < 0) return false;
-        uint64_t *so = seqs + bp.seq_off;
-        const uint32_t nseq = bp.nseq, regen = bp.regen;
-        uint64_t lsum = 0;
-        for (uint32_t i = 0; i < nseq; i++) {
-            // a cell is {next_base u16 | nb u8 << 16 | add_bits u8 << 24, base_value u32} (SeqEntry), one 8-byte load each
-            const Cell2 el = ld_cell(tll + st_ll), eo = ld_cell(tof + st_of), em = ld_cell(tml + st_ml);
-            b.refill();
-            const uint32_t ofv = eo.y + b.read((int)(eo.x >> 24));
-            b.refill();
-            const uint32_t ml = em.y + b.read((int)(em.x >> 24));
-            const uint32_t ll = el.y + b.read((int)(el.x >> 24));
-            uint32_t offset;
-            if (ofv > 3) {
-                offset = ofv - 3;
-                r2 = r1, r1 = r0, r0 = offset;
-            } else {
-                const uint32_t idx = ofv - 1 + (ll == 0 ? 1 : 0);
-                if (idx == 0) {
-                    offset = r0;
-                } else {
-                    if (idx == 3 && r0 == 1) return false;  // offset 0: libzstd patches it up; let it decide
-                    offset = idx == 1 ? r1 : idx == 2 ? r2 : r0 - 1;
-                    if (idx != 1) r2 = r1;
-                    r1 = r0, r0 = offset;
-                }
-            }
-            if (i + 1 < nseq) {
-                b.refill();
-                st_ll = (el.x & 0xFFFF) + b.read((int)((el.x >> 16) & 0xFF));
-                st_ml = (em.x & 0xFFFF) + b.read((int)((em.x >> 16) & 0xFF));
-                st_of = (eo.x & 0xFFFF) + b.read((int)((eo.x >> 16) & 0xFF));
-            }
-            lsum += ll;
-            if (b.left < 0 || lsum > regen || offset >= (1u << 27) || ll >= (1u << 18) || ml >= (1u << 18)) return false;
-            so[i] = seq_pack(ll, ml, offset);
-        }
-        if (b.left != 0) return false;
+ZD_HD uint32_t pack_cell(uint2 g, int which) {  // g: a SeqEntry as stored by the parse step
+    const uint32_t next_base = g.x & 0xFFFF, nb = (g.x >> 16) & 0xFF, add = g.x >> 24, base = g.y;
+    uint32_t code;
+    if (which == 1) {
+        code = add;  // offset code: base = 1 << code
+    } else if (which == 0) {
+        code = add == 0 ? base : add == 1 ? 16 + (base - 16) / 2 : add == 2 ? 20 + (base - 24) / 4 : add == 3 ? 22 + (base - 32) / 8
+               : add == 4 ? 24u : add == 6 ? 25u : add + 19;
+    } else {
+        code = add == 0 ? base - 3 : add == 1 ? 32 + (base - 35) / 2 : add == 2 ? 36 + (base - 43) / 4 : add == 3 ? 38 + (base - 51) / 8
+               : add == 4 ? 40 + (base - 67) / 16 : add == 5 ? 42u : add == 7 ? 43u : add + 36;
     }
-    return true;
+    return next_base | nb << 10 | add << 14 | (code & 63) << 19;
 }
 
-// ---------------------------------------------------------------- execution, one THREAD per frame
-// A warp-per-frame executor spends ~1,300 cycles per sequence on a chain of dependent loads, shared-memory round trips and warp
-// barriers (11 ms per ciphertext frame, measured) while 31 of its lanes have next to nothing to copy: a ciphertext's typical
-// sequence is five literal bytes and a three-byte match.  Here one thread keeps the output position, the word being assembled
-// and the previous word in REGISTERS, appends up to eight bytes per step with shifts, and stores aligned 64-bit words; a match
-// whose source lies in the last 8..15 bytes (offset 8: the zero bytes of the previous residue) never touches memory.  Thirty-two
-// frames share a warp, so the batch's frames all run at once.
-struct Sink64 {
-    uint64_t *dst;  // 8-byte aligned; the caller leaves room up to the next multiple of 8 after the content
-    uint64_t acc;   // bytes [pos & ~7, pos) of the word being assembled, low byte first, upper bytes zero
-    uint64_t prev;  // the word before it
-    size_t pos;
-    ZD_HD void put(uint64_t v, int k) {  // appends the k (1..8) low bytes of v; the other bytes of v are zero
-        const int a = (int)(pos & 7);
-        acc |= v << (8 * a);
-        if (a + k >= 8) {
-            dst[pos >> 3] = acc;
-            prev = acc;
-            acc = a ? v >> (8 * (8 - a)) : 0;
+// PTX shifts clamp at 32: a shift by 32 yields 0.  The host must do the same (x86 would shift by n mod 32).
+ZD_HD uint32_t shl32(uint32_t v, uint32_t n) {
+#if defined(__CUDA_ARCH__)
+    uint32_t r;
+    asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
+    return r;
+#else
+    return n >= 32 ? 0u : v << n;
+#endif
+}
+ZD_HD uint32_t shr32(uint32_t v, uint32_t n) {
+#if defined(__CUDA_ARCH__)
+    uint32_t r;
+    asm("shr.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
+    return r;
+#else
+    return n >= 32 ? 0u : v >> n;
+#endif
+}
+
+// backward bit reader on aligned 32-bit words (Back32) with the next word already in a register
+struct Back32P {
+    const uint32_t *wp, *w0;
+    uint32_t lo_bits, nextw, nextmask;  // the prefetched word is masked when it is CONSUMED: nothing waits for the load before
+    uint64_t c;   // unread bits, left-aligned
+    int avail;    // how many of them are valid
+    int left;     // stream bits not yet consumed (negative after an over-read; a stream is < 2^20 bits)
+    ZD_HD void fetch() {
+        nextw = 0, nextmask = 0;
+        if (wp >= w0) {
+            nextw = ZD_LDG32(wp);
+            nextmask = wp == w0 ? ~((1u << lo_bits) - 1) : 0xFFFFFFFFu;
         }
-        pos += (size_t)k;
     }
-    // k (1..8) bytes that are already part of the output, starting at absolute position p (p + k <= pos), upper bytes garbage.
-    // *k is reduced when the range would straddle the flushed / register boundary.
-    ZD_HD uint64_t get(size_t p, int *k) const {
-        const size_t wordpos = pos & ~(size_t)7;
-        if (p + 8 >= wordpos) {  // inside (prev, acc)
-            const unsigned sh = (unsigned)(p + 8 - wordpos) * 8;  // 0..127
-            if (sh == 0) return prev;
-            if (sh < 64) return (prev >> sh) | (acc << (64 - sh));
-            return acc >> (sh - 64);
+    ZD_HD bool init(const uint8_t *base, size_t len) {
+        if (len == 0 || len > (1u << 17)) return false;
+        const uint8_t last = base[len - 1];
+        if (last == 0) return false;
+        const uintptr_t a = (uintptr_t)base;
+        w0 = (const uint32_t *)(a & ~(uintptr_t)3);
+        lo_bits = (uint32_t)(a & 3) * 8;
+        left = (int)(len - 1) * 8 + highbit(last);
+        const uint32_t abs_top = lo_bits + (uint32_t)left;
+        const uint32_t r = abs_top & 31;
+        wp = w0 + (abs_top >> 5);
+        c = 0;
+        avail = 0;
+        if (r) {
+            uint32_t w = ZD_LDG32(wp) & ((1u << r) - 1);
+            if (wp == w0 && lo_bits) w &= ~((1u << lo_bits) - 1);
+            c = (uint64_t)w << (64 - r);
+            avail = (int)r;
         }
-        const size_t room = wordpos - p;  // bytes of the range that are in memory for sure
-        if ((size_t)*k > room) *k = (int)room;
-        const uint64_t *w = dst + (p >> 3);
-        const unsigned sh = (unsigned)(p & 7) * 8;
-        const uint64_t lo = w[0];
-        if (sh == 0) return lo;
-        return (lo >> sh) | (w[1] << (64 - sh));
+        wp--;
+        fetch();
+        return true;
     }
-    ZD_HD void finish() {
-        if (pos & 7) dst[pos >> 3] = acc;
+    ZD_HD void refill() {  // afterwards avail >= 32
+        if (avail < 32) {
+            c |= (uint64_t)(nextw & nextmask) << (32 - avail);
+            avail += 32;
+            wp--;
+            fetch();
+        }
+    }
+    ZD_HD uint32_t read(int n) {  // n in [0, 32], n <= avail
+        const uint32_t v = (uint32_t)((c >> 1) >> (63 - n));
+        c <<= n;
+        avail -= n;
+        left -= n;
+        return v;
     }
 };
-ZD_HD uint64_t low_bytes(uint64_t v, int k) { return k >= 8 ? v : v & ((1ull << (8 * k)) - 1); }
-// n bytes of read-only input at src (any alignment, readable kPad bytes around) appended to the sink
-ZD_HD void sink_copy(Sink64 &o, const uint8_t *src, size_t n) {
-    size_t done = 0;
-    while (done < n) {
-        const int k = n - done < 8 ? (int)(n - done) : 8;
-        o.put(low_bytes(window_at(src + done, 0), k), k);
-        done += (size_t)k;
-    }
-}
-ZD_HD void sink_fill(Sink64 &o, uint8_t v, size_t n) {
-    const uint64_t rep = 0x0101010101010101ull * v;
-    size_t done = 0;
-    while (done < n) {
-        const int k = n - done < 8 ? (int)(n - done) : 8;
-        o.put(low_bytes(rep, k), k);
-        done += (size_t)k;
-    }
-}
 
-ZD_FN int plan2_exec(const uint8_t *src, const Plan2 *plan, const uint64_t *seqs, const uint8_t *lits, uint8_t *dst, size_t *dlen) {
-    if (plan->status != kZdOk || plan->seq_bad || plan->huf_bad[0] || plan->huf_bad[1] || plan->huf_bad[2] || plan->huf_bad[3])
-        return kZdFallback;
-    const size_t window = plan->window, cap = plan->content;
-    const size_t block_max = window < kBlockMax ? window : kBlockMax;
-    Sink64 o{(uint64_t *)dst, 0, 0, 0};
-    for (uint32_t bi = 0; bi < plan->nblocks; bi++) {
-        const Block2 &bp = plan->blocks[bi];
-        if (bp.type != 2) {
-            if (bp.size > cap - o.pos) return kZdFallback;
-            if (bp.type == 0) sink_copy(o, src + bp.src_off, bp.size);
-            else sink_fill(o, byte_at(src, bp.src_off), bp.size);
-            continue;
+// The sequences of one block -> (literal length, match length, resolved offset) records at `so`, and the block's verdict.  The
+// per-sequence checks are monotone (bits left, literal total) or independent of the other sequences (value ranges), so they are
+// accumulated and judged once after the loop; a sequence whose six bit fields fit the 32 bits a single refill guarantees - all
+// but a handful - takes them from one register.  The repeat offsets r0_, r1_, r2_ carry over from one block to the next.
+ZD_HD bool seq_block(const uint8_t *src, const Block2 &bp, const uint32_t *tll, const uint32_t *tof, const uint32_t *tml,
+                     const uint32_t *lut, uint64_t *so, uint32_t &r0_, uint32_t &r1_, uint32_t &r2_) {
+    Back32P b;
+    if (!b.init(src + bp.bs_off, bp.bs_len)) return false;
+    b.refill();
+    uint32_t st_ll = b.read((int)bp.ll_log), st_of = b.read((int)bp.of_log), st_ml = b.read((int)bp.ml_log);
+    if (b.left < 0) return false;
+    const uint32_t nseq = bp.nseq, regen = bp.regen;
+    uint32_t r0 = r0_, r1 = r1_, r2 = r2_;
+    uint32_t lsum = 0, badacc = 0;  // (lsum: < 2^18 per term, < 2^16 terms)
+    for (uint32_t i = 0; i < nseq; i++) {
+        const uint32_t el = tll[st_ll], eo = tof[st_of], em = tml[st_ml];
+        const uint32_t keep = i + 1 < nseq ? 0xFu : 0u;  // the last sequence reads no state bits
+        const uint32_t a_of = (eo >> 14) & 31, a_ml = (em >> 14) & 31, a_ll = (el >> 14) & 31;
+        const uint32_t n_ll = (el >> 10) & keep, n_ml = (em >> 10) & keep, n_of = (eo >> 10) & keep;
+        const uint32_t s1 = a_of + a_ml, s2 = s1 + a_ll, s3 = s2 + n_ll, s4 = s3 + n_ml, tot = s4 + n_of;
+        uint32_t x_of, x_ml, x_ll, y_ll, y_ml, y_of;
+        b.refill();
+        if (tot <= 32) {
+            const uint32_t hi = (uint32_t)(b.c >> 32);
+            x_of = shr32(hi, 32 - a_of);
+            x_ml = shr32(shl32(hi, a_of), 32 - a_ml);
+            x_ll = shr32(shl32(hi, s1), 32 - a_ll);
+            y_ll = shr32(shl32(hi, s2), 32 - n_ll);
+            y_ml = shr32(shl32(hi, s3), 32 - n_ml);
+            y_of = shr32(shl32(hi, s4), 32 - n_of);
+            b.c <<= tot;
+            b.avail -= (int)tot;
+            b.left -= (int)tot;
+        } else {
+            x_of = b.read((int)a_of);
+            b.refill();
+            x_ml = b.read((int)a_ml);
+            x_ll = b.read((int)a_ll);
+            b.refill();
+            y_ll = b.read((int)n_ll);
+            y_ml = b.read((int)n_ml);
+            y_of = b.read((int)n_of);
         }
-        const uint8_t *lit = bp.lit_mode == 0 ? src + bp.lit_off : lits + bp.lit_off;
-        const int lit_rle = bp.lit_mode == 1 ? bp.lit_rle : -1;
-        size_t lpos = 0;
-        const size_t block_start = o.pos, regen = bp.regen;
-        const uint64_t *so = seqs + bp.seq_off;
-        for (uint32_t i = 0; i < bp.nseq; i++) {
-#if defined(__CUDA_ARCH__)
-            const uint64_t e = __ldg((const unsigned long long *)(so + i));
-#else
-            const uint64_t e = so[i];
-#endif
-            const uint32_t ll = (uint32_t)(e & 0x3FFFF), ml = (uint32_t)((e >> 18) & 0x3FFFF), offset = (uint32_t)(e >> 36);
-            if (ll > regen - lpos) return kZdFallback;
-            if ((size_t)ll + ml > cap - o.pos || o.pos + ll + ml - block_start > block_max) return kZdFallback;
-            if (offset > o.pos + ll || offset > window || offset == 0) return kZdFallback;
-            if (lit_rle >= 0) sink_fill(o, (uint8_t)lit_rle, ll);
-            else sink_copy(o, lit + lpos, ll);
-            lpos += ll;
-            uint32_t rest = ml;
-            while (rest) {
-                int k = rest < 8 ? (int)rest : 8;
-                if ((uint32_t)k > offset) k = (int)offset;  // an overlapping match repeats its own output: at most one period per step
-                const uint64_t v = o.get(o.pos - offset, &k);
-                o.put(low_bytes(v, k), k);
-                rest -= (uint32_t)k;
+        st_ll = (el & 0x3FF) + y_ll;
+        st_ml = (em & 0x3FF) + y_ml;
+        st_of = (eo & 0x3FF) + y_of;
+        const uint32_t ofv = (1u << a_of) + x_of, ml = lut[36 + (em >> 19)] + x_ml, ll = lut[el >> 19] + x_ll;
+        uint32_t offset;
+        if (ofv > 3) {
+            offset = ofv - 3;
+            r2 = r1, r1 = r0, r0 = offset;
+        } else {
+            const uint32_t idx = ofv - 1 + (ll == 0 ? 1 : 0);
+            if (idx == 0) {
+                offset = r0;
+            } else {
+                if (idx == 3 && r0 == 1) return false;  // offset 0: libzstd patches it up; let it decide
+                offset = idx == 1 ? r1 : idx == 2 ? r2 : r0 - 1;
+                if (idx != 1) r2 = r1;
+                r1 = r0, r0 = offset;
             }
         }
-        const size_t tail = regen - lpos;
-        if (tail > cap - o.pos || o.pos + tail - block_start > block_max) return kZdFallback;
-        if (lit_rle >= 0) sink_fill(o, (uint8_t)lit_rle, tail);
-        else sink_copy(o, lit + lpos, tail);
+        lsum += ll;
+        badacc |= (offset >> 27) | ((ll | ml) >> 18) | (lsum >> 30);
+        so[i] = seq_pack(ll & 0x3FFFF, ml & 0x3FFFF, offset);
     }
-    if (o.pos != cap) return kZdFallback;
-    o.finish();
-    *dlen = o.pos;
-    return kZdOk;
+    r0_ = r0, r1_ = r1, r2_ = r2;
+    return b.left == 0 && badacc == 0 && lsum <= regen;
 }
 
 }  // namespace zd

@@ -1,21 +1,21 @@
-// Device zstd inflate, fourth generation (device-only; same contract as zstd_dec.h / zstd_plan2.h: kJobOk means byte-identical
-// to libzstd, everything else goes back to the host).
+// Device zstd inflate: the sequence chains and the execution, after zstd_plan2.h's parse and Huffman steps (device-only; same
+// contract as zstd_dec.h: kJobOk means byte-identical to libzstd, everything else goes back to the host).
 //
-// What the third generation (zstd_plan2.h) left on the table, measured on level-3 ciphertext frames (raw literals, 16,354
-// sequences of ~4 literal + ~4 match bytes, three 512/256/512-cell FSE tables per frame):
-//   * the sequence chain read its FSE tables from global memory at 0.5 MB per lane stride (three dependent L2 round trips per
-//     sequence) with 32 frames diverging inside one warp;
-//   * execution was one THREAD per frame: 16 k sequences one after the other although only the match copies depend on each other.
+// Measured on level-3 ciphertext frames (raw literals, 16,354 sequences of ~4 literal + ~4 match bytes, three 512/256/512-cell
+// FSE tables per frame), a thread per frame for both steps (profiles/r2_codec.md) leaves two things on the table:
+//   * a sequence chain that reads its FSE tables from global memory at 0.5 MB per lane stride makes three dependent L2 round
+//     trips per sequence, with 32 frames diverging inside one warp;
+//   * execution by one THREAD per frame runs 16 k sequences one after the other although only the match copies depend on each other.
 // Here:
 //   k_zd3_seq   four frames per warp (a one-lane warp costs as many issue slots as a full one, and shared memory - 5 KB of FSE
 //               tables per frame as 4-byte cells - bounds the frames per SM either way): each frame's tables are staged in shared
 //               memory, the bit reader keeps the next stream word prefetched, a sequence's six bit fields come out of one register
+//               (zstd_plan2.h seq_block)
 //   k_zd3_exec  one CTA (1,024 threads) per frame, the frame's output assembled in shared memory: prefix sums give every
 //               sequence its literal and output positions, literals are copied in parallel, pointer jumping moves every match's
 //               source back along its chain of pending matches (zstd_exec3.h), and the copies go through a per-byte "pending"
 //               bitmap (a match is copied once none of its source bytes is pending; dependencies point backwards only, so the
 //               earliest pending match is always ready); the payload leaves with 16-byte stores
-// Parsing (headers, table construction) and the Huffman streams stay zstd_plan2.h's plan2_parse / plan2_huf.
 #pragma once
 #include "codec_kernels.h"
 #include "zstd_plan2.h"
@@ -27,172 +27,17 @@ using zd::Block2;
 using zd::Plan2;
 using zd::Tables2;
 
-constexpr int kSeqFrames = 4;                        // frames per warp of k_zd3_seq: lanes 0, 8, 16, 24 walk one chain each
-constexpr int kTabCells = 512 + 256 + 512;           // LL (log <= 9), OF (<= 8), ML (<= 9)
-constexpr int kLutCells = 36 + 53;                   // base values of the literal-length and match-length codes (one copy per CTA)
-constexpr size_t kSeqSmem = ((size_t)kSeqFrames * kTabCells + kLutCells) * sizeof(uint32_t);  // 20.4 KB per one-warp CTA: 11 CTAs per SM
-
-// A table cell in shared memory: next state base (10 bits) | state bits << 10 (4) | value bits << 14 (5) | code << 19 (6).  The
-// value's BASE is a function of the code alone (RFC 8878 3.1.1.3.2.1.1) and is not on the chain that links one sequence to the
-// next - only the bit counts are - so it comes from a small per-CTA table after the fact and a cell is 4 bytes instead of 8.
-__device__ __forceinline__ uint32_t pack_cell(uint2 g, int which) {  // g: a SeqEntry as stored by the parse step
-    const uint32_t next_base = g.x & 0xFFFF, nb = (g.x >> 16) & 0xFF, add = g.x >> 24, base = g.y;
-    uint32_t code;
-    if (which == 1) {
-        code = add;  // offset code: base = 1 << code
-    } else if (which == 0) {
-        code = add == 0 ? base : add == 1 ? 16 + (base - 16) / 2 : add == 2 ? 20 + (base - 24) / 4 : add == 3 ? 22 + (base - 32) / 8
-               : add == 4 ? 24u : add == 6 ? 25u : add + 19;
-    } else {
-        code = add == 0 ? base - 3 : add == 1 ? 32 + (base - 35) / 2 : add == 2 ? 36 + (base - 43) / 4 : add == 3 ? 38 + (base - 51) / 8
-               : add == 4 ? 40 + (base - 67) / 16 : add == 5 ? 42u : add == 7 ? 43u : add + 36;
-    }
-    return next_base | nb << 10 | add << 14 | (code & 63) << 19;
-}
-
-__device__ __forceinline__ uint32_t shl32(uint32_t v, uint32_t n) {  // PTX shifts clamp at 32: a shift by 32 yields 0
-    uint32_t r;
-    asm("shl.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
-    return r;
-}
-__device__ __forceinline__ uint32_t shr32(uint32_t v, uint32_t n) {
-    uint32_t r;
-    asm("shr.b32 %0, %1, %2;" : "=r"(r) : "r"(v), "r"(n));
-    return r;
-}
-
-// backward bit reader on aligned 32-bit words (zstd_plan2.h Back32) with the next word already in a register
-struct Back32P {
-    const uint32_t *wp, *w0;
-    uint32_t lo_bits, nextw, nextmask;  // the prefetched word is masked when it is CONSUMED: nothing waits for the load before
-    uint64_t c;   // unread bits, left-aligned
-    int avail;    // how many of them are valid
-    int left;     // stream bits not yet consumed (negative after an over-read; a stream is < 2^20 bits)
-    __device__ __forceinline__ void fetch() {
-        nextw = 0, nextmask = 0;
-        if (wp >= w0) {
-            nextw = __ldg(wp);
-            nextmask = wp == w0 ? ~((1u << lo_bits) - 1) : 0xFFFFFFFFu;
-        }
-    }
-    __device__ __forceinline__ bool init(const uint8_t *base, size_t len) {
-        if (len == 0 || len > (1u << 17)) return false;
-        const uint8_t last = base[len - 1];
-        if (last == 0) return false;
-        const uintptr_t a = (uintptr_t)base;
-        w0 = (const uint32_t *)(a & ~(uintptr_t)3);
-        lo_bits = (uint32_t)(a & 3) * 8;
-        left = (int)(len - 1) * 8 + (31 - __clz((int)last));
-        const uint32_t abs_top = lo_bits + (uint32_t)left;
-        const uint32_t r = abs_top & 31;
-        wp = w0 + (abs_top >> 5);
-        c = 0;
-        avail = 0;
-        if (r) {
-            uint32_t w = __ldg(wp) & ((1u << r) - 1);
-            if (wp == w0 && lo_bits) w &= ~((1u << lo_bits) - 1);
-            c = (uint64_t)w << (64 - r);
-            avail = (int)r;
-        }
-        wp--;
-        fetch();
-        return true;
-    }
-    __device__ __forceinline__ void refill() {  // afterwards avail >= 32
-        if (avail < 32) {
-            c |= (uint64_t)(nextw & nextmask) << (32 - avail);
-            avail += 32;
-            wp--;
-            fetch();
-        }
-    }
-    __device__ __forceinline__ uint32_t read(int n) {  // n in [0, 32], n <= avail
-        const uint32_t v = (uint32_t)((c >> 1) >> (63 - n));
-        c <<= n;
-        avail -= n;
-        left -= n;
-        return v;
-    }
-};
-
-// The sequences of one block: plan2_seq's results and verdict.  Its per-sequence checks are monotone (bits left, literal
-// total) or independent of the other sequences (value ranges), so they are accumulated and judged once after the loop; a
-// sequence whose six bit fields fit the 32 bits a single refill guarantees - all but a handful - takes them from one register.
-__device__ __forceinline__ bool seq_block(const uint8_t *src, const Block2 &bp, const uint32_t *tll, const uint32_t *tof,
-                                          const uint32_t *tml, const uint32_t *lut, uint64_t *so, uint32_t &r0_, uint32_t &r1_,
-                                          uint32_t &r2_) {
-    Back32P b;
-    if (!b.init(src + bp.bs_off, bp.bs_len)) return false;
-    b.refill();
-    uint32_t st_ll = b.read((int)bp.ll_log), st_of = b.read((int)bp.of_log), st_ml = b.read((int)bp.ml_log);
-    if (b.left < 0) return false;
-    const uint32_t nseq = bp.nseq, regen = bp.regen;
-    uint32_t r0 = r0_, r1 = r1_, r2 = r2_;
-    uint32_t lsum = 0, badacc = 0;  // (lsum: < 2^18 per term, < 2^16 terms)
-    for (uint32_t i = 0; i < nseq; i++) {
-        const uint32_t el = tll[st_ll], eo = tof[st_of], em = tml[st_ml];
-        const uint32_t keep = i + 1 < nseq ? 0xFu : 0u;  // the last sequence reads no state bits
-        const uint32_t a_of = (eo >> 14) & 31, a_ml = (em >> 14) & 31, a_ll = (el >> 14) & 31;
-        const uint32_t n_ll = (el >> 10) & keep, n_ml = (em >> 10) & keep, n_of = (eo >> 10) & keep;
-        const uint32_t s1 = a_of + a_ml, s2 = s1 + a_ll, s3 = s2 + n_ll, s4 = s3 + n_ml, tot = s4 + n_of;
-        uint32_t x_of, x_ml, x_ll, y_ll, y_ml, y_of;
-        b.refill();
-        if (tot <= 32) {
-            const uint32_t hi = (uint32_t)(b.c >> 32);
-            x_of = shr32(hi, 32 - a_of);
-            x_ml = shr32(shl32(hi, a_of), 32 - a_ml);
-            x_ll = shr32(shl32(hi, s1), 32 - a_ll);
-            y_ll = shr32(shl32(hi, s2), 32 - n_ll);
-            y_ml = shr32(shl32(hi, s3), 32 - n_ml);
-            y_of = shr32(shl32(hi, s4), 32 - n_of);
-            b.c <<= tot;
-            b.avail -= (int)tot;
-            b.left -= (int)tot;
-        } else {
-            x_of = b.read((int)a_of);
-            b.refill();
-            x_ml = b.read((int)a_ml);
-            x_ll = b.read((int)a_ll);
-            b.refill();
-            y_ll = b.read((int)n_ll);
-            y_ml = b.read((int)n_ml);
-            y_of = b.read((int)n_of);
-        }
-        st_ll = (el & 0x3FF) + y_ll;
-        st_ml = (em & 0x3FF) + y_ml;
-        st_of = (eo & 0x3FF) + y_of;
-        const uint32_t ofv = (1u << a_of) + x_of, ml = lut[36 + (em >> 19)] + x_ml, ll = lut[el >> 19] + x_ll;
-        uint32_t offset;
-        if (ofv > 3) {
-            offset = ofv - 3;
-            r2 = r1, r1 = r0, r0 = offset;
-        } else {
-            const uint32_t idx = ofv - 1 + (ll == 0 ? 1 : 0);
-            if (idx == 0) {
-                offset = r0;
-            } else {
-                if (idx == 3 && r0 == 1) return false;  // offset 0: libzstd patches it up; let it decide
-                offset = idx == 1 ? r1 : idx == 2 ? r2 : r0 - 1;
-                if (idx != 1) r2 = r1;
-                r1 = r0, r0 = offset;
-            }
-        }
-        lsum += ll;
-        badacc |= (offset >> 27) | ((ll | ml) >> 18) | (lsum >> 30);
-        so[i] = zd::seq_pack(ll & 0x3FFFF, ml & 0x3FFFF, offset);
-    }
-    r0_ = r0, r1_ = r1, r2_ = r2;
-    return b.left == 0 && badacc == 0 && lsum <= regen;
-}
+constexpr int kSeqFrames = 4;  // frames per warp of k_zd3_seq: lanes 0, 8, 16, 24 walk one chain each
+constexpr size_t kSeqSmem = ((size_t)kSeqFrames * zd::kTabCells + zd::kLutCells) * sizeof(uint32_t);  // 20.4 KB per one-warp CTA: 11 CTAs per SM
 
 // One warp, up to kSeqFrames frames: slot s = lane / 8; its eight lanes stage the block's tables, lane 8 s walks the chain.
-// `tabs_smem`: kSeqFrames x kTabCells cells.  Returns the slot's verdict to its eight lanes.
+// `tabs_smem`: kSeqFrames x kTabCells cells, then the kLutCells base values.  Returns the slot's verdict to its eight lanes.
 __device__ __forceinline__ bool seq_frames(const uint8_t *src, const Plan2 *plan, const Tables2 *tabs, uint64_t *seqs, bool have,
                                            uint32_t *tabs_smem) {
     const int lane = threadIdx.x & 31, sub = lane & 7;
-    uint32_t *T = tabs_smem + (size_t)(lane >> 3) * kTabCells;
-    uint32_t *lut = tabs_smem + (size_t)kSeqFrames * kTabCells;
-    for (int c = lane; c < kLutCells; c += 32) lut[c] = c < 36 ? zd::ll_base(c) : zd::ml_base(c - 36);
+    uint32_t *T = tabs_smem + (size_t)(lane >> 3) * zd::kTabCells;
+    uint32_t *lut = tabs_smem + (size_t)kSeqFrames * zd::kTabCells;
+    for (int c = lane; c < zd::kLutCells; c += 32) lut[c] = c < 36 ? zd::ll_base(c) : zd::ml_base(c - 36);
     uint32_t r0 = 1, r1 = 4, r2 = 8;
     bool ok = have;
     for (uint32_t bi = 0; bi < zd::kP2MaxBlocks; bi++) {
@@ -205,13 +50,13 @@ __device__ __forceinline__ bool seq_frames(const uint8_t *src, const Plan2 *plan
             } else {
                 const uint2 *gll = (const uint2 *)tabs->ll[bp->ll_tab], *gof = (const uint2 *)tabs->of[bp->of_tab],
                             *gml = (const uint2 *)tabs->ml[bp->ml_tab];
-                for (uint32_t k = sub; k < (1u << bp->ll_log); k += 8) T[k] = pack_cell(__ldg(gll + k), 0);
-                for (uint32_t k = sub; k < (1u << bp->of_log); k += 8) T[512 + k] = pack_cell(__ldg(gof + k), 1);
-                for (uint32_t k = sub; k < (1u << bp->ml_log); k += 8) T[768 + k] = pack_cell(__ldg(gml + k), 2);
+                for (uint32_t k = sub; k < (1u << bp->ll_log); k += 8) T[k] = zd::pack_cell(__ldg(gll + k), 0);
+                for (uint32_t k = sub; k < (1u << bp->of_log); k += 8) T[512 + k] = zd::pack_cell(__ldg(gof + k), 1);
+                for (uint32_t k = sub; k < (1u << bp->ml_log); k += 8) T[768 + k] = zd::pack_cell(__ldg(gml + k), 2);
             }
         }
         __syncwarp();
-        if (run && ok && sub == 0) ok = seq_block(src, *bp, T, T + 512, T + 768, lut, seqs + bp->seq_off, r0, r1, r2);
+        if (run && ok && sub == 0) ok = zd::seq_block(src, *bp, T, T + 512, T + 768, lut, seqs + bp->seq_off, r0, r1, r2);
         ok = __shfl_sync(0xFFFFFFFFu, (int)ok, lane & ~7) != 0;
     }
     return ok;

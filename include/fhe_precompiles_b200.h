@@ -246,11 +246,12 @@ int32_t fhe_b200_write_ciphertext(const uint64_t *words, const char *data_type, 
  * 0 uses libcrypto's when the machine has it.  Exposed so that tests can pin both against a known-good SHA-512. */
 void fhe_b200_sha512(const uint8_t *bytes, size_t len, int32_t portable, uint8_t out[64]);
 int32_t fhe_b200_set_zstd_writer(int32_t mode);
-/* Device-side zstd inflate of n ciphertext-payload frames (codec_kernels.cu, zstd_dec.h): what fhe_b200_batch uses for the
- * operands of a tile.  frames[i] / lens[i] are host buffers; `out` receives n payloads of 131,169 bytes; status[i] = 1 when
- * the frame was inflated (byte-identical to libzstd), 2 when the strict decoder hands it back to the host (unsupported
- * feature, malformed frame, or content that is not a 131,169-byte payload).  The batch surface additionally
- * checks the 97-byte prefix and every residue (k_ct_unpack); this entry point stops at the payload bytes.  elapsed_ms: kernels only. */
+/* Device-side zstd inflate of n ciphertext-payload frames (codec_kernels.cu: k_zd2_parse, k_zd3_huf, k_zd3_seq, k_zd3_exec):
+ * what fhe_b200_batch uses for the operands of a tile.  frames[i] / lens[i] are host buffers; `out` receives n payloads of
+ * 131,169 bytes; status[i] = 1 when the frame was inflated (byte-identical to libzstd), 2 when the strict decoder hands it
+ * back to the host (unsupported feature, malformed frame, or content that is not a 131,169-byte payload).  The batch surface
+ * additionally checks the 97-byte prefix and every residue (k_ct_unpack); this entry point stops at the payload bytes.
+ * elapsed_ms: kernels only. */
 int32_t fhe_b200_zstd_inflate(int32_t device, const uint8_t *const *frames, const size_t *lens, size_t n, uint8_t *out,
                               int32_t *status, float *elapsed_ms);
 void fhe_b200_parms_id(int32_t which, uint64_t out[4]);

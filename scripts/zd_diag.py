@@ -1,4 +1,5 @@
-"""Device zstd inflate timing: batch-oriented pipeline (FHE_B200_ZSTD_TWO_PHASE=2, default), two-phase (1), one warp per frame (0)."""
+"""Device zstd inflate timing (fhe_b200_zstd_inflate): ciphertext, text and structured frames, and batches of 32 to 8,192
+level-3 ciphertext frames."""
 import os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -17,12 +18,9 @@ p = ct()
 cts = [ct() for _ in range(16)]
 frs = [z.compress(c, 3) for c in cts]
 t = bytes(rng.choice(list(b"abcdefgh \n"), size=Z.PAYLOAD).astype(np.uint8))
-for mode in (sys.argv[1:] or ("3", "2", "1", "0")):
-    os.environ["FHE_B200_ZSTD_TWO_PHASE"] = mode
-    print("two_phase =", mode)
-    run("warm", [frs[0]], [cts[0]])
-    run("ct_l3 x1", [frs[0]], [cts[0]])
-    run("text_l3 x1", [z.compress(t, 3)], [t])
-    run("structured x1", [F.zstd_structured_frame(cts[0])], [cts[0]])
-    for n in (32, 256, 1024, 4096, 8192) if mode != "0" else (32, 1024):
-        run(f"ct_l3 x{n}", [frs[i % 16] for i in range(n)], [cts[i % 16] for i in range(n)])
+run("warm", [frs[0]], [cts[0]])
+run("ct_l3 x1", [frs[0]], [cts[0]])
+run("text_l3 x1", [z.compress(t, 3)], [t])
+run("structured x1", [F.zstd_structured_frame(cts[0])], [cts[0]])
+for n in (32, 256, 1024, 4096, 8192):
+    run(f"ct_l3 x{n}", [frs[i % 16] for i in range(n)], [cts[i % 16] for i in range(n)])

@@ -1,4 +1,4 @@
-"""Device zstd inflate (k_zstd_inflate) against libzstd: ciphertext-payload-sized frames of several kinds and levels,
+"""Device zstd inflate (fhe_b200_zstd_inflate) against libzstd: ciphertext-payload-sized frames of several kinds and levels,
 corrupted frames, and the kernel's throughput.  Needs a GPU."""
 import ctypes
 import json

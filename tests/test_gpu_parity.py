@@ -339,17 +339,15 @@ def test_batch_tiles_equal_single_calls(keys):
     assert all(got[k] == want[i] for k, i in enumerate(order))
 
 
-@pytest.mark.parametrize("two_phase", ["0", "1", "2", "3"])
-def test_device_zstd_inflate_matches_libzstd(dev, two_phase, monkeypatch):
-    """k_zstd_inflate (0) / k_zstd_plan + k_zstd_execute (1) / k_zd2_parse + k_zd2_decode + k_zd2_exec (2) / k_zd2_parse + k_zd3_seq + k_zd3_exec (3, the default; csrc/zstd_dec.h
-    and zstd_plan2.h on the device): ciphertext-payload frames written by libzstd at several levels, by the
-    structured writer, other content of the same size (Huffman literals, RLE, raw blocks) and corrupted frames. A frame the
-    device accepts must be byte-identical to libzstd's output; everything else must be handed back (status 2)."""
+def test_device_zstd_inflate_matches_libzstd(dev):
+    """The device zstd decoder (k_zd2_parse, k_zd3_huf, k_zd3_seq, k_zd3_exec): ciphertext-payload frames written by libzstd
+    at several levels, by the structured writer, other content of the same size (Huffman literals, RLE, raw blocks) and
+    corrupted frames. A frame the device accepts must be byte-identical to libzstd's output; everything else must be handed
+    back (status 2)."""
     import ctypes
 
     from fhe_precompiles_b200 import _lib
 
-    monkeypatch.setenv("FHE_B200_ZSTD_TWO_PHASE", two_phase)  # read by the entry point on every call
     L = _lib.lib()
     z = F.zstd()
     rng = np.random.default_rng(2024)

@@ -1,7 +1,7 @@
-"""The device zstd decoder's source (csrc/zstd_dec.h), built for the host, against libzstd: every fixture blob of the
-reference (written by SEAL's bundled zstd 1.4.x, including Huffman, treeless and repeat-mode blocks), random data of many
-shapes at many levels, structured frames, and mutated frames.  Contract under test: status 0 => bytes identical to libzstd's;
-anything else is a hand-back to the host (status 1), never a wrong answer.  CPU only."""
+"""The device zstd decoder's source (csrc/zstd_dec.h, zstd_plan2.h, zstd_exec3.h), built for the host by tests/zd_host.cpp,
+against libzstd: every fixture blob of the reference (written by SEAL's bundled zstd 1.4.x, including Huffman, treeless and
+repeat-mode blocks), random data of many shapes at many levels, structured frames, and mutated frames.  Contract under test:
+status 0 => bytes identical to libzstd's; anything else is a hand-back to the host (status 1), never a wrong answer.  CPU only."""
 import ctypes
 import os
 import subprocess
@@ -14,7 +14,7 @@ from oracle import formats as F
 
 
 @pytest.fixture(scope="module")
-def zd_lib(tmp_path_factory):
+def zd(tmp_path_factory):
     out = tmp_path_factory.mktemp("zd") / "libzd_host.so"
     src = os.path.join(ROOT, "tests", "zd_host.cpp")
     inc = os.path.join(ROOT, "fhe_precompiles_b200", "csrc")
@@ -22,38 +22,19 @@ def zd_lib(tmp_path_factory):
     lib = ctypes.CDLL(str(out))
     cap = 1 << 21
     buf = ctypes.create_string_buffer(cap)
+    fn = lib.zd_decode
+    fn.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t),
+                   ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_long)]
 
-    def make(fn):
-        fn.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]
+    def decode(frame: bytes):
+        n, rounds, polls = ctypes.c_size_t(), ctypes.c_int(), ctypes.c_long()
+        rc = fn(frame, len(frame), buf, cap, ctypes.byref(n), ctypes.byref(rounds), ctypes.byref(polls))
+        assert rc != 2, "the parallel executor's copy phase stopped making progress"
+        decode.rounds, decode.polls = rounds.value, polls.value
+        return rc, (buf.raw[: n.value] if rc == 0 else None)
 
-        def decode(frame: bytes):
-            n = ctypes.c_size_t()
-            rc = fn(frame, len(frame), buf, cap, ctypes.byref(n))
-            return rc, (buf.raw[: n.value] if rc == 0 else None)
-
-        return decode
-
-    def make_v3():
-        fn = lib.zd_decode_v3
-        fn.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t),
-                       ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_long)]
-
-        def decode(frame: bytes):
-            n, rounds, polls = ctypes.c_size_t(), ctypes.c_int(), ctypes.c_long()
-            rc = fn(frame, len(frame), buf, cap, ctypes.byref(n), ctypes.byref(rounds), ctypes.byref(polls))
-            assert rc != 2, "the parallel executor's copy phase stopped making progress"
-            decode.rounds, decode.polls = rounds.value, polls.value
-            return rc, (buf.raw[: n.value] if rc == 0 else None)
-
-        decode.max_content = 131169  # one ciphertext payload: what k_zd3_exec holds in shared memory
-        return decode
-
-    return {"fused": make(lib.zd_decode), "two_phase": make(lib.zd_decode_two_phase), "v2": make(lib.zd_decode_v2), "v3": make_v3()}
-
-
-@pytest.fixture(params=["fused", "two_phase", "v2", "v3"])
-def zd(request, zd_lib):
-    return zd_lib[request.param]
+    decode.max_content = 131169  # one ciphertext payload: what k_zd3_exec holds in shared memory
+    return decode
 
 
 def _reference(frame: bytes):
@@ -85,7 +66,7 @@ def test_reference_fixtures_decode_identically(zd):
     for fr in frames:
         rc, got = zd(fr)
         want = F.zstd().decompress(fr)
-        if len(want) > getattr(zd, "max_content", 1 << 30):
+        if len(want) > zd.max_content:
             assert rc == 1  # (keys: the parallel executor holds one ciphertext payload)
             continue
         assert rc == 0 and got == want
@@ -113,13 +94,13 @@ def test_random_frames_at_many_levels(zd):
                 fr = z.compress(data, lvl)
                 rc, got = zd(fr)
                 assert rc in (0, 1) and (rc == 1 or got == data), (len(data), lvl)
-                if len(data) > getattr(zd, "max_content", 1 << 30):
+                if len(data) > zd.max_content:
                     assert rc == 1
                     continue
                 ok += rc == 0
                 total += 1
     payload = b"\x07" * 97 + np.stack([rng.integers(0, 1 << 36, 4096, dtype=np.uint64) for _ in range(4)]).tobytes()
-    assert ok >= total - 6, "only frames beyond the two-phase plan's limits (blocks, sequences) may be handed back"
+    assert ok >= total - 6, "only frames beyond the decoder's limits (blocks, sequences) may be handed back"
     rc, got = zd(F.zstd_structured_frame(payload))
     assert rc == 0 and got == payload
 
@@ -155,11 +136,10 @@ def test_mutated_frames_never_decode_wrongly(zd):
     assert accepted > 100 and handed_back > 100
 
 
-def test_parallel_executor_resolves_ciphertext_frames_by_jumping(zd_lib):
+def test_parallel_executor_resolves_ciphertext_frames_by_jumping(zd):
     """zstd_exec3.h on what it is built for: a level-3 ciphertext frame has ~16 k matches in 16 dependency chains ~1,000 long
     (the top-nibble tails), most 5-byte matches read a literal followed by a match.  The pointer jumping (with the one split)
     must leave next to nothing to the copy phase's polling, in a logarithmic number of rounds."""
-    zd = zd_lib["v3"]
     rng = np.random.default_rng(8)
     q = (0xFFFFEE001, 0xFFFFC4001)
     z = F.zstd()

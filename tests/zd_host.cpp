@@ -1,73 +1,17 @@
-// Host build of the device zstd decoder (fhe_precompiles_b200/csrc/zstd_dec.h) for tests/test_zstd_dec.py: the same source
-// that k_zstd_inflate runs, compiled with g++ so that it can be compared with libzstd and fuzzed without a GPU.
+// Host build of the device zstd decoder (fhe_precompiles_b200/csrc: zstd_dec.h, zstd_plan2.h, zstd_exec3.h) for
+// tests/test_zstd_dec.py: the same source that k_zd2_parse, k_zd3_huf, k_zd3_seq and k_zd3_exec run, compiled with g++ so that
+// it can be compared with libzstd and fuzzed without a GPU.  Where a kernel spreads a step over many threads, the threads are
+// played one after the other between the kernel's barriers.
+#include <algorithm>
 #include <cstring>
 #include <vector>
 
-#include "zstd_dec.h"
-
-extern "C" int zd_decode(const uint8_t *src, size_t slen, uint8_t *dst, size_t cap, size_t *dlen) {
-    static thread_local fheb::zd::Work *w = nullptr;
-    if (!w) {
-        w = new fheb::zd::Work();
-        fheb::zd::work_bind(w, nullptr);
-    }
-    std::vector<uint8_t> buf(slen + 2 * fheb::zd::kPad, 0xAA);  // the decoder reads aligned words around the frame
-    memcpy(buf.data() + fheb::zd::kPad, src, slen);
-    return fheb::zd::decode_frame(buf.data() + fheb::zd::kPad, slen, dst, cap, dlen, w);
-}
-
-// the two-phase pipeline (plan_frame + execute_plan), scalar on the host
-extern "C" int zd_decode_two_phase(const uint8_t *src, size_t slen, uint8_t *dst, size_t cap, size_t *dlen) {
-    static thread_local fheb::zd::Work *w = nullptr;
-    static thread_local fheb::zd::FramePlan *plan = nullptr;
-    static thread_local std::vector<uint64_t> seqs(fheb::zd::kPlanMaxSeqs);
-    if (!w) {
-        w = new fheb::zd::Work();
-        fheb::zd::work_bind(w, nullptr);
-        plan = new fheb::zd::FramePlan();
-    }
-    std::vector<uint8_t> buf(slen + 2 * fheb::zd::kPad, 0xAA), lits(cap + 8);
-    memcpy(buf.data() + fheb::zd::kPad, src, slen);
-    const uint8_t *f = buf.data() + fheb::zd::kPad;
-    if (fheb::zd::plan_frame(f, slen, cap, w, plan, seqs.data(), lits.data()) != fheb::zd::kZdOk) return 1;
-    return fheb::zd::execute_plan(f, plan, seqs.data(), lits.data(), dst, dlen);
-}
-
-// the batch-oriented pipeline (zstd_plan2.h): parse -> four Huffman stream "threads" + the sequence "thread" -> execution
-#include "zstd_plan2.h"
-extern "C" int zd_decode_v2(const uint8_t *src, size_t slen, uint8_t *dst, size_t cap, size_t *dlen) {
-    using namespace fheb::zd;
-    static thread_local Work *w = nullptr;
-    static thread_local Plan2 *plan = nullptr;
-    static thread_local Tables2 *tabs = nullptr;
-    static thread_local std::vector<uint64_t> seqs(kP2MaxSeqs);
-    if (!w) {
-        w = new Work();
-        plan = new Plan2();
-        tabs = new Tables2();
-    }
-    work_bind(w, nullptr);
-    // an odd leading pad so that stream starts land on every alignment
-    static thread_local unsigned shift = 0;
-    shift = (shift + 1) & 7;
-    std::vector<uint8_t> buf(slen + 2 * kPad + 8, 0xAA), lits(cap + 16);
-    uint8_t *f = buf.data() + kPad + shift;
-    memcpy(f, src, slen);
-    if (plan2_parse(f, slen, cap, w, plan, tabs) != kZdOk) return 1;
-    for (int k = 0; k < 4; k++) plan->huf_bad[k] = plan2_huf(f, plan, tabs, lits.data(), k) ? 0 : 1;
-    plan->seq_bad = plan2_seq(f, plan, tabs, seqs.data()) ? 0 : 1;
-    // the executor stores aligned 64-bit words: an aligned bounce buffer with room up to the next multiple of 8
-    std::vector<uint64_t> out((cap + 15) / 8);
-    const int rc = plan2_exec(f, plan, seqs.data(), lits.data(), (uint8_t *)out.data(), dlen);
-    if (rc == 0) memcpy(dst, out.data(), *dlen);
-    return rc;
-}
-
-// the fourth generation's execution (zstd_exec3.h, k_zd3_exec on the device): the same per-sequence steps, the CTA's 1,024
-// threads played one after the other between the barriers of the kernel.  *rounds = jump rounds of the busiest pass, *polls =
-// the number of times a thread found its source still pending in step 3 (0 when the jumping resolved everything).
 #include "zstd_exec3.h"
-extern "C" int zd_decode_v3(const uint8_t *src, size_t slen, uint8_t *dst, size_t cap, size_t *dlen, int *rounds, long *polls) {
+#include "zstd_plan2.h"
+
+// parse -> Huffman streams -> sequence chains -> execution.  *rounds = jump rounds of the busiest pass of the execution, *polls =
+// the number of times a thread found its source still pending in its step 3 (0 when the jumping resolved everything).
+extern "C" int zd_decode(const uint8_t *src, size_t slen, uint8_t *dst, size_t cap, size_t *dlen, int *rounds, long *polls) {
     using namespace fheb::zd;
     using namespace fheb::zd3;
     static thread_local Work *w = nullptr;
@@ -88,7 +32,28 @@ extern "C" int zd_decode_v3(const uint8_t *src, size_t slen, uint8_t *dst, size_
     if (plan2_parse(f, slen, cap, w, plan, tabs) != kZdOk) return 1;
     for (int k = 0; k < 4; k++)
         if (!plan2_huf(f, plan, tabs, lits.data(), k)) return 1;
-    if (!plan2_seq(f, plan, tabs, seqs.data())) return 1;
+    {  // k_zd3_seq (zstd_plan3.cuh seq_frames) for one frame slot
+        std::vector<uint32_t> tab(kTabCells), lut(kLutCells);
+        for (int c = 0; c < kLutCells; c++) lut[c] = c < 36 ? ll_base(c) : ml_base(c - 36);
+        const auto stage = [](uint32_t *dst, const SeqEntry *src, uint32_t log, int which) {
+            for (uint32_t k = 0; k < (1u << log); k++) {
+                uint2 g;  // the device's 8-byte load of a cell
+                memcpy(&g, src + k, sizeof g);
+                dst[k] = pack_cell(g, which);
+            }
+        };
+        uint32_t r0 = 1, r1 = 4, r2 = 8;
+        for (uint32_t bi = 0; bi < plan->nblocks; bi++) {
+            const Block2 &bp = plan->blocks[bi];
+            if (bp.type != 2 || bp.nseq == 0) continue;
+            if (bp.ll_log > 9 || bp.of_log > 8 || bp.ml_log > 9) return 1;
+            stage(tab.data(), tabs->ll[bp.ll_tab], bp.ll_log, 0);
+            stage(tab.data() + 512, tabs->of[bp.of_tab], bp.of_log, 1);
+            stage(tab.data() + 768, tabs->ml[bp.ml_tab], bp.ml_log, 2);
+            if (!seq_block(f, bp, tab.data(), tab.data() + 512, tab.data() + 768, lut.data(), seqs.data() + bp.seq_off, r0, r1, r2))
+                return 1;
+        }
+    }
     if (plan->content > kExecOutBytes - 31) return 1;
     const int T = kExecThreads;
     std::vector<uint8_t> out(kExecOutBytes, 0xEE);
