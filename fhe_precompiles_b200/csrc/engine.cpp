@@ -604,7 +604,10 @@ void Engine::relinearize(int device, const uint64_t *c3, const uint64_t *rk, uin
 
 // ---------------------------------------------------------------- host-buffer batch (H2D | kernels | D2H overlapped)
 // Chunk schedule of the host pipelines: full chunks in the middle, a short first one (the kernels start after 0.5 ms of copies
-// instead of 1.3) and a short last one (less to drain) - both still >= kFusedTailMinOps ops, so that they run the fused tails.
+// instead of 1.3) and a short last one (less to drain), both of kFusedTailMinOps ops or more where n allows.  For
+// kFusedTailMinOps < n < 2 kFusedTailMinOps the remainder after the first chunk is shorter and runs the split tails (n = 150:
+// 96 fused + 54 split).  With a pipeline chunk of 96 ops or fewer every chunk runs them, and with one just above 96 the
+// next-to-last chunk can be short (97 on 300 ops: 96 / 97 / 11 / 96).  tests/test_edge_parity.py pins these schedules.
 // A function of (off, n, chunk) only: every loop over the same batch sees the same chunks.
 static size_t pipe_chunk(size_t off, size_t n, size_t chunk) {
     const size_t rem = n - off, edge = kFusedTailMinOps;
