@@ -105,6 +105,10 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_upload_frames.restype = i32
     L.fhe_b200_download_frames.argtypes = [i32, vp, sz, vp, vp]
     L.fhe_b200_download_frames.restype = i32
+    L.fhe_b200_upload_ciphertexts.argtypes = [i32, i32, vp, vp, sz, vp, vp]
+    L.fhe_b200_upload_ciphertexts.restype = i32
+    L.fhe_b200_download_ciphertexts.argtypes = [i32, i32, vp, sz, vp, vp, vp]
+    L.fhe_b200_download_ciphertexts.restype = i32
     L.fhe_b200_frame_bytes.argtypes = []
     L.fhe_b200_frame_bytes.restype = sz
     L.fhe_b200_frame_stride.argtypes = []

@@ -441,6 +441,24 @@ int32_t fhe_b200_upload_frames(int32_t device, const uint8_t *frames, size_t str
 int32_t fhe_b200_download_frames(int32_t device, const uint64_t *d_words, size_t n, uint8_t *out_frames, int32_t *status) {
     DEV_GUARD(Engine::get().download_frames(device, d_words, n, out_frames, status));
 }
+// kind numbered as in fhe_b200_data_type_kind; the host arrays may be NULL only when n == 0
+static void check_ciphertext_args(const char *fn, int32_t kind, size_t n, bool arrays) {
+    if (kind < 0 || kind > 3)
+        throw std::runtime_error(std::string(fn) + ": unknown kind " + std::to_string(kind) + " (0 u256, 1 u64, 2 i64, 3 frac64)");
+    if (n && !arrays) throw std::runtime_error(std::string(fn) + ": null host array");
+}
+int32_t fhe_b200_upload_ciphertexts(int32_t device, int32_t kind, const uint8_t *const *cts, const size_t *lens, size_t n,
+                                    uint64_t *d_words, int32_t *status) {
+    DEV_GUARD(check_ciphertext_args("fhe_b200_upload_ciphertexts", kind, n, cts && lens && status);
+              if (n) Engine::get().upload_ciphertexts(device, (Kind)kind, cts, lens, n, d_words, status));
+}
+int32_t fhe_b200_download_ciphertexts(int32_t device, int32_t kind, const uint64_t *d_words, size_t n, uint8_t **outputs,
+                                      int64_t *output_lengths, int32_t *status) {
+    std::string row_error;
+    DEV_GUARD(check_ciphertext_args("fhe_b200_download_ciphertexts", kind, n, outputs && output_lengths && status);
+              if (n) Engine::get().download_ciphertexts(device, (Kind)kind, d_words, n, outputs, output_lengths, status, &row_error);
+              if (!row_error.empty()) set_error(row_error.c_str()));
+}
 size_t fhe_b200_frame_bytes(void) { return kPackedFrameBytes; }
 size_t fhe_b200_frame_stride(void) { return kPackedFrameStride; }
 int32_t fhe_b200_ntt(int32_t device, uint64_t *data, size_t n_limbs, const int32_t *mods, int32_t n_mods, int32_t inverse,

@@ -573,6 +573,23 @@ bool inflate_ct_payload(Span frame, uint8_t *dst) {
     return !z.isError(r) && r == want;
 }
 
+bool inflate_ct_blob(Span blob, uint8_t *dst) {
+    SealHeader h;
+    if (!parse_seal_header(blob.p, blob.n, &h) || h.size < kSealHeader || h.size > blob.n) return false;
+    const Span body{blob.p + kSealHeader, (size_t)h.size - kSealHeader};
+    const size_t want = kCtHeaderBytes + 8 * kCtWords;
+    if (h.compr == 0) {
+        if (body.n != want) return false;
+        memcpy(dst, body.p, want);
+        return true;
+    }
+    if (h.compr == 1) {
+        uLongf dl = (uLongf)want;
+        return uncompress(dst, &dl, body.p, (uLong)body.n) == Z_OK && dl == want;
+    }
+    return h.compr == 2 && inflate_ct_payload(body, dst);
+}
+
 void canonical_ct_prefix(uint8_t *p) {
     const HostContext &H = HostContext::get();
     memcpy(p, H.parms_id_data, 32);

@@ -60,6 +60,8 @@ int classify_ciphertext_blob(Span blob, Span *frame, uint8_t *compr);
 // libzstd inflate of a ciphertext frame straight into `dst` (131,169 bytes, e.g. pinned staging); false unless the frame
 // holds exactly a payload of that size.  The content is validated on the device (k_ct_unpack).
 bool inflate_ct_payload(Span frame, uint8_t *dst);
+// the same for a whole SEAL blob of any compr_mode (none: copied, zlib, zstd); false unless it holds exactly such a payload
+bool inflate_ct_blob(Span blob, uint8_t *dst);
 // the 97 bytes every valid size-2 data-level coefficient-form ciphertext payload starts with
 void canonical_ct_prefix(uint8_t *prefix97);
 // bincode(Ciphertext) around an already compressed payload `body` (SEAL header with view.compr_mode added here)

@@ -181,11 +181,14 @@ __global__ void __launch_bounds__(256) k_unpack40(const uint8_t *frames, const C
 }
 
 // words -> complete structured frame (kPackedFrameBytes); flag = 1 when the first 16 words are equal (the host writer hands
-// constant data to libzstd, and so must the caller)
-__global__ void __launch_bounds__(256) k_ct_pack40(const u64 *words, uint8_t *frames, int32_t *constant_flag, const uint8_t *prefix) {
+// constant data to libzstd, and so must the caller).  Output j starts at out + j * out_stride with the `head_len` bytes of
+// `head` (the bincode + SEAL envelope of a complete Ciphertext, or nothing), and its frame follows them.
+__global__ void __launch_bounds__(256) k_ct_pack40(const u64 *words, uint8_t *out, size_t out_stride, const uint8_t *head, int head_len,
+                                                   int32_t *constant_flag, const uint8_t *prefix) {
     const int j = blockIdx.x;
     const u64 *w = words + (size_t)j * kCodecCtWords;
-    uint8_t *f = frames + (size_t)j * kPackedFrameStride;
+    uint8_t *f = out + (size_t)j * out_stride + head_len;
+    if (blockIdx.y == 0 && (int)threadIdx.x < head_len) f[(int)threadIdx.x - head_len] = head[threadIdx.x];  // head_len <= 256
     if (blockIdx.y == 0 && threadIdx.x == 0) {
         frame40_fixed<true>(f);
         u64 diff = 0;
@@ -253,8 +256,14 @@ cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const
 }
 
 cudaError_t launch_codec_pack(const u64 *words, uint8_t *frames, int32_t *constant_flag, const uint8_t *prefix, int n, cudaStream_t s) {
+    return launch_codec_pack(words, frames, kPackedFrameStride, nullptr, 0, constant_flag, prefix, n, s);
+}
+
+cudaError_t launch_codec_pack(const u64 *words, uint8_t *out, size_t out_stride, const uint8_t *head, int head_len, int32_t *constant_flag,
+                              const uint8_t *prefix, int n, cudaStream_t s) {
     if (n == 0) return cudaSuccess;
-    k_ct_pack40<<<dim3(n, kSplit), 256, 0, s>>>(words, frames, constant_flag, prefix);
+    if (head_len < 0 || head_len > kPackHeadMax || out_stride < (size_t)head_len + kPackedFrameBytes) return cudaErrorInvalidValue;
+    k_ct_pack40<<<dim3(n, kSplit), 256, 0, s>>>(words, out, out_stride, head, head_len, constant_flag, prefix);
     g_codec_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }

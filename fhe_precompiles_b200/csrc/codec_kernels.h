@@ -38,6 +38,11 @@ cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const
 // n result ciphertexts -> n structured frames (kPackedFrameStride apart); constant_flag[i] = 1 if the host must use libzstd instead
 cudaError_t launch_codec_pack(const uint64_t *words, uint8_t *frames, int32_t *constant_flag, const uint8_t *prefix, int n,
                               cudaStream_t s);
+// the same into rows of `out_stride` bytes that start with the head_len (<= kPackHeadMax) bytes at `head` (device memory), the
+// frame right behind them: complete serialized ciphertexts when `head` is their constant bincode + SEAL envelope
+constexpr int kPackHeadMax = 256;
+cudaError_t launch_codec_pack(const uint64_t *words, uint8_t *out, size_t out_stride, const uint8_t *head, int head_len,
+                              int32_t *constant_flag, const uint8_t *prefix, int n, cudaStream_t s);
 uint64_t codec_launch_count();
 
 }  // namespace fheb

@@ -71,6 +71,12 @@ void parallel_for(size_t count, size_t grain, F &&fn) {
     }
     HostPool::get().run(std::min(width - 1, (count + grain - 1) / grain - 1), body);
 }
+// the Params every precompile result carries (testnet.rs:8-14) in sunscreen's bincode layout
+void testnet_params(uint8_t out[kParamsBytes]) {
+    uint64_t w[6] = {(uint64_t)kN, 3, kModulus[MQ0], kModulus[MQ1], kModulus[MP], kT};
+    memcpy(out, w, 48);
+    memset(out + 48, 0, 8);
+}
 // FHE_B200_TILE_PROFILE=<n >= 1>: wall time of binary_tile's phases summed over all tile workers, printed when the process exits;
 // the first n calls (warm-up: lanes, pinned buffers, key upload) are not counted
 struct TileProfile {
@@ -837,6 +843,250 @@ void Engine::download_frames(int device, const uint64_t *d_words, size_t n, uint
         for (size_t i = 0; i < n; i++) status[i] = X.h_status[i] ? 2 : 0;
 }
 
+// ---------------------------------------------------------------- sunscreen Ciphertexts <-> device-resident ciphertexts
+void Engine::xfer_host_stage(XferPipe &X, size_t bytes) {
+    for (auto &sl : X.slot) {
+        if (sl.h_stage_bytes >= bytes) continue;
+        cuda_throw(cudaStreamSynchronize(sl.stream), "sync before staging regrow");
+        cudaFreeHost(sl.h_stage);
+        sl.h_stage = nullptr, sl.h_stage_bytes = 0;
+        cuda_throw(cudaMallocHost((void **)&sl.h_stage, bytes), "cudaMallocHost");
+        sl.h_stage_bytes = bytes;
+    }
+}
+
+namespace {
+// what a precompile result of `kind` carries besides its words: the kind's data_type, the testnet Params, compr_mode zstd
+CipherView result_view(Kind kind) {
+    CipherView v;
+    v.data_type = data_type_of(kind);
+    testnet_params(v.params);
+    v.compr_mode = 2;
+    return v;
+}
+}  // namespace
+
+// Per ciphertext, on the host pool: bincode framing, data_type and the SEAL blob's header (a few hundred bytes).  Then, per chunk,
+// one job per ciphertext for launch_codec_inflate, which validates the 97-byte prefix and every residue and writes d_words:
+//   structured frame -> kJobPacked;  libzstd frame -> kJobZstd (device decoder) when the chunk brings device_zstd_min_frames_ of
+//   them, else inflated here -> kJobPayload;  compr_mode none -> kJobPayload as it is;  zlib -> inflated here -> kJobPayload.
+// Staging of a chunk, the same on the host (pinned) and on the device: [frames | payloads], so that one copy moves both.  Every
+// ciphertext that is not accepted on that path -- and every one the device hands back -- is decoded by decode_ciphertext, whose
+// code is the status (the device never turns a valid ciphertext into a rejection).
+void Engine::upload_ciphertexts(int device, Kind kind, const uint8_t *const *cts, const size_t *lens, size_t n, uint64_t *d_words,
+                                int32_t *status) {
+    if (n == 0) return;
+    device_context(device);
+    const size_t frames_cap = kXferChunk * kFrameSlotBytes, stage_bytes = frames_cap + kXferChunk * kPayloadStride;
+    XferPipe &X = xfer_pipe(device, n, stage_bytes);
+    std::lock_guard<std::mutex> lk(X.mu);
+    for (auto &sl : X.slot) cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");  // (idle unless a call before this one threw)
+    xfer_host_stage(X, stage_bytes);
+    enum : uint8_t { kDone, kHost, kPacked, kZstd, kPayload };  // route of a ciphertext
+    std::vector<uint8_t> route(n);
+    std::vector<Span> blob(n), frame(n);
+    std::vector<size_t> at(n);  // staging offset of a frame, or the payload job of a ciphertext
+    std::vector<int32_t> st(n, 0);
+    struct Pending {
+        size_t off = 0, c = 0;
+        int jobs = 0;
+        bool live = false;
+    } pend[2];
+
+    // a chunk's results: ciphertexts handed back by the device join the host route; the host decodes, checks and uploads them
+    const auto finish = [&](int b) {
+        Pending &p = pend[b];
+        XferSlot &sl = X.slot[b];
+        p.live = false;
+        for (int j = 0; j < p.jobs; j++)
+            if (X.h_status[p.off + j] == kJobFallback) route[p.off + (size_t)sl.h_jobs[j].slot] = kHost;
+        std::vector<size_t> host;
+        for (size_t i = p.off; i < p.off + p.c; i++)
+            if (route[i] == kHost) host.push_back(i);
+        if (host.empty()) return;
+        std::vector<std::vector<uint64_t>> words(host.size());
+        parallel_for(host.size(), 1, [&](size_t h) {
+            const size_t i = host[h];
+            CipherView v;
+            words[h].resize(kCtWords);
+            const int32_t rc = decode_ciphertext(Span{cts[i], lens[i]}, &v, words[h].data());
+            st[i] = rc ? rc : data_type_matches(v.data_type, kind) ? kOk : kErrSunscreen;
+        });
+        for (size_t h = 0; h < host.size(); h++)
+            if (st[host[h]] == kOk)
+                cuda_throw(cudaMemcpyAsync(d_words + host[h] * kCtWords, words[h].data(), kCtWords * 8, cudaMemcpyHostToDevice, sl.stream),
+                           "H2D host-decoded ciphertext");
+        cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");
+    };
+
+    size_t k = 0;
+    for (size_t off = 0; off < n; off += kXferChunk, k++) {
+        const size_t c = std::min(kXferChunk, n - off);
+        const int b = (int)(k & 1);
+        XferSlot &sl = X.slot[b];
+        cudaStream_t s = sl.stream;
+        if (pend[b].live) {  // this slot's staging, jobs and status are free again once its previous chunk is done
+            cuda_throw(cudaStreamSynchronize(s), "slot sync");
+            finish(b);
+        }
+        // (A) framing, data_type and blob header of every ciphertext of the chunk
+        parallel_for(c, 8, [&](size_t t) {
+            const size_t i = off + t;
+            CipherView v;
+            const int32_t rc = parse_ciphertext_framing(Span{cts[i], lens[i]}, &v, &blob[i]);
+            if (rc) {
+                st[i] = rc, route[i] = kDone;
+                return;
+            }
+            uint8_t compr = 0;
+            const int cls = data_type_matches(v.data_type, kind) ? classify_ciphertext_blob(blob[i], &frame[i], &compr) : -1;
+            if (cls == 2) route[i] = kPacked;
+            else if (cls == 1) route[i] = frame[i].n + 2 * kFramePad <= kFrameSlotBytes ? kZstd : kHost;
+            else if (cls == 0) route[i] = kPayload;
+            else route[i] = kHost;  // a wrong data_type or a malformed SEAL header: decode_ciphertext has the code
+        });
+        // (B) the engine's rule for libzstd frames; then jobs: payloads first (payload slot = job), frames behind them
+        size_t lib_frames = 0;
+        for (size_t i = off; i < off + c; i++) lib_frames += route[i] == kZstd;
+        const bool dev_zstd = device_zstd_ == 1 || (device_zstd_ == 2 && lib_frames >= device_zstd_min_frames_);
+        int jobs = 0;
+        for (size_t i = off; i < off + c; i++) {
+            if (route[i] == kZstd && !dev_zstd) route[i] = kPayload;
+            if (route[i] != kPayload) continue;
+            at[i] = (size_t)jobs;
+            sl.h_jobs[jobs++] = CodecJob{0, 0, kJobPayload, (int32_t)(i - off), 0};
+        }
+        const int payload_jobs = jobs;
+        size_t fcur = 0;
+        bool any_zstd = false, any_packed = false;
+        for (size_t i = off; i < off + c; i++) {
+            if (route[i] != kPacked && route[i] != kZstd) continue;
+            at[i] = fcur + kFramePad;
+            sl.h_jobs[jobs++] = CodecJob{at[i], (uint32_t)frame[i].n, route[i] == kPacked ? kJobPacked : kJobZstd, (int32_t)(i - off), 0};
+            (route[i] == kPacked ? any_packed : any_zstd) = true;
+            fcur += (frame[i].n + 2 * kFramePad + 15) & ~(size_t)15;
+        }
+        const size_t pay_base = (fcur + 255) & ~(size_t)255;
+        // (C) frames into the staging as they are, payloads inflated (or copied) into their slots
+        parallel_for(c, 2, [&](size_t t) {
+            const size_t i = off + t;
+            if (route[i] == kPacked || route[i] == kZstd) {
+                memcpy(sl.h_stage + at[i], frame[i].p, frame[i].n);
+            } else if (route[i] == kPayload && !inflate_ct_blob(blob[i], sl.h_stage + pay_base + at[i] * kPayloadStride)) {
+                route[i] = kHost;
+                sl.h_jobs[at[i]].kind = kJobNone;
+            }
+        });
+        // (D) one copy of the staging, the jobs, the codec kernels straight into d_words, the job status back
+        if (jobs) {
+            const size_t bytes = payload_jobs ? pay_base + (size_t)payload_jobs * kPayloadStride : fcur;
+            if (any_zstd && !sl.d_work) cuda_throw(cudaMalloc(&sl.d_work, kXferChunk * codec_work_bytes()), "cudaMalloc");
+            cuda_throw(cudaMemcpyAsync(sl.d_jobs, sl.h_jobs, (size_t)jobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
+            cuda_throw(cudaMemcpyAsync(sl.d_frames, sl.h_stage, bytes, cudaMemcpyHostToDevice, s), "H2D ciphertexts");
+            cuda_throw(launch_codec_inflate(sl.d_frames, sl.d_frames + pay_base, sl.d_jobs, sl.d_status, sl.d_work, X.d_prefix,
+                                            d_words + off * kCtWords, nullptr, jobs, any_zstd, any_packed, payload_jobs > 0, s),
+                       "ciphertext unpack");
+            cuda_throw(cudaMemcpyAsync(X.h_status + off, sl.d_status, (size_t)jobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H status");
+        }
+        pend[b] = Pending{off, c, jobs, true};
+    }
+    for (int b = 0; b < 2; b++) {
+        const int oldest = (int)((k + (size_t)b) & 1);  // (in chunk order)
+        if (!pend[oldest].live) continue;
+        cuda_throw(cudaStreamSynchronize(X.slot[oldest].stream), "xfer sync");
+        finish(oldest);
+    }
+    if (status) memcpy(status, st.data(), n * sizeof(int32_t));
+}
+
+// Structured writer: k_ct_pack40 writes every row as the complete Ciphertext (the kind's constant envelope, then the frame) and
+// one copy per chunk brings the final bytes back; constant (transparent) results take encode_ciphertext, as on the byte surface.
+// Default writer (SEAL's own bytes, libzstd level 3 on the host cores): one copy of the words per chunk, encode_ciphertext on
+// the host pool.  Either way the host works on chunk k while the device and PCIe work on chunk k + 1.
+void Engine::download_ciphertexts(int device, Kind kind, const uint64_t *d_words, size_t n, uint8_t **outputs, int64_t *output_lengths,
+                                  int32_t *status, std::string *row_error) {
+    if (n == 0) return;
+    device_context(device);
+    const CipherView view = result_view(kind);
+    const bool structured = zstd_writer() == 1;
+    const size_t head = wrapped_ciphertext_size(view, kPackedFrameBytes) - kPackedFrameBytes, whole = head + kPackedFrameBytes;
+    if (head > (size_t)kPackHeadMax) throw std::runtime_error("download_ciphertexts: data_type too long");
+    const size_t row = structured ? (whole + 15) & ~(size_t)15 : kCtWords * 8;
+    XferPipe &X = xfer_pipe(device, n, kXferChunk * row);
+    std::lock_guard<std::mutex> lk(X.mu);
+    for (auto &sl : X.slot) cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");  // (idle unless a call before this one threw)
+    xfer_host_stage(X, kXferChunk * row);
+    if (structured) {
+        std::vector<uint8_t> zero(kPackedFrameBytes, 0), env(whole);
+        wrap_ciphertext_blob_to(view, zero.data(), kPackedFrameBytes, env.data());
+        if (!X.d_head) cuda_throw(cudaMalloc((void **)&X.d_head, kPackHeadMax), "cudaMalloc");
+        cuda_throw(cudaMemcpy(X.d_head, env.data(), head, cudaMemcpyHostToDevice), "upload envelope");
+    }
+    std::mutex err_mu;
+    struct Pending {
+        size_t off = 0, c = 0;
+        bool live = false;
+    } pend[2];
+    const auto finish = [&](int b) {
+        Pending &p = pend[b];
+        XferSlot &sl = X.slot[b];
+        p.live = false;
+        cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");  // the chunk's bytes (or words) and constant flags are here
+        std::vector<std::vector<uint64_t>> constant(p.c);           // words of the constant results (structured writer)
+        bool any_constant = false;
+        if (structured)
+            for (size_t t = 0; t < p.c; t++)
+                if (X.h_status[p.off + t]) {
+                    constant[t].resize(kCtWords);
+                    any_constant = true;
+                    cuda_throw(cudaMemcpyAsync(constant[t].data(), d_words + (p.off + t) * kCtWords, kCtWords * 8, cudaMemcpyDeviceToHost, sl.stream),
+                               "D2H constant result");
+                }
+        if (any_constant) cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");
+        parallel_for(p.c, 4, [&](size_t t) {
+            const size_t i = p.off + t;
+            outputs[i] = nullptr, output_lengths[i] = 0, status[i] = -1;
+            try {
+                thread_local std::vector<uint8_t> bytes;
+                const uint8_t *src = sl.h_stage + t * row;
+                size_t len = whole;
+                if (!structured || !constant[t].empty()) {
+                    encode_ciphertext(view, structured ? constant[t].data() : reinterpret_cast<const uint64_t *>(src), &bytes);
+                    src = bytes.data(), len = bytes.size();
+                }
+                uint8_t *o = (uint8_t *)malloc(len);
+                if (!o) throw std::runtime_error("download_ciphertexts: out of host memory");
+                memcpy(o, src, len);
+                outputs[i] = o, output_lengths[i] = (int64_t)len, status[i] = 0;
+            } catch (const std::exception &e) {
+                std::lock_guard<std::mutex> g(err_mu);
+                if (row_error && row_error->empty()) *row_error = "download_ciphertexts: ciphertext " + std::to_string(i) + ": " + e.what();
+            }
+        });
+    };
+    size_t k = 0;
+    for (size_t off = 0; off < n; off += kXferChunk, k++) {
+        const size_t c = std::min(kXferChunk, n - off);
+        const int b = (int)(k & 1);
+        XferSlot &sl = X.slot[b];
+        cudaStream_t s = sl.stream;
+        if (pend[b].live) finish(b);
+        if (structured) {
+            cuda_throw(launch_codec_pack(d_words + off * kCtWords, sl.d_frames, row, X.d_head, (int)head, sl.d_status, X.d_prefix, (int)c, s),
+                       "ciphertext pack");
+            cuda_throw(cudaMemcpyAsync(sl.h_stage, sl.d_frames, (c - 1) * row + whole, cudaMemcpyDeviceToHost, s), "D2H ciphertexts");
+            cuda_throw(cudaMemcpyAsync(X.h_status + off, sl.d_status, c * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H flags");
+        } else {
+            cuda_throw(cudaMemcpyAsync(sl.h_stage, d_words + off * kCtWords, c * kCtWords * 8, cudaMemcpyDeviceToHost, s), "D2H words");
+        }
+        pend[b] = Pending{off, c, true};
+    }
+    for (int b = 0; b < 2; b++) {
+        const int oldest = (int)((k + (size_t)b) & 1);
+        if (pend[oldest].live) finish(oldest);
+    }
+}
+
 // ---------------------------------------------------------------- byte surface, one call
 namespace {
 struct LaneGuard {
@@ -1456,11 +1706,6 @@ Seed512 seed_from_hash(const std::vector<uint8_t> &msg) {
     Seed512 s;
     memcpy(s.w, h, 64);
     return s;
-}
-void testnet_params(uint8_t out[kParamsBytes]) {
-    uint64_t w[6] = {(uint64_t)kN, 3, kModulus[MQ0], kModulus[MQ1], kModulus[MP], kT};
-    memcpy(out, w, 48);
-    memset(out + 48, 0, 8);
 }
 }  // namespace
 

@@ -165,6 +165,15 @@ class Engine {
     // PCIe once at each end: frames (host) -> validated limb arrays on the device, and back.  Synchronous, chunk-pipelined.
     void upload_frames(int device, const uint8_t *frames, size_t stride, size_t n, uint64_t *d_words, int32_t *status);
     void download_frames(int device, const uint64_t *d_words, size_t n, uint8_t *out_frames, int32_t *status);
+    // The same from / to complete sunscreen Ciphertexts of `kind`, in whatever form the precompiles accept (libzstd, structured,
+    // zlib or uncompressed SEAL blobs) and write.  upload: status[i] = 0 or the code c_fhe_add_cipherK_cipherK returns for
+    // ciphertext i as its first operand (the words of that row are then undefined).  download: outputs[i] malloc'ed, byte for byte
+    // what a precompile of `kind` returns for these words under the current zstd writer; status[i] = -1 where a row failed
+    // (its message in *row_error).  Synchronous, in chunks of kXferChunk over the two transfer slots.
+    void upload_ciphertexts(int device, Kind kind, const uint8_t *const *cts, const size_t *lens, size_t n, uint64_t *d_words,
+                            int32_t *status);
+    void download_ciphertexts(int device, Kind kind, const uint64_t *d_words, size_t n, uint8_t **outputs, int64_t *output_lengths,
+                              int32_t *status, std::string *row_error);
 
     // Optional per-kernel timing of mul_relin(): CUDA events around every launch on the caller's stream.
     // kernel ids: see kKernelNames.  report() synchronises the device.
@@ -272,9 +281,15 @@ class Engine {
         size_t d_frames_bytes = 0;
         struct CodecJob *d_jobs = nullptr, *h_jobs = nullptr;
         int32_t *d_status = nullptr;
+        // upload_ciphertexts / download_ciphertexts: pinned mirror of d_frames (the scattered ciphertexts are gathered here, then
+        // cross PCIe in one copy), and the device zstd decoder's workspace; both allocated on first use
+        uint8_t *h_stage = nullptr;
+        size_t h_stage_bytes = 0;
+        void *d_work = nullptr;
     };
     struct XferPipe {
         uint8_t *d_prefix = nullptr;
+        uint8_t *d_head = nullptr;  // download_ciphertexts: the envelope in front of every structured frame (kPackHeadMax bytes)
         int32_t *h_status = nullptr;
         size_t h_status_cap = 0;
         XferSlot slot[2];
@@ -283,6 +298,7 @@ class Engine {
     static constexpr size_t kXferChunk = 256;
     std::vector<std::unique_ptr<XferPipe>> xfers_;
     XferPipe &xfer_pipe(int device, size_t n, size_t slot_bytes);
+    void xfer_host_stage(XferPipe &X, size_t bytes);  // XferSlot::h_stage of at least `bytes`; X.mu held
 
     struct TimedLaunch {
         int kernel;

@@ -158,6 +158,47 @@ def download_frames(ct: torch.Tensor, out: torch.Tensor = None):
     return out, status
 
 
+def upload_ciphertexts(cts: Sequence[bytes], kind: str, device: int = 0):
+    """sunscreen Ciphertext bytes of `kind` (what the c_fhe_* precompiles return and take, in any of the forms they accept) ->
+    (ct [n,2,2,4096] int64 on `device`, status [n] int32 host): status[i] is 0, or the code c_fhe_add_cipher<kind>_cipher<kind>
+    returns with ciphertext i as its first operand (row i of ct is then undefined)."""
+    k = _value_kind(kind)
+    if isinstance(cts, (bytes, bytearray)) or not all(isinstance(c, bytes) for c in cts):
+        raise TypeError("upload_ciphertexts takes a sequence of bytes objects")
+    n = len(cts)
+    dev = torch.device("cuda", device)
+    torch.cuda.current_stream(dev).synchronize()  # the library writes ct on its own streams
+    ct = torch.empty((n, 2, 2, N), dtype=torch.int64, device=dev)
+    status = torch.zeros((n,), dtype=torch.int32)
+    ptrs = (ctypes.c_char_p * n)(*cts)  # pointers into the bytes objects themselves: no copy
+    lens = (ctypes.c_size_t * n)(*(len(c) for c in cts))
+    _check(_lib.lib().fhe_b200_upload_ciphertexts(device, k, ptrs, lens, n, ct.data_ptr(), status.data_ptr()))
+    return ct, status
+
+
+def download_ciphertexts(ct: torch.Tensor, kind: str):
+    """ct [n,2,2,4096] int64 on a CUDA device -> (list of n sunscreen Ciphertext bytes of `kind`, status [n] int32 host): byte
+    for byte what a c_fhe_* precompile of that kind returns for these words under the current zstd writer.  status[i] = -1
+    (and b"") where row i failed."""
+    k = _value_kind(kind)
+    dev = _dev(ct)
+    if ct.dtype != torch.int64 or ct.dim() != 4 or tuple(ct.shape[1:]) != (2, 2, N):
+        raise ValueError("download_ciphertexts: ct must be int64 [n, 2, 2, 4096]")
+    n = ct.shape[0]
+    torch.cuda.current_stream(dev).synchronize()  # the library copies on its own streams: ct must be complete
+    L = _lib.lib()
+    outs = (ctypes.c_void_p * n)()
+    lens = (ctypes.c_int64 * n)()
+    status = torch.zeros((n,), dtype=torch.int32)
+    _check(L.fhe_b200_download_ciphertexts(dev, k, ct.data_ptr(), n, outs, lens, status.data_ptr()))
+    result = []
+    for i in range(n):
+        result.append(ctypes.string_at(outs[i], lens[i]) if outs[i] else b"")
+        if outs[i]:
+            L.fhe_free(outs[i])
+    return result, status
+
+
 def frame_bytes() -> int:
     return int(_lib.lib().fhe_b200_frame_bytes())
 

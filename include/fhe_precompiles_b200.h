@@ -179,7 +179,8 @@ int32_t fhe_b200_mul_relin_host(int32_t device, const uint64_t *a, const uint64_
                                 size_t n);
 /* Same op on SERIALIZED operands. Operand i of an array is the zstd frame at frames + i * stride: the compressed body of a
  * ciphertext as this library serializes it (a "structured frame": fhe_b200_frame_bytes() = 82,054 bytes, at byte 148 of the
- * packed `Ciphertext`; what every precompile here returns and what chained calls carry). Frames cross PCIe as they are (5 bytes
+ * packed `Ciphertext`; what the precompiles here return under the structured writer, fhe_b200_set_zstd_writer(1) -- the default
+ * writer returns SEAL's libzstd frames, which fhe_b200_upload_ciphertexts takes). Frames cross PCIe as they are (5 bytes
  * per residue instead of 8), are validated and unpacked on the GPU, and result i is written as a frame at
  * out_frames + i * fhe_b200_frame_stride(). Pin the buffers for full PCIe rate. status[i]: 0 done; 1 an operand is not a
  * structured frame or fails SEAL's range checks (result undefined: send that call through c_fhe_mul_*); 2 the result is not
@@ -197,6 +198,24 @@ int32_t fhe_b200_mul_relin_frames(int32_t device, const uint8_t *a_frames, const
  * Replaces bincode::deserialize / serialize of a Ciphertext around a sequence of Runtime::run calls (fhe.rs:21-30). */
 int32_t fhe_b200_upload_frames(int32_t device, const uint8_t *frames, size_t stride, size_t n, uint64_t *d_words, int32_t *status);
 int32_t fhe_b200_download_frames(int32_t device, const uint64_t *d_words, size_t n, uint8_t *out_frames, int32_t *status);
+/* The same from and to the bytes callers actually hold: bincode(sunscreen::Ciphertext), what every c_fhe_* precompile returns.
+ * upload: n Ciphertexts of `kind` (host buffers cts[i] / lens[i], as a binary precompile receives them: SEAL's libzstd frames,
+ *   structured frames, zlib or uncompressed blobs) -> d_words [n][2][2][4096] on `device`.  status[i] (host): 0, or the lib.rs
+ *   code that c_fhe_add_cipherK_cipherK returns when ciphertext i is its first operand (3 bad framing / SEAL blob / residue >= q,
+ *   7 data_type is not kind's, size != 2 or NTT form).  The words of a rejected row are undefined.  Framing is read on the host;
+ *   large batches of libzstd frames are inflated on the GPU (as fhe_b200_batch does), and the GPU validates and unpacks every
+ *   ciphertext.
+ * download: d_words [n][2][2][4096] on `device` -> n malloc'd Ciphertexts of `kind` (release each with fhe_free).  Output i is
+ *   byte-identical to what a c_fhe_* precompile of that kind returns for a result with these words, under the current
+ *   fhe_b200_set_zstd_writer mode (testnet Params, compr_mode zstd): under the structured writer the GPU writes the complete
+ *   bytes; under the default writer the host cores compress with libzstd, as SEAL does.  status[i]: 0, or -1 when that row
+ *   failed (outputs[i] NULL, message in fhe_b200_last_error).
+ * `kind` is numbered as in fhe_b200_data_type_kind.  Both are synchronous and return 0, or -1 for an unknown kind, a missing
+ * device or a CUDA failure; n == 0 does nothing. */
+int32_t fhe_b200_upload_ciphertexts(int32_t device, int32_t kind, const uint8_t *const *cts, const size_t *lens, size_t n,
+                                    uint64_t *d_words, int32_t *status);
+int32_t fhe_b200_download_ciphertexts(int32_t device, int32_t kind, const uint64_t *d_words, size_t n, uint8_t **outputs,
+                                      int64_t *output_lengths, int32_t *status);
 size_t fhe_b200_frame_bytes(void);
 size_t fhe_b200_frame_stride(void);
 /* Integer-pipe peak of `device` in 1e12 multiply-adds/s, measured by a register-only microbenchmark
