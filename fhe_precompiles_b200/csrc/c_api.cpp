@@ -208,11 +208,11 @@ int64_t fhe_b200_batch(fhe_b200_call *calls, size_t n, int32_t host_threads) {
     if (nt == 0) nt = 1;
     if (const char *e = getenv("FHE_B200_BATCH_THREADS"))
         if (host_threads <= 0 && atoi(e) > 0) nt = (size_t)atoi(e);
-    size_t tile = Engine::get().tile_ops_for(n);
-    const size_t big = Engine::get().big_tile_ops_for(n);
+    size_t tile = Engine::get().tile_ops();
+    const size_t big = Engine::big_tile_ops_for(n);
     bool serial_loops = true;
     size_t budget = 0;  // big tiles: the batch's thread budget, divided among the tile workers for their per-call loops
-    if (Engine::get().device_codec() && big > tile && n >= 2 * big) {
+    if (big > tile) {
         // a large batch: few big tiles (each stages its calls on the whole host pool and launches thousands of operand frames
         // at once), a handful of them in flight so that one tile's host phases overlap another's device phases
         tile = big;

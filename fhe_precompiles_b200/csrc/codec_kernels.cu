@@ -217,15 +217,10 @@ size_t codec_work_bytes() { return sizeof(JobScratch); }
 
 cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs, int32_t *status, void *work,
                                  const uint8_t *prefix, u64 *dst_a, u64 *dst_b, int n_jobs, bool any_zstd, bool any_packed,
-                                 bool any_payload, cudaStream_t s, int phase) {
+                                 bool any_payload, cudaStream_t s) {
     if (n_jobs == 0) return cudaSuccess;
-    const bool had_zstd = any_zstd;
-    if (phase != kCodecUnpack) {
-        cudaError_t ce = cudaMemsetAsync(status, 0, (size_t)n_jobs * sizeof(int32_t), s);  // kJobPending
-        if (ce != cudaSuccess) return ce;
-    } else {
-        any_zstd = false;  // (decoded by the kCodecDecode call)
-    }
+    cudaError_t ce = cudaMemsetAsync(status, 0, (size_t)n_jobs * sizeof(int32_t), s);  // kJobPending
+    if (ce != cudaSuccess) return ce;
     if (any_zstd) {
         static std::atomic<int> configured{0};  // (per process; the attributes are per function and device-independent in effect)
         int dev = 0, sms = 148;
@@ -243,8 +238,7 @@ cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const
                                                                                                     (JobScratch *)work, n_jobs);
         g_codec_launches.fetch_add(4, std::memory_order_relaxed);
     }
-    if (phase == kCodecDecode) return cudaGetLastError();
-    if ((had_zstd || any_payload) && dst_a) {  // (the standalone inflate entry point stops at the payloads)
+    if ((any_zstd || any_payload) && dst_a) {  // (the standalone inflate entry point stops at the payloads)
         k_ct_unpack<<<dim3(n_jobs, kSplit), 256, 0, s>>>(payloads, jobs, status, prefix, dst_a, dst_b);
         g_codec_launches.fetch_add(1, std::memory_order_relaxed);
     }

@@ -29,12 +29,9 @@ struct CodecJob {
 
 size_t codec_work_bytes();  // decoder workspace per job
 // inflate + validate + unpack every job into dst_a / dst_b slots; status[j] = kJobOk or kJobFallback
-// `phase`: kCodecAll, or the two halves separately - kCodecDecode (clear status[], run the zstd decoder) and kCodecUnpack
-// (validate + unpack payloads and structured frames) - so that a tile can inflate part of its frames on the host between them
-enum : int { kCodecAll = 0, kCodecDecode = 1, kCodecUnpack = 2 };
 cudaError_t launch_codec_inflate(const uint8_t *frames, uint8_t *payloads, const CodecJob *jobs, int32_t *status, void *work,
                                  const uint8_t *prefix, uint64_t *dst_a, uint64_t *dst_b, int n_jobs, bool any_zstd,
-                                 bool any_packed, bool any_payload, cudaStream_t s, int phase = kCodecAll);
+                                 bool any_packed, bool any_payload, cudaStream_t s);
 // n result ciphertexts -> n structured frames (kPackedFrameStride apart); constant_flag[i] = 1 if the host must use libzstd instead
 cudaError_t launch_codec_pack(const uint64_t *words, uint8_t *frames, int32_t *constant_flag, const uint8_t *prefix, int n,
                               cudaStream_t s);

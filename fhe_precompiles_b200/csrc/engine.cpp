@@ -77,40 +77,6 @@ void testnet_params(uint8_t out[kParamsBytes]) {
     memcpy(out, w, 48);
     memset(out + 48, 0, 8);
 }
-// FHE_B200_TILE_PROFILE=<n >= 1>: wall time of binary_tile's phases summed over all tile workers, printed when the process exits;
-// the first n calls (warm-up: lanes, pinned buffers, key upload) are not counted
-struct TileProfile {
-    static constexpr int kPhases = 8;
-    std::atomic<uint64_t> ns[kPhases];
-    std::atomic<uint64_t> tiles{0}, calls{0}, seen{0};
-    uint64_t skip = 0;
-    bool on = false;
-    TileProfile() {
-        for (auto &v : ns) v = 0;
-        const char *e = getenv("FHE_B200_TILE_PROFILE");
-        on = e && atoll(e) >= 1;
-        skip = on ? (uint64_t)atoll(e) : 0;
-    }
-    ~TileProfile() {
-        if (!on || !tiles.load()) return;
-        static const char *names[kPhases] = {"unpack+key", "framing", "plan", "stage", "enqueue", "device wait", "wrap", "host pass"};
-        fprintf(stderr, "[fhe_b200 tile profile] %llu tiles, %llu calls; us per call (summed over workers):", (unsigned long long)tiles.load(),
-                (unsigned long long)calls.load());
-        for (int k = 0; k < kPhases; k++) fprintf(stderr, " %s %.1f", names[k], ns[k].load() * 1e-3 / (double)calls.load());
-        fprintf(stderr, "\n");
-    }
-};
-TileProfile g_tile_profile;
-struct PhaseClock {
-    std::chrono::steady_clock::time_point t = std::chrono::steady_clock::now();
-    bool counted = false;
-    void lap(int phase) {
-        if (!counted) return;
-        const auto now = std::chrono::steady_clock::now();
-        g_tile_profile.ns[phase] += (uint64_t)std::chrono::duration_cast<std::chrono::nanoseconds>(now - t).count();
-        t = now;
-    }
-};
 }  // namespace
 
 Engine &Engine::get() {
@@ -127,29 +93,6 @@ Engine::Engine() {
         throw std::runtime_error("fhe_b200: no CUDA device visible; this library has no CPU fallback");
     size_t max_dev = env_size("FHE_B200_MAX_DEVICES", (size_t)n_devices_);
     if ((size_t)n_devices_ > max_dev) n_devices_ = (int)max_dev;
-    {
-        const char *v = getenv("FHE_B200_HELPER_DECODE");
-        helper_decode_ = !(v && *v == '0');
-        v = getenv("FHE_B200_DEVICE_CODEC");
-        device_codec_ = !(v && *v == '0');
-        // libzstd-written operand frames of a tile are inflated on the GPU (codec_kernels.cu, zstd_plan3.cuh): 0 never, 1 always,
-        // 2 (default) when the tile brings at least FHE_B200_DEVICE_ZSTD_MIN_FRAMES of them.  fhe_b200_batch cuts a large batch
-        // into tiles of zstd_tile_ops() calls so that the default applies to it; single calls and small batches inflate on the
-        // host (a frame is a 16 k-step chain: ~3 ms on the GPU however few frames there are, 0.11 ms on a host core).
-        v = getenv("FHE_B200_DEVICE_ZSTD");
-        device_zstd_ = (v && *v == '1') ? 1 : (v && *v == '0') ? 0 : 2;
-        v = getenv("FHE_B200_CALL_GRAPHS");
-        call_graphs_ = !(v && *v == '0');
-    }
-    device_zstd_min_frames_ = env_size("FHE_B200_DEVICE_ZSTD_MIN_FRAMES", 128);
-    zstd_tile_ops_ = env_size("FHE_B200_ZSTD_TILE_OPS", 128);
-    zstd_tile_min_batch_ = env_size("FHE_B200_ZSTD_TILE_MIN_BATCH", 2048);
-    {
-        const char *v = getenv("FHE_B200_HOST_INFLATE_PCT");  // share of a tile's libzstd frames the host cores inflate meanwhile
-        host_inflate_pct_ = (v && *v) ? (size_t)std::min(100, std::max(0, atoi(v))) : 0;
-    }
-    big_tile_set_ = getenv("FHE_B200_BIG_TILE_OPS") != nullptr;
-    big_tile_ops_ = env_size("FHE_B200_BIG_TILE_OPS", 0);  // fixed big-tile size (0: never); default: engine.h big_tile_ops_for
     tile_ops_ = env_size("FHE_B200_TILE_OPS", 16);
     if (tile_ops_ < 1) tile_ops_ = 1;
     chunk_ops_ = env_size("FHE_B200_CHUNK_OPS", 4096);
@@ -868,7 +811,7 @@ CipherView result_view(Kind kind) {
 
 // Per ciphertext, on the host pool: bincode framing, data_type and the SEAL blob's header (a few hundred bytes).  Then, per chunk,
 // one job per ciphertext for launch_codec_inflate, which validates the 97-byte prefix and every residue and writes d_words:
-//   structured frame -> kJobPacked;  libzstd frame -> kJobZstd (device decoder) when the chunk brings device_zstd_min_frames_ of
+//   structured frame -> kJobPacked;  libzstd frame -> kJobZstd (device decoder) when the chunk brings kDeviceZstdMinFrames of
 //   them, else inflated here -> kJobPayload;  compr_mode none -> kJobPayload as it is;  zlib -> inflated here -> kJobPayload.
 // Staging of a chunk, the same on the host (pinned) and on the device: [frames | payloads], so that one copy moves both.  Every
 // ciphertext that is not accepted on that path -- and every one the device hands back -- is decoded by decode_ciphertext, whose
@@ -948,7 +891,7 @@ void Engine::upload_ciphertexts(int device, Kind kind, const uint8_t *const *cts
         // (B) the engine's rule for libzstd frames; then jobs: payloads first (payload slot = job), frames behind them
         size_t lib_frames = 0;
         for (size_t i = off; i < off + c; i++) lib_frames += route[i] == kZstd;
-        const bool dev_zstd = device_zstd_ == 1 || (device_zstd_ == 2 && lib_frames >= device_zstd_min_frames_);
+        const bool dev_zstd = lib_frames >= kDeviceZstdMinFrames;
         int jobs = 0;
         for (size_t i = off; i < off + c; i++) {
             if (route[i] == kZstd && !dev_zstd) route[i] = kPayload;
@@ -1210,7 +1153,7 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
     };
     // every size and pointer above is fixed for a given call shape on this lane (payload slots, structured frames and the
     // result frame have constant sizes), so the sequence is replayed as a CUDA graph: ~13 launches and copies become one
-    if (call_graphs_ && !timed) {
+    if (!timed) {
         cudaGraphExec_t exec = nullptr;
         for (const auto &g : lane->graphs)
             if (g.op == (int)it.op && g.shape == (int)it.shape && g.kind0 == kinds[0] && g.kind1 == kinds[1] && g.rk == d_rk) {
@@ -1278,7 +1221,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
     if (timed && !lane->ev[0])
         for (auto &e : lane->ev) cuda_throw(cudaEventCreate(&e), "cudaEventCreate");
 
-    if (cnt == 1 && device_codec_ && helper_decode_ && single_call_fast(lane, items[0], timed, t_start)) return;
+    if (cnt == 1 && single_call_fast(lane, items[0], timed, t_start)) return;
 
     // device work classes; ct-ct first so that the second operand array is one prefix of the slots
     enum Cls { kMulCt = 0, kAddCt, kSubCt, kMulPt, kAddPt, kSubCtPt, kSubPtCt };
@@ -1294,9 +1237,6 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
     std::vector<Prep> prep(cnt);
     std::vector<size_t> order;
     order.reserve(cnt);
-    PhaseClock pc;
-    if (g_tile_profile.on && g_tile_profile.seen.fetch_add(cnt) >= g_tile_profile.skip)
-        pc.counted = true, g_tile_profile.tiles++, g_tile_profile.calls += cnt;
 
     // pass 1, reference order (pack.rs:261-263): framing, then the public key (a ~400 KB comparison with the cached key per call:
     // shared with pool threads when the tile is large)
@@ -1322,7 +1262,6 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
     });
     for (size_t i = 0; i < cnt; i++)
         if (prep[i].live) order.push_back(i);
-    pc.lap(0);
     const double t_unpack = us_since(t_start);
     struct Run {
         int cls;
@@ -1363,7 +1302,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
     // compressed frames; the GPU inflates, validates, computes and packs the result frame.  Whatever is not perfectly
     // ordinary -- and every operand the strict device decoder hands back -- is left for the host pass below, which
     // reproduces the reference's checks and error codes in their order.
-    if (device_codec_ && cnt >= 2 && !order.empty()) {
+    if (cnt >= 2 && !order.empty()) {
         ensure_codec(lane);
         std::vector<Run> runs;
         std::vector<size_t> slot_item, rest;
@@ -1400,16 +1339,14 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             }
             g.clean = clean;
         });
-        pc.lap(1);
-        // (B) serial: slots, jobs and staging offsets.  libzstd-written frames go to the device decoder when it is on -- always
-        // (FHE_B200_DEVICE_ZSTD=1) or, by default, when the tile brings enough frames to fill the GPU -- except for the share
-        // the host cores inflate meanwhile (FHE_B200_HOST_INFLATE_PCT): both decoders work on the same tile at once.
+        // (B) serial: slots, jobs and staging offsets.  libzstd-written frames go to the device decoder when the tile brings
+        // enough of them to fill the GPU, else all of them are inflated on the host
         size_t lib_frames = 0;
         for (const Stg &g : stg)
             if (g.clean)
                 for (int k = 0; k < g.nct; k++) lib_frames += g.kinds[k] == 1;
-        const bool dev_zstd = device_zstd_ == 1 || (device_zstd_ == 2 && lib_frames >= device_zstd_min_frames_);
-        size_t slots = 0, ctct_slots = 0, fcur = 0, seen_lib = 0;
+        const bool dev_zstd = lib_frames >= kDeviceZstdMinFrames;
+        size_t slots = 0, ctct_slots = 0, fcur = 0;
         int njobs = 0;
         bool any_zstd = false, any_packed = false, any_payload = false;
         std::vector<size_t> slot_stg;
@@ -1425,13 +1362,8 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             g.slot = slots;
             g.job0 = njobs;
             for (int k = 0; k < g.nct; k++) {
-                bool host = g.kinds[k] == 1 && !dev_zstd;
-                if (g.kinds[k] == 1 && dev_zstd) {  // Bresenham split of the libzstd frames between host and device
-                    host = (seen_lib + 1) * host_inflate_pct_ / 100 != seen_lib * host_inflate_pct_ / 100;
-                    seen_lib++;
-                }
-                g.on_host[k] = host;
-                if (host) {
+                g.on_host[k] = g.kinds[k] == 1 && !dev_zstd;
+                if (g.on_host[k]) {
                     lane->h_jobs[njobs++] = CodecJob{0, 0, kJobPayload, (int32_t)slots, k};  // payload slot = job index
                     any_payload = true;
                     continue;
@@ -1448,10 +1380,9 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             slot_item.push_back(i);
             slot_stg.push_back(oi);
         }
-        pc.lap(2);
         if (slots) {
-            // (C) bytes into the pinned staging -- frames as they are, encoded scalars -- and the device decoder is started on the
-            // frames; (C2) the payloads the host inflates follow while the GPU decodes (hybrid tiles: FHE_B200_HOST_INFLATE_PCT)
+            // (C) bytes into the pinned staging -- frames as they are, encoded scalars; (C2) the frames cross to the device while
+            // the host inflates the libzstd frames of a tile that is too small for the device decoder
             const auto fail_slot = [&](Stg &g) {
                 g.bad = true;
                 for (int c = 0; c < g.nct; c++) lane->h_jobs[g.job0 + c].kind = kJobNone;  // the kernels skip it; its slot computes on stale data
@@ -1465,16 +1396,10 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
                 if (it.shape != Shape::CtCt && encode_scalar(it.kind, it.shape == Shape::CtPt ? p.sb : p.sa, lane->h_plain + k * kN) != kOk)
                     fail_slot(g);
             });
-            pc.lap(3);
-            const bool split_codec = any_zstd && any_payload;  // decode on the device first, inflate the host's share meanwhile
             if (njobs) {
                 if (fcur) cuda_throw(cudaMemcpyAsync(lane->d_frames, lane->h_frames, fcur, cudaMemcpyHostToDevice, s), "H2D frames");
                 cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)njobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
             }
-            if (split_codec)
-                cuda_throw(launch_codec_inflate(lane->d_frames, lane->d_payloads, lane->d_jobs, lane->d_status, lane->d_work, lane->d_prefix,
-                                                lane->d_a, lane->d_b, njobs, any_zstd, any_packed, any_payload, s, kCodecDecode),
-                           "codec decode");
             if (any_payload) {
                 std::atomic<bool> any_failed{false};
                 parallel_for(slots, 2, [&](size_t k) {
@@ -1508,8 +1433,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
                                            (slots - ctct_slots) * kN * 2, cudaMemcpyHostToDevice, s),
                            "H2D plain");
             cuda_throw(launch_codec_inflate(lane->d_frames, lane->d_payloads, lane->d_jobs, lane->d_status, lane->d_work, lane->d_prefix,
-                                            lane->d_a, lane->d_b, njobs, any_zstd, any_packed, any_payload, s,
-                                            split_codec ? kCodecUnpack : kCodecAll),
+                                            lane->d_a, lane->d_b, njobs, any_zstd, any_packed, any_payload, s),
                        "codec inflate");
             launch_runs(runs);
             int32_t *d_cflag = lane->d_status + 2 * lane->cap, *h_cflag = lane->h_status + 2 * lane->cap;
@@ -1524,9 +1448,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             if (njobs)
                 cuda_throw(cudaMemcpyAsync(lane->h_status, lane->d_status, (size_t)njobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s),
                            "D2H status");
-            pc.lap(4);
             cuda_throw(cudaStreamSynchronize(s), "stream sync");
-            pc.lap(5);
             // (D) in parallel: results into their own buffers; calls the device handed back are collected for the host pass
             std::vector<uint8_t> redo(slots, 0);
             parallel_for(slots, 4, [&](size_t k) {
@@ -1575,7 +1497,6 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
         }
         std::stable_sort(rest.begin(), rest.end(), by_class);
         order.swap(rest);
-        pc.lap(6);
     }
 
     // ---- host pass: operands into adjacent staging slots, class by class; a call that fails here gives its slot to the next
@@ -1591,7 +1512,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
         int32_t rc = 0;
         if (it.shape == Shape::CtCt) {
             CipherView vb;
-            if (cnt == 1 && helper_decode_) {
+            if (cnt == 1) {
                 // a single call: inflate the second operand on a pool thread while this one inflates the first (a tile
                 // already keeps every core busy).  If no pool thread is free the caller does both, in order.
                 int32_t rcs[2] = {0, 0};
@@ -1647,7 +1568,6 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
         TileItem &it = items[slot_item[k]];
         it.rc = encode_ciphertext(prep[slot_item[k]].va, lane->h_out + k * kCtWords, &it.out);
     }
-    pc.lap(7);
     if (timed) {
         CallBreakdown &b = tl_breakdown;
         float ms[3] = {0, 0, 0};

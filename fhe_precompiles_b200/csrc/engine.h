@@ -120,29 +120,24 @@ class Engine {
     void binary_tile(TileItem *items, size_t cnt);
     size_t tile_ops() const { return tile_ops_; }
     size_t lane_device_count() const { return lane_devices_.size(); }  // GPUs the byte surface spreads its lanes over
-    // tile size for a batch of n calls: large batches run in tiles big enough for the device zstd decoder to take their operand
-    // frames (device_zstd_ == 2), everything else in tile_ops_
-    size_t tile_ops_for(size_t n) const {
-        return (device_codec_ && device_zstd_ == 2 && n >= zstd_tile_min_batch_ && zstd_tile_ops_ > tile_ops_) ? zstd_tile_ops_ : tile_ops_;
-    }
     // the calling thread is one of many tile workers: binary_tile keeps its per-call loops on it instead of sharing them with the pool
     static void set_thread_serial_loops(bool on);
     // ... or may share them with at most `threads` - 1 pool threads (0: no limit): a batch divides its thread budget among its workers
     static void set_thread_loop_width(size_t threads);
-    // tile size of a large batch: big tiles put thousands of operand frames in flight per launch (the device zstd decoder's
-    // throughput comes from frames in flight) and their staging loops are shared with the host pool
-    // Big tiles: a large batch runs as a few tiles of this many calls, each staging its calls on the whole host pool and
-    // launching thousands of operand frames at once (the device zstd decoder's rate grows with the frames per launch: 183 k
-    // frames/s at 1,024, 431 k at 8,192).  FHE_B200_BIG_TILE_OPS fixes the size (0 there: never); by default a batch of
-    // >= 2,048 calls takes an eighth of itself, between 256 and 1,024 calls.
-    size_t big_tile_ops_for(size_t n) const {
-        if (big_tile_set_) return big_tile_ops_;
-        if (!(device_codec_ && device_zstd_ == 2 && n >= zstd_tile_min_batch_)) return 0;
+    // libzstd-written operand frames of a tile (or transfer chunk) are inflated on the GPU when it brings at least this many of
+    // them, else on the host: a frame is a 16 k-step chain, ~3 ms on the GPU however few frames there are, 0.11 ms on a host core
+    static constexpr size_t kDeviceZstdMinFrames = 128;
+    static constexpr size_t kZstdTileMinBatch = 2048;
+    // Big tiles: a batch of >= kZstdTileMinBatch calls runs as a few tiles of an eighth of itself, between 256 and 1,024 calls
+    // (0: smaller batches), each staging its calls on the whole host pool and launching thousands of operand frames at once (the
+    // device zstd decoder's rate grows with the frames per launch: 183 k frames/s at 1,024, 431 k at 8,192).  Never more than
+    // n / 2: a batch in big tiles has at least two of them.
+    static size_t big_tile_ops_for(size_t n) {
+        if (n < kZstdTileMinBatch) return 0;
         size_t b = 256;
         while (b < 1024 && 2 * b <= n / 8) b *= 2;
         return b;
     }
-    bool device_codec() const { return device_codec_; }
     // per-call phase timing of binary_tile (host clock around the codec phases, CUDA events around the copies and the
     // kernels on the lane's stream); off by default
     void set_call_timing(bool on) { call_timing_ = on; }
@@ -221,17 +216,8 @@ class Engine {
     void ensure_capacity(Lane *lane, size_t cap);
     void ensure_codec(Lane *lane);
     bool single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono::steady_clock::time_point t_start);
-    bool device_codec_ = true;  // FHE_B200_DEVICE_CODEC=0: tiles decode and encode everything on the host
-    bool call_graphs_ = true;   // FHE_B200_CALL_GRAPHS=0: the single-call fast path launches its kernels one by one
     void drop_graphs(Lane *lane);
-    // libzstd-written operand frames inflated on the GPU (codec_kernels.cu): 0 never, 1 always, 2 (default) when a tile brings at
-    // least device_zstd_min_frames_ of them; host_inflate_pct_ % of those frames are inflated by the host cores meanwhile
-    int device_zstd_ = 2;
-    size_t device_zstd_min_frames_ = 128, host_inflate_pct_ = 0;
-    size_t zstd_tile_ops_ = 128, zstd_tile_min_batch_ = 2048;
-    size_t tile_ops_ = 16, big_tile_ops_ = 0;
-    bool big_tile_set_ = false;
-    bool helper_decode_ = true;  // FHE_B200_HELPER_DECODE=0 turns the helper-thread inflate of single calls off
+    size_t tile_ops_ = 16;
     std::atomic<bool> call_timing_{false};
     std::vector<int> lane_devices_;
     Lane *acquire_lane();

@@ -1,8 +1,9 @@
 """Byte-surface throughput of a LARGE batch (fhe_b200_batch, mul_cipheri64_cipheri64, operands as SEAL writes them: libzstd level-3
-frames; every call carries its own copy of the public key) under the engine's staging knobs.  The library reads the knobs at
-load time, so every configuration runs in its own process:
+frames; every call carries its own copy of the public key) by batch size and result writer (FHE_B200_ZSTD_WRITER).  Below 2,048
+calls the batch runs in 16-call tiles whose operands the host inflates, from 2,048 on in big tiles whose operands the GPU
+inflates.  Every configuration runs in its own process:
     python scripts/byte_surface_bench.py                      # sweep (parent)
-    python scripts/byte_surface_bench.py child <calls>        # one configuration, knobs from the environment
+    python scripts/byte_surface_bench.py child <calls>        # one configuration, writer from the environment
 Checks the first and last results against the single-call symbol."""
 import ctypes
 import json
@@ -54,8 +55,8 @@ def child(n: int, distinct: int = int(os.environ.get("BSB_DISTINCT", "256"))) ->
         for i in range(n):
             L.fhe_free(arr[i].output)
         rates.append(n / dt_)
-    knobs = {k: os.environ.get(k, "default") for k in ("FHE_B200_DEVICE_ZSTD", "FHE_B200_HOST_INFLATE_PCT", "FHE_B200_BIG_TILE_OPS", "FHE_B200_ZSTD_WRITER")}
-    print(json.dumps({"calls": n, "cores": os.cpu_count(), **knobs, "calls_per_s_by_rep": [round(r) for r in rates], "best": round(max(rates[1:]))}),
+    writer = os.environ.get("FHE_B200_ZSTD_WRITER", "default")
+    print(json.dumps({"calls": n, "cores": os.cpu_count(), "FHE_B200_ZSTD_WRITER": writer, "calls_per_s_by_rep": [round(r) for r in rates], "best": round(max(rates[1:]))}),
           flush=True)
 
 
@@ -63,20 +64,7 @@ def main() -> None:
     if len(sys.argv) > 1 and sys.argv[1] == "child":
         child(int(sys.argv[2]))
         return
-    sweeps = [
-        (4096, {}),                                                                       # default: 16-call tiles, host inflate
-        (4096, {"FHE_B200_BIG_TILE_OPS": "512"}),                                          # big tiles, host inflate only
-        (4096, {"FHE_B200_BIG_TILE_OPS": "512", "FHE_B200_DEVICE_ZSTD": "2", "FHE_B200_HOST_INFLATE_PCT": "0"}),   # device inflate only
-        (4096, {"FHE_B200_BIG_TILE_OPS": "512", "FHE_B200_DEVICE_ZSTD": "2"}),             # hybrid, 35 % on the host
-        (4096, {"FHE_B200_BIG_TILE_OPS": "1024", "FHE_B200_DEVICE_ZSTD": "2", "FHE_B200_HOST_INFLATE_PCT": "50"}),
-        (8192, {"FHE_B200_BIG_TILE_OPS": "1024", "FHE_B200_DEVICE_ZSTD": "2", "FHE_B200_HOST_INFLATE_PCT": "25"}),
-    ]
-    if len(sys.argv) > 1 and sys.argv[1] == "sweep3":  # the fourth-generation device decoder (zstd_plan3.cuh)
-        sweeps = [(4096, {}), (4096, {"FHE_B200_ZSTD_WRITER": "1"})]
-        for big in ("128", "256", "512"):
-            for pct in ("0", "25", "50"):
-                sweeps.append((8192, {"FHE_B200_BIG_TILE_OPS": big, "FHE_B200_DEVICE_ZSTD": "2", "FHE_B200_HOST_INFLATE_PCT": pct,
-                                      "FHE_B200_DEVICE_ZSTD_MIN_FRAMES": "64", "FHE_B200_ZSTD_WRITER": "1"}))
+    sweeps = [(n, {"FHE_B200_ZSTD_WRITER": w}) for w in ("0", "1") for n in (1024, 2048, 4096, 8192)]
     for n, env in sweeps:
         e = dict(os.environ)
         e.update(env)

@@ -391,49 +391,65 @@ def test_device_zstd_inflate_matches_libzstd(dev):
             assert payloads[i] is not None and raw[i * size : (i + 1) * size] == payloads[i], i
 
 
-@pytest.mark.parametrize("host_pct,writer", [("0", "0"), ("40", "0"), ("40", "1")])
-def test_batch_tiles_with_device_zstd(keys, host_pct, writer):
-    """FHE_B200_DEVICE_ZSTD=1: the operands of a tile are inflated by the device decoder (k_zd2_parse / k_zd3_seq / k_zd3_exec)
-    instead of libzstd - all of them, or (FHE_B200_HOST_INFLATE_PCT=40) a hybrid tile whose device share is decoded while the
-    host inflates the rest.  Same statuses and bytes as the single-call symbols, with either result writer (the knobs are read
-    when the engine starts, hence the subprocess)."""
-    import subprocess
-    import sys
+def test_big_tiles_with_device_zstd_equal_single_calls(keys):
+    """24 distinct calls - add / sub / mul x ct.ct / ct.pt / pt.ct over the four kinds, second operands alternately libzstd and
+    structured frames, some operands truncated or with a flipped bit - repeated to 2,064 calls.  fhe_b200_batch runs them as
+    eight 256-call big tiles whose libzstd operand frames the device decoder (k_zd2_parse / k_zd3_huf / k_zd3_seq / k_zd3_exec)
+    inflates, and a 16-call tail that libzstd inflates on the host.  Under either result writer every status and every output
+    byte equals the single-call symbols'."""
+    from fhe_precompiles_b200 import FHE, FheError, _lib, pack
 
-    code = """
-import sys
-sys.path.insert(0, %r); sys.path.insert(0, %r)
-import numpy as np
-from helpers import KeySet, KINDS, encrypt_value, precompile_name, value_of
-from fhe_precompiles_b200 import FHE, FheError, pack
-from oracle import formats as F
-keys = KeySet.load()
-calls = []
-for i in range(24):
-    kind = KINDS[i %% 4]; op = ("add", "sub", "mul")[(i // 4) %% 3]; shape = ("ctct", "ctpt", "ptct")[(i // 2) %% 3]
-    va, vb = value_of(kind, 2 + i %% 5), value_of(kind, 1 + i %% 3)
-    ca = F.make_ciphertext(kind, encrypt_value(keys, kind, va, 700 + i)).to_bytes()
-    cb = F.make_ciphertext(kind, encrypt_value(keys, kind, vb, 800 + i)).to_bytes(structured=bool(i & 1))
-    sc = pack.SERIALIZE[kind](vb)
-    args = {"ctct": (ca, cb), "ctpt": (ca, sc), "ptct": (sc, cb)}[shape]
-    data = pack.pack_binary_operation(keys.pub_bytes, *args)
-    if i %% 9 == 4: data = pack.pack_binary_operation(keys.pub_bytes, ca[:-9], args[1]) if shape != "ptct" else data[:11]
-    if i %% 9 == 7:
-        bad = bytearray(ca); bad[-300] ^= 0x10
-        data = pack.pack_binary_operation(keys.pub_bytes, bytes(bad), args[1]) if shape != "ptct" else data
-    calls.append((precompile_name(op, shape, kind), data))
-want = []
-for name, data in calls:
-    try: want.append((0, getattr(FHE, name)(data)))
-    except FheError as e: want.append((e.code, b""))
-got = FHE.run_batch(calls, host_threads=2)
-assert got == want, [(g[0], w[0]) for g, w in zip(got, want)]
-assert sum(1 for st, _ in want if st == 0) >= 16 and any(st for st, _ in want)
-print("device-zstd tiles ok")
-""" % (ROOT, os.path.join(ROOT, "tests"))
-    env = dict(os.environ, FHE_B200_DEVICE_ZSTD="1", FHE_B200_HOST_INFLATE_PCT=host_pct, FHE_B200_ZSTD_WRITER=writer)
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "device-zstd tiles ok" in r.stdout, r.stdout + r.stderr
+    calls, shapes = [], []
+    for i in range(24):
+        kind, op, shape = KINDS[i % 4], ("add", "sub", "mul")[(i // 4) % 3], ("ctct", "ctpt", "ptct")[(i // 2) % 3]
+        va, vb = value_of(kind, 2 + i % 5), value_of(kind, 1 + i % 3)
+        ca = F.make_ciphertext(kind, encrypt_value(keys, kind, va, 700 + i)).to_bytes()
+        cb = F.make_ciphertext(kind, encrypt_value(keys, kind, vb, 800 + i)).to_bytes(structured=bool(i & 1))
+        sc = pack.SERIALIZE[kind](vb)
+        args = {"ctct": (ca, cb), "ctpt": (ca, sc), "ptct": (sc, cb)}[shape]
+        data = pack.pack_binary_operation(keys.pub_bytes, *args)
+        if i % 9 == 4:
+            data = pack.pack_binary_operation(keys.pub_bytes, ca[:-9], args[1]) if shape != "ptct" else data[:11]
+        if i % 9 == 7:
+            bad = bytearray(ca)
+            bad[-300] ^= 0x10
+            data = pack.pack_binary_operation(keys.pub_bytes, bytes(bad), args[1]) if shape != "ptct" else data
+        calls.append((precompile_name(op, shape, kind), data))
+        shapes.append(shape)
+
+    def seal_frames(shape: str, data: bytes) -> int:
+        """libzstd frames this call brings to its tile's count: none unless every ciphertext operand parses, else the operands
+        whose bytes are exactly what SEAL writes (never more than the engine counts)"""
+        try:
+            _, a, b = F.unpack_binary_operation(data)
+            cts = {"ctct": (a, b), "ctpt": (a,), "ptct": (b,)}[shape]
+            return sum(F.Ciphertext.from_bytes(c).to_bytes() == c for c in cts)
+        except (EOFError, ValueError):
+            return 0
+
+    n, tile = 2064, 256  # Engine::big_tile_ops_for(2,064)
+    frames = [seal_frames(sh, data) for sh, (_, data) in zip(shapes, calls)]
+    per_tile = [sum(frames[i % 24] for i in range(t, t + tile)) for t in range(0, n - tile + 1, tile)]
+    assert len(per_tile) == 8 and min(per_tile) >= 128, per_tile  # kDeviceZstdMinFrames: every big tile decodes on the device
+    assert n - 8 * tile == 16  # the tail brings at most 32 frames: the host inflates them
+    batch = [calls[i % 24] for i in range(n)]
+    L = _lib.lib()
+    prev = L.fhe_b200_set_zstd_writer(-1)
+    try:
+        for mode in (0, 1):
+            L.fhe_b200_set_zstd_writer(mode)
+            want = []
+            for name, data in calls:
+                try:
+                    want.append((0, getattr(FHE, name)(data)))
+                except FheError as e:
+                    want.append((e.code, b""))
+            assert sum(1 for st, _ in want if st == 0) >= 16 and any(st for st, _ in want)
+            got = FHE.run_batch(batch)
+            wrong = [i for i in range(n) if got[i] != want[i % 24]]
+            assert not wrong, (mode, [(i, got[i][0], want[i % 24][0]) for i in wrong[:8]])
+    finally:
+        L.fhe_b200_set_zstd_writer(prev)
 
 
 def test_writer_modes_and_chained_calls(keys):
