@@ -5,7 +5,7 @@
 #include <chrono>
 #include <functional>
 
-#include "codec_kernels.h"
+#include "codec_stage.h"
 #include "host_pool.h"
 
 #include <cstdlib>
@@ -120,6 +120,7 @@ void Engine::create_lanes() {
         for (size_t i = 0; i < lanes_per_dev; i++) {
             std::unique_ptr<Lane> l(new Lane());
             l->device = d;
+            l->d_prefix = ct_prefix(d);
             cuda_throw(cudaStreamCreateWithFlags(&l->stream, cudaStreamNonBlocking), "cudaStreamCreate");
             ensure_capacity(l.get(), 1);
             lanes_.push_back(std::move(l));
@@ -171,13 +172,21 @@ void Engine::ensure_codec(Lane *l) {
     cuda_throw(cudaMalloc((void **)&l->d_jobs, ops * sizeof(CodecJob)), "cudaMalloc");
     cuda_throw(cudaMalloc((void **)&l->d_status, 3 * cap * sizeof(int32_t)), "cudaMalloc");
     cuda_throw(cudaMalloc(&l->d_work, ops * codec_work_bytes()), "cudaMalloc");
-    if (!l->d_prefix) {
+    l->codec_cap = cap;
+}
+
+// the caller has selected `device`
+const uint8_t *Engine::ct_prefix(int device) {
+    std::lock_guard<std::mutex> lk(prefix_mu_);
+    if (d_prefix_.size() < (size_t)n_devices_) d_prefix_.resize((size_t)n_devices_, nullptr);
+    uint8_t *&p = d_prefix_[(size_t)device];
+    if (!p) {
         uint8_t prefix[kCtPrefixBytes];
         canonical_ct_prefix(prefix);
-        cuda_throw(cudaMalloc((void **)&l->d_prefix, kCtPrefixBytes), "cudaMalloc");
-        cuda_throw(cudaMemcpy(l->d_prefix, prefix, kCtPrefixBytes, cudaMemcpyHostToDevice), "upload prefix");
+        cuda_throw(cudaMalloc((void **)&p, kCtPrefixBytes), "cudaMalloc");
+        cuda_throw(cudaMemcpy(p, prefix, kCtPrefixBytes, cudaMemcpyHostToDevice), "upload prefix");
     }
-    l->codec_cap = cap;
+    return p;
 }
 
 Lane *Engine::acquire_lane() {
@@ -567,15 +576,14 @@ static size_t pipe_chunk(size_t off, size_t n, size_t chunk) {
     return chunk;
 }
 
-void Engine::mul_relin_host(int device, const uint64_t *a, const uint64_t *b, const uint64_t *rk, uint64_t *out, size_t n) {
-    device_context(device);
+Engine::HostPipe &Engine::host_pipe(int device, const uint64_t *rk, std::unique_lock<std::mutex> &lk) {
     {
-        std::lock_guard<std::mutex> lk(arena_mu_);
+        std::lock_guard<std::mutex> g(arena_mu_);
         if (pipes_.size() < (size_t)n_devices_) pipes_.resize((size_t)n_devices_);
         if (!pipes_[(size_t)device]) pipes_[(size_t)device].reset(new HostPipe());
     }
     HostPipe &P = *pipes_[(size_t)device];
-    std::lock_guard<std::mutex> lk(P.mu);
+    lk = std::unique_lock<std::mutex>(P.mu);
     if (!P.chunk) P.chunk = env_size("FHE_B200_PIPE_CHUNK_OPS", 256);  // (sweep r2w: frames 282 k ops/s at 256 against 260 k at 128; limb arrays equal within noise)
     if (!P.d_rk) cuda_throw(cudaMalloc((void **)&P.d_rk, kRkWords * 8), "cudaMalloc(rk)");
     for (auto &sl : P.slot) {
@@ -587,9 +595,15 @@ void Engine::mul_relin_host(int device, const uint64_t *a, const uint64_t *b, co
             cuda_throw(cudaMalloc((void **)&sl.d_scratch, P.chunk * kScratchLimbsPerOp * kN * 8), "cudaMalloc");
         }
     }
-    P.ready = true;
     cuda_throw(cudaMemcpyAsync(P.d_rk, rk, kRkWords * 8, cudaMemcpyHostToDevice, P.slot[0].stream), "H2D rk");
     cuda_throw(cudaStreamSynchronize(P.slot[0].stream), "sync rk");
+    return P;
+}
+
+void Engine::mul_relin_host(int device, const uint64_t *a, const uint64_t *b, const uint64_t *rk, uint64_t *out, size_t n) {
+    device_context(device);
+    std::unique_lock<std::mutex> lk;
+    HostPipe &P = host_pipe(device, rk, lk);
     size_t i = 0;
     for (size_t off = 0, c = 0; off < n; off += c, i++) {
         c = pipe_chunk(off, n, P.chunk);
@@ -614,30 +628,11 @@ void Engine::mul_relin_frames(int device, const uint8_t *fa, const uint8_t *fb, 
                               size_t n, int32_t *status) {
     if (stride < kPackedFrameBytes) throw std::runtime_error("mul_relin_frames: stride smaller than a structured frame");
     device_context(device);
-    {
-        std::lock_guard<std::mutex> lk(arena_mu_);
-        if (pipes_.size() < (size_t)n_devices_) pipes_.resize((size_t)n_devices_);
-        if (!pipes_[(size_t)device]) pipes_[(size_t)device].reset(new HostPipe());
-    }
-    HostPipe &P = *pipes_[(size_t)device];
-    std::lock_guard<std::mutex> lk(P.mu);
-    if (!P.chunk) P.chunk = env_size("FHE_B200_PIPE_CHUNK_OPS", 256);  // (sweep r2w: frames 282 k ops/s at 256 against 260 k at 128; limb arrays equal within noise)
-    if (!P.d_rk) cuda_throw(cudaMalloc((void **)&P.d_rk, kRkWords * 8), "cudaMalloc(rk)");
-    if (!P.d_prefix) {
-        uint8_t prefix[kCtPrefixBytes];
-        canonical_ct_prefix(prefix);
-        cuda_throw(cudaMalloc((void **)&P.d_prefix, kCtPrefixBytes), "cudaMalloc");
-        cuda_throw(cudaMemcpy(P.d_prefix, prefix, kCtPrefixBytes, cudaMemcpyHostToDevice), "upload prefix");
-    }
+    const uint8_t *prefix = ct_prefix(device);
+    std::unique_lock<std::mutex> lk;
+    HostPipe &P = host_pipe(device, rk, lk);
     const size_t region = P.chunk * stride;  // one operand array of a chunk
     for (auto &sl : P.slot) {
-        if (!sl.stream) cuda_throw(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking), "cudaStreamCreate");
-        if (!sl.d_a) {
-            cuda_throw(cudaMalloc((void **)&sl.d_a, P.chunk * kCtWords * 8), "cudaMalloc");
-            cuda_throw(cudaMalloc((void **)&sl.d_b, P.chunk * kCtWords * 8), "cudaMalloc");
-            cuda_throw(cudaMalloc((void **)&sl.d_out, P.chunk * kCtWords * 8), "cudaMalloc");
-            cuda_throw(cudaMalloc((void **)&sl.d_scratch, P.chunk * kScratchLimbsPerOp * kN * 8), "cudaMalloc");
-        }
         if (sl.frame_stride != stride) {  // staging [pad | a frames | pad | b frames | pad], jobs interleaved a0 b0 a1 b1 ...
             cudaFree(sl.d_frames), cudaFree(sl.d_outframes), cudaFree(sl.d_jobs), cudaFree(sl.d_status);
             cuda_throw(cudaMalloc((void **)&sl.d_frames, 2 * region + 3 * kFramePad), "cudaMalloc");
@@ -654,14 +649,11 @@ void Engine::mul_relin_frames(int device, const uint8_t *fa, const uint8_t *fb, 
             sl.frame_stride = stride;
         }
     }
-    P.ready = true;
     if (P.h_status_cap < 3 * n) {
         if (P.h_status) cudaFreeHost(P.h_status);
         cuda_throw(cudaMallocHost((void **)&P.h_status, 3 * n * sizeof(int32_t)), "cudaMallocHost");
         P.h_status_cap = 3 * n;
     }
-    cuda_throw(cudaMemcpyAsync(P.d_rk, rk, kRkWords * 8, cudaMemcpyHostToDevice, P.slot[0].stream), "H2D rk");
-    cuda_throw(cudaStreamSynchronize(P.slot[0].stream), "sync rk");
     size_t k = 0;
     for (size_t off = 0, c = 0; off < n; off += c, k++) {
         c = pipe_chunk(off, n, P.chunk);
@@ -671,13 +663,13 @@ void Engine::mul_relin_frames(int device, const uint8_t *fa, const uint8_t *fb, 
         const size_t bytes = (c - 1) * stride + kPackedFrameBytes;
         cuda_throw(cudaMemcpyAsync(sl.d_frames + kFramePad, fa + off * stride, bytes, cudaMemcpyHostToDevice, s), "H2D frames a");
         cuda_throw(cudaMemcpyAsync(sl.d_frames + 2 * kFramePad + region, fb + off * stride, bytes, cudaMemcpyHostToDevice, s), "H2D frames b");
-        cuda_throw(launch_codec_inflate(sl.d_frames, nullptr, sl.d_jobs, sl.d_status, nullptr, P.d_prefix, sl.d_a, sl.d_b, (int)(2 * c), false,
+        cuda_throw(launch_codec_inflate(sl.d_frames, nullptr, sl.d_jobs, sl.d_status, nullptr, prefix, sl.d_a, sl.d_b, (int)(2 * c), false,
                                         true, false, s),
                    "frame unpack");
         ScratchMap m(sl.d_scratch, P.chunk);
         enqueue_mul(sl.d_a, sl.d_b, m, c, s, false);
         enqueue_relin(m.c3, P.d_rk, sl.d_out, m, c, s, false);
-        cuda_throw(launch_codec_pack(sl.d_out, sl.d_outframes, sl.d_status + 2 * P.chunk, P.d_prefix, (int)c, s), "frame pack");
+        cuda_throw(launch_codec_pack(sl.d_out, sl.d_outframes, sl.d_status + 2 * P.chunk, prefix, (int)c, s), "frame pack");
         cuda_throw(cudaMemcpyAsync(fout + off * kPackedFrameStride, sl.d_outframes, (c - 1) * kPackedFrameStride + kPackedFrameBytes,
                                    cudaMemcpyDeviceToHost, s),
                    "D2H frames");
@@ -706,12 +698,6 @@ Engine::XferPipe &Engine::xfer_pipe(int device, size_t n, size_t slot_bytes) {
         if (!xfers_[(size_t)device]) xfers_[(size_t)device].reset(new XferPipe());
     }
     XferPipe &X = *xfers_[(size_t)device];
-    if (!X.d_prefix) {
-        uint8_t prefix[kCtPrefixBytes];
-        canonical_ct_prefix(prefix);
-        cuda_throw(cudaMalloc((void **)&X.d_prefix, kCtPrefixBytes), "cudaMalloc");
-        cuda_throw(cudaMemcpy(X.d_prefix, prefix, kCtPrefixBytes, cudaMemcpyHostToDevice), "upload prefix");
-    }
     for (auto &sl : X.slot) {
         if (!sl.stream) {
             cuda_throw(cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking), "cudaStreamCreate");
@@ -741,6 +727,7 @@ void Engine::upload_frames(int device, const uint8_t *frames, size_t stride, siz
     if (n == 0) return;
     if (stride < kPackedFrameBytes) throw std::runtime_error("upload_frames: stride smaller than a structured frame");
     device_context(device);
+    const uint8_t *prefix = ct_prefix(device);
     XferPipe &X = xfer_pipe(device, n, kXferChunk * stride + 2 * kFramePad);
     std::lock_guard<std::mutex> lk(X.mu);
     size_t k = 0;
@@ -753,7 +740,7 @@ void Engine::upload_frames(int device, const uint8_t *frames, size_t stride, siz
         cuda_throw(cudaMemcpyAsync(sl.d_jobs, sl.h_jobs, c * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
         cuda_throw(cudaMemcpyAsync(sl.d_frames + kFramePad, frames + off * stride, (c - 1) * stride + kPackedFrameBytes, cudaMemcpyHostToDevice, s),
                    "H2D frames");
-        cuda_throw(launch_codec_inflate(sl.d_frames, nullptr, sl.d_jobs, sl.d_status, nullptr, X.d_prefix, d_words + off * kCtWords, nullptr,
+        cuda_throw(launch_codec_inflate(sl.d_frames, nullptr, sl.d_jobs, sl.d_status, nullptr, prefix, d_words + off * kCtWords, nullptr,
                                         (int)c, false, true, false, s),
                    "frame unpack");
         cuda_throw(cudaMemcpyAsync(X.h_status + off, sl.d_status, c * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H status");
@@ -768,6 +755,7 @@ void Engine::upload_frames(int device, const uint8_t *frames, size_t stride, siz
 void Engine::download_frames(int device, const uint64_t *d_words, size_t n, uint8_t *out_frames, int32_t *status) {
     if (n == 0) return;
     device_context(device);
+    const uint8_t *prefix = ct_prefix(device);
     XferPipe &X = xfer_pipe(device, n, kXferChunk * kPackedFrameStride);
     std::lock_guard<std::mutex> lk(X.mu);
     size_t k = 0;
@@ -775,7 +763,7 @@ void Engine::download_frames(int device, const uint64_t *d_words, size_t n, uint
         const size_t c = std::min(kXferChunk, n - off);
         XferSlot &sl = X.slot[k & 1];
         cudaStream_t s = sl.stream;
-        cuda_throw(launch_codec_pack(d_words + off * kCtWords, sl.d_frames, sl.d_status, X.d_prefix, (int)c, s), "frame pack");
+        cuda_throw(launch_codec_pack(d_words + off * kCtWords, sl.d_frames, sl.d_status, prefix, (int)c, s), "frame pack");
         cuda_throw(cudaMemcpyAsync(out_frames + off * kPackedFrameStride, sl.d_frames, (c - 1) * kPackedFrameStride + kPackedFrameBytes,
                                    cudaMemcpyDeviceToHost, s),
                    "D2H frames");
@@ -807,28 +795,55 @@ CipherView result_view(Kind kind) {
     v.compr_mode = 2;
     return v;
 }
+
+// One ciphertext operand as the codec staging sees it: its bincode framing, data_type and SEAL header (a few hundred bytes).
+struct Operand {
+    Route route = Route::Reject;
+    int32_t rc = kOk;   // Reject: the framing's error code
+    CipherView view;    // compr_mode: the blob's
+    Span blob, frame;   // the SEAL blob; its zstd frame (Zstd, Packed)
+};
+// The route of ciphertext `ct` as an operand of `kind`.  Which routes take the device path is the caller's choice.
+Route classify_operand(Span ct, Kind kind, Operand *op) {
+    if ((op->rc = parse_ciphertext_framing(ct, &op->view, &op->blob))) return op->route = Route::Reject;
+    uint8_t compr = 0;
+    const int cls = data_type_matches(op->view.data_type, kind) ? classify_ciphertext_blob(op->blob, &op->frame, &compr) : -1;
+    if (cls < 0) return op->route = Route::Host;
+    op->view.compr_mode = compr;
+    if (cls == 0) return op->route = Route::Blob;
+    if (op->frame.n + 2 * kFramePad > kFrameSlotBytes) return op->route = Route::Host;
+    return op->route = cls == 2 ? Route::Packed : Route::Zstd;
+}
+// Operand `op`, planned as job j of `jobs`, into the pinned staging: a frame copied to frames + its offset, or a payload the
+// host inflates into payloads + j * kPayloadStride.  False if the inflate fails.
+bool stage_operand(const Operand &op, const CodecJob *jobs, int32_t j, uint8_t *frames, uint8_t *payloads) {
+    if (jobs[j].kind == kJobPayload) {
+        uint8_t *dst = payloads + (size_t)j * kPayloadStride;
+        return op.route == Route::Blob ? inflate_ct_blob(op.blob, dst) : inflate_ct_payload(op.frame, dst);
+    }
+    memcpy(frames + jobs[j].src_off, op.frame.p, op.frame.n);
+    return true;
+}
 }  // namespace
 
-// Per ciphertext, on the host pool: bincode framing, data_type and the SEAL blob's header (a few hundred bytes).  Then, per chunk,
-// one job per ciphertext for launch_codec_inflate, which validates the 97-byte prefix and every residue and writes d_words:
-//   structured frame -> kJobPacked;  libzstd frame -> kJobZstd (device decoder) when the chunk brings kDeviceZstdMinFrames of
-//   them, else inflated here -> kJobPayload;  compr_mode none -> kJobPayload as it is;  zlib -> inflated here -> kJobPayload.
-// Staging of a chunk, the same on the host (pinned) and on the device: [frames | payloads], so that one copy moves both.  Every
-// ciphertext that is not accepted on that path -- and every one the device hands back -- is decoded by decode_ciphertext, whose
+// Per ciphertext, on the host pool: classify_operand.  Then, per chunk, one job per ciphertext the device path accepts (Blob,
+// Zstd, Packed), laid out by plan_codec_jobs, for launch_codec_inflate, which validates the 97-byte prefix and every residue
+// and writes d_words.  Staging of a chunk, the same on the host (pinned) and on the device: [frames | payloads], so that one
+// copy moves both.  Every other ciphertext -- and every one the device hands back -- is decoded by decode_ciphertext, whose
 // code is the status (the device never turns a valid ciphertext into a rejection).
 void Engine::upload_ciphertexts(int device, Kind kind, const uint8_t *const *cts, const size_t *lens, size_t n, uint64_t *d_words,
                                 int32_t *status) {
     if (n == 0) return;
     device_context(device);
+    const uint8_t *prefix = ct_prefix(device);
     const size_t frames_cap = kXferChunk * kFrameSlotBytes, stage_bytes = frames_cap + kXferChunk * kPayloadStride;
     XferPipe &X = xfer_pipe(device, n, stage_bytes);
     std::lock_guard<std::mutex> lk(X.mu);
     for (auto &sl : X.slot) cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");  // (idle unless a call before this one threw)
     xfer_host_stage(X, stage_bytes);
-    enum : uint8_t { kDone, kHost, kPacked, kZstd, kPayload };  // route of a ciphertext
-    std::vector<uint8_t> route(n);
-    std::vector<Span> blob(n), frame(n);
-    std::vector<size_t> at(n);  // staging offset of a frame, or the payload job of a ciphertext
+    std::vector<Operand> ops(n);
+    std::vector<StageOperand> sop(kXferChunk);
+    std::vector<int32_t> job(kXferChunk);
     std::vector<int32_t> st(n, 0);
     struct Pending {
         size_t off = 0, c = 0;
@@ -842,10 +857,10 @@ void Engine::upload_ciphertexts(int device, Kind kind, const uint8_t *const *cts
         XferSlot &sl = X.slot[b];
         p.live = false;
         for (int j = 0; j < p.jobs; j++)
-            if (X.h_status[p.off + j] == kJobFallback) route[p.off + (size_t)sl.h_jobs[j].slot] = kHost;
+            if (X.h_status[p.off + j] == kJobFallback) ops[p.off + (size_t)sl.h_jobs[j].slot].route = Route::Host;
         std::vector<size_t> host;
         for (size_t i = p.off; i < p.off + p.c; i++)
-            if (route[i] == kHost) host.push_back(i);
+            if (ops[i].route == Route::Host) host.push_back(i);
         if (host.empty()) return;
         std::vector<std::vector<uint64_t>> words(host.size());
         parallel_for(host.size(), 1, [&](size_t h) {
@@ -874,64 +889,32 @@ void Engine::upload_ciphertexts(int device, Kind kind, const uint8_t *const *cts
         }
         // (A) framing, data_type and blob header of every ciphertext of the chunk
         parallel_for(c, 8, [&](size_t t) {
-            const size_t i = off + t;
-            CipherView v;
-            const int32_t rc = parse_ciphertext_framing(Span{cts[i], lens[i]}, &v, &blob[i]);
-            if (rc) {
-                st[i] = rc, route[i] = kDone;
-                return;
-            }
-            uint8_t compr = 0;
-            const int cls = data_type_matches(v.data_type, kind) ? classify_ciphertext_blob(blob[i], &frame[i], &compr) : -1;
-            if (cls == 2) route[i] = kPacked;
-            else if (cls == 1) route[i] = frame[i].n + 2 * kFramePad <= kFrameSlotBytes ? kZstd : kHost;
-            else if (cls == 0) route[i] = kPayload;
-            else route[i] = kHost;  // a wrong data_type or a malformed SEAL header: decode_ciphertext has the code
+            Operand &o = ops[off + t];
+            if (classify_operand(Span{cts[off + t], lens[off + t]}, kind, &o) == Route::Reject) st[off + t] = o.rc;
+            sop[t] = StageOperand{o.route, o.frame.n, (int32_t)t, 0};
         });
-        // (B) the engine's rule for libzstd frames; then jobs: payloads first (payload slot = job), frames behind them
-        size_t lib_frames = 0;
-        for (size_t i = off; i < off + c; i++) lib_frames += route[i] == kZstd;
-        const bool dev_zstd = lib_frames >= kDeviceZstdMinFrames;
-        int jobs = 0;
-        for (size_t i = off; i < off + c; i++) {
-            if (route[i] == kZstd && !dev_zstd) route[i] = kPayload;
-            if (route[i] != kPayload) continue;
-            at[i] = (size_t)jobs;
-            sl.h_jobs[jobs++] = CodecJob{0, 0, kJobPayload, (int32_t)(i - off), 0};
-        }
-        const int payload_jobs = jobs;
-        size_t fcur = 0;
-        bool any_zstd = false, any_packed = false;
-        for (size_t i = off; i < off + c; i++) {
-            if (route[i] != kPacked && route[i] != kZstd) continue;
-            at[i] = fcur + kFramePad;
-            sl.h_jobs[jobs++] = CodecJob{at[i], (uint32_t)frame[i].n, route[i] == kPacked ? kJobPacked : kJobZstd, (int32_t)(i - off), 0};
-            (route[i] == kPacked ? any_packed : any_zstd) = true;
-            fcur += (frame[i].n + 2 * kFramePad + 15) & ~(size_t)15;
-        }
-        const size_t pay_base = (fcur + 255) & ~(size_t)255;
-        // (C) frames into the staging as they are, payloads inflated (or copied) into their slots
+        // (B) the jobs; (C) frames into the staging as they are, payloads inflated (or copied) into their slots
+        const StagePlan plan = plan_codec_jobs(sop.data(), c, sl.h_jobs, job.data());
+        const size_t pay_base = (plan.frame_bytes + 255) & ~(size_t)255;
         parallel_for(c, 2, [&](size_t t) {
-            const size_t i = off + t;
-            if (route[i] == kPacked || route[i] == kZstd) {
-                memcpy(sl.h_stage + at[i], frame[i].p, frame[i].n);
-            } else if (route[i] == kPayload && !inflate_ct_blob(blob[i], sl.h_stage + pay_base + at[i] * kPayloadStride)) {
-                route[i] = kHost;
-                sl.h_jobs[at[i]].kind = kJobNone;
+            if (job[t] >= 0 && !stage_operand(ops[off + t], sl.h_jobs, job[t], sl.h_stage, sl.h_stage + pay_base)) {
+                ops[off + t].route = Route::Host;
+                sl.h_jobs[job[t]].kind = kJobNone;
             }
         });
         // (D) one copy of the staging, the jobs, the codec kernels straight into d_words, the job status back
-        if (jobs) {
-            const size_t bytes = payload_jobs ? pay_base + (size_t)payload_jobs * kPayloadStride : fcur;
-            if (any_zstd && !sl.d_work) cuda_throw(cudaMalloc(&sl.d_work, kXferChunk * codec_work_bytes()), "cudaMalloc");
-            cuda_throw(cudaMemcpyAsync(sl.d_jobs, sl.h_jobs, (size_t)jobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
+        if (plan.jobs) {
+            const size_t bytes = plan.payloads ? pay_base + (size_t)plan.payloads * kPayloadStride : plan.frame_bytes;
+            if (plan.any_zstd && !sl.d_work) cuda_throw(cudaMalloc(&sl.d_work, kXferChunk * codec_work_bytes()), "cudaMalloc");
+            cuda_throw(cudaMemcpyAsync(sl.d_jobs, sl.h_jobs, (size_t)plan.jobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
             cuda_throw(cudaMemcpyAsync(sl.d_frames, sl.h_stage, bytes, cudaMemcpyHostToDevice, s), "H2D ciphertexts");
-            cuda_throw(launch_codec_inflate(sl.d_frames, sl.d_frames + pay_base, sl.d_jobs, sl.d_status, sl.d_work, X.d_prefix,
-                                            d_words + off * kCtWords, nullptr, jobs, any_zstd, any_packed, payload_jobs > 0, s),
+            cuda_throw(launch_codec_inflate(sl.d_frames, sl.d_frames + pay_base, sl.d_jobs, sl.d_status, sl.d_work, prefix,
+                                            d_words + off * kCtWords, nullptr, plan.jobs, plan.any_zstd, plan.any_packed, plan.payloads > 0, s),
                        "ciphertext unpack");
-            cuda_throw(cudaMemcpyAsync(X.h_status + off, sl.d_status, (size_t)jobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H status");
+            cuda_throw(cudaMemcpyAsync(X.h_status + off, sl.d_status, (size_t)plan.jobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s),
+                       "D2H status");
         }
-        pend[b] = Pending{off, c, jobs, true};
+        pend[b] = Pending{off, c, plan.jobs, true};
     }
     for (int b = 0; b < 2; b++) {
         const int oldest = (int)((k + (size_t)b) & 1);  // (in chunk order)
@@ -955,6 +938,7 @@ void Engine::download_ciphertexts(int device, Kind kind, const uint64_t *d_words
     const size_t head = wrapped_ciphertext_size(view, kPackedFrameBytes) - kPackedFrameBytes, whole = head + kPackedFrameBytes;
     if (head > (size_t)kPackHeadMax) throw std::runtime_error("download_ciphertexts: data_type too long");
     const size_t row = structured ? (whole + 15) & ~(size_t)15 : kCtWords * 8;
+    const uint8_t *prefix = ct_prefix(device);
     XferPipe &X = xfer_pipe(device, n, kXferChunk * row);
     std::lock_guard<std::mutex> lk(X.mu);
     for (auto &sl : X.slot) cuda_throw(cudaStreamSynchronize(sl.stream), "xfer sync");  // (idle unless a call before this one threw)
@@ -1015,7 +999,7 @@ void Engine::download_ciphertexts(int device, Kind kind, const uint64_t *d_words
         cudaStream_t s = sl.stream;
         if (pend[b].live) finish(b);
         if (structured) {
-            cuda_throw(launch_codec_pack(d_words + off * kCtWords, sl.d_frames, row, X.d_head, (int)head, sl.d_status, X.d_prefix, (int)c, s),
+            cuda_throw(launch_codec_pack(d_words + off * kCtWords, sl.d_frames, row, X.d_head, (int)head, sl.d_status, prefix, (int)c, s),
                        "ciphertext pack");
             cuda_throw(cudaMemcpyAsync(sl.h_stage, sl.d_frames, (c - 1) * row + whole, cudaMemcpyDeviceToHost, s), "D2H ciphertexts");
             cuda_throw(cudaMemcpyAsync(X.h_status + off, sl.d_status, c * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H flags");
@@ -1064,30 +1048,21 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
     if (unpack_binary_operation(it.in, &pk, &sa, &sb)) return false;
     const int nct = it.shape == Shape::CtCt ? 2 : 1;
     const Span cts[2] = {it.shape == Shape::PtCt ? sb : sa, sb};
-    CipherView views[2];
-    Span frames[2];
-    int kinds[2] = {0, 0};
+    Operand ops[2];
+    StageOperand sop[2];
     for (int k = 0; k < nct; k++) {
-        Span blob;
-        uint8_t compr = 0;
-        if (parse_ciphertext_framing(cts[k], &views[k], &blob) != kOk || !data_type_matches(views[k].data_type, it.kind)) return false;
-        kinds[k] = classify_ciphertext_blob(blob, &frames[k], &compr);
-        if (kinds[k] < 1 || frames[k].n + 2 * kFramePad > kFrameSlotBytes) return false;
-        views[k].compr_mode = compr;
+        const Route r = classify_operand(cts[k], it.kind, &ops[k]);
+        if (r != Route::Zstd && r != Route::Packed) return false;
+        sop[k] = StageOperand{r, ops[k].frame.n, 0, k};
     }
     if (zstd_writer() != 1) return false;
     ensure_codec(lane);
     cudaStream_t s = lane->stream;
 
-    // operand k is job k: payload slot k (libzstd frames, inflated here) or a structured frame copied as it is
-    const size_t frame_off[2] = {kFramePad, kFramePad + kFrameSlotBytes};  // fixed places: the copies below are replayed as a graph
-    const auto stage = [&](int k) -> bool {
-        if (kinds[k] == 2) {
-            memcpy(lane->h_frames + frame_off[k], frames[k].p, frames[k].n);
-            return true;
-        }
-        return inflate_ct_payload(frames[k], lane->h_payloads + (size_t)k * kPayloadStride);
-    };
+    // libzstd frames are inflated here (two never reach kDeviceZstdMinFrames), and a structured frame has one size: the plan,
+    // and so every copy below, is fixed for a pair of routes and is replayed as a graph
+    int32_t job[2];
+    const StagePlan plan = plan_codec_jobs(sop, (size_t)nct, lane->h_jobs, job);
     const bool need_relin = it.op == Op::Mul && it.shape == Shape::CtCt;
     const uint64_t *d_rk = nullptr;
     KeyPin pin;
@@ -1097,7 +1072,7 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
     const std::function<void()> work = [&] {  // tasks: first operand, second operand (ct x ct only), key comparison
         for (int t; (t = next.fetch_add(1)) < 3;) {
             if (t == 2) key_rc = relin_key(pk, lane->device, &d_rk, need_relin, &pin);
-            else if (t < nct) staged[t] = stage(t);
+            else if (t < nct) staged[t] = stage_operand(ops[t], lane->h_jobs, job[t], lane->h_frames, lane->h_payloads);
         }
     };
     HostPool::get().run((size_t)nct, work);
@@ -1105,31 +1080,19 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
     if (it.shape != Shape::CtCt && encode_scalar(it.kind, it.shape == Shape::CtPt ? sb : sa, lane->h_plain) != kOk) return false;
     const double t_decode = us_since(t_start);
 
-    bool any_payload = false, any_packed = false;
-    for (int k = 0; k < nct; k++) {
-        lane->h_jobs[k] = CodecJob{frame_off[k], (uint32_t)frames[k].n, kinds[k] == 2 ? kJobPacked : kJobPayload, 0, k};
-        (kinds[k] == 2 ? any_packed : any_payload) = true;
-    }
     int32_t *d_cflag = lane->d_status + nct, *h_cflag = lane->h_status + nct;  // right behind the job status: one copy back
     const auto enqueue = [&](bool ev) {
         if (ev) cudaEventRecord(lane->ev[0], s);
         cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)nct * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
-        for (int k = 0; k < nct; k++)
-            if (kinds[k] == 2)  // a structured frame has one size
-                cuda_throw(cudaMemcpyAsync(lane->d_frames + frame_off[k] - kFramePad, lane->h_frames + frame_off[k] - kFramePad,
-                                           kPackedFrameBytes + 2 * kFramePad, cudaMemcpyHostToDevice, s),
-                           "H2D frame");
-        if (any_payload) {  // slots 0 and 1 are adjacent: one copy covers both when both are payloads
-            const int first = kinds[0] == 2 ? 1 : 0, last = (nct == 2 && kinds[1] != 2) ? 1 : 0;
-            if (last >= first)
-                cuda_throw(cudaMemcpyAsync(lane->d_payloads + (size_t)first * kPayloadStride, lane->h_payloads + (size_t)first * kPayloadStride,
-                                           (size_t)(last - first + 1) * kPayloadStride, cudaMemcpyHostToDevice, s),
-                           "H2D payloads");
-        }
+        if (plan.frame_bytes)
+            cuda_throw(cudaMemcpyAsync(lane->d_frames, lane->h_frames, plan.frame_bytes, cudaMemcpyHostToDevice, s), "H2D frames");
+        if (plan.payloads)
+            cuda_throw(cudaMemcpyAsync(lane->d_payloads, lane->h_payloads, (size_t)plan.payloads * kPayloadStride, cudaMemcpyHostToDevice, s),
+                       "H2D payloads");
         if (it.shape != Shape::CtCt) cuda_throw(cudaMemcpyAsync(lane->d_plain, lane->h_plain, kN * 2, cudaMemcpyHostToDevice, s), "H2D plain");
         if (ev) cudaEventRecord(lane->ev[1], s);
         cuda_throw(launch_codec_inflate(lane->d_frames, lane->d_payloads, lane->d_jobs, lane->d_status, lane->d_work, lane->d_prefix, lane->d_a,
-                                        lane->d_b, nct, false, any_packed, any_payload, s),
+                                        lane->d_b, nct, plan.any_zstd, plan.any_packed, plan.payloads > 0, s),
                    "codec unpack");
         if (it.shape == Shape::CtCt) {
             if (it.op == Op::Mul) {
@@ -1151,12 +1114,12 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
         cuda_throw(cudaMemcpyAsync(lane->h_status, lane->d_status, (size_t)(nct + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H status");
         if (ev) cudaEventRecord(lane->ev[3], s);
     };
-    // every size and pointer above is fixed for a given call shape on this lane (payload slots, structured frames and the
-    // result frame have constant sizes), so the sequence is replayed as a CUDA graph: ~13 launches and copies become one
+    // every size and pointer above is fixed for a given call shape and pair of routes on this lane (the result frame has a
+    // constant size too), so the sequence is replayed as a CUDA graph: ~13 launches and copies become one
     if (!timed) {
         cudaGraphExec_t exec = nullptr;
         for (const auto &g : lane->graphs)
-            if (g.op == (int)it.op && g.shape == (int)it.shape && g.kind0 == kinds[0] && g.kind1 == kinds[1] && g.rk == d_rk) {
+            if (g.op == (int)it.op && g.shape == (int)it.shape && g.route0 == (int)ops[0].route && g.route1 == (int)ops[1].route && g.rk == d_rk) {
                 exec = g.exec;
                 count_launches(g.launches);
             }
@@ -1175,7 +1138,7 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
             cuda_throw(cudaStreamEndCapture(s, &graph), "end capture");
             cuda_throw(cudaGraphInstantiate(&exec, graph, 0), "graph instantiate");
             cudaGraphDestroy(graph);
-            lane->graphs.push_back(Lane::CallGraph{(int)it.op, (int)it.shape, kinds[0], kinds[1], d_rk, exec,
+            lane->graphs.push_back(Lane::CallGraph{(int)it.op, (int)it.shape, (int)ops[0].route, (int)ops[1].route, d_rk, exec,
                                                    launch_count() + codec_launch_count() - before});
         }
         cuda_throw(cudaGraphLaunch(exec, s), "graph launch");
@@ -1189,9 +1152,9 @@ bool Engine::single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono:
     if (h_cflag[0]) {  // constant result (a transparent ciphertext): the host writer's libzstd path
         cuda_throw(cudaMemcpyAsync(lane->h_out, lane->d_out, kCtWords * 8, cudaMemcpyDeviceToHost, s), "D2H");
         cuda_throw(cudaStreamSynchronize(s), "stream sync");
-        it.rc = encode_ciphertext(views[0], lane->h_out, &it.out);
+        it.rc = encode_ciphertext(ops[0].view, lane->h_out, &it.out);
     } else {
-        wrap_ciphertext_blob(views[0], lane->h_outframes, kPackedFrameBytes, &it.out);
+        wrap_ciphertext_blob(ops[0].view, lane->h_outframes, kPackedFrameBytes, &it.out);
         it.rc = kOk;
     }
     if (timed) {
@@ -1307,49 +1270,31 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
         std::vector<Run> runs;
         std::vector<size_t> slot_item, rest;
         const bool pack_on_device = zstd_writer() == 1;
-        // (A) per call, in parallel: bincode framing, type check, classification of the SEAL blobs
+        // (A) per call, in parallel: classify_operand; a call takes the device path when all its operands are Zstd or Packed
         struct Stg {
             bool clean = false;
-            int nct = 0, kinds[2] = {0, 0};
-            Span frames[2];
-            CipherView views[2];
-            bool on_host[2] = {false, false};  // libzstd-written frame inflated on the host (else staged for the device decoder)
-            int job0 = 0;
-            size_t slot = 0, off[2] = {0, 0};
-            std::atomic<bool> bad{false};      // staging failed: the host pass redoes the call
+            int nct = 0;
+            Operand ops[2];
+            size_t op0 = 0;                // its first operand in the plan: operand c is staged as job[op0 + c]
+            std::atomic<bool> bad{false};  // staging failed: the host pass redoes the call
         };
         std::vector<Stg> stg(order.size());
         parallel_for(order.size(), 8, [&](size_t oi) {
             const size_t i = order[oi];
             TileItem &it = items[i];
-            Prep &p = prep[i];
             Stg &g = stg[oi];
-            bool clean = p.key_rc == 0;
-            const Span cts[2] = {it.shape == Shape::PtCt ? p.sb : p.sa, p.sb};
-            const int want_ct = it.shape == Shape::CtCt ? 2 : 1;
-            for (int k = 0; clean && k < want_ct; k++) {
-                Span blob;
-                uint8_t compr = 0;
-                clean = parse_ciphertext_framing(cts[k], &g.views[k], &blob) == kOk && data_type_matches(g.views[k].data_type, it.kind);
-                if (!clean) break;
-                g.kinds[k] = classify_ciphertext_blob(blob, &g.frames[k], &compr);
-                clean = g.kinds[k] >= 1 && g.frames[k].n + 2 * kFramePad <= kFrameSlotBytes;
-                g.views[k].compr_mode = compr;
-                g.nct++;
+            const Span cts[2] = {it.shape == Shape::PtCt ? prep[i].sb : prep[i].sa, prep[i].sb};
+            g.nct = it.shape == Shape::CtCt ? 2 : 1;
+            g.clean = prep[i].key_rc == 0;
+            for (int k = 0; g.clean && k < g.nct; k++) {
+                const Route r = classify_operand(cts[k], it.kind, &g.ops[k]);
+                g.clean = r == Route::Zstd || r == Route::Packed;
             }
-            g.clean = clean;
         });
-        // (B) serial: slots, jobs and staging offsets.  libzstd-written frames go to the device decoder when the tile brings
-        // enough of them to fill the GPU, else all of them are inflated on the host
-        size_t lib_frames = 0;
-        for (const Stg &g : stg)
-            if (g.clean)
-                for (int k = 0; k < g.nct; k++) lib_frames += g.kinds[k] == 1;
-        const bool dev_zstd = lib_frames >= kDeviceZstdMinFrames;
-        size_t slots = 0, ctct_slots = 0, fcur = 0;
-        int njobs = 0;
-        bool any_zstd = false, any_packed = false, any_payload = false;
+        // (B) serial: slots, then the jobs of every clean call's operands
+        size_t slots = 0, ctct_slots = 0;
         std::vector<size_t> slot_stg;
+        std::vector<StageOperand> sop;
         for (size_t oi = 0; oi < order.size(); oi++) {
             const size_t i = order[oi];
             Stg &g = stg[oi];
@@ -1358,21 +1303,9 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
                 rest.push_back(i);
                 continue;
             }
-            p.va = g.views[0];
-            g.slot = slots;
-            g.job0 = njobs;
-            for (int k = 0; k < g.nct; k++) {
-                g.on_host[k] = g.kinds[k] == 1 && !dev_zstd;
-                if (g.on_host[k]) {
-                    lane->h_jobs[njobs++] = CodecJob{0, 0, kJobPayload, (int32_t)slots, k};  // payload slot = job index
-                    any_payload = true;
-                    continue;
-                }
-                g.off[k] = fcur + kFramePad;
-                lane->h_jobs[njobs++] = CodecJob{g.off[k], (uint32_t)g.frames[k].n, g.kinds[k] == 2 ? kJobPacked : kJobZstd, (int32_t)slots, k};
-                (g.kinds[k] == 2 ? any_packed : any_zstd) = true;
-                fcur += (g.frames[k].n + 2 * kFramePad + 15) & ~(size_t)15;
-            }
+            p.va = g.ops[0].view;
+            g.op0 = sop.size();
+            for (int k = 0; k < g.nct; k++) sop.push_back(StageOperand{g.ops[k].route, g.ops[k].frame.n, (int32_t)slots, k});
             const uint64_t *rk = p.cls == kMulCt ? p.d_rk : nullptr;
             if (runs.empty() || runs.back().cls != p.cls || runs.back().d_rk != rk) runs.push_back(Run{p.cls, rk, slots, slots});
             runs.back().end = ++slots;
@@ -1380,60 +1313,53 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             slot_item.push_back(i);
             slot_stg.push_back(oi);
         }
+        std::vector<int32_t> job(sop.size());
+        const StagePlan plan = plan_codec_jobs(sop.data(), sop.size(), lane->h_jobs, job.data());
         if (slots) {
             // (C) bytes into the pinned staging -- frames as they are, encoded scalars; (C2) the frames cross to the device while
             // the host inflates the libzstd frames of a tile that is too small for the device decoder
             const auto fail_slot = [&](Stg &g) {
                 g.bad = true;
-                for (int c = 0; c < g.nct; c++) lane->h_jobs[g.job0 + c].kind = kJobNone;  // the kernels skip it; its slot computes on stale data
+                for (int c = 0; c < g.nct; c++) lane->h_jobs[job[g.op0 + c]].kind = kJobNone;  // the kernels skip it; its slot computes on stale data
             };
             parallel_for(slots, 2, [&](size_t k) {
                 Stg &g = stg[slot_stg[k]];
                 TileItem &it = items[slot_item[k]];
                 Prep &p = prep[slot_item[k]];
                 for (int c = 0; c < g.nct; c++)
-                    if (!g.on_host[c]) memcpy(lane->h_frames + g.off[c], g.frames[c].p, g.frames[c].n);
+                    if (lane->h_jobs[job[g.op0 + c]].kind != kJobPayload)
+                        stage_operand(g.ops[c], lane->h_jobs, job[g.op0 + c], lane->h_frames, lane->h_payloads);
                 if (it.shape != Shape::CtCt && encode_scalar(it.kind, it.shape == Shape::CtPt ? p.sb : p.sa, lane->h_plain + k * kN) != kOk)
                     fail_slot(g);
             });
-            if (njobs) {
-                if (fcur) cuda_throw(cudaMemcpyAsync(lane->d_frames, lane->h_frames, fcur, cudaMemcpyHostToDevice, s), "H2D frames");
-                cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)njobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
-            }
-            if (any_payload) {
+            if (plan.frame_bytes)
+                cuda_throw(cudaMemcpyAsync(lane->d_frames, lane->h_frames, plan.frame_bytes, cudaMemcpyHostToDevice, s), "H2D frames");
+            cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)plan.jobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
+            if (plan.payloads) {
                 std::atomic<bool> any_failed{false};
                 parallel_for(slots, 2, [&](size_t k) {
                     Stg &g = stg[slot_stg[k]];
                     if (g.bad) return;
-                    for (int c = 0; c < g.nct; c++)
-                        if (g.on_host[c] && !inflate_ct_payload(g.frames[c], lane->h_payloads + (size_t)(g.job0 + c) * kPayloadStride)) {
+                    for (int c = 0; c < g.nct; c++) {
+                        const int32_t j = job[g.op0 + c];
+                        if (lane->h_jobs[j].kind == kJobPayload && !stage_operand(g.ops[c], lane->h_jobs, j, lane->h_frames, lane->h_payloads)) {
                             fail_slot(g);
                             any_failed = true;
                             break;
                         }
+                    }
                 });
                 if (any_failed)  // (the first copy of the job list may or may not have seen the cleared kinds: either is fine)
-                    cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)njobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
-            }
-            // payloads inflated on the host: one copy per run of adjacent payload slots
-            for (int j0 = 0; j0 < njobs;) {
-                if (lane->h_jobs[j0].kind != kJobPayload) {
-                    j0++;
-                    continue;
-                }
-                int j1 = j0 + 1;
-                while (j1 < njobs && lane->h_jobs[j1].kind == kJobPayload) j1++;
-                cuda_throw(cudaMemcpyAsync(lane->d_payloads + (size_t)j0 * kPayloadStride, lane->h_payloads + (size_t)j0 * kPayloadStride,
-                                           (size_t)(j1 - j0) * kPayloadStride, cudaMemcpyHostToDevice, s),
+                    cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)plan.jobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
+                cuda_throw(cudaMemcpyAsync(lane->d_payloads, lane->h_payloads, (size_t)plan.payloads * kPayloadStride, cudaMemcpyHostToDevice, s),
                            "H2D payloads");
-                j0 = j1;
             }
             if (slots > ctct_slots)
                 cuda_throw(cudaMemcpyAsync(lane->d_plain + ctct_slots * kN, lane->h_plain + ctct_slots * kN,
                                            (slots - ctct_slots) * kN * 2, cudaMemcpyHostToDevice, s),
                            "H2D plain");
             cuda_throw(launch_codec_inflate(lane->d_frames, lane->d_payloads, lane->d_jobs, lane->d_status, lane->d_work, lane->d_prefix,
-                                            lane->d_a, lane->d_b, njobs, any_zstd, any_packed, any_payload, s),
+                                            lane->d_a, lane->d_b, plan.jobs, plan.any_zstd, plan.any_packed, plan.payloads > 0, s),
                        "codec inflate");
             launch_runs(runs);
             int32_t *d_cflag = lane->d_status + 2 * lane->cap, *h_cflag = lane->h_status + 2 * lane->cap;
@@ -1445,9 +1371,8 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             } else {
                 cuda_throw(cudaMemcpyAsync(lane->h_out, lane->d_out, slots * kCtWords * 8, cudaMemcpyDeviceToHost, s), "D2H");
             }
-            if (njobs)
-                cuda_throw(cudaMemcpyAsync(lane->h_status, lane->d_status, (size_t)njobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s),
-                           "D2H status");
+            cuda_throw(cudaMemcpyAsync(lane->h_status, lane->d_status, (size_t)plan.jobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s),
+                       "D2H status");
             cuda_throw(cudaStreamSynchronize(s), "stream sync");
             // (D) in parallel: results into their own buffers; calls the device handed back are collected for the host pass
             std::vector<uint8_t> redo(slots, 0);
@@ -1455,7 +1380,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
                 const size_t i = slot_item[k];
                 Stg &g = stg[slot_stg[k]];
                 bool ok = !g.bad;
-                for (int j = g.job0; ok && j < g.job0 + g.nct; j++) ok = lane->h_status[j] != kJobFallback;
+                for (int c = 0; ok && c < g.nct; c++) ok = lane->h_status[job[g.op0 + c]] != kJobFallback;
                 if (!ok) {
                     redo[k] = 1;
                     return;

@@ -42,7 +42,7 @@ struct Lane {
     // device codec staging for tiles (allocated when a tile first uses it): compressed operand frames in, structured frames out
     size_t codec_cap = 0;
     uint8_t *h_frames = nullptr, *d_frames = nullptr, *h_payloads = nullptr, *d_payloads = nullptr, *h_outframes = nullptr, *d_outframes = nullptr;
-    uint8_t *d_prefix = nullptr;
+    const uint8_t *d_prefix = nullptr;  // the engine's canonical ciphertext prefix on this lane's device
     struct CodecJob *h_jobs = nullptr, *d_jobs = nullptr;
     int32_t *h_status = nullptr, *d_status = nullptr;  // [2 * cap] job status, then [cap] constant-result flags
     void *d_work = nullptr;
@@ -50,7 +50,7 @@ struct Lane {
     // CUDA graphs of the single-call fast path (copies + codec kernels + arithmetic), captured once per call shape and relin
     // key on this lane's buffers; dropped whenever the buffers are reallocated
     struct CallGraph {
-        int op, shape, kind0, kind1;
+        int op, shape, route0, route1;
         const uint64_t *rk;
         cudaGraphExec_t exec;
         uint64_t launches;  // kernels inside, for the launch counter
@@ -124,9 +124,6 @@ class Engine {
     static void set_thread_serial_loops(bool on);
     // ... or may share them with at most `threads` - 1 pool threads (0: no limit): a batch divides its thread budget among its workers
     static void set_thread_loop_width(size_t threads);
-    // libzstd-written operand frames of a tile (or transfer chunk) are inflated on the GPU when it brings at least this many of
-    // them, else on the host: a frame is a 16 k-step chain, ~3 ms on the GPU however few frames there are, 0.11 ms on a host core
-    static constexpr size_t kDeviceZstdMinFrames = 128;
     static constexpr size_t kZstdTileMinBatch = 2048;
     // Big tiles: a batch of >= kZstdTileMinBatch calls runs as a few tiles of an eighth of itself, between 256 and 1,024 calls
     // (0: smaller batches), each staging its calls on the whole host pool and launching thousands of operand frames at once (the
@@ -250,16 +247,20 @@ class Engine {
         size_t frame_stride = 0;
     };
     struct HostPipe {
-        bool ready = false;
         size_t chunk = 0;
         uint64_t *d_rk = nullptr;
-        uint8_t *d_prefix = nullptr;
         int32_t *h_status = nullptr;  // pinned, 3 per op of the largest call so far
         size_t h_status_cap = 0;
         PipeSlot slot[kPipeSlots];
         std::mutex mu;
     };
     std::vector<std::unique_ptr<HostPipe>> pipes_;
+    // the device's host pipeline with its streams and per-slot chunk buffers, `rk` uploaded; returns with `lk` holding its mu
+    HostPipe &host_pipe(int device, const uint64_t *rk, std::unique_lock<std::mutex> &lk);
+    // the 97 bytes every valid ciphertext payload starts with (canonical_ct_prefix), on `device`: the codec kernels check them
+    std::vector<uint8_t *> d_prefix_;
+    std::mutex prefix_mu_;
+    const uint8_t *ct_prefix(int device);
     // staging of upload_frames / download_frames: two slots per device, alternating chunks
     struct XferSlot {
         cudaStream_t stream = nullptr;
@@ -274,7 +275,6 @@ class Engine {
         void *d_work = nullptr;
     };
     struct XferPipe {
-        uint8_t *d_prefix = nullptr;
         uint8_t *d_head = nullptr;  // download_ciphertexts: the envelope in front of every structured frame (kPackHeadMax bytes)
         int32_t *h_status = nullptr;
         size_t h_status_cap = 0;
