@@ -279,17 +279,6 @@ __global__ void __launch_bounds__(kThreads, 3) k_ext_ntt_d(u64 *__restrict__ ntt
         default: ntt_dual_body<2>(limb, smem, t); break;
     }
 }
-// one lane of the dyadic tensor: operands in [0, 4s) -> product(s) mod s in [0, 2s)
-template <int NP>
-__device__ __forceinline__ u32 dual_mulsum(const u32 (&x)[NP], const u32 (&y)[NP], u32 s, u32 mu61) {
-    u64 P = 0;
-#pragma unroll
-    for (int k = 0; k < NP; k++) {
-        const u32 a = csub32(csub32(x[k], 2 * s), s), b = csub32(csub32(y[k], 2 * s), s);  // canonical: a b < 2^60
-        P = mad_wide(a, b, P);
-    }
-    return csub32(barrett61(P, mu61, s), 2 * s);
-}
 // the dyadic tensor of dual word D for output polynomial d + its inverse transform, left in registers (lanes in [0, 2s))
 template <int D, bool kTrailSync>
 __device__ __forceinline__ void tensor_intt_dual_regs(const u64 *__restrict__ nb, int d, u64 (&v)[1][8], u64 *smem, int t) {

@@ -154,6 +154,17 @@ __device__ __forceinline__ u32 shoup32(u32 x, u32 w, u32 ws, u32 s) { return x *
 __device__ __forceinline__ u32 csub32(u32 x, u32 m) { return min(x, x - m); }                                // [0, 2m) -> [0, m)
 // V < 2^61 -> V mod s in [0, 4s): q^ = floor(floor(V / 2^29) mu / 2^32), mu = floor(2^61 / s), is low by at most 3
 __device__ __forceinline__ u32 barrett61(u64 V, u32 mu61, u32 s) { return (u32)V - __umulhi((u32)(V >> 29), mu61) * s; }
+// one lane of the dyadic tensor: operands in [0, 4s) -> product(s) mod s in [0, 2s)
+template <int NP>
+__device__ __forceinline__ u32 dual_mulsum(const u32 (&x)[NP], const u32 (&y)[NP], u32 s, u32 mu61) {
+    u64 P = 0;
+#pragma unroll
+    for (int k = 0; k < NP; k++) {
+        const u32 a = csub32(csub32(x[k], 2 * s), s), b = csub32(csub32(y[k], 2 * s), s);  // canonical: a b < 2^60
+        P = mad_wide(a, b, P);
+    }
+    return csub32(barrett61(P, mu61, s), 2 * s);
+}
 // forward butterfly on both lanes: inputs in [0, 4s), outputs in [0, 4s)
 template <class M>
 __device__ __forceinline__ void dual_fwd_bfly(u64 &X, u64 &Y, u64 w, u64 ws) {
@@ -247,11 +258,12 @@ __device__ __forceinline__ u64 fold_k32(u64 x) {
     const u32 k = (u32)(x >> M::kBits);
     return (x & M::kMask) + (u64)(k * (u32)M::kC);
 }
+// canonical when floor(x / 2^b) c fits 32 bits: small primes x < 2^50, 61-bit primes any x
 template <class M>
 __device__ __forceinline__ u64 canon_k32(u64 x) {
     return csub<M>(fold_k32<M>(x), M::q);
 }
-// canonical residue of x when fold(x) < 2q: small primes x < 2^55, 61-bit primes any x
+// canonical residue of x when fold(x) < 2q: small primes x < 2^54 (at 2^55 q1's fold reaches 2^37.5 > 2q), 61-bit primes any x
 template <class M>
 __device__ __forceinline__ u64 canon(u64 x) {
     return csub<M>(fold<M>(x), M::q);

@@ -43,7 +43,8 @@ __device__ __forceinline__ int pass_upper(int t) {
 
 // ---------------------------------------------------------------- butterflies
 // forward (Cooley-Tukey): (X, Y) -> (X + wY, X - wY), lazily.  G = global stage index 0..11.
-//  small primes: T = wY in [0,5q) (approximate Shoup quotient); bounds grow by 5q per stage (< 2^43 after 12), never reduced.
+//  small primes: T = wY in [0,5q) (approximate Shoup quotient); bounds grow by 5q per stage, never reduced: inputs < 2^42 stay
+//                 below 2^42 + 60q < 2^44 (< 2^43 from canonical inputs), inside shoup_acc<M, 2>'s x < 2^44.
 //  61-bit primes: T in [0,2q); stage inputs grow 2q -> 4q -> 6q -> 8q (< 2^64) and X is folded back below 2q
 //                 (3 instructions: q = 2^61 - c) on every third stage.
 template <class M, int G>
@@ -51,7 +52,7 @@ __device__ __forceinline__ void fwd_bfly(u64 &X, u64 &Y, u64 w, u64 ws) {
     if constexpr (M::kDual) {
         dual_fwd_bfly<M>(X, Y, w, ws);
     } else if constexpr (M::kSmall) {
-        const u64 Xo = shoup_acc<M, 2>(X, Y, w, ws);  // Y < 2^43 throughout the forward transform
+        const u64 Xo = shoup_acc<M, 2>(X, Y, w, ws);  // Y < 2^42 + 55q < 2^44 throughout the forward transform
         Y = (X + X + 5 * M::q) - Xo;  // X + 5q - T
         X = Xo;
     } else {
@@ -211,7 +212,7 @@ __device__ __forceinline__ void smem_load(const u64 *smem, u64 (&v)[NP][8], int 
 // Forward NTT of NP polynomials.
 //  in : v holds coefficients elem_index<0>(t, r) = r*512 + t   (natural order; small primes < 2^42, large < 2q)
 //  out: v holds NTT values at positions elem_index<9>(t, r) = 8*t + r, reduced to [0, q) if kCanon
-//       (else small primes < in + 48q, large primes < 8q).  Large-prime inputs must be < 2q.
+//       (else small primes < in + 60q, large primes < 8q).  Large-prime inputs must be < 2q.
 template <class M, int NP, bool kCanon, bool kTrailSync = true>
 __device__ __forceinline__ void ntt_forward(u64 (&v)[NP][8], u64 *smem, const ulonglong2 *__restrict__ tw, int t) {
     fwd_pass<M, NP, 0>(v, tw, pass_upper<0>(t));
@@ -231,7 +232,7 @@ __device__ __forceinline__ void ntt_forward(u64 (&v)[NP][8], u64 *smem, const ul
 #pragma unroll
         for (int p = 0; p < NP; p++)
 #pragma unroll
-            for (int r = 0; r < 8; r++) v[p][r] = canon_k32<M>(v[p][r]);  // small: < 2^43; large: < 8q
+            for (int r = 0; r < 8; r++) v[p][r] = canon_k32<M>(v[p][r]);  // small: < 2^44; large: < 8q
     }
     if (kTrailSync) __syncthreads();  // smem may be reused by the caller
 }
