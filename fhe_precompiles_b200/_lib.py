@@ -81,6 +81,8 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_mul_relin.argtypes = [i32, vp, vp, vp, vp, sz, vp]
     L.fhe_b200_encrypt.argtypes = [i32, vp, vp, vp, vp, sz, vp]
     L.fhe_b200_encrypt.restype = i32
+    L.fhe_b200_encrypt_keyed.argtypes = [i32, vp, sz, vp, vp, vp, vp, sz, vp]
+    L.fhe_b200_encrypt_keyed.restype = i32
     L.fhe_b200_seal_sample.argtypes = [i32, vp, vp, sz, vp]
     L.fhe_b200_seal_sample.restype = i32
     L.fhe_b200_seal_op_words.argtypes = []

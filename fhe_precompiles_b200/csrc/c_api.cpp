@@ -80,6 +80,10 @@ extern "C" const uint8_t fhe_b200_network_pub_end[];
 extern "C" const uint8_t fhe_b200_network_pri[];
 extern "C" const uint8_t fhe_b200_network_pri_end[];
 
+// a call of a tile left to its single-call symbol (binary_tile decides every call it is given)
+bool runs_single(const TileItem &) { return false; }
+bool runs_single(const ThresholdItem &it) { return it.single; }
+
 struct OpDesc {
     const char *name;
     int32_t (*fn)(const uint8_t *, size_t, uint8_t **, int64_t *);
@@ -194,6 +198,15 @@ static bool binary_desc(int32_t index, Op *op, Shape *shape, Kind *kind) {
     return true;
 }
 
+// ops 36..47: encrypt_*, reencrypt_*, decrypt_* for u256, u64, i64, frac64
+static bool threshold_desc(int32_t index, Threshold *op, Kind *kind) {
+    if (index < 36 || index >= 48) return false;
+    static const Threshold ops[3] = {Threshold::Encrypt, Threshold::Reencrypt, Threshold::Decrypt};
+    *op = ops[(index - 36) / 4];
+    *kind = (Kind)((index - 36) % 4);
+    return true;
+}
+
 static size_t env_or(const char *name, size_t dflt) {
     const char *e = getenv(name);
     return (e && atoll(e) > 0) ? (size_t)atoll(e) : dflt;
@@ -202,7 +215,8 @@ static size_t env_or(const char *name, size_t dflt) {
 int64_t fhe_b200_batch(fhe_b200_call *calls, size_t n, int32_t host_threads) {
     if (!calls || n == 0) return 0;
     // Workers take TILES of consecutive calls: the binary precompiles of a tile share one lane, one H2D / D2H per operand
-    // array and one batched kernel sequence per operation class (Engine::binary_tile), so launch and synchronisation cost
+    // array and one batched kernel sequence per operation class (Engine::binary_tile), and its threshold calls share another
+    // lane, one batched decryption and one batched encryption (Engine::threshold_tile), so launch and synchronisation cost
     // is paid per tile, not per call.  Two workers per core: while one waits on its lane another runs the codec.
     size_t nt = host_threads > 0 ? (size_t)host_threads : 2 * (size_t)std::thread::hardware_concurrency();
     if (nt == 0) nt = 1;
@@ -234,9 +248,56 @@ int64_t fhe_b200_batch(fhe_b200_call *calls, size_t n, int32_t host_threads) {
     // budget (one of several ranks on the host) divides it among its tile workers
     const size_t loop_width =
         (budget && budget < std::thread::hardware_concurrency()) ? std::max<size_t>(1, (budget + nt - 1) / nt) : 0;
+    const Span net_pub{fhe_b200_network_pub, (size_t)(fhe_b200_network_pub_end - fhe_b200_network_pub)};
+    const Span net_pri{fhe_b200_network_pri, (size_t)(fhe_b200_network_pri_end - fhe_b200_network_pri)};
+    // one tile of calls (binary or threshold), then its results into the caller-owned buffers (a malloc + an 82 KB copy per call):
+    // shared with the pool when this worker runs a big tile, like the tile's own per-call loops
+    const auto run_tile = [&](auto &items, const std::vector<size_t> &which, const auto &run) {
+        if (items.empty()) return;
+        try {
+            run();
+        } catch (const std::exception &e) {
+            set_error(e.what());
+            for (auto &it : items) it.rc = kErrSunscreen;
+        } catch (...) {
+            set_error("unknown exception");
+            for (auto &it : items) it.rc = kErrSunscreen;
+        }
+        const auto finish_one = [&](size_t k) {
+            fhe_b200_call &c = calls[which[k]];
+            if (runs_single(items[k])) {  // a call the tile left to the single-call symbol: its status, output and error
+                c.status = kOps[c.op].fn(c.bytes, c.bytes_length, &c.output, &c.output_length);
+                return;
+            }
+            if (items[k].out_malloc) {  // written in place by the tile: the caller frees it with fhe_free
+                if (items[k].rc == 0) {
+                    c.status = 0, c.output = items[k].out_malloc, c.output_length = (int64_t)items[k].out_malloc_len;
+                    items[k].out_malloc = nullptr;
+                    return;
+                }
+                free(items[k].out_malloc);
+                items[k].out_malloc = nullptr;
+            }
+            c.status = finish(items[k].rc, items[k].out, &c.output, &c.output_length);
+            std::vector<uint8_t>().swap(items[k].out);
+        };
+        if (!serial_loops && items.size() >= 64) {
+            std::atomic<size_t> nextk{0};
+            const std::function<void()> body = [&] {
+                for (size_t k; (k = nextk.fetch_add(8)) < items.size();)
+                    for (size_t j = k; j < std::min(items.size(), k + 8); j++) finish_one(j);
+            };
+            const size_t width = std::min<size_t>(loop_width ? loop_width : std::thread::hardware_concurrency(), items.size() / 8);
+            if (width < 2) body();
+            else HostPool::get().run(width - 1, body);
+        } else {
+            for (size_t k = 0; k < items.size(); k++) finish_one(k);
+        }
+    };
     auto worker = [&]() {
         std::vector<TileItem> items;
-        std::vector<size_t> which;
+        std::vector<ThresholdItem> titems;
+        std::vector<size_t> which, twhich;
         struct SerialLoops {
             bool on;
             explicit SerialLoops(bool v, size_t width) : on(v) {
@@ -254,15 +315,22 @@ int64_t fhe_b200_batch(fhe_b200_call *calls, size_t n, int32_t host_threads) {
             const size_t lo = t * tile, hi = std::min(n, lo + tile);
             items.clear();
             which.clear();
+            titems.clear();
+            twhich.clear();
             for (size_t i = lo; i < hi; i++) {
                 fhe_b200_call &c = calls[i];
                 Op op;
                 Shape shape;
                 Kind kind;
+                Threshold top;
                 if (binary_desc(c.op, &op, &shape, &kind)) {
                     items.push_back(TileItem{op, shape, kind, Span{c.bytes, c.bytes_length}, {}, 0});
                     items.back().take_malloc = true;
                     which.push_back(i);
+                } else if (threshold_desc(c.op, &top, &kind)) {
+                    titems.push_back(ThresholdItem{top, kind, Span{c.bytes, c.bytes_length}, {}, 0});
+                    titems.back().take_malloc = true;
+                    twhich.push_back(i);
                 } else if (c.op < 0 || c.op >= kNumOps) {
                     c.status = kErrSunscreen;
                     c.output = nullptr;
@@ -271,45 +339,8 @@ int64_t fhe_b200_batch(fhe_b200_call *calls, size_t n, int32_t host_threads) {
                     c.status = kOps[c.op].fn(c.bytes, c.bytes_length, &c.output, &c.output_length);
                 }
             }
-            if (!items.empty()) {
-                try {
-                    Engine::get().binary_tile(items.data(), items.size());
-                } catch (const std::exception &e) {
-                    set_error(e.what());
-                    for (auto &it : items) it.rc = kErrSunscreen;
-                } catch (...) {
-                    set_error("unknown exception");
-                    for (auto &it : items) it.rc = kErrSunscreen;
-                }
-                // results into caller-owned buffers (a malloc + an 82 KB copy per call): shared with the pool when this worker
-                // runs a big tile, like the tile's own per-call loops
-                const auto finish_one = [&](size_t k) {
-                    fhe_b200_call &c = calls[which[k]];
-                    if (items[k].out_malloc) {  // written in place by the tile: the caller frees it with fhe_free
-                        if (items[k].rc == 0) {
-                            c.status = 0, c.output = items[k].out_malloc, c.output_length = (int64_t)items[k].out_malloc_len;
-                            items[k].out_malloc = nullptr;
-                            return;
-                        }
-                        free(items[k].out_malloc);
-                        items[k].out_malloc = nullptr;
-                    }
-                    c.status = finish(items[k].rc, items[k].out, &c.output, &c.output_length);
-                    std::vector<uint8_t>().swap(items[k].out);
-                };
-                if (!serial_loops && items.size() >= 64) {
-                    std::atomic<size_t> nextk{0};
-                    const std::function<void()> body = [&] {
-                        for (size_t k; (k = nextk.fetch_add(8)) < items.size();)
-                            for (size_t j = k; j < std::min(items.size(), k + 8); j++) finish_one(j);
-                    };
-                    const size_t width = std::min<size_t>(loop_width ? loop_width : std::thread::hardware_concurrency(), items.size() / 8);
-                    if (width < 2) body();
-                    else HostPool::get().run(width - 1, body);
-                } else {
-                    for (size_t k = 0; k < items.size(); k++) finish_one(k);
-                }
-            }
+            run_tile(items, which, [&] { Engine::get().binary_tile(items.data(), items.size()); });
+            run_tile(titems, twhich, [&] { Engine::get().threshold_tile(titems.data(), titems.size(), net_pub, net_pri); });
             for (size_t i = lo; i < hi; i++)
                 if (calls[i].status) failed.fetch_add(1);
         }
@@ -362,6 +393,11 @@ int32_t fhe_b200_int_peak(int32_t device, int32_t wide, double *tera_mads_per_s)
 int32_t fhe_b200_encrypt(int32_t device, const uint64_t *pk, const uint16_t *plain, const uint64_t *seeds, uint64_t *ct, size_t n,
                          void *stream) {
     DEV_GUARD(Engine::get().encrypt_device(device, pk, plain, seeds, ct, n, (cudaStream_t)stream));
+}
+int32_t fhe_b200_encrypt_keyed(int32_t device, const uint64_t *pks, size_t n_keys, const int32_t *key_index, const uint16_t *plain,
+                               const uint64_t *seeds, uint64_t *ct, size_t n, void *stream) {
+    DEV_GUARD(if (n && (!pks || !n_keys || !key_index)) throw std::runtime_error("fhe_b200_encrypt_keyed: no keys or no key indices");
+              Engine::get().encrypt_keyed_device(device, pks, key_index, plain, seeds, ct, n, (cudaStream_t)stream));
 }
 int32_t fhe_b200_seal_sample(int32_t device, uint64_t *streams, int32_t *failed, size_t n, void *stream) {
     DEV_GUARD(device_context(device); cuda_throw(launch_seal_sample(streams, nullptr, failed, n, (cudaStream_t)stream), "seal_sample"));

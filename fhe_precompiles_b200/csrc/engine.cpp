@@ -1510,6 +1510,10 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
 // ---------------------------------------------------------------- device-resident encrypt / decrypt
 void Engine::encrypt_device(int device, const uint64_t *pk, const uint16_t *plain, const uint64_t *seeds, uint64_t *ct, size_t n,
                             cudaStream_t s) {
+    encrypt_keyed_device(device, pk, nullptr, plain, seeds, ct, n, s);
+}
+void Engine::encrypt_keyed_device(int device, const uint64_t *pks, const int32_t *key_index, const uint16_t *plain,
+                                  const uint64_t *seeds, uint64_t *ct, size_t n, cudaStream_t s) {
     device_context(device);
     if (n == 0) return;
     const size_t chunk = chunk_ops_ < n ? chunk_ops_ : n;
@@ -1517,7 +1521,9 @@ void Engine::encrypt_device(int device, const uint64_t *pk, const uint16_t *plai
     uint64_t *encbuf = lease.st->p;
     for (size_t off = 0; off < n; off += chunk) {
         const size_t c = n - off < chunk ? n - off : chunk;
-        cuda_throw(launch_encrypt(pk, plain + off * kN, seeds + off * 8, encbuf, ct + off * kCtWords, c, s), "encrypt");
+        cuda_throw(launch_encrypt_keyed(pks, key_index ? key_index + off : nullptr, plain + off * kN, seeds + off * 8, encbuf,
+                                        ct + off * kCtWords, c, s),
+                   "encrypt");
     }
 }
 void Engine::decrypt_device(int device, const uint64_t *ct, const uint64_t *sk, uint16_t *plain, size_t n, cudaStream_t s,
@@ -1646,6 +1652,216 @@ int32_t Engine::reencrypt(Kind kind, Span in, Span, Span net_pri, std::vector<ui
     msg.insert(msg.end(), in.p, in.p + in.n);
     msg.insert(msg.end(), scalar.begin(), scalar.end());
     return encrypt_plain(kind, Span{scalar.data(), scalar.size()}, pk, seed_from_hash(msg).w, &view, lane, out);
+}
+
+
+// ---------------------------------------------------------------- threshold calls of the batch surface, a tile at a time
+// (1) per call, on the host pool: framing, the target key of a reencrypt (pinned for the tile), the route of the ciphertext
+// operand.  (2) one codec pass and one launch_decrypt over every decrypt / reencrypt operand.  (3) per call: the decrypted
+// scalars, then the seeds and plaintexts of every encryption.  (4) one launch_encrypt_keyed over every encrypt / reencrypt row,
+// each under its own key, and the result writer as binary_tile's.  A call whose operand is not a libzstd or structured frame of
+// its kind, or that the device decoder hands back, is marked `single`: the caller runs it as the single call, which owns those
+// codes, once the tile has released its lane.
+void Engine::threshold_tile(ThresholdItem *items, size_t cnt, Span net_pub, Span net_pri) {
+    for (size_t i = 0; i < cnt; i++) items[i].single = cnt == 1;  // a lone call gains nothing from the tile
+    if (cnt < 2) return;
+    Lane *lane = acquire_lane();
+    LaneGuard guard{this, lane, &Engine::release_lane};
+    threshold_on_lane(lane, items, cnt, net_pub, net_pri);
+}
+
+void Engine::threshold_on_lane(Lane *lane, ThresholdItem *items, size_t cnt, Span net_pub, Span net_pri) {
+    cuda_throw(cudaSetDevice(lane->device), "cudaSetDevice");
+    ensure_capacity(lane, cnt);
+    ensure_codec(lane);
+    cudaStream_t s = lane->stream;
+    const size_t cap = lane->cap;
+    struct Prep {
+        Span a, b;             // encrypt: plain, public data; reencrypt: target key, public data
+        Operand op;            // decrypt / reencrypt: the ciphertext
+        const uint64_t *d_pk = nullptr;
+        KeyPin pin;
+        std::vector<uint8_t> scalar;  // reencrypt: the decrypted value
+        bool live = false;
+    };
+    std::vector<Prep> prep(cnt);
+
+    // (1)
+    parallel_for(cnt, 4, [&](size_t i) {
+        ThresholdItem &it = items[i];
+        Prep &p = prep[i];
+        it.rc = kOk;
+        Span ct = it.in;
+        if (it.op == Threshold::Encrypt) {
+            p.live = (it.rc = unpack_two_arguments(it.in, &p.a, &p.b)) == kOk;
+            return;
+        }
+        if (it.op == Threshold::Reencrypt) {  // reference order: key, ciphertext, public data (pack.rs:261-263)
+            if ((it.rc = unpack_binary_operation(it.in, &p.a, &ct, &p.b))) return;
+            if ((it.rc = public_key(p.a, lane->device, &p.d_pk, &p.pin))) return;
+        }
+        const Route r = classify_operand(ct, it.kind, &p.op);
+        if (r == Route::Zstd || r == Route::Packed) p.live = true;
+        else it.single = true;
+    });
+
+    // (2)
+    std::vector<size_t> dec_item;
+    std::vector<StageOperand> sop;
+    for (size_t i = 0; i < cnt; i++)
+        if (prep[i].live && items[i].op != Threshold::Encrypt) {
+            sop.push_back(StageOperand{prep[i].op.route, prep[i].op.frame.n, (int32_t)dec_item.size(), 0});
+            dec_item.push_back(i);
+        }
+    const size_t D = dec_item.size();
+    if (D) {
+        std::vector<int32_t> job(D);
+        std::vector<uint8_t> bad(D, 0);
+        const StagePlan plan = plan_codec_jobs(sop.data(), D, lane->h_jobs, job.data());
+        parallel_for(D, 2, [&](size_t k) {
+            if (!stage_operand(prep[dec_item[k]].op, lane->h_jobs, job[k], lane->h_frames, lane->h_payloads)) {
+                bad[k] = 1;
+                lane->h_jobs[job[k]].kind = kJobNone;
+            }
+        });
+        if (plan.frame_bytes)
+            cuda_throw(cudaMemcpyAsync(lane->d_frames, lane->h_frames, plan.frame_bytes, cudaMemcpyHostToDevice, s), "H2D frames");
+        if (plan.payloads)
+            cuda_throw(cudaMemcpyAsync(lane->d_payloads, lane->h_payloads, (size_t)plan.payloads * kPayloadStride, cudaMemcpyHostToDevice, s),
+                       "H2D payloads");
+        cuda_throw(cudaMemcpyAsync(lane->d_jobs, lane->h_jobs, (size_t)plan.jobs * sizeof(CodecJob), cudaMemcpyHostToDevice, s), "H2D jobs");
+        cuda_throw(launch_codec_inflate(lane->d_frames, lane->d_payloads, lane->d_jobs, lane->d_status, lane->d_work, lane->d_prefix, lane->d_a,
+                                        nullptr, plan.jobs, plan.any_zstd, plan.any_packed, plan.payloads > 0, s),
+                   "codec inflate");
+        int32_t *d_exh = lane->d_status + 2 * cap, *h_exh = lane->h_status + 2 * cap;  // behind the job status
+        cuda_throw(launch_decrypt(lane->d_a, network_sk(lane->device, net_pri), lane->d_scratch, lane->d_plain, D, s, d_exh), "decrypt");
+        uint16_t *h_dec = reinterpret_cast<uint16_t *>(lane->h_a);  // decrypted plaintexts; h_plain stages the encryptions' below
+        cuda_throw(cudaMemcpyAsync(h_dec, lane->d_plain, D * kN * 2, cudaMemcpyDeviceToHost, s), "D2H plain");
+        cuda_throw(cudaMemcpyAsync(h_exh, d_exh, D * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H noise flags");
+        cuda_throw(cudaMemcpyAsync(lane->h_status, lane->d_status, (size_t)plan.jobs * sizeof(int32_t), cudaMemcpyDeviceToHost, s),
+                   "D2H status");
+        cuda_throw(cudaStreamSynchronize(s), "stream sync");
+        // (3a) the decrypted scalars; a noise budget of 0 is sunscreen's decryption failure (fhe.rs:643, 696)
+        parallel_for(D, 8, [&](size_t k) {
+            const size_t i = dec_item[k];
+            ThresholdItem &it = items[i];
+            Prep &p = prep[i];
+            p.live = false;
+            if (bad[k] || lane->h_status[job[k]] == kJobFallback) it.single = true;
+            else if (h_exh[k]) it.rc = kErrFailedDecryption;
+            else if (it.op == Threshold::Decrypt) decode_scalar(it.kind, h_dec + k * kN, kN, &it.out);
+            else decode_scalar(it.kind, h_dec + k * kN, kN, &p.scalar), p.live = true;
+        });
+    }
+
+    // (3b) encryption rows: encrypts under the network key, reencrypts under their target keys
+    std::vector<size_t> enc_item;
+    std::vector<const uint64_t *> keys;  // distinct keys of the tile, in the order of their first row
+    std::map<const uint64_t *, int32_t> key_slot;
+    const uint64_t *d_net_pk = nullptr;
+    KeyPin net_pin;
+    uint64_t *h_seeds = lane->h_b;
+    int32_t *h_kidx = reinterpret_cast<int32_t *>(lane->h_b + cap * 8);
+    for (size_t i = 0; i < cnt; i++) {
+        if (!prep[i].live) continue;
+        const uint64_t *pk = prep[i].d_pk;
+        if (items[i].op == Threshold::Encrypt) {
+            if (!d_net_pk && public_key(net_pub, lane->device, &d_net_pk, &net_pin) != kOk)
+                throw std::runtime_error("fhe_b200: embedded network public key is corrupt");
+            pk = d_net_pk;
+        }
+        const auto ins = key_slot.emplace(pk, (int32_t)keys.size());
+        if (ins.second) keys.push_back(pk);
+        h_kidx[enc_item.size()] = ins.first->second;
+        enc_item.push_back(i);
+    }
+    const size_t E = enc_item.size();
+    if (E == 0) return;
+    parallel_for(E, 4, [&](size_t e) {
+        const size_t i = enc_item[e];
+        ThresholdItem &it = items[i];
+        Prep &p = prep[i];
+        std::vector<uint8_t> msg(p.b.p, p.b.p + p.b.n);
+        Span scalar = p.a;
+        if (it.op == Threshold::Encrypt) {  // seed = SHA-512(public_data || constant || plain bytes)   (fhe.rs:600-611)
+            msg.insert(msg.end(), kSeedConstant, kSeedConstant + 64);
+            msg.insert(msg.end(), p.a.p, p.a.p + p.a.n);
+        } else {  // seed = SHA-512(public_data || whole input || plain bytes)   (fhe.rs:676, 646-649)
+            msg.insert(msg.end(), it.in.p, it.in.p + it.in.n);
+            msg.insert(msg.end(), p.scalar.begin(), p.scalar.end());
+            scalar = Span{p.scalar.data(), p.scalar.size()};
+        }
+        const int32_t rc = encode_scalar(it.kind, scalar, lane->h_plain + e * kN);
+        if (rc) {  // the row still computes, on whatever its staging holds; nobody reads it
+            it.rc = rc == kErrSunscreen ? kErrFailedEncryption : rc;
+            p.live = false;
+            return;
+        }
+        memcpy(h_seeds + e * 8, seed_from_hash(msg).w, 64);
+    });
+
+    // (4) per-lane layout inside d_scratch: sampler streams [cap][6][N] | seeds [cap][8] | key indices [cap] | keys [k][2][3][N].
+    // The keys start on a 256-byte boundary whatever the lane's capacity: k_encrypt_seal reads them 16 bytes at a time.
+    uint64_t *encbuf = lane->d_scratch, *d_seeds = encbuf + cap * 6 * kN;
+    int32_t *d_kidx = reinterpret_cast<int32_t *>(d_seeds + cap * 8);
+    uint64_t *d_keys = d_seeds + ((cap * 9 + 31) & ~(size_t)31);
+    static_assert(6 * kN + 9 + 31 + 2 * 6 * kN <= kScratchLimbsPerOp * kN, "per call: its stream, seed, index, the padding and up to two keys (k <= cap + 1)");
+    int32_t *d_failed = lane->d_status + cap, *h_failed = lane->h_status + cap;
+    int32_t *d_cflag = lane->d_status + 2 * cap, *h_cflag = lane->h_status + 2 * cap;
+    for (size_t j = 0; j < keys.size(); j++)
+        cuda_throw(cudaMemcpyAsync(d_keys + j * kPkWords, keys[j], kPkWords * 8, cudaMemcpyDeviceToDevice, s), "D2D key");
+    cuda_throw(cudaMemcpyAsync(lane->d_plain, lane->h_plain, E * kN * 2, cudaMemcpyHostToDevice, s), "H2D plain");
+    cuda_throw(cudaMemcpyAsync(d_seeds, h_seeds, E * 64, cudaMemcpyHostToDevice, s), "H2D seeds");
+    cuda_throw(cudaMemcpyAsync(d_kidx, h_kidx, E * sizeof(int32_t), cudaMemcpyHostToDevice, s), "H2D key indices");
+    cuda_throw(launch_encrypt_keyed(d_keys, d_kidx, lane->d_plain, d_seeds, encbuf, lane->d_out, E, s, d_failed), "encrypt");
+    const bool pack_on_device = zstd_writer() == 1;
+    if (pack_on_device) {
+        cuda_throw(launch_codec_pack(lane->d_out, lane->d_outframes, d_cflag, lane->d_prefix, (int)E, s), "codec pack");
+        cuda_throw(cudaMemcpyAsync(lane->h_outframes, lane->d_outframes, E * kPackedFrameStride, cudaMemcpyDeviceToHost, s), "D2H frames");
+        cuda_throw(cudaMemcpyAsync(h_cflag, d_cflag, E * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H flags");
+    } else {
+        cuda_throw(cudaMemcpyAsync(lane->h_out, lane->d_out, E * kCtWords * 8, cudaMemcpyDeviceToHost, s), "D2H");
+    }
+    cuda_throw(cudaMemcpyAsync(h_failed, d_failed, E * sizeof(int32_t), cudaMemcpyDeviceToHost, s), "D2H sampler flags");
+    cuda_throw(cudaStreamSynchronize(s), "stream sync");
+    const CipherView enc_view[4] = {result_view(Kind::U256), result_view(Kind::U64), result_view(Kind::I64), result_view(Kind::Frac64)};
+    std::vector<uint8_t> constant(E, 0);
+    parallel_for(E, 4, [&](size_t e) {
+        const size_t i = enc_item[e];
+        ThresholdItem &it = items[i];
+        Prep &p = prep[i];
+        if (!p.live) return;
+        const CipherView &view = it.op == Threshold::Encrypt ? enc_view[(int)it.kind] : p.op.view;
+        if (h_failed[e]) {
+            it.rc = kErrFailedEncryption;  // PRNG stream window exhausted (~24 sigma)
+        } else if (!pack_on_device) {
+            it.rc = encode_ciphertext(view, lane->h_out + e * kCtWords, &it.out);
+        } else if (h_cflag[e]) {
+            constant[e] = 1;  // constant result (a transparent ciphertext): the host writer's libzstd path, below
+        } else {
+            const uint8_t *frame = lane->h_outframes + e * kPackedFrameStride;
+            uint8_t *direct = nullptr;
+            if (it.take_malloc) {
+                it.out_malloc_len = wrapped_ciphertext_size(view, kPackedFrameBytes);
+                direct = (uint8_t *)malloc(it.out_malloc_len);
+            }
+            if (direct) {
+                wrap_ciphertext_blob_to(view, frame, kPackedFrameBytes, direct);
+                it.out_malloc = direct;
+            } else {
+                wrap_ciphertext_blob(view, frame, kPackedFrameBytes, &it.out);
+            }
+            it.rc = kOk;
+        }
+    });
+    for (size_t e = 0; e < E; e++)
+        if (constant[e]) {
+            const size_t i = enc_item[e];
+            cuda_throw(cudaMemcpyAsync(lane->h_out, lane->d_out + e * kCtWords, kCtWords * 8, cudaMemcpyDeviceToHost, s), "D2H");
+            cuda_throw(cudaStreamSynchronize(s), "stream sync");
+            items[i].rc = encode_ciphertext(items[i].op == Threshold::Encrypt ? enc_view[(int)items[i].kind] : prep[i].op.view,
+                                            lane->h_out, &items[i].out);
+        }
 }
 
 }  // namespace fheb

@@ -78,6 +78,20 @@ struct TileItem {
     size_t out_malloc_len = 0;
 };
 
+// one call of the threshold-network precompiles (encrypt_*, reencrypt_*, decrypt_*) inside a tile of the batch surface
+enum class Threshold : int { Encrypt = 0, Reencrypt = 1, Decrypt = 2 };
+struct ThresholdItem {
+    Threshold op;
+    Kind kind;
+    Span in;
+    std::vector<uint8_t> out;
+    int32_t rc = 0;
+    bool take_malloc = false;  // as TileItem
+    uint8_t *out_malloc = nullptr;
+    size_t out_malloc_len = 0;
+    bool single = false;  // set by threshold_tile: the tile did not take the call, whose caller runs it as the single call
+};
+
 struct KeyEntry {
     std::vector<uint8_t> bytes;  // exact PublicKey bytes this entry was parsed from
     uint64_t tag = 0;            // cheap pre-filter
@@ -177,6 +191,11 @@ class Engine {
     int32_t encrypt(Kind kind, Span in, Span net_pub, Span net_pri, std::vector<uint8_t> *out);
     int32_t reencrypt(Kind kind, Span in, Span net_pub, Span net_pri, std::vector<uint8_t> *out);
     int32_t decrypt(Kind kind, Span in, Span net_pub, Span net_pri, std::vector<uint8_t> *out);
+    // `cnt` independent threshold calls on ONE lane: one batched decryption over every decrypt_* / reencrypt_* operand and one
+    // batched encryption (a key per row) over every encrypt_* / reencrypt_* result.  Per-call results and error codes are exactly
+    // those of the three functions above.  A call whose operand is not perfectly ordinary (or a tile of one) is left marked
+    // `single`, with no result: the caller runs it as the single call after this returns.
+    void threshold_tile(ThresholdItem *items, size_t cnt, Span net_pub, Span net_pri);
 
     // scratch arena for `ops` concurrent multiply+relin ops, one per (device, caller stream): grown on demand, leased while
     // a caller enqueues, evicted (after synchronising its stream) when more than FHE_B200_SCRATCH_ARENAS are idle on a device
@@ -203,6 +222,9 @@ class Engine {
     // device-resident batched encrypt / decrypt (pointers on `device`)
     void encrypt_device(int device, const uint64_t *pk, const uint16_t *plain, const uint64_t *seeds, uint64_t *ct, size_t n,
                         cudaStream_t s);
+    // the same with a key per op: pks [k][2][3][N], key_index [n] ints in [0, k) (device data, not checked)
+    void encrypt_keyed_device(int device, const uint64_t *pks, const int32_t *key_index, const uint16_t *plain, const uint64_t *seeds,
+                              uint64_t *ct, size_t n, cudaStream_t s);
     // exhausted (optional, [n] ints on the device): 1 where the invariant noise budget is 0 (the plaintext is then garbage)
     void decrypt_device(int device, const uint64_t *ct, const uint64_t *sk, uint16_t *plain, size_t n, cudaStream_t s,
                         int32_t *exhausted = nullptr);
@@ -213,6 +235,8 @@ class Engine {
     void ensure_capacity(Lane *lane, size_t cap);
     void ensure_codec(Lane *lane);
     bool single_call_fast(Lane *lane, TileItem &it, bool timed, std::chrono::steady_clock::time_point t_start);
+    // threshold_tile's device passes on `lane`
+    void threshold_on_lane(Lane *lane, ThresholdItem *items, size_t cnt, Span net_pub, Span net_pri);
     void drop_graphs(Lane *lane);
     size_t tile_ops_ = 16;
     std::atomic<bool> call_timing_{false};

@@ -1129,11 +1129,13 @@ __device__ __forceinline__ void encrypt_seal_body(const u64 *__restrict__ pk, co
         store_natural(ct + (size_t)(j * 2 + MI) * kN, w[j], t);
     }
 }
-__global__ void __launch_bounds__(kThreads, 1) k_encrypt_seal(const u64 *__restrict__ pk, const u64 *__restrict__ scratch,
-                                                               size_t op_stride, const unsigned short *__restrict__ plain,
-                                                               u64 *__restrict__ ct) {
+// pks [k][2][3][N]: op i encrypts under pks + key_index[i] * 6N, or under pks itself when key_index is null
+__global__ void __launch_bounds__(kThreads, 1) k_encrypt_seal(const u64 *__restrict__ pks, const int *__restrict__ key_index,
+                                                               const u64 *__restrict__ scratch, size_t op_stride,
+                                                               const unsigned short *__restrict__ plain, u64 *__restrict__ ct) {
     extern __shared__ __align__(16) u64 smem[];
     const size_t op = blockIdx.y;
+    const u64 *pk = pks + (key_index ? (size_t)key_index[op] : 0) * (6 * kN);
     const signed char *smp = reinterpret_cast<const signed char *>(scratch + op * op_stride + kSealStreamWords);
     const unsigned short *pl = plain + op * kN;
     u64 *out = ct + op * 4 * kN;
@@ -1406,16 +1408,20 @@ cudaError_t launch_decrypt(const u64 *ct, const u64 *sk, u64 *xbuf, unsigned sho
     g_launches.fetch_add(2, std::memory_order_relaxed);
     return cudaGetLastError();
 }
-cudaError_t launch_encrypt(const u64 *pk, const unsigned short *plain, const u64 *seeds, u64 *encbuf, u64 *ct, size_t n_ops,
-                           cudaStream_t s, int *failed) {
+cudaError_t launch_encrypt_keyed(const u64 *pks, const int *key_index, const unsigned short *plain, const u64 *seeds, u64 *encbuf,
+                                 u64 *ct, size_t n_ops, cudaStream_t s, int *failed) {
     if (n_ops == 0) return cudaSuccess;
     static_assert(kSealStreamWords + 3 * kN / 8 <= 6 * kN, "per-op encryption scratch is [6][N] words");
     const size_t stride = 6 * kN;
     k_seal_prng<<<(unsigned)n_ops, 512, 0, s>>>(seeds, encbuf, stride);
     k_seal_sample<<<(unsigned)n_ops, 512, 0, s>>>(encbuf, stride, failed);
-    k_encrypt_seal<<<dim3(2, (unsigned)n_ops), kThreads, kSmem2, s>>>(pk, encbuf, stride, plain, ct);
+    k_encrypt_seal<<<dim3(2, (unsigned)n_ops), kThreads, kSmem2, s>>>(pks, key_index, encbuf, stride, plain, ct);
     g_launches.fetch_add(3, std::memory_order_relaxed);
     return cudaGetLastError();
+}
+cudaError_t launch_encrypt(const u64 *pk, const unsigned short *plain, const u64 *seeds, u64 *encbuf, u64 *ct, size_t n_ops,
+                           cudaStream_t s, int *failed) {
+    return launch_encrypt_keyed(pk, nullptr, plain, seeds, encbuf, ct, n_ops, s, failed);
 }
 cudaError_t launch_seal_sample(u64 *streams, signed char *samples, int *failed, size_t n_ops, cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;

@@ -41,6 +41,10 @@ cudaError_t launch_decrypt(const u64 *ct, const u64 *sk, u64 *xbuf, unsigned sho
 // failed[op] (optional) = 1 if the op's PRNG stream window ran out (never observed: ~24 sigma)
 cudaError_t launch_encrypt(const u64 *pk, const unsigned short *plain, const u64 *seeds, u64 *encbuf, u64 *ct, size_t n_ops,
                            cudaStream_t s, int *failed = nullptr);
+// the same with a key per op: pks [k][2][3][N], key_index [n_ops] device ints in [0, k) (not checked: an index outside the
+// key array is the caller's error, as a bad pointer is); op i encrypts under pks + key_index[i] * 2 * 3 * N
+cudaError_t launch_encrypt_keyed(const u64 *pks, const int *key_index, const unsigned short *plain, const u64 *seeds, u64 *encbuf,
+                                 u64 *ct, size_t n_ops, cudaStream_t s, int *failed = nullptr);
 // SEAL's samplers (ternary u, clipped-normal e0 / e1) on caller-supplied streams of 32-bit draws: op i owns
 // kSealOpWords = 28 * 512 + 3 * N / 8 words at streams + i * kSealOpWords -- 28,672 draws followed by room for the three
 // int8 sample polynomials, which the kernel writes there.  failed[i] = 1 if the draws ran out.

@@ -254,9 +254,29 @@ def encrypt(pk: torch.Tensor, plain: torch.Tensor, seeds: torch.Tensor) -> torch
     _dev(plain)
     _dev(seeds)
     n = plain.shape[0]
-    assert plain.dtype == torch.int16 and seeds.dtype == torch.int64 and tuple(seeds.shape) == (n, 8)
+    assert plain.dtype == torch.int16 and tuple(plain.shape) == (n, N)
+    assert seeds.dtype == torch.int64 and tuple(seeds.shape) == (n, 8)
     ct = torch.empty((n, 2, 2, N), dtype=torch.int64, device=pk.device)
     _check(_lib.lib().fhe_b200_encrypt(dev, pk.data_ptr(), plain.data_ptr(), seeds.data_ptr(), ct.data_ptr(), n, _stream(dev)))
+    return ct
+
+
+def encrypt_keyed(pks: torch.Tensor, key_index: torch.Tensor, plain: torch.Tensor, seeds: torch.Tensor) -> torch.Tensor:
+    """encrypt() with a key per row: pks [k,2,3,4096] int64, key_index [n] int32 in [0, k), plain [n,4096] int16, seeds [n,8]
+    int64 (all on one CUDA device) -> ct [n,2,2,4096]; row i is encrypt(pks[key_index[i]], ...) of that row.  The indices are
+    not checked on the device: one outside [0, k) is the caller's error."""
+    dev = _dev(pks)
+    _dev(key_index)
+    _dev(plain)
+    _dev(seeds)
+    n = plain.shape[0]
+    assert pks.dim() == 4 and tuple(pks.shape[1:]) == (2, 3, N) and pks.dtype == torch.int64
+    assert key_index.dtype == torch.int32 and tuple(key_index.shape) == (n,)
+    assert plain.dtype == torch.int16 and tuple(plain.shape) == (n, N)
+    assert seeds.dtype == torch.int64 and tuple(seeds.shape) == (n, 8)
+    ct = torch.empty((n, 2, 2, N), dtype=torch.int64, device=pks.device)
+    _check(_lib.lib().fhe_b200_encrypt_keyed(dev, pks.data_ptr(), pks.shape[0], key_index.data_ptr(), plain.data_ptr(), seeds.data_ptr(),
+                                             ct.data_ptr(), n, _stream(dev)))
     return ct
 
 

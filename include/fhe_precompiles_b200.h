@@ -115,7 +115,10 @@ typedef struct fhe_b200_call {
 int32_t fhe_b200_op_index(const char *name);
 const char *fhe_b200_op_name(int32_t index);
 /* Runs n independent precompile calls, codec on `host_threads` host threads (0 = all cores), arithmetic
- * sharded over every visible GPU. Returns the number of calls whose status != 0. */
+ * sharded over every visible GPU. Returns the number of calls whose status != 0.  Consecutive calls form tiles: the 36
+ * binary precompiles of a tile run as batched kernels, and so do its encrypt_* / reencrypt_* / decrypt_* calls (one
+ * decryption over every ciphertext operand, one encryption over every result, each row under its own key);
+ * public_key_bytes runs as the single call.  Each status and output equals what the single c_fhe_* call returns. */
 int64_t fhe_b200_batch(fhe_b200_call *calls, size_t n, int32_t host_threads);
 
 /* Device-resident entry points. All pointers are device memory on `device`; `stream` is a cudaStream_t
@@ -147,6 +150,13 @@ int32_t fhe_b200_mul_relin(int32_t device, const uint64_t *a, const uint64_t *b,
 int32_t fhe_b200_encrypt(int32_t device, const uint64_t *pk, const uint16_t *plain, const uint64_t *seeds, uint64_t *ct, size_t n,
                          void *stream);
 int32_t fhe_b200_decrypt(int32_t device, const uint64_t *ct, const uint64_t *sk, uint16_t *plain, size_t n, void *stream);
+/* fhe_b200_encrypt with a key per op: pks [n_keys][2][3][4096] (each as fhe_b200_encrypt's pk), key_index [n] int32 on the
+ * device; op i encrypts plain[i] with seeds[i] under pks + key_index[i] * 2 * 3 * 4096, bit for bit what fhe_b200_encrypt
+ * computes for that row under that key.  For a batch whose rows go to different users, e.g. the re-encryptions of a block.
+ * The indices are device data and are not checked: an index outside [0, n_keys) is the caller's error, as a bad pointer is.
+ * n == 0 launches nothing; -1 (fhe_b200_last_error) for a missing device, missing keys or indices, or a failed launch. */
+int32_t fhe_b200_encrypt_keyed(int32_t device, const uint64_t *pks, size_t n_keys, const int32_t *key_index, const uint16_t *plain,
+                               const uint64_t *seeds, uint64_t *ct, size_t n, void *stream);
 /* The sampling stage of fhe_b200_encrypt on its own, on caller-supplied draws instead of the Blake2xb stream: op i owns
  * fhe_b200_seal_op_words() device words at streams + i * that -- 28,672 32-bit draws (little-endian word pairs) followed by
  * room for the three int8[4096] polynomials u, e0, e1, which are written there in SEAL's order (sample_poly_ternary, then
