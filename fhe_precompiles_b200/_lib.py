@@ -79,6 +79,10 @@ def lib() -> ctypes.CDLL:
     L.fhe_b200_plain_addsub.argtypes = [i32, vp, vp, vp, sz, i32, vp]
     L.fhe_b200_multiply_plain.argtypes = [i32, vp, vp, vp, sz, vp]
     L.fhe_b200_mul_relin.argtypes = [i32, vp, vp, vp, vp, sz, vp]
+    L.fhe_b200_mul_relin_keyed.argtypes = [i32, vp, vp, vp, sz, vp, vp, sz, vp]
+    L.fhe_b200_mul_relin_keyed.restype = i32
+    L.fhe_b200_relinearize_keyed.argtypes = [i32, vp, vp, sz, vp, vp, sz, vp]
+    L.fhe_b200_relinearize_keyed.restype = i32
     L.fhe_b200_encrypt.argtypes = [i32, vp, vp, vp, vp, sz, vp]
     L.fhe_b200_encrypt.restype = i32
     L.fhe_b200_encrypt_keyed.argtypes = [i32, vp, sz, vp, vp, vp, vp, sz, vp]

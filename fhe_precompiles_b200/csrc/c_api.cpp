@@ -387,6 +387,16 @@ int32_t fhe_b200_mul_relin(int32_t device, const uint64_t *a, const uint64_t *b,
                            size_t n, void *stream) {
     DEV_GUARD(Engine::get().mul_relin(device, a, b, rk, out, n, (cudaStream_t)stream));
 }
+int32_t fhe_b200_mul_relin_keyed(int32_t device, const uint64_t *a, const uint64_t *b, const uint64_t *rks, size_t n_keys,
+                                 const int32_t *key_index, uint64_t *out, size_t n, void *stream) {
+    DEV_GUARD(if (n && (!rks || !n_keys || !key_index)) throw std::runtime_error("fhe_b200_mul_relin_keyed: no keys or no key indices");
+              Engine::get().mul_relin_keyed(device, a, b, rks, n_keys, key_index, out, n, (cudaStream_t)stream));
+}
+int32_t fhe_b200_relinearize_keyed(int32_t device, const uint64_t *c3, const uint64_t *rks, size_t n_keys, const int32_t *key_index,
+                                   uint64_t *out, size_t n, void *stream) {
+    DEV_GUARD(if (n && (!rks || !n_keys || !key_index)) throw std::runtime_error("fhe_b200_relinearize_keyed: no keys or no key indices");
+              Engine::get().relinearize_keyed(device, c3, rks, n_keys, key_index, out, n, (cudaStream_t)stream));
+}
 int32_t fhe_b200_int_peak(int32_t device, int32_t wide, double *tera_mads_per_s) {
     DEV_GUARD(device_context(device); cuda_throw(measure_int_peak(wide, tera_mads_per_s), "int_peak"));
 }

@@ -138,7 +138,9 @@ void Engine::ensure_capacity(Lane *l, size_t cap) {
     if (l->cap >= cap) return;
     drop_graphs(l);
     cudaFreeHost(l->h_a), cudaFreeHost(l->h_b), cudaFreeHost(l->h_out), cudaFreeHost(l->h_plain);
+    cudaFreeHost(l->h_rk_ptrs), cudaFreeHost(l->h_rk_index);
     cudaFree(l->d_a), cudaFree(l->d_b), cudaFree(l->d_out), cudaFree(l->d_plain), cudaFree(l->d_scratch);
+    cudaFree(l->d_rk_ptrs), cudaFree(l->d_rk_index);
     l->cap = 0;
     const size_t ct = cap * kCtWords * 8;
     cuda_throw(cudaMallocHost((void **)&l->h_a, ct), "cudaMallocHost");
@@ -150,6 +152,10 @@ void Engine::ensure_capacity(Lane *l, size_t cap) {
     cuda_throw(cudaMalloc((void **)&l->d_out, ct), "cudaMalloc");
     cuda_throw(cudaMalloc((void **)&l->d_plain, cap * kN * 2), "cudaMalloc");
     cuda_throw(cudaMalloc((void **)&l->d_scratch, cap * kScratchLimbsPerOp * kN * 8), "cudaMalloc");
+    cuda_throw(cudaMallocHost((void **)&l->h_rk_ptrs, cap * sizeof(uint64_t *)), "cudaMallocHost");
+    cuda_throw(cudaMallocHost((void **)&l->h_rk_index, cap * sizeof(int32_t)), "cudaMallocHost");
+    cuda_throw(cudaMalloc((void **)&l->d_rk_ptrs, cap * sizeof(uint64_t *)), "cudaMalloc");
+    cuda_throw(cudaMalloc((void **)&l->d_rk_index, cap * sizeof(int32_t)), "cudaMalloc");
     l->cap = cap;
 }
 
@@ -275,7 +281,7 @@ KeyEntry *Engine::find_or_parse_key(Span pk, int32_t *rc) {
     e->d_rk.assign((size_t)n_devices_, nullptr);
     e->d_pk.assign((size_t)n_devices_, nullptr);
     e->users = 1;
-    const size_t cap = env_size("FHE_B200_KEY_CACHE", 8);
+    const size_t cap = env_size("FHE_B200_KEY_CACHE", 256);  // a block's users: ~1 MB of host memory each, ~0.6 MB per device
 
     std::lock_guard<std::mutex> lk(key_mu_);
     for (auto &o : keys_)  // another thread may have inserted the same key meanwhile
@@ -507,17 +513,37 @@ void Engine::enqueue_mul(const uint64_t *a, const uint64_t *b, const ScratchMap 
         TIMED(1, launch_floor_sk(m.tens, m.c3, c, s), "floor_sk");
     }
 }
-// relinearise c size-3 ciphertexts c3 -> out
+// A prepared dual-base key takes 12 limbs; its preparation passes through 24 limbs of temporaries (coefficient form, lifted).
+// A fused chunk runs them through its tensor region (15 limbs per op, dead once c3 exists) in groups of keys that fit.
+constexpr size_t kPreparedKeyLimbs = 12, kPrepareTmpLimbs = 24;
+static_assert(kPrepareTmpLimbs <= 15 * kFusedTailMinOps, "a fused chunk's tensor region holds the temporaries of one key at least");
+
+// relinearise c size-3 ciphertexts c3 -> out, under rk or (keys) under a key per op
 void Engine::enqueue_relin(const uint64_t *c3, const uint64_t *rk, uint64_t *out, const ScratchMap &m, size_t c, cudaStream_t s,
-                           bool timed) {
+                           bool timed, RelinKeys *keys) {
     if (c >= kFusedTailMinOps) {
         // the whole key switch on the dual base; m.tens (15 limbs per op, dead once c3 exists) holds the lifted key
-        TIMED(10, launch_rk_prepare_ksd(rk, m.tens, s), "rk_prepare_ksd");
+        const uint64_t *rkd = m.tens + 24 * kN;
+        if (!keys) {
+            TIMED(10, launch_rk_prepare_ksd(rk, m.tens, s), "rk_prepare_ksd");
+        } else {
+            if (!keys->ready) {
+                size_t group = 15 * c / kPrepareTmpLimbs;
+                if (group > kMaxPrepareKeys) group = kMaxPrepareKeys;
+                for (size_t k0 = 0; k0 < keys->n_keys; k0 += group) {
+                    const size_t g = keys->n_keys - k0 < group ? keys->n_keys - k0 : group;
+                    TIMED(10, launch_rk_prepare_keys(nullptr, keys->raw + k0, g, m.tens, keys->prepared + k0 * kPreparedKeyLimbs * kN, s),
+                          "rk_prepare_ksd");
+                }
+                keys->ready = true;
+            }
+            rkd = keys->prepared;
+        }
         TIMED(11, launch_digit_ntt_ksd(c3, m.dig, c, s), "digit_ntt_ksd");
-        TIMED(15, launch_ks_tail_ksd(m.dig, m.tens + 24 * kN, c3, out, c, s), "ks_tail_ksd");
+        TIMED(15, launch_ks_tail_ksd(m.dig, rkd, c3, out, c, s, keys ? keys->key_index : nullptr), "ks_tail_ksd");
     } else {
         TIMED(6, launch_digit_ntt(c3, m.dig, c, s), "digit_ntt");
-        TIMED(7, launch_ks_intt(m.dig, rk, m.ks, c, s), "ks_intt");
+        TIMED(7, launch_ks_intt_keyed(m.dig, rk, keys ? keys->raw : nullptr, keys ? keys->key_index : nullptr, m.ks, c, s), "ks_intt");
         TIMED(3, launch_relin_finish(c3, m.ks, out, c, s), "relin_finish");
     }
 }
@@ -557,6 +583,44 @@ void Engine::relinearize(int device, const uint64_t *c3, const uint64_t *rk, uin
     for (size_t off = 0; off < n; off += chunk) {
         const size_t c = n - off < chunk ? n - off : chunk;
         enqueue_relin(c3 + off * 6 * kN, rk, out + off * kCtWords, m, c, s, false);
+    }
+}
+
+void Engine::mul_relin_keyed(int device, const uint64_t *a, const uint64_t *b, const uint64_t *rks, size_t n_keys,
+                             const int32_t *key_index, uint64_t *out, size_t n, cudaStream_t s) {
+    keyed_chunks(device, a, b, nullptr, rks, n_keys, key_index, out, n, s);
+}
+void Engine::relinearize_keyed(int device, const uint64_t *c3, const uint64_t *rks, size_t n_keys, const int32_t *key_index,
+                               uint64_t *out, size_t n, cudaStream_t s) {
+    keyed_chunks(device, nullptr, nullptr, c3, rks, n_keys, key_index, out, n, s);
+}
+// The arena holds the chunk's scratch, then the K prepared keys (only when full chunks run the fused tails) and the table of the
+// K key pointers; the keys are prepared once, by the first fused chunk, and every chunk may use any of them.
+void Engine::keyed_chunks(int device, const uint64_t *a, const uint64_t *b, const uint64_t *c3, const uint64_t *rks, size_t n_keys,
+                          const int32_t *key_index, uint64_t *out, size_t n, cudaStream_t s) {
+    if (n == 0) return;
+    device_context(device);
+    const size_t chunk = chunk_ops_ < n ? chunk_ops_ : n;
+    const size_t prepared_limbs = chunk >= kFusedTailMinOps ? n_keys * kPreparedKeyLimbs : 0;
+    const size_t table_limbs = (n_keys * sizeof(uint64_t *) + kN * 8 - 1) / (kN * 8);
+    const size_t extra_ops = (prepared_limbs + table_limbs + kScratchLimbsPerOp - 1) / kScratchLimbsPerOp;
+    ScratchLease lease{this, lease_scratch(device, s, chunk + extra_ops), &Engine::release_scratch};
+    ScratchMap m(lease.st->p, chunk);
+    RelinKeys keys;
+    keys.n_keys = n_keys;
+    keys.prepared = lease.st->p + chunk * kScratchLimbsPerOp * kN;
+    const uint64_t **table = reinterpret_cast<const uint64_t **>(keys.prepared + prepared_limbs * kN);
+    keys.raw = table;
+    cuda_throw(launch_key_table(rks, kRkWords, n_keys, table, s), "key_table");
+    for (size_t off = 0; off < n; off += chunk) {
+        const size_t c = n - off < chunk ? n - off : chunk;
+        keys.key_index = key_index + off;
+        if (a) {
+            enqueue_mul(a + off * kCtWords, b + off * kCtWords, m, c, s, timing_);
+            enqueue_relin(m.c3, nullptr, out + off * kCtWords, m, c, s, timing_, &keys);
+        } else {
+            enqueue_relin(c3 + off * 6 * kN, nullptr, out + off * kCtWords, m, c, s, false, &keys);
+        }
     }
 }
 
@@ -1226,16 +1290,28 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
     for (size_t i = 0; i < cnt; i++)
         if (prep[i].live) order.push_back(i);
     const double t_unpack = us_since(t_start);
+    // one run per class: a pass launches all its ct-ct multiplies as one run, whatever keys they use
     struct Run {
         int cls;
-        const uint64_t *d_rk;
         size_t begin, end;
     };
+    // the multiply run's keys: the distinct keys in order of first appearance, and each slot's index into them
+    struct RunKeys {
+        std::vector<const uint64_t *> keys;
+        std::vector<int32_t> index;
+        void add(const uint64_t *rk) {
+            if (keys.empty() || keys.back() != rk) keys.push_back(rk);  // the class is sorted by key
+            index.push_back((int32_t)keys.size() - 1);
+        }
+    };
+    // ops sharing a key sit next to each other: their key reads hit in L2
     const auto by_class = [&](size_t x, size_t y) {
         if (prep[x].cls != prep[y].cls) return prep[x].cls < prep[y].cls;
         return prep[x].cls == kMulCt && prep[x].d_rk < prep[y].d_rk;
     };
-    const auto launch_runs = [&](const std::vector<Run> &rs) {
+    // a tile has at most one key per op, so its prepared keys fit the extension buffer, dead once the tensor product exists
+    static_assert(kPreparedKeyLimbs <= 20, "prepared keys (one per op at most) in nttbuf (20 limbs per op)");
+    const auto launch_runs = [&](const std::vector<Run> &rs, RunKeys &rk) {
         for (const Run &r : rs) {
             const size_t c = r.end - r.begin;
             const uint64_t *a = lane->d_a + r.begin * kCtWords;
@@ -1246,7 +1322,22 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
                 case kMulCt: {
                     ScratchMap m(lane->d_scratch, c);
                     enqueue_mul(a, b, m, c, s, false);
-                    enqueue_relin(m.c3, r.d_rk, o, m, c, s, false);
+                    if (rk.keys.size() == 1) {
+                        enqueue_relin(m.c3, rk.keys[0], o, m, c, s, false);
+                        break;
+                    }
+                    const size_t k = rk.keys.size();
+                    memcpy(lane->h_rk_ptrs, rk.keys.data(), k * sizeof(uint64_t *));
+                    memcpy(lane->h_rk_index, rk.index.data(), c * sizeof(int32_t));
+                    cuda_throw(cudaMemcpyAsync(lane->d_rk_ptrs, lane->h_rk_ptrs, k * sizeof(uint64_t *), cudaMemcpyHostToDevice, s), "H2D keys");
+                    cuda_throw(cudaMemcpyAsync(lane->d_rk_index, lane->h_rk_index, c * sizeof(int32_t), cudaMemcpyHostToDevice, s),
+                               "H2D key indices");
+                    RelinKeys keys;
+                    keys.raw = lane->d_rk_ptrs;
+                    keys.n_keys = k;
+                    keys.prepared = m.nttbuf;
+                    keys.key_index = lane->d_rk_index;
+                    enqueue_relin(m.c3, nullptr, o, m, c, s, false, &keys);
                     break;
                 }
                 case kAddCt: cuda_throw(launch_eltwise(a, b, o, c, 0, s), "eltwise"); break;
@@ -1268,6 +1359,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
     if (cnt >= 2 && !order.empty()) {
         ensure_codec(lane);
         std::vector<Run> runs;
+        RunKeys run_keys;
         std::vector<size_t> slot_item, rest;
         const bool pack_on_device = zstd_writer() == 1;
         // (A) per call, in parallel: classify_operand; a call takes the device path when all its operands are Zstd or Packed
@@ -1306,8 +1398,8 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             p.va = g.ops[0].view;
             g.op0 = sop.size();
             for (int k = 0; k < g.nct; k++) sop.push_back(StageOperand{g.ops[k].route, g.ops[k].frame.n, (int32_t)slots, k});
-            const uint64_t *rk = p.cls == kMulCt ? p.d_rk : nullptr;
-            if (runs.empty() || runs.back().cls != p.cls || runs.back().d_rk != rk) runs.push_back(Run{p.cls, rk, slots, slots});
+            if (p.cls == kMulCt) run_keys.add(p.d_rk);
+            if (runs.empty() || runs.back().cls != p.cls) runs.push_back(Run{p.cls, slots, slots});
             runs.back().end = ++slots;
             if (p.cls <= kSubCt) ctct_slots = slots;
             slot_item.push_back(i);
@@ -1361,7 +1453,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             cuda_throw(launch_codec_inflate(lane->d_frames, lane->d_payloads, lane->d_jobs, lane->d_status, lane->d_work, lane->d_prefix,
                                             lane->d_a, lane->d_b, plan.jobs, plan.any_zstd, plan.any_packed, plan.payloads > 0, s),
                        "codec inflate");
-            launch_runs(runs);
+            launch_runs(runs, run_keys);
             int32_t *d_cflag = lane->d_status + 2 * lane->cap, *h_cflag = lane->h_status + 2 * lane->cap;
             if (pack_on_device) {
                 cuda_throw(launch_codec_pack(lane->d_out, lane->d_outframes, d_cflag, lane->d_prefix, (int)slots, s), "codec pack");
@@ -1426,6 +1518,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
 
     // ---- host pass: operands into adjacent staging slots, class by class; a call that fails here gives its slot to the next
     std::vector<Run> runs;
+    RunKeys run_keys;
     std::vector<size_t> slot_item;
     size_t slots = 0, ctct_slots = 0;
     for (size_t i : order) {
@@ -1465,8 +1558,8 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
             p.live = false;
             continue;
         }
-        const uint64_t *rk = p.cls == kMulCt ? p.d_rk : nullptr;
-        if (runs.empty() || runs.back().cls != p.cls || runs.back().d_rk != rk) runs.push_back(Run{p.cls, rk, slots, slots});
+        if (p.cls == kMulCt) run_keys.add(p.d_rk);
+        if (runs.empty() || runs.back().cls != p.cls) runs.push_back(Run{p.cls, slots, slots});
         runs.back().end = ++slots;
         if (p.cls <= kSubCt) ctct_slots = slots;
         slot_item.push_back(i);
@@ -1483,7 +1576,7 @@ void Engine::binary_tile(TileItem *items, size_t cnt) {
                                    cudaMemcpyHostToDevice, s),
                    "H2D plain");
     if (timed) cudaEventRecord(lane->ev[1], s);
-    launch_runs(runs);
+    launch_runs(runs, run_keys);
     if (timed) cudaEventRecord(lane->ev[2], s);
     cuda_throw(cudaMemcpyAsync(lane->h_out, lane->d_out, slots * kCtWords * 8, cudaMemcpyDeviceToHost, s), "D2H");
     if (timed) cudaEventRecord(lane->ev[3], s);

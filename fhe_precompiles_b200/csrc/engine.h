@@ -29,6 +29,15 @@ struct ScratchMap {
         : tens(base), c3(tens + c * 15 * kN), ks(c3 + c * 6 * kN), nttbuf(ks + c * 6 * kN), dig(nttbuf + c * 20 * kN) {}
 };
 
+// the keys of a key switch with a key per op: op i of a chunk runs under key key_index[i] of n_keys
+struct RelinKeys {
+    const uint64_t *const *raw = nullptr;  // device array of n_keys device pointers to SEAL-form keys [2][2][3][N] (split tails)
+    size_t n_keys = 0;
+    uint64_t *prepared = nullptr;  // [n_keys][12][N] dual-base keys (fused tails), filled by the first chunk that runs them
+    bool ready = false;            // `prepared` holds the keys
+    const int32_t *key_index = nullptr;  // device ints of the chunk's ops (not checked)
+};
+
 // A lane = one stream + staging for `cap` calls (1 until a tile of the batch surface needs more).
 struct Lane {
     int device = 0;
@@ -38,6 +47,9 @@ struct Lane {
     uint16_t *h_plain = nullptr;                                // pinned, cap * kN
     uint64_t *d_a = nullptr, *d_b = nullptr, *d_out = nullptr, *d_scratch = nullptr;
     uint16_t *d_plain = nullptr;
+    // a tile's ct-ct multiplies under more than one key: its distinct keys and each slot's index into them (cap entries each)
+    const uint64_t **h_rk_ptrs = nullptr, **d_rk_ptrs = nullptr;
+    int32_t *h_rk_index = nullptr, *d_rk_index = nullptr;
     bool busy = false;
     // device codec staging for tiles (allocated when a tile first uses it): compressed operand frames in, structured frames out
     size_t codec_cap = 0;
@@ -159,6 +171,13 @@ class Engine {
                    cudaStream_t s);
     void multiply(int device, const uint64_t *a, const uint64_t *b, uint64_t *out3, size_t n, cudaStream_t s);
     void relinearize(int device, const uint64_t *c3, const uint64_t *rk, uint64_t *out, size_t n, cudaStream_t s);
+    // the same with a key per row: rks [n_keys][2][2][3][N], key_index [n] device ints in [0, n_keys) (not checked); row i is
+    // bit for bit mul_relin / relinearize of that row under rks[key_index[i]].  All n_keys keys are prepared, once per call, into
+    // n_keys x 12 limbs of the stream's scratch arena (which keeps its size): the caller passes the keys its rows use.
+    void mul_relin_keyed(int device, const uint64_t *a, const uint64_t *b, const uint64_t *rks, size_t n_keys, const int32_t *key_index,
+                         uint64_t *out, size_t n, cudaStream_t s);
+    void relinearize_keyed(int device, const uint64_t *c3, const uint64_t *rks, size_t n_keys, const int32_t *key_index, uint64_t *out,
+                           size_t n, cudaStream_t s);
 
     // host-buffer batched entry point: a, b, out are host memory (pinned for full PCIe rate), rk host words.
     // H2D, kernels and D2H of consecutive chunks overlap on `kPipeSlots` streams.  Synchronous.
@@ -316,8 +335,12 @@ class Engine {
     };
     bool timing_ = false;
     void enqueue_mul(const uint64_t *a, const uint64_t *b, const ScratchMap &m, size_t c, cudaStream_t s, bool timed);
+    // keys (optional): a key per op instead of rk
     void enqueue_relin(const uint64_t *c3, const uint64_t *rk, uint64_t *out, const ScratchMap &m, size_t c, cudaStream_t s,
-                       bool timed);
+                       bool timed, RelinKeys *keys = nullptr);
+    // mul_relin_keyed (a, b) or relinearize_keyed (c3)
+    void keyed_chunks(int device, const uint64_t *a, const uint64_t *b, const uint64_t *c3, const uint64_t *rks, size_t n_keys,
+                      const int32_t *key_index, uint64_t *out, size_t n, cudaStream_t s);
     void timed_launch(int kernel, cudaStream_t s, bool timed, cudaError_t e0, const char *what);
     std::vector<TimedLaunch> timed_;
     std::mutex timed_mu_;

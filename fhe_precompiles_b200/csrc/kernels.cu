@@ -504,11 +504,14 @@ __device__ __forceinline__ void ks_intt_body(const u64 *__restrict__ dg, const u
     ntt_inverse<M, 1, true, false>(v, smem, kt.twi[MI], t, kc.ninv[MI], kc.ninv_w[MI]);
     store_natural(dst, v[0], t);
 }
+// rk: every op's key, or (key_index non-null) op i reads the key rks[key_index[i]]
 __global__ void __launch_bounds__(kThreads, 2) k_ks_intt(const u64 *__restrict__ dig, const u64 *__restrict__ rk,
+                                                          const u64 *const *__restrict__ rks, const int *__restrict__ key_index,
                                                           u64 *__restrict__ ks) {
     extern __shared__ __align__(16) u64 smem[];
     const size_t op = blockIdx.y;
     const int k = blockIdx.x / 3, J = blockIdx.x % 3;
+    if (key_index) rk = rks[key_index[op]];
     const u64 *dg = dig + op * 6 * kN;
     u64 *dst = ks + (op * 6 + blockIdx.x) * kN;
     const int t = threadIdx.x;
@@ -525,7 +528,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks_intt(const u64 *__restrict__
 // P), 0 <= RK < 3 Q.  |U_k| < 2 N 2^36 2^111 = 2^160 << S / 2, so U_k is carried exactly by the six dual primes: 6 forward + 6
 // inverse DUAL transforms instead of 6 + 6 on 36/37-bit primes, and U_k mod (q0, q1, P) follows by the same CRT-with-rounding
 // as in k_floor_sk_d.  Same bits as SEAL (the oracle follows SEAL; prototyped in Python first).
-//   k_rk_intt_ksd / k_rk_lift_ksd / k_rk_ntt_ksd : the key -> coefficient form -> integer lift mod s_i -> dual NTT (per call)
+//   k_rk_intt_ksd / k_rk_lift_ksd / k_rk_ntt_ksd : the key -> coefficient form -> integer lift mod s_i -> dual NTT (per call;
+//                     K keys in the same three launches, key-major: [K][12][N] at each stage)
 //   k_digit_ntt_ksd : dual NTT of the two digits ([c2]_{q_j} as integers)          grid (6 = j*3+w, ops) -> dig [op][2][3][N]
 //   k_ks_tail_ksd   : MAC with the lifted key + inverse dual NTTs, U mod (P, q0, q1), rounded division by P, add to (c0, c1)
 //                     grid (2 = k, ops) -> out [op][2][2][N]
@@ -538,18 +542,22 @@ __device__ __forceinline__ void rk_intt_body(const u64 *__restrict__ src, u64 *_
     ntt_inverse<M, 1, true, false>(v, smem, kt.twi[MI], t, kc.ninv[MI], kc.ninv_w[MI]);
     store_natural(dst, v[0], t);
 }
-__global__ void __launch_bounds__(kThreads, 2) k_rk_intt_ksd(const u64 *__restrict__ rk, u64 *__restrict__ coef) {
+// grid (12 limbs, K keys): key y is rk itself (K = 1, rks null) or rks[y]
+__global__ void __launch_bounds__(kThreads, 2) k_rk_intt_ksd(const u64 *__restrict__ rk, const u64 *const *__restrict__ rks,
+                                                              u64 *__restrict__ coef) {
     extern __shared__ __align__(16) u64 smem[];
     const int limb = blockIdx.x, t = threadIdx.x;
+    if (rks) rk = rks[blockIdx.y];
+    coef += (size_t)blockIdx.y * 12 * kN;
     switch (limb % 3) {
         case 0: rk_intt_body<MQ0>(rk + (size_t)limb * kN, coef + (size_t)limb * kN, smem, t); break;
         case 1: rk_intt_body<MQ1>(rk + (size_t)limb * kN, coef + (size_t)limb * kN, smem, t); break;
         default: rk_intt_body<MP>(rk + (size_t)limb * kN, coef + (size_t)limb * kN, smem, t); break;
     }
 }
-// coef [4 = j*2+k][3 moduli][N] -> lifted [4][3 dual words][N], every lane in [0, 4s)
+// coef [K][4 = j*2+k][3 moduli][N] -> lifted [K][4][3 dual words][N], every lane in [0, 4s)
 __global__ void __launch_bounds__(256) k_rk_lift_ksd(const u64 *__restrict__ coef, u64 *__restrict__ lifted) {
-    const int g = blockIdx.x * 256 + threadIdx.x;  // 4 * N threads
+    const int g = blockIdx.x * 256 + threadIdx.x;  // K * 4 * N threads
     const int jk = g / kN, i = g % kN;
     const u64 *c = coef + (size_t)jk * 3 * kN + i;
     const u64 y[3] = {shoup<Mod<MQ0>>(c[0], kc.lk_C[0].w, kc.lk_C[0].ws), shoup<Mod<MQ1>>(c[kN], kc.lk_C[1].w, kc.lk_C[1].ws),
@@ -571,6 +579,7 @@ __global__ void __launch_bounds__(256) k_rk_lift_ksd(const u64 *__restrict__ coe
     o[kN] = pack64(lane[2], lane[3]);
     o[2 * kN] = pack64(lane[4], lane[5]);
 }
+// grid 12 K: limb x of key x / 12
 __global__ void __launch_bounds__(kThreads, 3) k_rk_ntt_ksd(const u64 *__restrict__ lifted, u64 *__restrict__ rkd) {
     extern __shared__ __align__(16) u64 smem[];
     const int limb = blockIdx.x, t = threadIdx.x;
@@ -683,12 +692,15 @@ __device__ __forceinline__ void ks_finish_coeff_ksd(u64 w0, u64 w1, u64 w2, u64 
 }
 
 // ---- the tail of the key switch in one kernel: one CTA per (output polynomial k, op), the three dual
-// words of U_k one after the other with the first two parked in shared memory (as k_tensor_floor_d): U_k never goes through HBM
+// words of U_k one after the other with the first two parked in shared memory (as k_tensor_floor_d): U_k never goes through HBM.
+// rkd: the prepared key of every op, or (key_index non-null) [K][12][N] with op i under key key_index[i]
 __global__ void __launch_bounds__(kThreads, 2) k_ks_tail_ksd(const u64 *__restrict__ dig, const u64 *__restrict__ rkd,
-                                                              const u64 *__restrict__ c3, u64 *__restrict__ out) {
+                                                              const int *__restrict__ key_index, const u64 *__restrict__ c3,
+                                                              u64 *__restrict__ out) {
     extern __shared__ __align__(16) u64 smem[];  // [3][kN]
     const size_t op = blockIdx.y;
     const int k = blockIdx.x, t = threadIdx.x;
+    if (key_index) rkd += (size_t)key_index[op] * 12 * kN;
     const u64 *dg = dig + op * 6 * kN;
     u64 *park0 = smem + kN, *park1 = smem + 2 * kN;
     {
@@ -1378,9 +1390,10 @@ cudaError_t launch_tensor_floor(const u64 *nttbuf, u64 *c3, size_t n_ops, cudaSt
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
-cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s) {
+cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s,
+                               const int *key_index) {
     if (n_ops == 0) return cudaSuccess;
-    k_ks_tail_ksd<<<dim3(2, (unsigned)n_ops), kThreads, kSmem3, s>>>(dig, rkd, c3, out);
+    k_ks_tail_ksd<<<dim3(2, (unsigned)n_ops), kThreads, kSmem3, s>>>(dig, rkd, key_index, c3, out);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
@@ -1391,8 +1404,12 @@ cudaError_t launch_digit_ntt(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t
     return cudaGetLastError();
 }
 cudaError_t launch_ks_intt(const u64 *dig, const u64 *rk, u64 *ks, size_t n_ops, cudaStream_t s) {
+    return launch_ks_intt_keyed(dig, rk, nullptr, nullptr, ks, n_ops, s);
+}
+cudaError_t launch_ks_intt_keyed(const u64 *dig, const u64 *rk, const u64 *const *rks, const int *key_index, u64 *ks, size_t n_ops,
+                                 cudaStream_t s) {
     if (n_ops == 0) return cudaSuccess;
-    k_ks_intt<<<dim3(6, (unsigned)n_ops), kThreads, kSmem1, s>>>(dig, rk, ks);
+    k_ks_intt<<<dim3(6, (unsigned)n_ops), kThreads, kSmem1, s>>>(dig, rk, rks, key_index, ks);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
@@ -1434,11 +1451,26 @@ cudaError_t launch_seal_sample(u64 *streams, signed char *samples, int *failed, 
 // the key of the key switch on the dual base, once per chunk; tmp = 36 limbs of scratch (coefficient-form key, lifted key,
 // dual-NTT key at tmp + 24 limbs)
 cudaError_t launch_rk_prepare_ksd(const u64 *rk, u64 *tmp, cudaStream_t s) {
-    u64 *coef = tmp, *lifted = tmp + 12 * kN, *rkd = tmp + 24 * kN;
-    k_rk_intt_ksd<<<12, kThreads, kSmem1, s>>>(rk, coef);
-    k_rk_lift_ksd<<<4 * kN / 256, 256, 0, s>>>(coef, lifted);
-    k_rk_ntt_ksd<<<12, kThreads, kSmem1, s>>>(lifted, rkd);
+    return launch_rk_prepare_keys(rk, nullptr, 1, tmp, tmp + 24 * kN, s);
+}
+cudaError_t launch_rk_prepare_keys(const u64 *rk, const u64 *const *rks, size_t n_keys, u64 *tmp, u64 *rkd, cudaStream_t s) {
+    if (n_keys == 0) return cudaSuccess;
+    if (n_keys > kMaxPrepareKeys) return cudaErrorInvalidValue;
+    u64 *coef = tmp, *lifted = tmp + n_keys * 12 * kN;
+    k_rk_intt_ksd<<<dim3(12, (unsigned)n_keys), kThreads, kSmem1, s>>>(rk, rks, coef);
+    k_rk_lift_ksd<<<(unsigned)(n_keys * 4 * kN / 256), 256, 0, s>>>(coef, lifted);
+    k_rk_ntt_ksd<<<(unsigned)(n_keys * 12), kThreads, kSmem1, s>>>(lifted, rkd);
     g_launches.fetch_add(3, std::memory_order_relaxed);
+    return cudaGetLastError();
+}
+__global__ void k_key_table(const u64 *rks, size_t stride, size_t n_keys, const u64 **table) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_keys) table[i] = rks + i * stride;
+}
+cudaError_t launch_key_table(const u64 *rks, size_t stride, size_t n_keys, const u64 **table, cudaStream_t s) {
+    if (n_keys == 0) return cudaSuccess;
+    k_key_table<<<(unsigned)((n_keys + 255) / 256), 256, 0, s>>>(rks, stride, n_keys, table);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
     return cudaGetLastError();
 }
 cudaError_t launch_digit_ntt_ksd(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s) {

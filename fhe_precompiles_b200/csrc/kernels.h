@@ -31,6 +31,10 @@ cudaError_t launch_tensor_floor(const u64 *nttbuf, u64 *c3, size_t n_ops, cudaSt
 // key switch on SEAL's key primes: launch_digit_ntt -> launch_ks_intt -> launch_relin_finish; dig, ks [n][2][3][N]
 cudaError_t launch_digit_ntt(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s);
 cudaError_t launch_ks_intt(const u64 *dig, const u64 *rk, u64 *ks, size_t n_ops, cudaStream_t s);
+// the same with a key per op: key_index [n_ops] device ints, op i under the key rks[key_index[i]] (rks: device array of device
+// pointers to keys [2][2][3][N]; indices not checked).  key_index null: every op under rk, as launch_ks_intt.
+cudaError_t launch_ks_intt_keyed(const u64 *dig, const u64 *rk, const u64 *const *rks, const int *key_index, u64 *ks, size_t n_ops,
+                                 cudaStream_t s);
 cudaError_t launch_relin_finish(const u64 *c3, const u64 *ks, u64 *out, size_t n_ops, cudaStream_t s);
 // decrypt n size-2 ciphertexts with sk [>=2 limbs][N] (NTT form): xbuf scratch [n][2][N], plain out [n][N] u16
 // exhausted (optional, [n_ops] ints on the device): set to 1 where the invariant noise budget is 0
@@ -53,8 +57,16 @@ cudaError_t launch_seal_sample(u64 *streams, signed char *samples, int *failed, 
 // key switch on the dual base: launch_rk_prepare_ksd (per chunk) -> launch_digit_ntt_ksd -> launch_ks_tail_ksd
 // tmp36: 36 limbs of scratch; the dual-NTT key ends up at tmp36 + 24 limbs
 cudaError_t launch_rk_prepare_ksd(const u64 *rk, u64 *tmp36, cudaStream_t s);
+// K keys in the same three launches: the keys rks[0 .. K) (a device array of device pointers), or rk itself when rks is null
+// (K = 1); tmp: 24 K limbs of scratch; rkd: the prepared keys [K][12][N].  K <= kMaxPrepareKeys.
+constexpr size_t kMaxPrepareKeys = 65535;
+cudaError_t launch_rk_prepare_keys(const u64 *rk, const u64 *const *rks, size_t n_keys, u64 *tmp, u64 *rkd, cudaStream_t s);
 cudaError_t launch_digit_ntt_ksd(const u64 *c3, u64 *dig, size_t n_ops, cudaStream_t s);
-cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s);
+// key_index (optional, [n_ops] device ints, not checked): op i under the prepared key rkd + key_index[i] * 12 * N
+cudaError_t launch_ks_tail_ksd(const u64 *dig, const u64 *rkd, const u64 *c3, u64 *out, size_t n_ops, cudaStream_t s,
+                               const int *key_index = nullptr);
+// table[i] = rks + i * stride for i < n_keys (device memory): the key table of contiguous keys
+cudaError_t launch_key_table(const u64 *rks, size_t stride, size_t n_keys, const u64 **table, cudaStream_t s);
 
 uint64_t launch_count();
 void count_launches(uint64_t n);  // kernels replayed through a CUDA graph (the launchers only count at capture time)

@@ -104,6 +104,45 @@ def mul_relin(a, b, rk, out=None):
     return out
 
 
+def _check_keyed(rks: torch.Tensor, key_index: torch.Tensor, n: int) -> None:
+    assert rks.dim() == 5 and tuple(rks.shape[1:]) == (2, 2, 3, N) and rks.dtype == torch.int64
+    assert key_index.dtype == torch.int32 and tuple(key_index.shape) == (n,)
+
+
+def mul_relin_keyed(a: torch.Tensor, b: torch.Tensor, rks: torch.Tensor, key_index: torch.Tensor, out=None) -> torch.Tensor:
+    """mul_relin() with a relinearisation key per row: a, b [n,2,2,4096], rks [k,2,2,3,4096] int64, key_index [n] int32 in
+    [0, k) (all on one CUDA device) -> [n,2,2,4096]; row i is mul_relin(a[i], b[i], rks[key_index[i]]).  The indices are not
+    checked on the device: one outside [0, k) is the caller's error.  All k keys are prepared and take 393 KB of scratch each:
+    pass the keys the rows use, not a whole table of users."""
+    dev = _dev(a)
+    _dev(b)
+    _dev(rks)
+    _dev(key_index)
+    n = a.shape[0]
+    assert a.dtype == torch.int64 and tuple(a.shape) == (n, 2, 2, N) and b.dtype == torch.int64 and tuple(b.shape) == (n, 2, 2, N)
+    _check_keyed(rks, key_index, n)
+    if out is None:
+        out = torch.empty_like(a)
+    assert out.dtype == torch.int64 and tuple(out.shape) == (n, 2, 2, N) and out.is_contiguous()
+    _check(_lib.lib().fhe_b200_mul_relin_keyed(dev, a.data_ptr(), b.data_ptr(), rks.data_ptr(), rks.shape[0], key_index.data_ptr(),
+                                               out.data_ptr(), n, _stream(dev)))
+    return out
+
+
+def relinearize_keyed(c3: torch.Tensor, rks: torch.Tensor, key_index: torch.Tensor) -> torch.Tensor:
+    """relinearize() with a key per row: c3 [n,3,2,4096], rks and key_index as in mul_relin_keyed() -> [n,2,2,4096]."""
+    dev = _dev(c3)
+    _dev(rks)
+    _dev(key_index)
+    n = c3.shape[0]
+    assert c3.dtype == torch.int64 and tuple(c3.shape) == (n, 3, 2, N)
+    _check_keyed(rks, key_index, n)
+    out = torch.empty((n, 2, 2, N), dtype=torch.int64, device=c3.device)
+    _check(_lib.lib().fhe_b200_relinearize_keyed(dev, c3.data_ptr(), rks.data_ptr(), rks.shape[0], key_index.data_ptr(), out.data_ptr(), n,
+                                                 _stream(dev)))
+    return out
+
+
 def ntt_(data: torch.Tensor, mods: Sequence[int], inverse: bool = False) -> torch.Tensor:
     """In-place batched NTT over data[..., 4096]; limb i (flattened) uses modulus mods[i % len(mods)]."""
     dev = _dev(data)

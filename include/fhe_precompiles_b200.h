@@ -139,6 +139,18 @@ int32_t fhe_b200_multiply(int32_t device, const uint64_t *a, const uint64_t *b, 
 int32_t fhe_b200_relinearize(int32_t device, const uint64_t *c3, const uint64_t *rk, uint64_t *out, size_t n, void *stream);
 int32_t fhe_b200_mul_relin(int32_t device, const uint64_t *a, const uint64_t *b, const uint64_t *rk, uint64_t *out,
                            size_t n, void *stream);
+/* fhe_b200_mul_relin / fhe_b200_relinearize with a relinearisation key per row: rks [n_keys][2][2][3][4096] (each as
+ * fhe_b200_mul_relin's rk), key_index [n] int32 on the device; row i is bit for bit fhe_b200_mul_relin (fhe_b200_relinearize) of
+ * that row under rks + key_index[i] * 2 * 2 * 3 * 4096.  For a batch whose rows belong to different users, e.g. the multiplies
+ * of a block: one call, the keys prepared once, instead of one call per key.  Every one of the n_keys keys is prepared, whether
+ * a row uses it or not, and the stream's scratch grows by n_keys x 393,216 bytes (kept for later calls on that stream): pass
+ * only the keys the batch uses, i.e. n_keys = the number of distinct keys of its rows, not a whole table of users.
+ * The indices are device data and are not checked: an index outside [0, n_keys) is the caller's error, as a bad pointer is.
+ * n == 0 launches nothing; -1 (fhe_b200_last_error) for a missing device, missing keys or indices, or a failed launch. */
+int32_t fhe_b200_mul_relin_keyed(int32_t device, const uint64_t *a, const uint64_t *b, const uint64_t *rks, size_t n_keys,
+                                 const int32_t *key_index, uint64_t *out, size_t n, void *stream);
+int32_t fhe_b200_relinearize_keyed(int32_t device, const uint64_t *c3, const uint64_t *rks, size_t n_keys, const int32_t *key_index,
+                                   uint64_t *out, size_t n, void *stream);
 /* Deterministic public-key encryption of n plaintexts (uint16 [n][4096]) under pk [2][3][4096] (NTT form, as in the key
  * file) with one 512-bit seed per op (seeds [n][8] words; the byte surface passes the eight little-endian words of its
  * SHA-512 digest, fhe.rs:611-616).  BIT-EXACT with the reference: this is sunscreen 0.8.1 `encrypt_deterministic` as the
